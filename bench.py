@@ -3,6 +3,7 @@
 
     python bench.py --gpus N --steps K --warmup W          # this repo's CUDA path
     python bench.py --impl reference --gpus N ...          # the reference's CPU (PyTorch) path, oracle port
+    python bench.py ... --dump-outputs DIR                 # also write the last timed step's outputs as DIR/*.npy
 
 One "step" = the loop body of train_unet.cu:5019-5037 on one synthetic batch: H2D batch copy (e2e only),
 timestep + noise draw, q-sample, U-Net forward, MSE, backward, (gradient all-reduce), AdamW.
@@ -221,6 +222,8 @@ def run_cuda(args):
     ms_step = ms_total / args.steps
     value = world * B / (ms_step * 1e-3)
     loss_now = tr.last_loss()
+    if args.dump_outputs and rank == 0:   # before the end-to-end leg below trains further
+        dump_outputs(args.dump_outputs, tr)
 
     # ---- end to end through the public API with HOST buffers: H2D of the batch + D2H of the loss every step
     import ctypes
@@ -323,6 +326,23 @@ def run_cuda(args):
     if use_dist:
         dist.barrier()
         dist.destroy_process_group()
+
+
+DUMP_SAMPLE = 1 << 22   # parameters kept in the dump: 16 MB in float32 of the 82 MB vector
+
+
+def dump_outputs(out_dir, tr):
+    """What the last timed step handed its caller, as float32 .npy files: the loss, the model output (B, C, H, W) and the
+    updated parameters at DUMP_SAMPLE positions drawn with a fixed seed.  (The fused AdamW clears the gradients, so a
+    training step returns none.)  The bench's inputs are seeded, so two builds run with the same arguments can be
+    compared file by file."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    idx = np.sort(np.random.default_rng(0).choice(tr.nparams, size=min(DUMP_SAMPLE, tr.nparams), replace=False))
+    arrays = {"loss": np.array([tr.last_loss()], dtype=np.float32), "output": tr.get_output(),
+              "params_sample": tr.get_params()[idx]}
+    for name, a in arrays.items():
+        np.save(os.path.join(out_dir, name + ".npy"), a)
 
 
 def conv_microbench(ub, pk):
@@ -486,7 +506,14 @@ def main():
     ap.add_argument("--no-reference-cuda", action="store_true")
     ap.add_argument("--no-prefetch", action="store_true",
                     help="end-to-end leg without ub_trainer_set_next_batch (synchronous H2D before every step)")
+    ap.add_argument("--dump-outputs", metavar="DIR",
+                    help="write the loss, model output and sampled updated parameters of the last timed step to DIR")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl == "reference":
+        # the CPU arm sizes its batch from a timing probe, so its inputs are not the same from run to run
+        ap.error("--dump-outputs applies to --impl cuda only")
     if args.impl == "reference":
         run_reference(args)
     else:
