@@ -206,9 +206,11 @@ int ub_groupnorm_nhwc_backward(const void* x_bf16, const void* dy_bf16, const fl
 
 /* Attention core in the native layout (what the trainer runs; replaces attention_forward1 / attention_backward,
  * dev/attention.cuh:6-22, without their permutes and (B,NH,T,T) matrices): qkv is NHWC bf16 [B*T][3C], channel order
- * [Q | K | V], each [NH][32]; out [B*T][C] bf16; lse [B][NH][T] fp32 (log2-domain logsumexp, saved for backward).
- * backward: dqkv [B*T][3C] bf16 from dout [B*T][C]; dsum [B][NH][T] is scratch.  Head size must be 32.
- * impl: 0 = tcgen05 kernels (needs T in {16,32,64,128,256} and an even NH), 1 = SIMT fp32 fallback (any T). */
+ * [Q | K | V], each [NH][HS] with head size HS = C / NH; out [B*T][C] bf16; lse [B][NH][T] fp32 (log2-domain
+ * logsumexp, saved for backward).  backward: dqkv [B*T][3C] bf16 from dout [B*T][C]; dsum [B][NH][T] is scratch.
+ * Head size 32 (C == NH * 32) or 64 (C == NH * 64); any other is rejected.
+ * impl: 0 = tcgen05 kernels: T in {16,32,64,128,256} and either HS = 32 with an even NH or HS = 64 with any NH;
+ *       1 = SIMT fp32 fallback (any T, either head size). */
 int ub_attention_nhwc_forward(const void* qkv_bf16, void* out_bf16, float* lse, int B, int T, int C, int NH, int impl);
 int ub_attention_nhwc_backward(const void* qkv_bf16, const void* out_bf16, const void* dout_bf16, const float* lse,
                                void* dqkv_bf16, float* dsum, int B, int T, int C, int NH, int impl);
@@ -228,7 +230,8 @@ typedef struct {
     int channel_mult[8]; /* {1,2,3,4} */
     int n_res_blocks;    /* 2 */
     int att_start_level; /* 2 : attention at levels >= this */
-    int head_size;       /* 32 */
+    int head_size;       /* 32; or 64 (guided-diffusion's num_head_channels = 64).  Like channel_mult, not stored in
+                            the checkpoint header: the caller sets it to what the model was trained with */
     int gn_n_groups;     /* 32 */
     int n_timesteps;     /* 1000, linear beta schedule 1e-4 .. 0.02 (train_unet.cu:3131-3147) */
     unsigned long long seed;

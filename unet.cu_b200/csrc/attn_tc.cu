@@ -1,21 +1,24 @@
-// Attention core on the 5th-gen tensor cores (tcgen05 + TMEM), head size 32, sequence length T <= 256.
+// Attention core on the 5th-gen tensor cores (tcgen05 + TMEM), head size 32 or 64, sequence length T <= 256.
 //
 // Replaces attention_forward1 / attention_backward (/root/reference/train_unet.cu:2553-2760: cuBLAS batched GEMMs
 // with materialised (B,NH,T,T) matrices and three permutes) on the internal NHWC bf16 qkv tensor
-// [B*T][3C], channel order [Q | K | V], each [NH][32] (dev/unet.py:75-87).
+// [B*T][3C], channel order [Q | K | V], each [NH][HS] (dev/unet.py:75-87).
 //
-// One CTA = 128 consecutive rows of the flattened (image, position) axis x one PAIR of heads.  A 64-channel TMA box
-// (128-byte swizzle) holds both heads of the pair; a head is selected by the K offset inside the swizzle row
-// (+64 B), exactly like a K step of the conv kernels.  All T <= 256 scores of a row fit in TMEM, so softmax is exact
-// (no online rescaling).  For T < 128 a tile spans 128/T images and the cross-image scores are masked.
+// One CTA = 128 consecutive rows of the flattened (image, position) axis x one 64-channel TMA box (128-byte swizzle)
+// of each of Q, K, V.  HS = 32: the box holds a PAIR of heads, a head is selected by the K offset inside the swizzle
+// row (+64 B), exactly like a K step of the conv kernels, and the CTA works through the two heads one after the
+// other.  HS = 64: the box holds exactly one head (any NH) and the head loop runs once.  All T <= 256 scores of a row
+// fit in TMEM, so softmax is exact (no online rescaling).  For T < 128 a tile spans 128/T images and the cross-image
+// scores are masked.
 //
 //   forward : S = Q K^T (K-major x K-major, N = keys) -> TMEM;  row threads: p = exp2(s - max), P (bf16) -> smem in
 //             the canonical K-major SW128 layout;  O = P V with V read MN-major straight from its natural layout.
 //   dq      : per 128-key chunk  S, dP = dO V^T -> TMEM;  dS = P o (dP - D) -> smem;  dQ += dS K (K MN-major).
 //   dkv     : rows are KEYS:  S^T = K Q^T, dP^T = V dO^T -> TMEM;  P^T, dS^T -> smem;  dV += P^T dO, dK += dS^T Q
 //             (dO, Q MN-major).  No atomics, no cross-CTA reduction: a CTA owns its 128 keys for all queries.
-// The PV-type MMAs use N = 64 (both heads' channels of the MN-major operand) and keep the 32 columns of the current
-// head: the wasted half costs 16 tensor cycles per MMA and saves a second descriptor mode.
+// The PV-type MMAs use N = 64 (the box's channels of the MN-major operand).  HS = 32 keeps the 32 columns of the
+// current head: the wasted half costs 16 tensor cycles per MMA and saves a second descriptor mode.  HS = 64 uses all
+// 64.  The score MMAs take K = HS in HS/16 steps of K = 16.
 //
 // Warp roles: warp 0 = TMA + MMA issue (one elected lane) + TMEM allocator; warps 1-8 = row threads (TMEM lane =
 // row; the two warps of a lane quadrant split the columns of every chunk).  mbarriers: load -> s (accumulators ready) -> p (operand written to smem) -> o (second MMA done).
@@ -38,7 +41,6 @@ namespace {
 constexpr int kThreads = 288;     // warp 0: TMA + MMA issue; warps 1-8: row threads, two warps per TMEM lane quadrant
 constexpr int kRowThreads = 256;  // (the two warps of a quadrant split the columns of every chunk)
 constexpr float kLog2e = 1.4426950408889634f;
-constexpr int HS = 32;
 
 __device__ __forceinline__ float ex2(float x) {
     float y;
@@ -49,6 +51,16 @@ __device__ __forceinline__ void fence_async_smem() { asm volatile("fence.proxy.a
 
 // byte offset of the 16-byte chunk `c16` (0..7) of row r inside a [rows][128 B] SWIZZLE_128B tile
 __device__ __forceinline__ uint32_t sw128(int r, int c16) { return uint32_t(r) * 128u + (uint32_t(c16 ^ (r & 7)) << 4); }
+
+// the N = HS/2 accumulator columns a row thread drains per head (HS = 32: 16, HS = 64: 32)
+template <int N>
+__device__ __forceinline__ void tmem_ld_half(uint32_t taddr, uint32_t (&v)[N]) {
+    static_assert(N == 16 || N == 32, "head size 32 or 64");
+    if constexpr (N == 16)
+        tmem_ld16(taddr, v);
+    else
+        tmem_ld32(taddr, v);
+}
 
 __device__ __forceinline__ uint32_t pack2(float a, float b) {
     const __nv_bfloat162 h = __floats2bfloat162_rn(a, b);
@@ -84,7 +96,7 @@ struct Tile {
     int row0;    // first row (flattened b*T + t) of the CTA
     int col0;    // first column row (flattened) of the column range
     int ncols;   // columns (keys for fwd/dq, queries for dkv): 128 or 256
-    int hp;      // head pair
+    int hp;      // 64-channel box: head pair (HS = 32) or head (HS = 64)
 };
 __device__ __forceinline__ Tile make_tile(const AttnTcParams& p) {
     Tile t;
@@ -129,7 +141,7 @@ __device__ __forceinline__ void prologue(Smem* sm, uint32_t ncols_tmem, int warp
 // =====================================================================================================
 // forward
 // =====================================================================================================
-template <bool MASK>
+template <int HS, bool MASK>
 __global__ void __launch_bounds__(kThreads) attn_tc_fwd_kernel(const __grid_constant__ AttnTcParams p) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -142,11 +154,13 @@ __global__ void __launch_bounds__(kThreads) attn_tc_fwd_kernel(const __grid_cons
     float* sl = sx + 512;                                              // [2 heads][2 halves][128] partial row sum
     Smem* sm = reinterpret_cast<Smem*>(sl + 512);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    constexpr int HPB = 64 / HS;  // heads per box
     const int C = p.NH * HS;
     const uint32_t tm_cols = t.ncols > 128 ? 512 : 256;
     const uint32_t o_col = t.ncols;  // O accumulator behind the scores
-    // head split (AttnTcParams::hsplit): gridDim.z == 2 and the CTA works on ONE head of its pair
-    const int h_lo = gridDim.z == 2 ? int(blockIdx.z) : 0, h_hi = gridDim.z == 2 ? int(blockIdx.z) + 1 : 2;
+    // head split (HS = 32 only, see attn_hsplit): gridDim.z == 2 and the CTA works on ONE head of its pair
+    const bool hsplit = HS == 32 && gridDim.z == 2;
+    const int h_lo = hsplit ? int(blockIdx.z) : 0, h_hi = hsplit ? int(blockIdx.z) + 1 : HPB;
     prologue(sm, tm_cols, warp, lane);
     const uint32_t tmem = sm->tmem_slot;
 
@@ -173,8 +187,8 @@ __global__ void __launch_bounds__(kThreads) attn_tc_fwd_kernel(const __grid_cons
             for (int h = h_lo; h < h_hi; ++h) {
                 if (elect_one_sync()) {
 #pragma unroll
-                    for (int k = 0; k < 2; ++k)
-                        umma_bf16(tmem, dQ + uint64_t(h * 4 + k * 2), dK + uint64_t(h * 4 + k * 2), id_s, k);
+                    for (int k = 0; k < HS / 16; ++k)
+                        umma_bf16(tmem, dQ + uint64_t(h * (HS / 8) + k * 2), dK + uint64_t(h * (HS / 8) + k * 2), id_s, k);
                     umma_commit(&sm->bar_s);
                 }
                 __syncwarp();
@@ -202,13 +216,20 @@ __global__ void __launch_bounds__(kThreads) attn_tc_fwd_kernel(const __grid_cons
             mbar_wait(&sm->bar_s, h - h_lo);
             tc_fence_after();
             float m = -1e30f;
-            for (int c0 = 32 * half; c0 < t.ncols; c0 += 64) {
+            auto chunk_max = [&](int c0) {
                 uint32_t v[32];
                 tmem_ld32(trow + c0, v);
                 tmem_ld_wait();
 #pragma unroll
                 for (int j = 0; j < 32; ++j)
                     if (same_image<MASK>(p, r, c0 + j)) m = fmaxf(m, __uint_as_float(v[j]));
+            };
+            if constexpr (HS == 32) {
+                for (int c0 = 32 * half; c0 < t.ncols; c0 += 64) chunk_max(c0);
+            } else {
+                // (without the head loop ptxas unrolls this loop and spills around the overlapping 32-register loads)
+#pragma unroll 1
+                for (int c0 = 32 * half; c0 < t.ncols; c0 += 64) chunk_max(c0);
             }
             sx[(h * 2 + half) * 128 + r] = m;
             asm volatile("bar.sync 1, 256;" ::: "memory");
@@ -238,16 +259,16 @@ __global__ void __launch_bounds__(kThreads) attn_tc_fwd_kernel(const __grid_cons
             if (h == h_hi - 1) pdl_trigger_late();  // all MMAs of this CTA are complete
             tc_fence_after();
             l += sl[(h * 2 + (half ^ 1)) * 128 + r];  // (ordered by the bar_p arrive / bar_o wait pair)
-            uint32_t o[16];
-            tmem_ld16(trow + o_col + h * 32 + half * 16, o);
+            uint32_t o[HS / 2];
+            tmem_ld_half(trow + o_col + h * HS + half * (HS / 2), o);
             tmem_ld_wait();
             tc_fence_before();
             if (rvalid) {
                 const float inv = 1.f / l;
-                const int head = t.hp * 2 + h;
-                __nv_bfloat16* op = p.out + size_t(gr) * p.ldo + head * HS + half * 16;
+                const int head = t.hp * HPB + h;
+                __nv_bfloat16* op = p.out + size_t(gr) * p.ldo + head * HS + half * (HS / 2);
 #pragma unroll
-                for (int j = 0; j < 2; ++j)
+                for (int j = 0; j < HS / 16; ++j)
                     reinterpret_cast<uint4*>(op)[j] = make_uint4(
                         pack2(__uint_as_float(o[8 * j]) * inv, __uint_as_float(o[8 * j + 1]) * inv),
                         pack2(__uint_as_float(o[8 * j + 2]) * inv, __uint_as_float(o[8 * j + 3]) * inv),
@@ -268,7 +289,7 @@ __global__ void __launch_bounds__(kThreads) attn_tc_fwd_kernel(const __grid_cons
 // =====================================================================================================
 // backward, dQ (rows = queries)
 // =====================================================================================================
-template <bool MASK>
+template <int HS, bool MASK>
 __global__ void __launch_bounds__(kThreads) attn_tc_dq_kernel(const __grid_constant__ AttnTcParams p) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -280,12 +301,14 @@ __global__ void __launch_bounds__(kThreads) attn_tc_dq_kernel(const __grid_const
     uint8_t* sdS = sV + size_t(t.ncols) * 128;  // [2][128][128 B]
     Smem* sm = reinterpret_cast<Smem*>(sdS + 32768);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    constexpr int HPB = 64 / HS;  // heads per box
     const int C = p.NH * HS;
-    const int h_lo = gridDim.z == 2 ? int(blockIdx.z) : 0, h_hi = gridDim.z == 2 ? int(blockIdx.z) + 1 : 2;  // head split
+    const bool hsplit = HS == 32 && gridDim.z == 2;  // head split
+    const int h_lo = hsplit ? int(blockIdx.z) : 0, h_hi = hsplit ? int(blockIdx.z) + 1 : HPB;
     prologue(sm, 512, warp, lane);
     const uint32_t tmem = sm->tmem_slot;
     const int nchunk = t.ncols / 128;
-    // TMEM columns: S [0,128)  dP [128,256)  dQ_h [256 + 64h, +64)
+    // TMEM columns: S [0,128)  dP [128,256)  dQ_h [256 + 64h, +64)  (HS = 64: one head, dQ [256, 320))
 
     if (warp == 0) {
         {
@@ -313,8 +336,8 @@ __global__ void __launch_bounds__(kThreads) attn_tc_dq_kernel(const __grid_const
                 for (int cc = 0; cc < nchunk; ++cc, ++it) {
                     if (elect_one_sync()) {
 #pragma unroll
-                        for (int k = 0; k < 2; ++k) {
-                            const uint64_t o = uint64_t(h * 4 + k * 2);
+                        for (int k = 0; k < HS / 16; ++k) {
+                            const uint64_t o = uint64_t(h * (HS / 8) + k * 2);
                             umma_bf16(tmem, dQ + o, dK + o + uint64_t(cc * 1024), id_s, k);
                             umma_bf16(tmem + 128, dG + o, dV + o + uint64_t(cc * 1024), id_s, k);
                         }
@@ -343,18 +366,18 @@ __global__ void __launch_bounds__(kThreads) attn_tc_dq_kernel(const __grid_const
         const float scale = rsqrtf(float(HS));
         const float c = scale * kLog2e;
         const int b = rvalid ? gr / p.T : 0, tt = rvalid ? gr % p.T : 0;
-        // D = rowsum(dO o O), L = logsumexp (log2 domain), per head of the pair
+        // D = rowsum(dO o O), L = logsumexp (log2 domain), per head of the box
         float Dv[2] = {0.f, 0.f}, Lv[2] = {0.f, 0.f};
         if (rvalid) {
 #pragma unroll
-            for (int h = 0; h < 2; ++h) {
+            for (int h = 0; h < HPB; ++h) {
                 if (h < h_lo || h >= h_hi) continue;
-                const int head = t.hp * 2 + h;
+                const int head = t.hp * HPB + h;
                 const uint4* gp = reinterpret_cast<const uint4*>(p.dout + size_t(gr) * p.lddo + head * HS);
                 const uint4* op = reinterpret_cast<const uint4*>(p.out + size_t(gr) * p.ldo + head * HS);
                 float d = 0.f;
 #pragma unroll
-                for (int j = 0; j < 4; ++j) {
+                for (int j = 0; j < HS / 8; ++j) {
                     float a[8], o[8];
                     unpack8(gp[j], a);
                     unpack8(op[j], o);
@@ -394,14 +417,14 @@ __global__ void __launch_bounds__(kThreads) attn_tc_dq_kernel(const __grid_const
             mbar_wait(&sm->bar_o, (it - 1) & 1);
             if (h == h_hi - 1) pdl_trigger_late();  // all MMAs of this CTA are complete
             tc_fence_after();
-            uint32_t o[16];
-            tmem_ld16(trow + 256 + h * 64 + h * 32 + half * 16, o);
+            uint32_t o[HS / 2];
+            tmem_ld_half(trow + 256 + h * 64 + h * HS + half * (HS / 2), o);
             tmem_ld_wait();
             tc_fence_before();
             if (rvalid) {
-                __nv_bfloat16* op = p.dqkv + size_t(gr) * p.ldd + (t.hp * 2 + h) * HS + half * 16;
+                __nv_bfloat16* op = p.dqkv + size_t(gr) * p.ldd + (t.hp * HPB + h) * HS + half * (HS / 2);
 #pragma unroll
-                for (int j = 0; j < 2; ++j)
+                for (int j = 0; j < HS / 16; ++j)
                     reinterpret_cast<uint4*>(op)[j] = make_uint4(
                         pack2(__uint_as_float(o[8 * j]) * scale, __uint_as_float(o[8 * j + 1]) * scale),
                         pack2(__uint_as_float(o[8 * j + 2]) * scale, __uint_as_float(o[8 * j + 3]) * scale),
@@ -418,7 +441,7 @@ __global__ void __launch_bounds__(kThreads) attn_tc_dq_kernel(const __grid_const
 // =====================================================================================================
 // backward, dK and dV (rows = keys, columns = queries)
 // =====================================================================================================
-template <bool MASK>
+template <int HS, bool MASK>
 __global__ void __launch_bounds__(kThreads) attn_tc_dkv_kernel(const __grid_constant__ AttnTcParams p) {
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
@@ -433,12 +456,15 @@ __global__ void __launch_bounds__(kThreads) attn_tc_dkv_kernel(const __grid_cons
     float* sD = sL + 2 * 256;
     Smem* sm = reinterpret_cast<Smem*>(sD + 2 * 256);
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
+    constexpr int HPB = 64 / HS;  // heads per box
     const int C = p.NH * HS;
-    const int h_lo = gridDim.z == 2 ? int(blockIdx.z) : 0, h_hi = gridDim.z == 2 ? int(blockIdx.z) + 1 : 2;  // head split
+    const bool hsplit = HS == 32 && gridDim.z == 2;  // head split
+    const int h_lo = hsplit ? int(blockIdx.z) : 0, h_hi = hsplit ? int(blockIdx.z) + 1 : HPB;
     prologue(sm, 512, warp, lane);
     const uint32_t tmem = sm->tmem_slot;
     const int nchunk = t.ncols / 128;
     // TMEM columns: S^T [0,128)  dP^T [128,256)  dK_h [256 + 64h, +64)  dV_h [384 + 64h, +64)
+    // (HS = 64: one head, dK [256, 320), dV [384, 448))
 
     if (warp == 0) {
         {
@@ -467,8 +493,8 @@ __global__ void __launch_bounds__(kThreads) attn_tc_dkv_kernel(const __grid_cons
                 for (int cc = 0; cc < nchunk; ++cc, ++it) {
                     if (elect_one_sync()) {
 #pragma unroll
-                        for (int k = 0; k < 2; ++k) {
-                            const uint64_t o = uint64_t(h * 4 + k * 2);
+                        for (int k = 0; k < HS / 16; ++k) {
+                            const uint64_t o = uint64_t(h * (HS / 8) + k * 2);
                             umma_bf16(tmem, dK + o, dQ + o + uint64_t(cc * 1024), id_s, k);
                             umma_bf16(tmem + 128, dV + o, dG + o + uint64_t(cc * 1024), id_s, k);
                         }
@@ -498,21 +524,21 @@ __global__ void __launch_bounds__(kThreads) attn_tc_dkv_kernel(const __grid_cons
         const uint32_t trow = tmem + (uint32_t(q * 32) << 16);
         const float scale = rsqrtf(float(HS));
         const float c = scale * kLog2e;
-        // logsumexp and D of every query column, both heads
-        for (int i = threadIdx.x - 32; i < 2 * t.ncols; i += kRowThreads) {
+        // logsumexp and D of every query column, every head of the box
+        for (int i = threadIdx.x - 32; i < HPB * t.ncols; i += kRowThreads) {
             const int h = i / t.ncols, col = i % t.ncols;
             const int gq = t.col0 + col;
             float L = 0.f, D = 0.f;
             if (gq < p.B * p.T) {
-                const int head = t.hp * 2 + h;
+                const int head = t.hp * HPB + h;
                 const size_t idx = (size_t(gq / p.T) * p.NH + head) * p.T + gq % p.T;
                 L = p.lse[idx];
-                // D = rowsum(dO o O) of the query, recomputed here (32 products) instead of read from the dq kernel's
+                // D = rowsum(dO o O) of the query, recomputed here (HS products) instead of read from the dq kernel's
                 // dsum: the two backward kernels then have no dependency and run concurrently (attn_tc_bwd)
                 const uint4* gp = reinterpret_cast<const uint4*>(p.dout + size_t(gq) * p.lddo + head * HS);
                 const uint4* op = reinterpret_cast<const uint4*>(p.out + size_t(gq) * p.ldo + head * HS);
 #pragma unroll
-                for (int j = 0; j < 4; ++j) {
+                for (int j = 0; j < HS / 8; ++j) {
                     float a[8], o[8];
                     unpack8(gp[j], a);
                     unpack8(op[j], o);
@@ -555,16 +581,16 @@ __global__ void __launch_bounds__(kThreads) attn_tc_dkv_kernel(const __grid_cons
             mbar_wait(&sm->bar_o, (it - 1) & 1);
             if (h == h_hi - 1) pdl_trigger_late();  // all MMAs of this CTA are complete
             tc_fence_after();
-            uint32_t dk[16], dv[16];
-            tmem_ld16(trow + 256 + h * 64 + h * 32 + half * 16, dk);
-            tmem_ld16(trow + 384 + h * 64 + h * 32 + half * 16, dv);
+            uint32_t dk[HS / 2], dv[HS / 2];
+            tmem_ld_half(trow + 256 + h * 64 + h * HS + half * (HS / 2), dk);
+            tmem_ld_half(trow + 384 + h * 64 + h * HS + half * (HS / 2), dv);
             tmem_ld_wait();
             tc_fence_before();
             if (rvalid) {
-                __nv_bfloat16* kp = p.dqkv + size_t(gr) * p.ldd + C + (t.hp * 2 + h) * HS + half * 16;
-                __nv_bfloat16* vp = p.dqkv + size_t(gr) * p.ldd + 2 * C + (t.hp * 2 + h) * HS + half * 16;
+                __nv_bfloat16* kp = p.dqkv + size_t(gr) * p.ldd + C + (t.hp * HPB + h) * HS + half * (HS / 2);
+                __nv_bfloat16* vp = p.dqkv + size_t(gr) * p.ldd + 2 * C + (t.hp * HPB + h) * HS + half * (HS / 2);
 #pragma unroll
-                for (int j = 0; j < 2; ++j) {
+                for (int j = 0; j < HS / 16; ++j) {
                     reinterpret_cast<uint4*>(kp)[j] = make_uint4(
                         pack2(__uint_as_float(dk[8 * j]) * scale, __uint_as_float(dk[8 * j + 1]) * scale),
                         pack2(__uint_as_float(dk[8 * j + 2]) * scale, __uint_as_float(dk[8 * j + 3]) * scale),
@@ -604,31 +630,38 @@ size_t smem_dkv(int ncols) { return 1024 + 32768 + size_t(ncols) * 256 + 65536 +
 
 }  // namespace
 
-bool attn_tc_supported(int T, int NH, int HSz) {
-    if (HSz != HS || (NH % 2) != 0) return false;
+// HS = 32 needs an even NH (a 64-channel box holds a pair of heads); HS = 64 takes any NH >= 1
+bool attn_tc_supported(int T, int NH, int HS) {
+    if (!((HS == 32 && NH >= 2 && NH % 2 == 0) || (HS == 64 && NH >= 1))) return false;
     return T == 256 || T == 128 || T == 64 || T == 32 || T == 16;
+}
+
+template <int HS>
+static void attn_tc_init_hs() {
+    cudaFuncSetAttribute(attn_tc_fwd_kernel<HS, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem_fwd(256)));
+    cudaFuncSetAttribute(attn_tc_dq_kernel<HS, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem_dq(256)));
+    cudaFuncSetAttribute(attn_tc_dkv_kernel<HS, false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem_dkv(256)));
+    cudaFuncSetAttribute(attn_tc_fwd_kernel<HS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem_fwd(128)));
+    cudaFuncSetAttribute(attn_tc_dq_kernel<HS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem_dq(128)));
+    cudaFuncSetAttribute(attn_tc_dkv_kernel<HS, true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem_dkv(128)));
 }
 
 void attn_tc_init() {
     static bool done = false;
     if (done) return;
-    cudaFuncSetAttribute(attn_tc_fwd_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem_fwd(256)));
-    cudaFuncSetAttribute(attn_tc_dq_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem_dq(256)));
-    cudaFuncSetAttribute(attn_tc_dkv_kernel<false>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem_dkv(256)));
-    cudaFuncSetAttribute(attn_tc_fwd_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem_fwd(128)));
-    cudaFuncSetAttribute(attn_tc_dq_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem_dq(128)));
-    cudaFuncSetAttribute(attn_tc_dkv_kernel<true>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(smem_dkv(128)));
+    attn_tc_init_hs<32>();
+    attn_tc_init_hs<64>();
     done = true;
 }
 
-int attn_tc_plan(AttnTcParams* p, const __nv_bfloat16* qkv, int ld, int B, int T, int NH, int HSz,
+int attn_tc_plan(AttnTcParams* p, const __nv_bfloat16* qkv, int ld, int B, int T, int NH, int HS,
                  __nv_bfloat16* out, int ldo, float* lse, const __nv_bfloat16* dout, int lddo, __nv_bfloat16* dqkv,
                  int ldd, float* dsum) {
     memset(p, 0, sizeof(*p));
-    if (!attn_tc_supported(T, NH, HSz)) return -20;
+    if (!attn_tc_supported(T, NH, HS)) return -20;
     const int C = NH * HS;
     if ((ldo % 8) || (ldd % 8) || (lddo % 8)) return -21;
-    p->qkv = qkv, p->ld = ld, p->B = B, p->T = T, p->NH = NH;
+    p->qkv = qkv, p->ld = ld, p->B = B, p->T = T, p->NH = NH, p->HS = HS;
     p->out = out, p->ldo = ldo, p->lse = lse, p->dout = dout, p->lddo = lddo, p->dqkv = dqkv, p->ldd = ldd;
     p->dsum = dsum;
     for (p->tshift = 0; (1 << p->tshift) < T; ++p->tshift) {
@@ -639,26 +672,45 @@ int attn_tc_plan(AttnTcParams* p, const __nv_bfloat16* qkv, int ld, int B, int T
     return r;
 }
 
-// Head split (UB_ATTN_HSPLIT bit mask: 1 forward, 2 dq, 4 dkv; default 1): a CTA owns 128 rows x a PAIR of heads (one
-// 64-channel box) and works through the two heads one after the other; with the split the pair is shared by two CTAs
-// (grid z) that each load the box and take one head.  T = 256: 192 one-per-SM CTAs are two waves on 148 SMs, 384 half
-// CTAs are three half-waves; T = 64: 64 CTAs become 128.
+// Head split (UB_ATTN_HSPLIT bit mask: 1 forward, 2 dq, 4 dkv; default 1), HS = 32 only: a CTA owns 128 rows x a PAIR
+// of heads (one 64-channel box) and works through the two heads one after the other; with the split the pair is shared
+// by two CTAs (grid z) that each load the box and take one head.  T = 256: 192 one-per-SM CTAs are two waves on 148
+// SMs, 384 half CTAs are three half-waves; T = 64: 64 CTAs become 128.  At HS = 64 a box is one head: nothing to split.
 static int attn_hsplit() {
     static const int v = getenv("UB_ATTN_HSPLIT") ? atoi(getenv("UB_ATTN_HSPLIT")) : 1;
     return v;
 }
 static dim3 attn_grid(const AttnTcParams& p, int bit) {
-    return dim3((p.B * p.T + 127) / 128, p.NH / 2, (attn_hsplit() & bit) ? 2 : 1);
+    return dim3((p.B * p.T + 127) / 128, p.NH * p.HS / 64, (p.HS == 32 && (attn_hsplit() & bit)) ? 2 : 1);
 }
 static int attn_ncols(const AttnTcParams& p) { return p.T >= 128 ? p.T : 128; }
 
+template <int HS>
+static void attn_tc_fwd_hs(const AttnTcParams& p, cudaStream_t st) {
+    if (p.T >= 128)
+        launch_pdl(attn_tc_fwd_kernel<HS, false>, dim3(attn_grid(p, 1)), dim3(kThreads), smem_fwd(attn_ncols(p)), st, p);
+    else
+        launch_pdl(attn_tc_fwd_kernel<HS, true>, dim3(attn_grid(p, 1)), dim3(kThreads), smem_fwd(attn_ncols(p)), st, p);
+}
+
 int attn_tc_fwd(const AttnTcParams& p, cudaStream_t st) {
     attn_tc_init();
-    if (p.T >= 128)
-        launch_pdl(attn_tc_fwd_kernel<false>, dim3(attn_grid(p, 1)), dim3(kThreads), smem_fwd(attn_ncols(p)), st, p);
+    if (p.HS == 64)
+        attn_tc_fwd_hs<64>(p, st);
     else
-        launch_pdl(attn_tc_fwd_kernel<true>, dim3(attn_grid(p, 1)), dim3(kThreads), smem_fwd(attn_ncols(p)), st, p);
+        attn_tc_fwd_hs<32>(p, st);
     return int(cudaGetLastError());
+}
+
+template <int HS>
+static void attn_tc_bwd_hs(const AttnTcParams& p, cudaStream_t st, cudaStream_t s2) {
+    if (p.T >= 128) {
+        launch_pdl(attn_tc_dkv_kernel<HS, false>, dim3(attn_grid(p, 4)), dim3(kThreads), smem_dkv(attn_ncols(p)), s2, p);
+        launch_pdl(attn_tc_dq_kernel<HS, false>, dim3(attn_grid(p, 2)), dim3(kThreads), smem_dq(attn_ncols(p)), st, p);
+    } else {
+        launch_pdl(attn_tc_dkv_kernel<HS, true>, dim3(attn_grid(p, 4)), dim3(kThreads), smem_dkv(attn_ncols(p)), s2, p);
+        launch_pdl(attn_tc_dq_kernel<HS, true>, dim3(attn_grid(p, 2)), dim3(kThreads), smem_dq(attn_ncols(p)), st, p);
+    }
 }
 
 // dq and dkv are independent (each recomputes S and D): with an auxiliary stream and two events the dkv kernel runs
@@ -672,13 +724,10 @@ int attn_tc_bwd(const AttnTcParams& p, cudaStream_t st, cudaStream_t aux, cudaEv
         cudaStreamWaitEvent(aux, ev_fork, 0);
         s2 = aux;
     }
-    if (p.T >= 128) {
-        launch_pdl(attn_tc_dkv_kernel<false>, dim3(attn_grid(p, 4)), dim3(kThreads), smem_dkv(attn_ncols(p)), s2, p);
-        launch_pdl(attn_tc_dq_kernel<false>, dim3(attn_grid(p, 2)), dim3(kThreads), smem_dq(attn_ncols(p)), st, p);
-    } else {
-        launch_pdl(attn_tc_dkv_kernel<true>, dim3(attn_grid(p, 4)), dim3(kThreads), smem_dkv(attn_ncols(p)), s2, p);
-        launch_pdl(attn_tc_dq_kernel<true>, dim3(attn_grid(p, 2)), dim3(kThreads), smem_dq(attn_ncols(p)), st, p);
-    }
+    if (p.HS == 64)
+        attn_tc_bwd_hs<64>(p, st, s2);
+    else
+        attn_tc_bwd_hs<32>(p, st, s2);
     if (s2 != st) {
         cudaEventRecord(ev_join, s2);
         cudaStreamWaitEvent(st, ev_join, 0);

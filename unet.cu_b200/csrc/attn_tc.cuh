@@ -1,4 +1,4 @@
-// tcgen05 attention core (head size 32, T in {16,32,64,128,256}) on the internal NHWC bf16 qkv tensor; see attn_tc.cu.
+// tcgen05 attention core (head size 32 with an even head count, or 64; T in {16,32,64,128,256}) on the internal NHWC bf16 qkv tensor; see attn_tc.cu.
 #pragma once
 #include <cuda.h>
 #include <cuda_bf16.h>
@@ -21,6 +21,7 @@ struct AttnTcParams {
     __nv_bfloat16* dqkv;  // [B*T][ldd], sections [dQ | dK | dV]
     int ldd;
     float* dsum;          // [B][NH][T] rowsum(dO o O), written by the dq kernel (the dkv kernel recomputes it)
+    int HS;               // head size, 32 or 64 (selects the kernel instantiation)
 };
 
 bool attn_tc_supported(int T, int NH, int HS);

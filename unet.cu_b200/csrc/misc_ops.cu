@@ -31,15 +31,18 @@ __device__ __forceinline__ void st8f(bf16* p, const float* f) {
 }
 
 // =====================================================================================================
-// attention core, head size 32, one thread per query (forward, dq) or per key (dk, dv)
+// attention core, head size 32 or 64, one row (query for forward / dq, key for dk, dv) per LPR = HS/32 lanes: a lane
+// owns 32 channels of its row, and the dot products of a row are combined with one shfl.xor.  (HS = 64 with one thread
+// per row would hold 4 x 64 fp32 values per thread in the dkv kernel and spill.)
 // =====================================================================================================
-static constexpr int HS = 32;
-static constexpr int KT = 256;  // keys (or queries) staged in smem per chunk
+static constexpr int kStage = 8192;  // fp32 values of one staged [KT][HS] operand: KT = kStage / HS rows per chunk
 
-// stage `n` rows of a 32-channel slice (row r at src + r*ld) into smem as fp32 [n][32]
+// stage `n` rows of an HS-channel slice (row r at src + r*ld) into smem as fp32 [n][HS]
+template <int HS>
 __device__ __forceinline__ void stage_rows(const bf16* src, int ld, int n, float* dst, float scale) {
-    for (int i = threadIdx.x; i < n * 4; i += blockDim.x) {
-        const int r = i >> 2, part = i & 3;
+    constexpr int kParts = HS / 8, kPartsLog2 = HS == 64 ? 3 : 2;  // 16-byte parts per row
+    for (int i = threadIdx.x; i < n * kParts; i += blockDim.x) {
+        const int r = i >> kPartsLog2, part = i & (kParts - 1);
         float f[8];
         ld8f(src + size_t(r) * ld + part * 8, f);
 #pragma unroll
@@ -47,44 +50,58 @@ __device__ __forceinline__ void stage_rows(const bf16* src, int ld, int n, float
     }
 }
 
-__global__ void __launch_bounds__(128) attn_fwd_kernel(const bf16* __restrict__ qkv, int ld, int T, int NH,
+// sum of a row's partial dot products over its LPR lanes (adjacent lanes)
+template <int LPR>
+__device__ __forceinline__ float row_sum(float a) {
+    if constexpr (LPR == 2) a += __shfl_xor_sync(0xffffffffu, a, 1);
+    return a;
+}
+
+// HS = 64 asks for one resident block (minBlocks 1): without that hint ptxas caps the kernel at 96 registers and spills
+// the row index across the key loop.  HS = 32 keeps the plain bound (minBlocks 0 = no hint).
+template <int HS>
+__global__ void __launch_bounds__(128, HS == 64 ? 1 : 0) attn_fwd_kernel(const bf16* __restrict__ qkv, int ld, int T, int NH,
                                                        bf16* __restrict__ out, int ldo, float* __restrict__ lse) {
+    constexpr int LPR = HS / 32, KT = kStage / HS;
     pdl_entry();
-    extern __shared__ float smf[];  // K [KT][32], V [KT][32]
+    extern __shared__ float smf[];  // K [KT][HS], V [KT][HS]
     float* sK = smf;
     float* sV = smf + KT * HS;
     const int h = blockIdx.y, b = blockIdx.z;
     const int C = NH * HS;
-    const int qi = blockIdx.x * blockDim.x + threadIdx.x;
+    const int part = LPR == 1 ? 0 : int(threadIdx.x) & (LPR - 1);  // this lane's 32 channels: [part*32, part*32+32)
+    const int qi = blockIdx.x * (blockDim.x / LPR) + threadIdx.x / LPR;
     const bool active = qi < T;
     const bf16* base = qkv + size_t(b) * T * ld;
-    float q[HS], acc[HS];
+    const int ch = h * HS + part * 32;
+    float q[32], acc[32];
     const float qscale = rsqrtf(float(HS)) * kLog2e;
     if (active) {
 #pragma unroll
-        for (int part = 0; part < 4; ++part) ld8f(base + size_t(qi) * ld + h * HS + part * 8, q + part * 8);
+        for (int p8 = 0; p8 < 4; ++p8) ld8f(base + size_t(qi) * ld + ch + p8 * 8, q + p8 * 8);
     }
 #pragma unroll
-    for (int d = 0; d < HS; ++d) q[d] = active ? q[d] * qscale : 0.f, acc[d] = 0.f;
+    for (int d = 0; d < 32; ++d) q[d] = active ? q[d] * qscale : 0.f, acc[d] = 0.f;
     float m = -1e30f, l = 0.f;
     for (int k0 = 0; k0 < T; k0 += KT) {
         const int nk = min(KT, T - k0);
         __syncthreads();
-        stage_rows(base + size_t(k0) * ld + C + h * HS, ld, nk, sK, 1.f);
-        stage_rows(base + size_t(k0) * ld + 2 * C + h * HS, ld, nk, sV, 1.f);
+        stage_rows<HS>(base + size_t(k0) * ld + C + h * HS, ld, nk, sK, 1.f);
+        stage_rows<HS>(base + size_t(k0) * ld + 2 * C + h * HS, ld, nk, sV, 1.f);
         __syncthreads();
         for (int j0 = 0; j0 < nk; j0 += 8) {
             float s[8];
             float cmax = -1e30f;
 #pragma unroll
             for (int jj = 0; jj < 8; ++jj) {
-                const float4* kr = reinterpret_cast<const float4*>(sK + (j0 + jj) * HS);
+                const float4* kr = reinterpret_cast<const float4*>(sK + (j0 + jj) * HS + part * 32);
                 float a = 0.f;
 #pragma unroll
                 for (int d4 = 0; d4 < 8; ++d4) {
                     const float4 kv = kr[d4];
                     a += q[d4 * 4] * kv.x + q[d4 * 4 + 1] * kv.y + q[d4 * 4 + 2] * kv.z + q[d4 * 4 + 3] * kv.w;
                 }
+                a = row_sum<LPR>(a);
                 s[jj] = (j0 + jj < nk) ? a : -1e30f;
                 cmax = fmaxf(cmax, s[jj]);
             }
@@ -92,7 +109,7 @@ __global__ void __launch_bounds__(128) attn_fwd_kernel(const bf16* __restrict__ 
                 const float corr = exp2f(m - cmax);
                 l *= corr;
 #pragma unroll
-                for (int d = 0; d < HS; ++d) acc[d] *= corr;
+                for (int d = 0; d < 32; ++d) acc[d] *= corr;
                 m = cmax;
             }
 #pragma unroll
@@ -100,7 +117,7 @@ __global__ void __launch_bounds__(128) attn_fwd_kernel(const bf16* __restrict__ 
                 if (j0 + jj >= nk) continue;  // never touch unstaged smem rows
                 const float p = exp2f(s[jj] - m);
                 l += p;
-                const float4* vr = reinterpret_cast<const float4*>(sV + (j0 + jj) * HS);
+                const float4* vr = reinterpret_cast<const float4*>(sV + (j0 + jj) * HS + part * 32);
 #pragma unroll
                 for (int d4 = 0; d4 < 8; ++d4) {
                     const float4 vv = vr[d4];
@@ -113,48 +130,55 @@ __global__ void __launch_bounds__(128) attn_fwd_kernel(const bf16* __restrict__ 
     if (active) {
         const float inv = 1.f / l;
 #pragma unroll
-        for (int d = 0; d < HS; ++d) acc[d] *= inv;
-        bf16* op = out + (size_t(b) * T + qi) * ldo + h * HS;
+        for (int d = 0; d < 32; ++d) acc[d] *= inv;
+        bf16* op = out + (size_t(b) * T + qi) * ldo + ch;
 #pragma unroll
-        for (int part = 0; part < 4; ++part) st8f(op + part * 8, acc + part * 8);
-        lse[(size_t(b) * NH + h) * T + qi] = m + log2f(l);
+        for (int p8 = 0; p8 < 4; ++p8) st8f(op + p8 * 8, acc + p8 * 8);
+        if (part == 0) lse[(size_t(b) * NH + h) * T + qi] = m + log2f(l);
     }
 }
 
-// dq: thread per query
+// dq: LPR lanes per query
+template <int HS>
 __global__ void __launch_bounds__(128) attn_bwd_dq_kernel(const bf16* __restrict__ qkv, int ld,
                                                           const bf16* __restrict__ out, int ldo,
                                                           const bf16* __restrict__ dout, int lddo,
                                                           const float* __restrict__ lse, int T, int NH,
                                                           bf16* __restrict__ dqkv, int ldd,
                                                           float* __restrict__ dsum) {
+    constexpr int LPR = HS / 32, KT = kStage / HS;
     pdl_entry();
     extern __shared__ float smf[];
     float* sK = smf;
     float* sV = smf + KT * HS;
     const int h = blockIdx.y, b = blockIdx.z;
     const int C = NH * HS;
-    const int qi = blockIdx.x * blockDim.x + threadIdx.x;
+    const int part = LPR == 1 ? 0 : int(threadIdx.x) & (LPR - 1);
+    const int qi = blockIdx.x * (blockDim.x / LPR) + threadIdx.x / LPR;
     const bool active = qi < T;
     const bf16* base = qkv + size_t(b) * T * ld;
-    float q[HS], dO[HS], dq[HS];
+    const int ch = h * HS + part * 32;
+    float q[32], dO[32], dq[32];
     const float scale = rsqrtf(float(HS));
     float Dv = 0.f, L = 0.f;
     if (active) {
-        float o[HS];
+        float o[32];
 #pragma unroll
-        for (int part = 0; part < 4; ++part) {
-            ld8f(base + size_t(qi) * ld + h * HS + part * 8, q + part * 8);
-            ld8f(dout + (size_t(b) * T + qi) * lddo + h * HS + part * 8, dO + part * 8);
-            ld8f(out + (size_t(b) * T + qi) * ldo + h * HS + part * 8, o + part * 8);
+        for (int p8 = 0; p8 < 4; ++p8) {
+            ld8f(base + size_t(qi) * ld + ch + p8 * 8, q + p8 * 8);
+            ld8f(dout + (size_t(b) * T + qi) * lddo + ch + p8 * 8, dO + p8 * 8);
+            ld8f(out + (size_t(b) * T + qi) * ldo + ch + p8 * 8, o + p8 * 8);
         }
 #pragma unroll
-        for (int d = 0; d < HS; ++d) Dv += dO[d] * o[d];
+        for (int d = 0; d < 32; ++d) Dv += dO[d] * o[d];
+    }
+    Dv = row_sum<LPR>(Dv);  // (both lanes of a row share `active`: the shuffle stays outside the branch)
+    if (active) {
         L = lse[(size_t(b) * NH + h) * T + qi];
-        dsum[(size_t(b) * NH + h) * T + qi] = Dv;
+        if (part == 0) dsum[(size_t(b) * NH + h) * T + qi] = Dv;
     }
 #pragma unroll
-    for (int d = 0; d < HS; ++d) {
+    for (int d = 0; d < 32; ++d) {
         q[d] = active ? q[d] * scale * kLog2e : 0.f;
         if (!active) dO[d] = 0.f;
         dq[d] = 0.f;
@@ -162,12 +186,12 @@ __global__ void __launch_bounds__(128) attn_bwd_dq_kernel(const bf16* __restrict
     for (int k0 = 0; k0 < T; k0 += KT) {
         const int nk = min(KT, T - k0);
         __syncthreads();
-        stage_rows(base + size_t(k0) * ld + C + h * HS, ld, nk, sK, 1.f);
-        stage_rows(base + size_t(k0) * ld + 2 * C + h * HS, ld, nk, sV, 1.f);
+        stage_rows<HS>(base + size_t(k0) * ld + C + h * HS, ld, nk, sK, 1.f);
+        stage_rows<HS>(base + size_t(k0) * ld + 2 * C + h * HS, ld, nk, sV, 1.f);
         __syncthreads();
         for (int j = 0; j < nk; ++j) {
-            const float4* kr = reinterpret_cast<const float4*>(sK + j * HS);
-            const float4* vr = reinterpret_cast<const float4*>(sV + j * HS);
+            const float4* kr = reinterpret_cast<const float4*>(sK + j * HS + part * 32);
+            const float4* vr = reinterpret_cast<const float4*>(sV + j * HS + part * 32);
             float s = 0.f, dp = 0.f;
 #pragma unroll
             for (int d4 = 0; d4 < 8; ++d4) {
@@ -176,6 +200,7 @@ __global__ void __launch_bounds__(128) attn_bwd_dq_kernel(const bf16* __restrict
                 s += q[d4 * 4] * kv.x + q[d4 * 4 + 1] * kv.y + q[d4 * 4 + 2] * kv.z + q[d4 * 4 + 3] * kv.w;
                 dp += dO[d4 * 4] * vv.x + dO[d4 * 4 + 1] * vv.y + dO[d4 * 4 + 2] * vv.z + dO[d4 * 4 + 3] * vv.w;
             }
+            s = row_sum<LPR>(s), dp = row_sum<LPR>(dp);
             const float ds = exp2f(s - L) * (dp - Dv);
 #pragma unroll
             for (int d4 = 0; d4 < 8; ++d4) {
@@ -187,40 +212,44 @@ __global__ void __launch_bounds__(128) attn_bwd_dq_kernel(const bf16* __restrict
     }
     if (active) {
 #pragma unroll
-        for (int d = 0; d < HS; ++d) dq[d] *= scale;
-        bf16* op = dqkv + (size_t(b) * T + qi) * ldd + h * HS;
+        for (int d = 0; d < 32; ++d) dq[d] *= scale;
+        bf16* op = dqkv + (size_t(b) * T + qi) * ldd + ch;
 #pragma unroll
-        for (int part = 0; part < 4; ++part) st8f(op + part * 8, dq + part * 8);
+        for (int p8 = 0; p8 < 4; ++p8) st8f(op + p8 * 8, dq + p8 * 8);
     }
 }
 
-// dk, dv: thread per key
+// dk, dv: LPR lanes per key
+template <int HS>
 __global__ void __launch_bounds__(128) attn_bwd_dkv_kernel(const bf16* __restrict__ qkv, int ld,
                                                            const bf16* __restrict__ dout, int lddo,
                                                            const float* __restrict__ lse,
                                                            const float* __restrict__ dsum, int T, int NH,
                                                            bf16* __restrict__ dqkv, int ldd) {
+    constexpr int LPR = HS / 32, KT = kStage / HS;
     pdl_entry();
-    extern __shared__ float smf[];  // Q(scaled) [KT][32], dO [KT][32], lse [KT], D [KT]
+    extern __shared__ float smf[];  // Q(scaled) [KT][HS], dO [KT][HS], lse [KT], D [KT]
     float* sQ = smf;
     float* sdO = smf + KT * HS;
     float* sL = smf + 2 * KT * HS;
     float* sD = sL + KT;
     const int h = blockIdx.y, b = blockIdx.z;
     const int C = NH * HS;
-    const int kj = blockIdx.x * blockDim.x + threadIdx.x;
+    const int part = LPR == 1 ? 0 : int(threadIdx.x) & (LPR - 1);
+    const int kj = blockIdx.x * (blockDim.x / LPR) + threadIdx.x / LPR;
     const bool active = kj < T;
     const bf16* base = qkv + size_t(b) * T * ld;
-    float k[HS], v[HS], dk[HS], dv[HS];
+    const int ch = h * HS + part * 32;
+    float k[32], v[32], dk[32], dv[32];
     if (active) {
 #pragma unroll
-        for (int part = 0; part < 4; ++part) {
-            ld8f(base + size_t(kj) * ld + C + h * HS + part * 8, k + part * 8);
-            ld8f(base + size_t(kj) * ld + 2 * C + h * HS + part * 8, v + part * 8);
+        for (int p8 = 0; p8 < 4; ++p8) {
+            ld8f(base + size_t(kj) * ld + C + ch + p8 * 8, k + p8 * 8);
+            ld8f(base + size_t(kj) * ld + 2 * C + ch + p8 * 8, v + p8 * 8);
         }
     }
 #pragma unroll
-    for (int d = 0; d < HS; ++d) {
+    for (int d = 0; d < 32; ++d) {
         if (!active) k[d] = 0.f, v[d] = 0.f;
         dk[d] = 0.f, dv[d] = 0.f;
     }
@@ -228,16 +257,16 @@ __global__ void __launch_bounds__(128) attn_bwd_dkv_kernel(const bf16* __restric
     for (int q0 = 0; q0 < T; q0 += KT) {
         const int nq = min(KT, T - q0);
         __syncthreads();
-        stage_rows(base + size_t(q0) * ld + h * HS, ld, nq, sQ, qscale);
-        stage_rows(dout + (size_t(b) * T + q0) * lddo + h * HS, lddo, nq, sdO, 1.f);
+        stage_rows<HS>(base + size_t(q0) * ld + h * HS, ld, nq, sQ, qscale);
+        stage_rows<HS>(dout + (size_t(b) * T + q0) * lddo + h * HS, lddo, nq, sdO, 1.f);
         for (int i = threadIdx.x; i < nq; i += blockDim.x) {
             sL[i] = lse[(size_t(b) * NH + h) * T + q0 + i];
             sD[i] = dsum[(size_t(b) * NH + h) * T + q0 + i];
         }
         __syncthreads();
         for (int i = 0; i < nq; ++i) {
-            const float4* qr = reinterpret_cast<const float4*>(sQ + i * HS);
-            const float4* gr = reinterpret_cast<const float4*>(sdO + i * HS);
+            const float4* qr = reinterpret_cast<const float4*>(sQ + i * HS + part * 32);
+            const float4* gr = reinterpret_cast<const float4*>(sdO + i * HS + part * 32);
             float s = 0.f, dp = 0.f;
 #pragma unroll
             for (int d4 = 0; d4 < 8; ++d4) {
@@ -246,6 +275,7 @@ __global__ void __launch_bounds__(128) attn_bwd_dkv_kernel(const bf16* __restric
                 s += k[d4 * 4] * qv.x + k[d4 * 4 + 1] * qv.y + k[d4 * 4 + 2] * qv.z + k[d4 * 4 + 3] * qv.w;
                 dp += v[d4 * 4] * gv.x + v[d4 * 4 + 1] * gv.y + v[d4 * 4 + 2] * gv.z + v[d4 * 4 + 3] * gv.w;
             }
+            s = row_sum<LPR>(s), dp = row_sum<LPR>(dp);
             const float p = exp2f(s - sL[i]);
             const float ds = p * (dp - sD[i]);
 #pragma unroll
@@ -262,45 +292,71 @@ __global__ void __launch_bounds__(128) attn_bwd_dkv_kernel(const bf16* __restric
     if (active) {
         // sQ holds q * scale * log2e, so sum(ds * sQ) = log2e * (scale * sum ds q): multiply by ln2
 #pragma unroll
-        for (int d = 0; d < HS; ++d) dk[d] *= kLn2;
-        bf16* okp = dqkv + (size_t(b) * T + kj) * ldd + C + h * HS;
-        bf16* ovp = dqkv + (size_t(b) * T + kj) * ldd + 2 * C + h * HS;
+        for (int d = 0; d < 32; ++d) dk[d] *= kLn2;
+        bf16* okp = dqkv + (size_t(b) * T + kj) * ldd + C + ch;
+        bf16* ovp = dqkv + (size_t(b) * T + kj) * ldd + 2 * C + ch;
 #pragma unroll
-        for (int part = 0; part < 4; ++part) {
-            st8f(okp + part * 8, dk + part * 8);
-            st8f(ovp + part * 8, dv + part * 8);
+        for (int p8 = 0; p8 < 4; ++p8) {
+            st8f(okp + p8 * 8, dk + p8 * 8);
+            st8f(ovp + p8 * 8, dv + p8 * 8);
         }
     }
 }
 
 static int attn_block_threads(int T) { return T >= 128 ? 128 : (T >= 64 ? 64 : 32); }
+static constexpr int kSmemKV = 2 * kStage * 4;                                        // fwd, dq
+template <int HS> static constexpr int smem_attn_dkv() { return (2 * kStage + 2 * (kStage / HS)) * 4; }
 
 void attn_init() {
     static bool cfg = false;
     if (cfg) return;
-    cudaFuncSetAttribute(attn_fwd_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * KT * HS * 4);
-    cudaFuncSetAttribute(attn_bwd_dq_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 2 * KT * HS * 4);
-    cudaFuncSetAttribute(attn_bwd_dkv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, (2 * KT * HS + 2 * KT) * 4);
+    cudaFuncSetAttribute(attn_fwd_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemKV);
+    cudaFuncSetAttribute(attn_bwd_dq_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemKV);
+    cudaFuncSetAttribute(attn_bwd_dkv_kernel<32>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_attn_dkv<32>());
+    cudaFuncSetAttribute(attn_fwd_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemKV);
+    cudaFuncSetAttribute(attn_bwd_dq_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, kSmemKV);
+    cudaFuncSetAttribute(attn_bwd_dkv_kernel<64>, cudaFuncAttributeMaxDynamicSharedMemorySize, smem_attn_dkv<64>());
     cfg = true;
 }
 
-int attn_fwd(const bf16* qkv, int ld, int B, int T, int NH, int HSz, bf16* out, int ldo, float* lse,
+// grid: (row blocks, NH, B); a block of bt threads covers bt / LPR rows
+template <int HS>
+static dim3 attn_simt_grid(int B, int T, int NH) {
+    const int rows = attn_block_threads(T) / (HS / 32);
+    return dim3((T + rows - 1) / rows, NH, B);
+}
+
+int attn_fwd(const bf16* qkv, int ld, int B, int T, int NH, int HS, bf16* out, int ldo, float* lse,
              cudaStream_t st) {
-    if (HSz != HS) return -20;
+    if (HS != 32 && HS != 64) return -20;
     attn_init();
     const int bt = attn_block_threads(T);
-    launch_pdl(attn_fwd_kernel, dim3(dim3((T + bt - 1) / bt, NH, B)), dim3(bt), 2 * KT * HS * 4, st, qkv, ld, T, NH, out, ldo, lse);
+    if (HS == 64)
+        launch_pdl(attn_fwd_kernel<64>, attn_simt_grid<64>(B, T, NH), dim3(bt), kSmemKV, st, qkv, ld, T, NH, out, ldo, lse);
+    else
+        launch_pdl(attn_fwd_kernel<32>, attn_simt_grid<32>(B, T, NH), dim3(bt), kSmemKV, st, qkv, ld, T, NH, out, ldo, lse);
     return int(cudaGetLastError());
 }
 
-int attn_bwd(const bf16* qkv, int ld, const bf16* out, int ldo, const bf16* dout, int lddo, const float* lse, int B,
-             int T, int NH, int HSz, bf16* dqkv, int ldd, float* dsum, cudaStream_t st) {
-    if (HSz != HS) return -20;
+template <int HS>
+static void attn_bwd_hs(const bf16* qkv, int ld, const bf16* out, int ldo, const bf16* dout, int lddo, const float* lse,
+                        int B, int T, int NH, bf16* dqkv, int ldd, float* dsum, cudaStream_t st) {
     const int bt = attn_block_threads(T);
-    dim3 grid((T + bt - 1) / bt, NH, B);
-    launch_pdl(attn_bwd_dq_kernel, dim3(grid), dim3(bt), 2 * KT * HS * 4, st, qkv, ld, out, ldo, dout, lddo, lse, T, NH, dqkv, ldd, dsum);
-    launch_pdl(attn_bwd_dkv_kernel, dim3(grid), dim3(bt), (2 * KT * HS + 2 * KT) * 4, st, qkv, ld, dout, lddo, lse, dsum, T, NH, dqkv,
-                                                                        ldd);
+    const dim3 grid = attn_simt_grid<HS>(B, T, NH);
+    launch_pdl(attn_bwd_dq_kernel<HS>, dim3(grid), dim3(bt), kSmemKV, st, qkv, ld, out, ldo, dout, lddo, lse, T, NH, dqkv,
+               ldd, dsum);
+    launch_pdl(attn_bwd_dkv_kernel<HS>, dim3(grid), dim3(bt), smem_attn_dkv<HS>(), st, qkv, ld, dout, lddo, lse, dsum, T,
+               NH, dqkv, ldd);
+}
+
+int attn_bwd(const bf16* qkv, int ld, const bf16* out, int ldo, const bf16* dout, int lddo, const float* lse, int B,
+             int T, int NH, int HS, bf16* dqkv, int ldd, float* dsum, cudaStream_t st) {
+    if (HS != 32 && HS != 64) return -20;
+    attn_init();
+    if (HS == 64)
+        attn_bwd_hs<64>(qkv, ld, out, ldo, dout, lddo, lse, B, T, NH, dqkv, ldd, dsum, st);
+    else
+        attn_bwd_hs<32>(qkv, ld, out, ldo, dout, lddo, lse, B, T, NH, dqkv, ldd, dsum, st);
     return int(cudaGetLastError());
 }
 

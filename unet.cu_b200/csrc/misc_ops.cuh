@@ -10,7 +10,7 @@ namespace ub {
 typedef __nv_bfloat16 bf16;
 
 // ---- attention core (replaces attention_forward1 / attention_backward, /root/reference/train_unet.cu:2553-2760)
-// qkv: NHWC bf16 [B*T][ld], channel order [Q | K | V], each [NH][HS] (dev/unet.py:75-87); HS must be 32.
+// qkv: NHWC bf16 [B*T][ld], channel order [Q | K | V], each [NH][HS] (dev/unet.py:75-87); HS = 32 or 64 (else -20).
 // out[B*T][ldo] (C = NH*HS channels); lse[B][NH][T] = log2-domain logsumexp of the scaled scores.
 void attn_init();
 int attn_fwd(const bf16* qkv, int ld, int B, int T, int NH, int HS, bf16* out, int ldo, float* lse, cudaStream_t st);

@@ -531,18 +531,26 @@ int ub_conv2d_nhwc_wgrad(const void* dout, const void* x, float* dweight, float*
 
 extern "C" {
 // ---- attention core, native layout
-int ub_attention_nhwc_forward(const void* qkv, void* out, float* lse, int B, int T, int C, int NH, int impl) {
-    if (NH < 1 || C != NH * 32) {
-        fail("attention_nhwc: head size must be 32 (C == NH * 32)");
-        return UB_ERR_SHAPE;
+// head size C / NH (32 or 64) if impl can run the shape, else 0 with the reason set
+static int attention_shape_check(int C, int NH, int T, int impl) {
+    const int HS = NH < 1 ? 0 : (C == NH * 32 ? 32 : (C == NH * 64 ? 64 : 0));
+    if (!HS) {
+        fail("attention_nhwc: head size must be 32 or 64 (C == NH * 32 or C == NH * 64)");
+        return 0;
     }
+    if (impl == 0 && !attn_tc_supported(T, NH, HS)) {
+        fail("attention_nhwc: the tcgen05 kernels need T in {16,32,64,128,256} and, at head size 32, an even NH");
+        return 0;
+    }
+    return HS;
+}
+
+int ub_attention_nhwc_forward(const void* qkv, void* out, float* lse, int B, int T, int C, int NH, int impl) {
+    const int HS = attention_shape_check(C, NH, T, impl);
+    if (!HS) return UB_ERR_SHAPE;
     if (impl == 0) {
-        if (!attn_tc_supported(T, NH, 32)) {
-            fail("attention_nhwc: the tcgen05 kernels need T in {16,32,64,128,256} and an even NH");
-            return UB_ERR_SHAPE;
-        }
         AttnTcParams p;
-        int r = attn_tc_plan(&p, (const bf16*)qkv, 3 * C, B, T, NH, 32, (bf16*)out, C, lse, nullptr, 0, nullptr, 0,
+        int r = attn_tc_plan(&p, (const bf16*)qkv, 3 * C, B, T, NH, HS, (bf16*)out, C, lse, nullptr, 0, nullptr, 0,
                              nullptr);
         if (r) {
             fail("attn_tc_plan failed (%d)", r);
@@ -550,23 +558,17 @@ int ub_attention_nhwc_forward(const void* qkv, void* out, float* lse, int B, int
         }
         attn_tc_fwd(p, ub_layer_stream());
     } else {
-        attn_fwd((const bf16*)qkv, 3 * C, B, T, NH, 32, (bf16*)out, C, lse, ub_layer_stream());
+        attn_fwd((const bf16*)qkv, 3 * C, B, T, NH, HS, (bf16*)out, C, lse, ub_layer_stream());
     }
     return finish(1);
 }
 int ub_attention_nhwc_backward(const void* qkv, const void* out, const void* dout, const float* lse, void* dqkv,
                                float* dsum, int B, int T, int C, int NH, int impl) {
-    if (NH < 1 || C != NH * 32) {
-        fail("attention_nhwc: head size must be 32 (C == NH * 32)");
-        return UB_ERR_SHAPE;
-    }
+    const int HS = attention_shape_check(C, NH, T, impl);
+    if (!HS) return UB_ERR_SHAPE;
     if (impl == 0) {
-        if (!attn_tc_supported(T, NH, 32)) {
-            fail("attention_nhwc: the tcgen05 kernels need T in {16,32,64,128,256} and an even NH");
-            return UB_ERR_SHAPE;
-        }
         AttnTcParams p;
-        int r = attn_tc_plan(&p, (const bf16*)qkv, 3 * C, B, T, NH, 32, (bf16*)const_cast<void*>(out), C,
+        int r = attn_tc_plan(&p, (const bf16*)qkv, 3 * C, B, T, NH, HS, (bf16*)const_cast<void*>(out), C,
                              const_cast<float*>(lse), (const bf16*)dout, C, (bf16*)dqkv, 3 * C, dsum);
         if (r) {
             fail("attn_tc_plan failed (%d)", r);
@@ -574,7 +576,7 @@ int ub_attention_nhwc_backward(const void* qkv, const void* out, const void* dou
         }
         attn_tc_bwd(p, ub_layer_stream());
     } else {
-        attn_bwd((const bf16*)qkv, 3 * C, (const bf16*)out, C, (const bf16*)dout, C, lse, B, T, NH, 32, (bf16*)dqkv,
+        attn_bwd((const bf16*)qkv, 3 * C, (const bf16*)out, C, (const bf16*)dout, C, lse, B, T, NH, HS, (bf16*)dqkv,
                  3 * C, dsum, ub_layer_stream());
     }
     return finish(2);

@@ -855,7 +855,8 @@ struct Builder {
             ep.bias = P(bq), ep.out = qkv.p, ep.ldo = qkv.ld;
             conv_op(true, {{g.p, C, g.ld, pq.wf, 1}}, H, W, 3 * C, ep);
         }
-        // tcgen05 attention core when the shape allows (T <= 256, even head count), SIMT fallback otherwise
+        // tcgen05 attention core when the shape allows (T <= 256; head size 64, or 32 with an even head count), SIMT
+        // fallback otherwise
         const bool tc = attn_tc_supported(Tn, NH, HSz);
         label("attn fwd T=%d C=%d", Tn, C);
         split([&](int h) {
@@ -1319,8 +1320,8 @@ static int validate_config(const UbConfig& c) {
         set_err("C_model must be a multiple of 64 (tcgen05 K blocks of 64 channels)");
         return UB_ERR_SHAPE;
     }
-    if (c.head_size != 32) {
-        set_err("head_size must be 32");
+    if (c.head_size != 32 && c.head_size != 64) {  // (C_model % 64 == 0: every level's C divides by either)
+        set_err("head_size must be 32 or 64");
         return UB_ERR_SHAPE;
     }
     if ((c.H >> (c.n_levels - 1)) < 1 || c.H % (1 << (c.n_levels - 1)) || c.W % (1 << (c.n_levels - 1))) {
