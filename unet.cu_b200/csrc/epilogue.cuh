@@ -147,7 +147,7 @@ __device__ __forceinline__ void epi_side_load(const EpiOut& e, bool valid, size_
 }
 __device__ __forceinline__ void epi_chunk_gn(const EpiOut& e, uint32_t taddr, const float* comb, const float* gconst,
                                              int cstride, bool valid, size_t pix, int n, int lane, float* red,
-                                             float* tr, uint4 (&xr)[2], int n_next, uint32_t* keep_pk = nullptr) {
+                                             float* tr, uint4 (&xr)[2], int n_next) {
     uint32_t v[16];
     epi_tmem_load16(e, taddr, v);
     uint4 xn[2];
@@ -218,10 +218,6 @@ __device__ __forceinline__ void epi_chunk_gn(const EpiOut& e, uint32_t taddr, co
         __nv_bfloat16* op = reinterpret_cast<__nv_bfloat16*>(e.out) + pix * e.ldo + n;
         reinterpret_cast<uint4*>(op)[0] = make_uint4(pk[0], pk[1], pk[2], pk[3]);
         reinterpret_cast<uint4*>(op)[1] = make_uint4(pk[4], pk[5], pk[6], pk[7]);
-        if (keep_pk) {  // (GroupNorm finish: the stored values stay in registers for pass 2)
-#pragma unroll
-            for (int i = 0; i < 8; ++i) keep_pk[i] = pk[i];
-        }
     } else {
 #pragma unroll
         for (int j = 0; j < 16; ++j) f[j] = 0.f, q[j] = 0.f;
@@ -356,174 +352,6 @@ __device__ __forceinline__ void epi_stage_gconst(float* gconst, const float* chs
 
 __device__ __forceinline__ void named_bar_sync(int id, int nthreads) {
     asm volatile("bar.sync %0, %1;" ::"r"(id), "r"(nthreads) : "memory");
-}
-
-// ---------------------------------------------------------------------------------------------------------------
-// GroupNorm finish (IgemmConvParams::gnf): the second half of a fused GroupNorm, run by the NTHREADS epilogue threads of
-// a CTA whose pixel tile holds whole images (gnf_cluster == 1) or one half of an image whose other half belongs to the
-// cluster peer (gnf_cluster == 2), after pass 1 (epi_row_keep) and a barrier.
-//   red  [4][BN][2]      column sums of the four TMEM lane quadrants (pass 1)
-//   tot  [2][TB][BN][2]  per-(image, channel) totals: [0] this CTA's, [1] stored here by the cluster peer (DSMEM)
-//   gcf  [TB][3][BN]     per-(image, channel) constants of pass 2
-//   gst  [2][BN]         gamma, beta of channels [n0, n0 + BN), staged while the main loop ran
-//   xbar                 mbarrier (count BN) the peer's threads arrive on after their remote stores
-// forward  (gnf == 1): totals = (sum y, sum y^2) -> a = act(y * A + Bb), A = gamma * rstd, Bb = beta - mean * A
-// backward (gnf == 2): totals = (sum dz, sum dz * xhat) -> dx = A * dz - Bc * x + Cc (+ add), the constants of
-//   gn_bwd_apply_dz_kernel (nhwc_ops.cu); dgamma / dbeta / the embedding column sums follow from the totals alone:
-//   sum_p dx = A * sum dz - Bc * sum x + HW * Cc.
-// Pass 2 works on the bf16 values pass 1 stored (kept in registers: keep = y or dz, xkeep = the GroupNorm input), so the
-// result is bit-identical to the separate kernel reading those tensors; there is no global-memory round trip between
-// the passes, only three CTA barriers (and the peer's arrivals).
-template <int MAXCH>
-__device__ __forceinline__ void epi_row_keep(const EpiOut& e, uint32_t trow, const float* comb, int BN, bool valid,
-                                             size_t pix, int n0, const float* gconst, int lane, float* red, float* tr,
-                                             int half, const uint4* side, uint32_t (&keep)[MAXCH][8],
-                                             uint4 (&xkeep)[MAXCH][2]) {
-    uint4 xr[2] = {side[0], side[1]};
-#pragma unroll
-    for (int i = 0; i < MAXCH; ++i) {
-        const int c0 = 16 * half + 32 * i;
-        if (c0 < BN) {
-            xkeep[i][0] = xr[0], xkeep[i][1] = xr[1];
-            epi_chunk_gn(e, trow + uint32_t(c0), comb + c0, gconst + c0, BN, valid, pix, n0 + c0, lane, red + 2 * c0, tr,
-                         xr, c0 + 32 < BN ? n0 + c0 + 32 : -1, keep[i]);
-        }
-    }
-}
-
-template <int NTHREADS, int MAXCH>
-__device__ __forceinline__ void epi_gn_finish(const IgemmConvParams& p, const float* red, float* tot, float* gcf,
-                                              const float* gst, const float* gconst, uint64_t* xbar, int n0, int b0,
-                                              int et, int lbw, int half, bool valid, size_t pix,
-                                              const uint32_t (&keep)[MAXCH][8], const uint4 (&xkeep)[MAXCH][2]) {
-    const int BN = p.BN, TB = p.TB, rpi = p.TW * p.TH, cpg = p.gnf_cpg;
-    const bool pair = p.gnf_cluster == 2;
-    const uint32_t rank = pair ? cluster_ctarank() : 0u;
-    float* tot_peer = tot + TB * BN * 2;
-    // the residual-gradient rows of pass 2 travel while the totals and constants are formed
-    uint4 va[MAXCH][2];
-    if (p.gnf == 2 && p.gnf_add && valid) {
-#pragma unroll
-        for (int i = 0; i < MAXCH; ++i) {
-            const int c0 = 16 * half + 32 * i;
-            if (c0 < BN) {
-                const uint4* ap = reinterpret_cast<const uint4*>(p.gnf_add + pix * p.gnf_ldadd + n0 + c0);
-                va[i][0] = ap[0], va[i][1] = ap[1];
-            }
-        }
-    }
-    if (pair) cluster_wait();  // the peer has initialised its barrier (every thread of the pair arrived after its prologue)
-    for (int idx = et; idx < TB * BN; idx += NTHREADS) {
-        const int img = idx / BN, c = idx - img * BN;
-        float s = 0.f, ss = 0.f;
-#pragma unroll
-        for (int q = 0; q < 4; ++q) {
-            const int iq = min((q * 32) / rpi, TB - 1);
-            if (iq == img) {
-                const float2 v = *reinterpret_cast<const float2*>(red + (size_t(q) * BN + c) * 2);
-                s += v.x, ss += v.y;
-            }
-        }
-        tot[idx * 2] = s, tot[idx * 2 + 1] = ss;
-        if (pair) {
-            st_cluster_v2(mapa_cluster(smem_u32(tot_peer + idx * 2), rank ^ 1u), s, ss);
-            mbar_arrive_remote(mapa_cluster(smem_u32(xbar), rank ^ 1u));
-        }
-    }
-    if (pair) mbar_wait_cluster(xbar, 0);
-    named_bar_sync(1, NTHREADS);
-    const float n = float(cpg) * float(p.H * p.W);
-    for (int idx = et; idx < TB * BN; idx += NTHREADS) {
-        const int img = idx / BN, c = idx - img * BN, ch = n0 + c;
-        const int g0 = (c / cpg) * cpg;
-        float* g3 = gcf + size_t(img) * 3 * BN;
-        if (p.gnf == 1) {
-            float s = 0.f, ss = 0.f;
-            for (int k = 0; k < cpg; ++k) {
-                const int i2 = (img * BN + g0 + k) * 2;
-                s += tot[i2] + (pair ? tot_peer[i2] : 0.f);
-                ss += tot[i2 + 1] + (pair ? tot_peer[i2 + 1] : 0.f);
-            }
-            const float mean = s / n;
-            const float var = fmaxf(ss / n - mean * mean, 0.f);
-            const float a = rsqrtf(var + 1e-5f) * gst[c];
-            g3[c] = a;
-            g3[BN + c] = gst[BN + c] - mean * a;
-        } else {
-            const float* gc = gconst + size_t(img) * 4 * BN;  // a, bb, rstd, mean * rstd of the forward pass
-            float m1 = 0.f, m2 = 0.f;
-            for (int k = 0; k < cpg; ++k) {
-                const int i2 = (img * BN + g0 + k) * 2;
-                const float gam = gst[g0 + k];
-                m1 += gam * (tot[i2] + (pair ? tot_peer[i2] : 0.f));
-                m2 += gam * (tot[i2 + 1] + (pair ? tot_peer[i2 + 1] : 0.f));
-            }
-            const float r = gc[2 * BN + c], mr = gc[3 * BN + c], A = gc[c];
-            const float c1 = r * m1 / n, c2 = r * m2 / n;
-            const float Bc = c2 * r, Cc = mr * c2 - c1;
-            g3[c] = A, g3[BN + c] = Bc, g3[2 * BN + c] = Cc;
-            if (b0 + img < p.B && rank == 0) {  // once per (image, channel)
-                const int i2 = (img * BN + c) * 2;
-                const float sd = tot[i2] + (pair ? tot_peer[i2] : 0.f);
-                const float sq = tot[i2 + 1] + (pair ? tot_peer[i2 + 1] : 0.f);
-                atomicAdd(p.gnf_dgamma + ch, sq);
-                atomicAdd(p.gnf_dbeta + ch, sd);
-                if (p.gnf_colsum) {
-                    const size_t bc = size_t(b0 + img) * p.Cout + ch;
-                    atomicAdd(p.gnf_colsum + bc, A * sd - Bc * p.gn_chsum[bc * 2] + float(p.H * p.W) * Cc);
-                }
-            }
-        }
-    }
-    named_bar_sync(1, NTHREADS);
-    if (!valid) return;
-    const uint32_t g3s = smem_u32(gcf + size_t(lbw) * 3 * BN), row = 4u * uint32_t(BN);
-    __nv_bfloat16* orow = p.gnf_out + pix * p.gnf_ldo + n0;
-#pragma unroll
-    for (int ci = 0; ci < MAXCH; ++ci) {
-        const int c0 = 16 * half + 32 * ci;
-        if (c0 < BN) {
-            uint32_t pk[8];
-#pragma unroll
-            for (int j = 0; j < 2; ++j) {
-                float y[8], x[8], ad[8], o[8];
-                unpack_bf16x8(make_uint4(keep[ci][j * 4], keep[ci][j * 4 + 1], keep[ci][j * 4 + 2], keep[ci][j * 4 + 3]), y);
-                if (p.gnf == 2) {
-                    unpack_bf16x8(xkeep[ci][j], x);
-                    if (p.gnf_add) unpack_bf16x8(va[ci][j], ad);
-                }
-#pragma unroll
-                for (int h4 = 0; h4 < 2; ++h4) {
-                    const uint32_t ga = g3s + 4u * uint32_t(c0 + j * 8 + h4 * 4);
-                    const float4 k0 = lds_v4(ga), k1 = lds_v4(ga + row);
-                    const float a4[4] = {k0.x, k0.y, k0.z, k0.w}, b4[4] = {k1.x, k1.y, k1.z, k1.w};
-                    if (p.gnf == 1) {
-#pragma unroll
-                        for (int i = 0; i < 4; ++i) {
-                            const float z = fmaf(y[h4 * 4 + i], a4[i], b4[i]);
-                            o[h4 * 4 + i] = p.gnf_silu ? z * epi_sigmoid(z) : z;
-                        }
-                    } else {
-                        const float4 k2 = lds_v4(ga + 2u * row);
-                        const float c4[4] = {k2.x, k2.y, k2.z, k2.w};
-#pragma unroll
-                        for (int i = 0; i < 4; ++i) {
-                            const int e = h4 * 4 + i;
-                            const float g = fmaf(a4[i], y[e], fmaf(-b4[i], x[e], c4[i]));
-                            o[e] = p.gnf_add ? ad[e] + g : g;
-                        }
-                    }
-                }
-#pragma unroll
-                for (int i = 0; i < 4; ++i) {
-                    const __nv_bfloat162 h2 = __floats2bfloat162_rn(o[2 * i], o[2 * i + 1]);
-                    pk[j * 4 + i] = *reinterpret_cast<const uint32_t*>(&h2);
-                }
-            }
-            reinterpret_cast<uint4*>(orow + c0)[0] = make_uint4(pk[0], pk[1], pk[2], pk[3]);
-            reinterpret_cast<uint4*>(orow + c0)[1] = make_uint4(pk[4], pk[5], pk[6], pk[7]);
-        }
-    }
 }
 
 }  // namespace ub

@@ -494,14 +494,6 @@ bool gn_slab_supported(int B, int HW, int C, int G, bool backward) {
     SlabPlan pl;
     return slab_plan(B, HW, C, G, backward, &pl);
 }
-// Measured (tools/gn_bench.py, profiles/r02f_gn_bench.txt): the slab kernels beat the two-pass kernels wherever a CTA's
-// share of the slab stays in registers and the cluster is small; image-sized slabs (64x64: clusters of 8, two waves of
-// one 512-thread CTA per SM) and loop-mode slabs lose to two streaming passes with thousands of CTAs in flight.
-bool gn_slab_preferred(int B, int HW, int C, int G) {
-    SlabPlan f, b;
-    if (!slab_plan(B, HW, C, G, false, &f) || !slab_plan(B, HW, C, G, true, &b)) return false;
-    return f.K > 0 && b.K > 0 && f.csz <= 4 && b.csz <= 4;
-}
 
 int gn_slab_fwd(const bf16* x, int ldx, const float* gamma, const float* beta, int B, int HW, int C, int G, int silu,
                 bf16* y, int ldy, float* chsum, cudaStream_t st) {

@@ -31,7 +31,6 @@ static constexpr int kMaxStages = 8;
 static constexpr int kConvThreads = 320;   // conv: TMA warp, MMA warp, 8 epilogue warps (2 per TMEM lane quadrant)
 static constexpr int kWgradThreads = 192;  // wgrad: TMA warp, MMA warp, 4 epilogue warps
 static constexpr int kEpiThreads = kConvThreads - 64;
-static constexpr int kGnfChunks = 3;  // GroupNorm finish: 16-column chunks per epilogue thread, i.e. BN <= 96
 
 // Phase timeline of igemm_conv_kernel (development only: -DUB_TRACE, tools/igemm_test.cu `trace` mode).  Per CTA:
 // [0] globaltimer at entry, [1] SM id, then SM clock at [2] entry [3] prologue done [4] griddepcontrol.wait passed
@@ -179,7 +178,7 @@ __device__ __forceinline__ void conv_produce_loop(const IgemmConvParams& p, int 
 // 8x8 / 16x16 levels) run NACC = 2: lane 0 of the last epilogue warp -- idle during the main loop -- issues the odd K
 // blocks into a second accumulator and the epilogue adds the two.  (An 11th warp for the second issuer capped the
 // two-CTA kernel at 80 registers; the spilling epilogue cost more in the step than the main loop won.)
-template <int NACC, bool MS = false, bool GNF = false>
+template <int NACC, bool MS = false>
 __device__ __forceinline__ void igemm_conv_body(const IgemmConvParams& p) {
     pdl_trigger();
 #ifdef UB_TRACE
@@ -201,10 +200,6 @@ __device__ __forceinline__ void igemm_conv_body(const IgemmConvParams& p) {
     float* comb = reinterpret_cast<float*>(reinterpret_cast<uint8_t*>(full_bar) + 256);
     float* gconst = comb + p.ncomb * p.BN;  // [ngimg][4][BN] GroupNorm constants (gn-bwd epilogue only)
     float* red = gconst + p.ngimg * 4 * p.BN;  // [4 warps][BN][2] column sums of the GroupNorm hooks
-    float* gnf_tot = red + p.nred * p.BN;      // GroupNorm finish (epi_gn_finish): [2][TB][BN][2] totals ...
-    float* gnf_gcf = gnf_tot + 4 * p.TB * p.BN;  // ... [TB][3][BN] constants ...
-    float* gnf_gst = gnf_gcf + 3 * p.TB * p.BN;  // ... and [2][BN] staged gamma / beta
-    uint64_t* gnf_xbar = tmem_full_bar + 4;    // byte 160 of the barrier block: the cluster peer's arrivals
 
     const int warp = threadIdx.x >> 5;
     const int lane = threadIdx.x & 31;
@@ -232,7 +227,6 @@ __device__ __forceinline__ void igemm_conv_body(const IgemmConvParams& p) {
         }
         mbar_init(tmem_full_bar, NACC);
         if constexpr (MS) mbar_init(tmem_full_bar + 2, 1);  // statistics MMAs complete (byte 144 of the barrier block)
-        if constexpr (GNF) mbar_init(gnf_xbar, uint32_t(p.BN));
         fence_mbar_init();
     }
     if (warp == 1) {
@@ -268,9 +262,6 @@ __device__ __forceinline__ void igemm_conv_body(const IgemmConvParams& p) {
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
-    if constexpr (GNF) {
-        if (p.gnf_cluster == 2) cluster_arrive();  // this CTA's barriers exist (the peer waits before it stores into us)
-    }
     if (threadIdx.x == 0) UB_TR(3, (unsigned long long)clock64());
     pdl_wait();  // everything above touched only kernel parameters, shared memory, TMEM (and prefetched weights)
     if (threadIdx.x == 0) UB_TR(4, (unsigned long long)clock64());
@@ -322,13 +313,6 @@ __device__ __forceinline__ void igemm_conv_body(const IgemmConvParams& p) {
         for (int i = 0; i < p.ngimg; ++i)
             epi_stage_gconst(gconst + i * 4 * p.BN, p.gn_chsum, p.gn_gamma, p.gn_beta, min(b0 + i, p.B - 1), p.Cout,
                              p.gn_cpg, p.H * p.W, n0, p.BN, et, kEpiThreads);
-        if constexpr (GNF) {
-            if (p.gnf) {
-                const float* gam = p.gnf == 1 ? p.gnf_gamma : p.gn_gamma;
-                const float* bet = p.gnf == 1 ? p.gnf_beta : p.gn_beta;
-                for (int c = et; c < p.BN; c += kEpiThreads) gnf_gst[c] = gam[n0 + c], gnf_gst[p.BN + c] = bet[n0 + c];
-            }
-        }
         named_bar_sync(1, kEpiThreads);
 
         const size_t pix = (size_t(b) * p.H + h) * p.W + w;
@@ -450,25 +434,7 @@ __device__ __forceinline__ void igemm_conv_body(const IgemmConvParams& p) {
                 if (threadIdx.x == 64) bulk_wait_group0();
             }
         }
-        bool done_gnf = false;
-        if constexpr (GNF) {
-            if (p.gnf) {  // hooked pass 1 with the stored values kept in registers, then the GroupNorm's second half
-                done_gnf = true;
-                const int lbw = min(lb, p.TB - 1);
-                uint32_t keep[kGnfChunks][8];
-                uint4 xkeep[kGnfChunks][2];
-                epi_row_keep<kGnfChunks>(eo, tmem_base + (uint32_t(q * 32) << 16),
-                                         comb + (p.ncomb > 1 ? min(lb, p.ncomb - 1) : 0) * p.BN, p.BN, valid, pix, n0,
-                                         gconst + lbw * 4 * p.BN, lane, red + size_t(q) * p.BN * 2,
-                                         reinterpret_cast<float*>(smem) + (warp - 2) * (32 * 36), half, side, keep, xkeep);
-                named_bar_sync(1, kEpiThreads);
-                epi_flush_stats(red, p.gn_x ? p.gn_S : p.stats, p.Cout, n0, p.BN, b0, p.B, p.TW * p.TH, p.TB, et,
-                                kEpiThreads);
-                epi_gn_finish<kEpiThreads, kGnfChunks>(p, red, gnf_tot, gnf_gcf, gnf_gst, gconst, gnf_xbar, n0, b0, et, lbw,
-                                                       half, valid, pix, keep, xkeep);
-            }
-        }
-        if (!done_ms && !done_gnf) {
+        if (!done_ms) {
         // GroupNorm hooks: all 32 pixels of a warp lie in one image of the tile (plan)
         const int lbw = min(lb, p.TB - 1);
         epi_row(eo, tmem_base + (uint32_t(q * 32) << 16), comb + (p.ncomb > 1 ? min(lb, p.ncomb - 1) : 0) * p.BN, p.BN,
@@ -506,10 +472,6 @@ __global__ void __launch_bounds__(kConvThreads, 2) igemm_conv_ms_kernel(const __
 }
 __global__ void __launch_bounds__(kConvThreads, 1) igemm_conv2_ms_kernel(const __grid_constant__ IgemmConvParams p) {
     igemm_conv_body<2, true>(p);
-}
-// two streams + GroupNorm finish in the epilogue (low-resolution levels, see IgemmConvParams::gnf)
-__global__ void __launch_bounds__(kConvThreads, 1) igemm_conv2_gnf_kernel(const __grid_constant__ IgemmConvParams p) {
-    igemm_conv_body<2, false, true>(p);
 }
 
 // =====================================================================================================
@@ -987,24 +949,8 @@ int igemm_conv_plan(IgemmConvParams* p, const ConvSegDesc* segs, int nseg, int B
     // Two CTAs per SM when possible (one CTA's epilogue overlaps the other's main loop): <= ~110 KiB each.
     // (the smem tail -- barriers, staged addends, GroupNorm constants and reduction scratch -- comes off the budget)
     const int tb_guess = (128 / (p->TW * p->TH)) < 1 ? 1 : 128 / (p->TW * p->TH);
-    // GroupNorm finish (IgemmConvParams::gnf) is possible when a hooked two-stream conv's tile holds whole images, or
-    // exactly half an image with the other half in the next pixel tile (a 2-CTA cluster along grid.x)
-    p->gnf_cluster = 0;
-    if (gn_hook && p->nacc == 2 && ep.out_mode == OUT_NHWC_BF16 && p->tiles_w == 1 && W == p->TW) {
-        // Measured round 2 (bench.py, B = 32): whole-image tiles only (8x8) 5.045 ms per step against 5.043 without
-        // -- the 34 GroupNorm launches it removes cost ~4 us each in the pipelined step, the longer epilogue costs
-        // the same -- and 5.15 ms with the 16x16 CTA pairs (their exchange adds 4-12 us per conv).  Parity-tested
-        // (UB_GN_FINISH=1 pytest), kept as an opt-in: UB_GN_FINISH=1, UB_GNF_NO_PAIR=1 for whole-image tiles only.
-        static const bool off = !(getenv("UB_GN_FINISH") && atoi(getenv("UB_GN_FINISH")) != 0);
-        if (!off && p->TH == H && p->TW * p->TH * p->TB <= 128 && (p->TB == 1 || (p->TW * p->TH) % 32 == 0))
-            p->gnf_cluster = 1;
-        else if (!off && !(getenv("UB_GNF_NO_PAIR") && atoi(getenv("UB_GNF_NO_PAIR"))) && p->TB == 1 && p->TH * 2 == H &&
-                 p->TW * p->TH == 128)
-            p->gnf_cluster = 2;
-    }
-    const int ngnf = p->gnf_cluster ? 7 * p->TB + 2 : 0;  // tot [2][TB][BN][2] + gcf [TB][3][BN] + gamma / beta
     const uint32_t tail = 1024u + uint32_t(kBarrierBytes) +
-                          uint32_t((ep.rowvec ? tb_guess : 1) + (ep.gn_x ? 4 * tb_guess : 0) + (gn_hook ? 8 : 0) + ngnf) *
+                          uint32_t((ep.rowvec ? tb_guess : 1) + (ep.gn_x ? 4 * tb_guess : 0) + (gn_hook ? 8 : 0)) *
                               uint32_t(BN) * 4u;
     int stages = int((113u * 1024u - tail) / p->stage_bytes);
     if (stages < 3) stages = int((227u * 1024u - tail) / p->stage_bytes);
@@ -1071,10 +1017,6 @@ int igemm_conv_plan(IgemmConvParams* p, const ConvSegDesc* segs, int nseg, int B
         }
     }
     p->nred = gn_hook ? 8 : 0;
-    p->gnf_cpg = Cout / (ep.gn_groups > 0 ? ep.gn_groups : 32);
-    if (p->gnf_cluster && (Cout % (ep.gn_groups > 0 ? ep.gn_groups : 32) != 0 || BN % p->gnf_cpg != 0 ||
-                           BN > 32 * kGnfChunks))
-        p->gnf_cluster = 0;
     {
         // tensor-core statistics + TMA output store (IgemmConvParams::ms) for the plain stats hook on full
         // 128-pixel tiles of one or two whole images with a 64- or 128-channel N tile, one or two MMA streams
@@ -1083,7 +1025,7 @@ int igemm_conv_plan(IgemmConvParams* p, const ConvSegDesc* segs, int nseg, int B
         static const bool want_ms = !(getenv("UB_EPI_MMA") && atoi(getenv("UB_EPI_MMA")) == 0);
         const bool full_tiles = W % p->TW == 0 && H % p->TH == 0 && p->TW * p->TH * p->TB == 128;
         const size_t need = size_t(2 * (BN / 64) + 1) * 16384;  // Y atoms, Y*Y atoms, ones tile in the dead stages
-        if (want_ms && !p->gnf_cluster && ep.stats && !ep.gn_x && p->out_mode == OUT_NHWC_BF16 && (BN == 64 || BN == 128) &&
+        if (want_ms && ep.stats && !ep.gn_x && p->out_mode == OUT_NHWC_BF16 && (BN == 64 || BN == 128) &&
             p->nacc <= 2 && (p->TB == 1 || (p->TB == 2 && (p->TW * p->TH) == 64)) && full_tiles &&
             need <= size_t(p->stages) * p->stage_bytes && p->nacc * BN + 64 <= (p->nacc == 1 ? 256 : 512) &&
             make_act_map(&p->tmO, reinterpret_cast<const __nv_bfloat16*>(ep.out), Cout, p->ldo, W, H, B, p->TW, p->TH,
@@ -1095,15 +1037,15 @@ int igemm_conv_plan(IgemmConvParams* p, const ConvSegDesc* segs, int nseg, int B
         // tile + TMA store (any whole-tile shape, N tiles of 64 .. 256 channels); UB_EPI_TMA_STORE=0 keeps the
         // per-thread stores
         static const bool want_st = !(getenv("UB_EPI_TMA_STORE") && atoi(getenv("UB_EPI_TMA_STORE")) == 0);
-        if (want_ms && want_st && !p->ms && !gn_hook && !p->gnf_cluster && p->out_mode == OUT_NHWC_BF16 && BN % 64 == 0 &&
+        if (want_ms && want_st && !p->ms && !gn_hook && p->out_mode == OUT_NHWC_BF16 && BN % 64 == 0 &&
             p->nacc <= 2 && full_tiles && size_t(BN / 64) * 16384 <= size_t(p->stages) * p->stage_bytes &&
             make_act_map(&p->tmO, reinterpret_cast<const __nv_bfloat16*>(ep.out), Cout, p->ldo, W, H, B, p->TW, p->TH,
                          p->TB) == 0)
             p->ms = 2;
     }
-    if (size_t(p->ncomb + 4 * p->ngimg + p->nred + ngnf) * BN * sizeof(float) > 24576) return -9;  // smem tail budget
+    if (size_t(p->ncomb + 4 * p->ngimg + p->nred) * BN * sizeof(float) > 24576) return -9;  // smem tail budget
     if (size_t(p->stages) * p->stage_bytes + 1024 + kBarrierBytes +
-            size_t(p->ncomb + 4 * p->ngimg + p->nred + ngnf) * BN * sizeof(float) > size_t(227) * 1024)
+            size_t(p->ncomb + 4 * p->ngimg + p->nred) * BN * sizeof(float) > size_t(227) * 1024)
         return -3;
     if (p->out_mode != OUT_NCHW_F32) {
         const int esz = p->out_mode == OUT_NHWC_BF16 ? 2 : 4;
@@ -1116,32 +1058,11 @@ int igemm_conv_plan(IgemmConvParams* p, const ConvSegDesc* segs, int nseg, int B
     return 0;
 }
 
-bool igemm_conv_gn_finish_fwd(IgemmConvParams* p, const float* gamma, const float* beta, int groups, int silu,
-                              __nv_bfloat16* out, int ldo) {
-    if (!p->gnf_cluster || p->gnf || !p->stats || p->gn_x || p->nacc != 2 || p->ms) return false;
-    if (groups < 1 || p->Cout % groups || p->BN % (p->Cout / groups) || !gamma || !beta || !out) return false;
-    if ((ldo % 8) != 0 || (reinterpret_cast<uintptr_t>(out) & 15)) return false;
-    p->gnf = 1, p->gnf_gamma = gamma, p->gnf_beta = beta, p->gnf_cpg = p->Cout / groups, p->gnf_silu = silu;
-    p->gnf_out = out, p->gnf_ldo = ldo;
-    return true;
-}
-bool igemm_conv_gn_finish_bwd(IgemmConvParams* p, const __nv_bfloat16* add_in, int ldadd, __nv_bfloat16* dx, int lddx,
-                              float* dgamma, float* dbeta, float* colsum) {
-    if (!p->gnf_cluster || p->gnf || !p->gn_x || p->nacc != 2 || p->ms) return false;
-    if (p->BN % p->gn_cpg || !dx || !dgamma || !dbeta) return false;
-    if ((lddx % 8) != 0 || (reinterpret_cast<uintptr_t>(dx) & 15)) return false;
-    if (add_in && ((ldadd % 8) != 0 || (reinterpret_cast<uintptr_t>(add_in) & 15))) return false;
-    p->gnf = 2, p->gnf_cpg = p->gn_cpg, p->gnf_add = add_in, p->gnf_ldadd = ldadd, p->gnf_out = dx, p->gnf_ldo = lddx;
-    p->gnf_dgamma = dgamma, p->gnf_dbeta = dbeta, p->gnf_colsum = colsum;
-    return true;
-}
-
 void igemm_init() {
     static bool done = false;
     if (done) return;
     cudaFuncSetAttribute(igemm_conv_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(227 * 1024));
     cudaFuncSetAttribute(igemm_conv2_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(227 * 1024));
-    cudaFuncSetAttribute(igemm_conv2_gnf_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(227 * 1024));
     cudaFuncSetAttribute(igemm_conv_ms_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(227 * 1024));
     cudaFuncSetAttribute(igemm_conv2_ms_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(227 * 1024));
     cudaFuncSetAttribute(igemm_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, int(227 * 1024));
@@ -1151,14 +1072,11 @@ void igemm_init() {
 int igemm_conv_launch(const IgemmConvParams& p, cudaStream_t st) {
     igemm_init();
     const size_t smem = size_t(p.stages) * p.stage_bytes + 1024 + kBarrierBytes +
-                        size_t(p.ncomb + 4 * p.ngimg + p.nred + (p.gnf_cluster ? 7 * p.TB + 2 : 0)) * p.BN * sizeof(float);
+                        size_t(p.ncomb + 4 * p.ngimg + p.nred) * p.BN * sizeof(float);
     dim3 grid(p.tiles_w * p.tiles_h * p.tiles_b, p.Cout / p.BN);
     auto kern = p.nacc == 2 ? igemm_conv2_kernel : igemm_conv_kernel;
     if (p.ms) kern = p.nacc == 2 ? igemm_conv2_ms_kernel : igemm_conv_ms_kernel;
-    if (p.gnf) kern = igemm_conv2_gnf_kernel;
-    static const bool force_cl2 = getenv("UB_FORCE_CLUSTER2") != nullptr;  // experiment: what does a cluster launch cost?
-    const int cl = (p.gnf && p.gnf_cluster == 2) || (force_cl2 && p.nacc == 2 && grid.x % 2 == 0) ? 2 : 1;
-    launch_pdl_cluster(kern, dim3(grid), dim3(kConvThreads), smem, st, cl, p);
+    launch_pdl(kern, dim3(grid), dim3(kConvThreads), smem, st, p);
     const cudaError_t e = cudaGetLastError();
     if (e != cudaSuccess)  // a failed launch must never pass silently (the output would simply be stale)
         fprintf(stderr, "[unet_b200] igemm_conv launch failed: %s (grid %u x %u, smem %zu, BN %d, stages %d)\n",

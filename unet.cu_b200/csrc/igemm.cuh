@@ -69,24 +69,6 @@ struct IgemmConvParams {
     // of channel c in TMEM lane c, and the Y tile goes to global memory with one TMA store per 64 channels.
     int ms;
     CUtensorMap tmO;                // output tensor, box (64, TW, TH, TB), SWIZZLE_128B (ms only)
-    // GroupNorm "finish" (low-resolution levels, igemm_conv2_kernel only): when the CTA's pixel tile holds whole images
-    // (8x8: two images per tile) or one half of an image whose other half is the cluster peer's tile (16x16), the
-    // statistics a hook accumulates are complete inside the CTA (pair) and the epilogue also runs the pass that
-    // normally is a kernel of its own -- forward: a = act(gn(y)) of the tensor it just stored (replaces gn_apply);
-    // backward: dx = gn'(dz) (+ residual gradient), dgamma / dbeta / the per-image column sums (replaces
-    // gn_bwd_apply_dz).  These levels are bound by kernel count x per-kernel latency, not by bytes.
-    int gnf_cluster;                // set by the plan: 0 = not eligible, 1 = whole images per tile, 2 = CTA pair per image
-    int gnf;                        // set by igemm_conv_gn_finish_*: 0 off, 1 forward, 2 backward
-    const float* gnf_gamma;         // forward: the consumer GroupNorm's scale / shift (backward uses gn_gamma / gn_beta)
-    const float* gnf_beta;
-    __nv_bfloat16* gnf_out;         // forward: act(gn(y)); backward: dx
-    int gnf_ldo;
-    int gnf_silu, gnf_cpg;
-    const __nv_bfloat16* gnf_add;   // backward: gradient added to dx (residual path), or nullptr
-    int gnf_ldadd;
-    float* gnf_dgamma;              // backward: [Cout] += sum over images of (sum dz*xhat)
-    float* gnf_dbeta;               //           [Cout] += sum dz
-    float* gnf_colsum;              // backward: [B][Cout] += per-image column sums of dx (embedding gradient), or nullptr
 };
 
 // persistent row-tile variant (igemm_rows.cu); same segments / epilogue as IgemmConvParams
@@ -196,13 +178,6 @@ void igemm_init();
 int igemm_conv_plan(IgemmConvParams* p, const ConvSegDesc* segs, int nseg, int B, int H, int W, int Cout,
                     const ConvEpilogue& ep);
 int igemm_conv_launch(const IgemmConvParams& p, cudaStream_t st);
-// GroupNorm finish (see IgemmConvParams::gnf): extend a planned conv whose epilogue carries the statistics hook
-// (forward) / the gn-bwd hook (backward).  Return false -- and leave the plan untouched -- when the plan is not
-// eligible (tile does not hold whole images, groups straddle the N tile, ...): the caller then emits the GroupNorm kernel.
-bool igemm_conv_gn_finish_fwd(IgemmConvParams* p, const float* gamma, const float* beta, int groups, int silu,
-                              __nv_bfloat16* out, int ldo);
-bool igemm_conv_gn_finish_bwd(IgemmConvParams* p, const __nv_bfloat16* add_in, int ldadd, __nv_bfloat16* dx, int lddx,
-                              float* dgamma, float* dbeta, float* colsum);
 
 bool igemm_rows_eligible(int B, int H, int W, int Cout);
 int igemm_rows_plan(IgemmRowsParams* p, const ConvSegDesc* segs, int nseg, int B, int H, int W, int Cout,

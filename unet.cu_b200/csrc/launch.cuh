@@ -73,28 +73,6 @@ inline bool pdl_enabled() {
     return on;
 }
 
-// the same with a thread-block cluster of `cluster_x` CTAs along grid.x
-template <typename... KArgs, typename... Args>
-inline cudaError_t launch_pdl_cluster(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
-                                      int cluster_x, Args&&... args) {
-    cudaLaunchConfig_t cfg = {};
-    cfg.gridDim = grid, cfg.blockDim = block, cfg.dynamicSmemBytes = smem, cfg.stream = st;
-    cudaLaunchAttribute at[2];
-    int n = 0;
-    if (pdl_enabled()) {
-        at[n].id = cudaLaunchAttributeProgrammaticStreamSerialization;
-        at[n].val.programmaticStreamSerializationAllowed = 1;
-        ++n;
-    }
-    if (cluster_x > 1) {
-        at[n].id = cudaLaunchAttributeClusterDimension;
-        at[n].val.clusterDim.x = unsigned(cluster_x), at[n].val.clusterDim.y = 1, at[n].val.clusterDim.z = 1;
-        ++n;
-    }
-    cfg.attrs = at, cfg.numAttrs = unsigned(n);
-    return cudaLaunchKernelEx(&cfg, kernel, std::forward<Args>(args)...);
-}
-
 template <typename... KArgs, typename... Args>
 inline cudaError_t launch_pdl(void (*kernel)(KArgs...), dim3 grid, dim3 block, size_t smem, cudaStream_t st,
                               Args&&... args) {

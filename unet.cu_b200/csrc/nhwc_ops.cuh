@@ -53,7 +53,6 @@ void gn_bwd_apply(const bf16* x, int ldx, const bf16* dy, int lddy, const float*
 //      groups of channels) held in registers in between: 1R + 1W forward, 2R (+1R) + 1W backward.  Return -1 when the
 //      shape is not supported (channel count not a multiple of 16, slab too large): use the two-pass kernels above.
 bool gn_slab_supported(int B, int HW, int C, int G, bool backward);
-bool gn_slab_preferred(int B, int HW, int C, int G);  // supported AND measured faster than the two-pass kernels
 void gn_slab_init();  // opt-in shared memory attributes; called by nhwc_ops_init() (before graph capture)
 // y = act(gn(x)); chsum[B][C][2] receives the per-(image, channel) sum / sum of squares (overwritten, for the backward)
 int gn_slab_fwd(const bf16* x, int ldx, const float* gamma, const float* beta, int B, int HW, int C, int G, int silu,

@@ -209,44 +209,6 @@ __device__ __forceinline__ void tmem_ld_wait() {
     asm volatile("tcgen05.wait::ld.sync.aligned;" ::: "memory");
 }
 
-// ---------------------------------------------------------------- thread-block clusters / distributed shared memory
-__device__ __forceinline__ uint32_t cluster_ctarank() {
-    uint32_t r;
-    asm volatile("mov.u32 %0, %%cluster_ctarank;" : "=r"(r));
-    return r;
-}
-// shared::cta address -> the same offset in the shared memory of CTA `rank` of this cluster (shared::cluster address)
-__device__ __forceinline__ uint32_t mapa_cluster(uint32_t saddr, uint32_t rank) {
-    uint32_t r;
-    asm volatile("mapa.shared::cluster.u32 %0, %1, %2;" : "=r"(r) : "r"(saddr), "r"(rank));
-    return r;
-}
-__device__ __forceinline__ void st_cluster_v2(uint32_t caddr, float a, float b) {
-    asm volatile("st.shared::cluster.v2.f32 [%0], {%1, %2};" ::"r"(caddr), "f"(a), "f"(b) : "memory");
-}
-// arrive on an mbarrier of another CTA of the cluster; orders this thread's earlier (remote) stores before it
-__device__ __forceinline__ void mbar_arrive_remote(uint32_t cbar) {
-    asm volatile("mbarrier.arrive.release.cluster.shared::cluster.b64 _, [%0];" ::"r"(cbar) : "memory");
-}
-// wait (cluster-scope acquire) on a barrier of THIS CTA that threads of other CTAs arrive on; traps instead of hanging
-__device__ __forceinline__ void mbar_wait_cluster(uint64_t* bar, uint32_t parity) {
-    uint32_t ok = 0;
-    for (uint32_t spin = 0; !ok; ++spin) {
-        asm volatile(
-            "{\n\t"
-            ".reg .pred P;\n\t"
-            "mbarrier.try_wait.parity.acquire.cluster.shared::cta.b64 P, [%1], %2;\n\t"
-            "selp.b32 %0, 1, 0, P;\n\t"
-            "}\n"
-            : "=r"(ok)
-            : "r"(smem_u32(bar)), "r"(parity)
-            : "memory");
-        if (spin > (1u << 26)) __trap();  // ~seconds: the peer CTA is gone -- fail loudly, do not hang the GPU
-    }
-}
-// all threads of all CTAs of the cluster arrive (non-blocking) / wait for everybody's arrival
-__device__ __forceinline__ void cluster_arrive() { asm volatile("barrier.cluster.arrive.release;" ::: "memory"); }
-__device__ __forceinline__ void cluster_wait() { asm volatile("barrier.cluster.wait.acquire;" ::: "memory"); }
 __device__ __forceinline__ uint4 ldg_v4(const void* p) {  // plain (coherent) 16-byte global load
     uint4 v;
     asm volatile("ld.global.v4.u32 {%0, %1, %2, %3}, [%4];" : "=r"(v.x), "=r"(v.y), "=r"(v.z), "=r"(v.w) : "l"(p));

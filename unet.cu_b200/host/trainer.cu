@@ -13,8 +13,6 @@
 #include <cstring>
 #include <algorithm>
 #include <functional>
-#include <map>
-#include <memory>
 #include <string>
 #include <vector>
 
@@ -117,17 +115,6 @@ struct UbTrainer {
     cudaStream_t aux_stream = nullptr;
     cudaEvent_t ev_aux_fork = nullptr, ev_aux_join = nullptr;
     bool attn_concurrent = true;
-    // Micro-batch pipelining: the main-stream ops that work image by image (conv fprop / dgrad, GroupNorm, attention,
-    // data movement) are emitted once per micro-batch of B / n_mb images -- batch-major views of the same buffers -- and
-    // micro-batch h > 0 runs on mb_streams[h - 1], a parallel branch of the captured graph.  The step is ~40 % batch-
-    // independent latency at B = 32 (5.17 ms at B = 32, 3.69 at 16, 2.96 at 8: profiles/r02_microbatch.txt); the idea
-    // was that two independent chains hide each other's latency.  They do not (5.30 ms with two chains): an experiment
-    // switch (UB_MICROBATCH), off by default.  Ops that need the whole batch (weight gradients on the side stream, loss,
-    // optimizer) join the chains first.
-    int n_mb = 1;
-    bool mb_fwd_only = false;  // UB_MICROBATCH_FWD: the chains exist in the forward pass only
-    int mb_max_hw = 0;         // UB_MICROBATCH_LOWRES: > 0 = chains only at levels of at most this many pixels per image
-    std::vector<cudaStream_t> mb_streams;
     std::vector<cudaEvent_t> side_events;
     size_t side_ev_next = 0;
     bool use_side = true;
@@ -208,7 +195,6 @@ struct UbTrainer {
         double bytes;   // ... or algorithmic bytes (memory-bound kernels)
         int side;       // 0 = main stream, 1 = weight-gradient branch (side stream), 2 = join marker
         std::string label;
-        int half = -1;  // >= 0: this op is micro-batch `half` of a per-image op (runs on that micro-batch's stream)
     };
     std::vector<OpInfo> fwd_info, bwd_info;
     int launches_fwd = 0, launches_bwd = 0, launches_misc = 0;
@@ -288,43 +274,7 @@ struct Builder {
     };
     std::vector<Node> nodes;
     std::vector<View> skipgrad;  // per node: gradient arriving from the up path
-    // UB_MICROBATCH_LOWRES = hw: micro-batch chains only at levels of at most hw pixels per image (the 8x8 / 16x16 levels
-    // run on less than half of the SMs and are bound by per-kernel latency); node_nh[i] = chains of node i
-    std::vector<int> node_nh;
-    void level_mb(int H, int W) {
-        if (T->mb_max_hw <= 0) return;
-        nh = (H * W <= T->mb_max_hw && T->n_mb > 1 && B % T->n_mb == 0) ? T->n_mb : 1;
-        Bh = B / nh;
-    }
-    void sync_nh() { node_nh.resize(nodes.size(), nh); }
-
-    // micro-batches (see UbTrainer::n_mb): nh chains of Bh images each
-    int nh = 1, Bh = 0;
-    int cur_half = -1;  // set while the ops of one micro-batch are being emitted (split())
-    explicit Builder(UbTrainer* t) : T(t), c(t->cfg), B(t->cfg.B) {
-        nh = t->n_mb > 0 && B % t->n_mb == 0 ? t->n_mb : 1;
-        Bh = B / nh;
-        level_mb(t->cfg.H, t->cfg.W);  // (UB_MICROBATCH_LOWRES: the full-resolution head of the step runs as one chain)
-    }
-    // emit the same op for every micro-batch: fn(h) pushes the ops of micro-batch h (views offset with mb())
-    template <class Fn>
-    void split(Fn fn) {
-        std::string lbl = next_label;
-        for (int h = 0; h < nh; ++h) {
-            cur_half = nh > 1 ? h : -1;
-            next_label = lbl;
-            fn(h);
-        }
-        cur_half = -1;
-        next_label.clear();
-    }
-    // micro-batch h of a batch-major view / per-image fp32 table with `per_img` floats per image
-    View mb(View v, int h) const {
-        if (v.p) v.p += size_t(h) * Bh * v.H * v.W * v.ld;
-        if (v.cs) v.cs += size_t(h) * Bh * v.C * 2;
-        return v;
-    }
-    float* mbf(float* p, int h, size_t per_img) const { return p ? p + size_t(h) * Bh * per_img : nullptr; }
+    explicit Builder(UbTrainer* t) : T(t), c(t->cfg), B(t->cfg.B) {}
 
     size_t take(size_t n) {
         size_t o = poff;
@@ -350,7 +300,7 @@ struct Builder {
            int side = 0) {
         if (!real()) return;
         T->fwd_ops.push_back(std::move(op)), T->launches_fwd += launches;
-        T->fwd_info.push_back({kind, launches, flops, bytes, side, next_label, side == 0 ? cur_half : -1}), next_label.clear();
+        T->fwd_info.push_back({kind, launches, flops, bytes, side, next_label}), next_label.clear();
     }
     // forward: the time-embedding chain runs on the side stream until its first consumer (conv1 of the first ResBlock)
     bool fwd_side_pending = false;
@@ -362,7 +312,7 @@ struct Builder {
             int side = 0) {
         if (!real()) return;
         T->bwd_ops.push_back(std::move(op)), T->launches_bwd += launches;
-        T->bwd_info.push_back({kind, launches, flops, bytes, side, next_label, side == 0 ? cur_half : -1}), next_label.clear();
+        T->bwd_info.push_back({kind, launches, flops, bytes, side, next_label}), next_label.clear();
     }
     std::string next_label;  // optional description of the next op pushed (per-op profile dump)
     void label(const char* fmt, ...) {
@@ -412,52 +362,32 @@ struct Builder {
         double k = 0, bytes = act_bytes(Cout, H, W);
         for (auto& sg : segs) k += double(sg.ntaps) * sg.Cin, bytes += act_bytes(sg.Cin, H, W) + 2.0 * sg.ntaps * sg.Cin * Cout;
         const double flops = 2.0 * B * H * W * Cout * k;
-        // one launch per micro-batch: batch-major views of the same buffers (operands, output, residual, per-image
-        // embedding vector / GroupNorm statistics)
-        split([&](int h) {
-            std::vector<ConvSegDesc> sh = segs;
-            for (auto& sg : sh) sg.x += size_t(h) * Bh * H * W * sg.ldx;
-            ConvEpilogue eh = ep;
-            const size_t opix = size_t(h) * Bh * H * W;
-            eh.out = (bf16*)ep.out + opix * (ep.ldo ? ep.ldo : Cout);
-            if (ep.residual) eh.residual = ep.residual + opix * (ep.ldr ? ep.ldr : Cout);
-            eh.rowvec = mbf(const_cast<float*>(ep.rowvec), h, Cout);
-            eh.stats = mbf(ep.stats, h, size_t(Cout) * 2);
-            if (ep.gn_x) {
-                eh.gn_x = ep.gn_x + opix * ep.gn_ldx;
-                eh.gn_chsum = mbf(const_cast<float*>(ep.gn_chsum), h, size_t(Cout) * 2);
-                eh.gn_S = mbf(ep.gn_S, h, size_t(Cout) * 2);
+        UbTrainer::Op op;
+        // persistent row-tile kernel for the 16x16 .. 128x128 levels, one-CTA-per-128-pixels kernel otherwise
+        IgemmRowsParams pr;
+        if (!no_rows && igemm_rows_eligible(B, H, W, Cout) &&
+            igemm_rows_plan(&pr, segs.data(), int(segs.size()), B, H, W, Cout, ep, sm_count()) == 0) {
+            op = [pr](cudaStream_t st) { igemm_rows_launch(pr, st); };
+            label("conv%s %s Cin=%d%s Cout=%d %dx%d rows BN=%d stages=%d/%d%s%s", segs[0].ntaps == 9 ? "3x3" : "1x1",
+                  fwd ? "fwd" : "dgrad", segs[0].Cin, segs.size() > 1 ? "+skip" : "", Cout, H, W, pr.BN, pr.a_stages,
+                  pr.w_stages, ep.stats ? " +stats" : "", ep.gn_x ? " +gnbwd" : "");
+        } else {
+            IgemmConvParams p;
+            int r = igemm_conv_plan(&p, segs.data(), int(segs.size()), B, H, W, Cout, ep);
+            if (r) {
+                set_err("igemm_conv_plan failed (%d) for %dx%d Cout=%d Cin0=%d", r, H, W, Cout, segs[0].Cin);
+                plan_errors++;
+                return;
             }
-            UbTrainer::Op op;
-            // persistent row-tile kernel for the 16x16 .. 128x128 levels, one-CTA-per-128-pixels kernel otherwise
-            IgemmRowsParams pr;
-            if (!no_rows && igemm_rows_eligible(Bh, H, W, Cout) &&
-                igemm_rows_plan(&pr, sh.data(), int(sh.size()), Bh, H, W, Cout, eh, sm_count()) == 0) {
-                op = [pr](cudaStream_t st) { igemm_rows_launch(pr, st); };
-                label("conv%s %s Cin=%d%s Cout=%d %dx%d rows BN=%d stages=%d/%d%s%s", segs[0].ntaps == 9 ? "3x3" : "1x1",
-                      fwd ? "fwd" : "dgrad", segs[0].Cin, segs.size() > 1 ? "+skip" : "", Cout, H, W, pr.BN, pr.a_stages,
-                      pr.w_stages, ep.stats ? " +stats" : "", ep.gn_x ? " +gnbwd" : "");
-            } else {
-                // (shared: a GroupNorm that consumes the output may still extend the plan, see gn_finish)
-                auto pp = std::make_shared<IgemmConvParams>();
-                IgemmConvParams& p = *pp;
-                int r = igemm_conv_plan(&p, sh.data(), int(sh.size()), Bh, H, W, Cout, eh);
-                if (r) {
-                    set_err("igemm_conv_plan failed (%d) for %dx%d Cout=%d Cin0=%d", r, H, W, Cout, segs[0].Cin);
-                    plan_errors++;
-                    return;
-                }
-                if (nh == 1 && p.gnf_cluster && (ep.stats || ep.gn_x)) gn_finish[ep.out] = pp;
-                op = [pp](cudaStream_t st) { igemm_conv_launch(*pp, st); };
-                label("conv%s %s Cin=%d%s Cout=%d %dx%d BN=%d stages=%d%s%s%s", segs[0].ntaps == 9 ? "3x3" : "1x1",
-                      fwd ? "fwd" : "dgrad", segs[0].Cin, segs.size() > 1 ? "+skip" : "", Cout, H, W, p.BN, p.stages,
-                      ep.stats ? " +stats" : "", ep.gn_x ? " +gnbwd" : "", p.ms == 2 ? " +tmast" : p.ms ? " +ms" : "");
-            }
-            if (fwd)
-                F(op, 1, UB_KIND_CONV, flops / nh, bytes / nh);
-            else
-                Bk(op, 1, UB_KIND_CONV, flops / nh, bytes / nh);
-        });
+            op = [p](cudaStream_t st) { igemm_conv_launch(p, st); };
+            label("conv%s %s Cin=%d%s Cout=%d %dx%d BN=%d stages=%d%s%s%s", segs[0].ntaps == 9 ? "3x3" : "1x1",
+                  fwd ? "fwd" : "dgrad", segs[0].Cin, segs.size() > 1 ? "+skip" : "", Cout, H, W, p.BN, p.stages,
+                  ep.stats ? " +stats" : "", ep.gn_x ? " +gnbwd" : "", p.ms == 2 ? " +tmast" : p.ms ? " +ms" : "");
+        }
+        if (fwd)
+            F(op, 1, UB_KIND_CONV, flops, bytes);
+        else
+            Bk(op, 1, UB_KIND_CONV, flops, bytes);
     }
     // Weight (and bias) gradient of a conv / linear layer on the side stream.  Every CTA adds its tile into an fp32
     // accumulator with TMA reduce-add boxes; 3x3 layers accumulate in [tap][o][c] and are transposed into the reference
@@ -499,51 +429,14 @@ struct Builder {
         size_t w, b;
         float *chsum, *S;
     };
-    // GroupNorm finish (IgemmConvParams::gnf): convs of the low-resolution levels whose epilogue can complete the
-    // GroupNorm that consumes their output (forward) / whose gn-bwd hook they carry (backward), keyed by output tensor.
-    // gn_fwd / gn_bwd extend the plan and emit no kernel of their own when the output's producer is registered here.
-    std::map<const void*, std::shared_ptr<IgemmConvParams>> gn_finish;
-    int gn_finished_fwd = 0, gn_finished_bwd = 0;
-    // statistics buffer of a tensor whose producer (a conv epilogue) accumulates them
-    // GroupNorm scheme (UB_GN_MODE), decided per tensor shape.  Measured round 2 (bench.py, B = 32, ms/step):
-    //   hooks 5.09 (default) | auto 5.23 | passes 5.47 | slab 6.05
-    //   hooks  statistics / gn-bwd pre-pass accumulated with atomics in the producing conv's epilogue + one apply pass
-    //          (costs ~0.5 ms per step inside the conv epilogues, profiles/r02d_ops_nohooks.txt, but every alternative
-    //          costs more on the GroupNorm side: the step is bound by kernel count x per-kernel latency, not bytes)
-    //   auto   single-pass slab kernels (csrc/gn_slab.cu: statistics + normalisation in one kernel, nothing in the conv
-    //          epilogues) wherever they beat the two-pass kernels stand-alone (gn_slab_preferred: below 64x64), hooks
-    //          elsewhere
-    //   slab   slab kernels wherever they are supported, `passes` elsewhere
-    //   passes separate statistics pass + apply pass, no hooks
-    static int gn_mode() {
-        static const int m = [] {
-            const char* e = getenv("UB_GN_MODE");
-            if (e && e[0] == 's') return 0;
-            if (e && e[0] == 'p') return 2;
-            if (e && e[0] == 'a') return 3;
-            return 1;
-        }();
-        return m;
-    }
-    bool use_slab(int C, int H, int W) const {
-        const int m = gn_mode();
-        if (m == 0) return gn_slab_supported(Bh, H * W, C, c.gn_n_groups, false) && gn_slab_supported(Bh, H * W, C, c.gn_n_groups, true);
-        return m == 3 && gn_slab_preferred(Bh, H * W, C, c.gn_n_groups);
-    }
-    // does the conv that produces a (C, H, W) tensor accumulate its GroupNorm statistics / run the gn-bwd pre-pass?
-    bool use_hooks(int C, int H, int W) const {
-        const int m = gn_mode();
-        return m == 1 || (m == 3 && !use_slab(C, H, W));
-    }
-    // The gn-bwd pre-pass hook (x read + silu' + two column sums in the dgrad epilogue) makes the 64x64 dgrad convs
-    // epilogue-bound (39 us against 24 us unhooked): above UB_GN_BWD_HOOK_MAX_HW pixels per image the backward uses the
-    // separate statistics pass instead (the forward statistics hook stays).
-    static int bwd_hook_max_hw() {
-        static const int v = getenv("UB_GN_BWD_HOOK_MAX_HW") ? atoi(getenv("UB_GN_BWD_HOOK_MAX_HW")) : (1 << 30);
-        return v;
-    }
-    bool use_bwd_hook(int C, int H, int W) const { return use_hooks(C, H, W) && H * W <= bwd_hook_max_hw(); }
-    float* stats_buf(int C, int H, int W) { return use_hooks(C, H, W) ? zf32(size_t(B) * C * 2) : nullptr; }
+    // GroupNorm: the conv that produces a normalised tensor accumulates its per-(image, channel) statistics in its
+    // epilogue (stats_buf), the dgrad conv that produces dL/dy runs the first half of the backward (gn_hook), and the
+    // GroupNorm itself is one apply pass each way.  Measured round 2 (bench.py, B = 32, ms/step): these hooks 5.09;
+    // separate statistics + apply passes 5.47; single-pass slab kernels (csrc/gn_slab.cu) 6.05 everywhere, 5.23 below
+    // 64x64 (where they beat the two-pass kernels stand-alone) with hooks above.  The hooks cost ~0.5 ms per step inside
+    // the conv epilogues (profiles/r02d_ops_nohooks.txt), but every alternative costs more on the GroupNorm side: the
+    // step is bound by kernel count x per-kernel latency, not bytes.
+    float* stats_buf(int C) { return zf32(size_t(B) * C * 2); }
     // ss (use_scale_shift_norm): per-image [scale | shift] rows applied after the normalisation (gn_scale_shift)
     GN gn_fwd(View x, View y, int silu, const float* ss = nullptr, DropArgs drop = DropArgs()) {
         GN g;
@@ -551,83 +444,33 @@ struct Builder {
         const bool have = x.cs != nullptr;  // the producer's epilogue already accumulated the statistics
         g.chsum = have ? x.cs : zf32(size_t(B) * x.C * 2);
         g.S = zf32(size_t(B) * x.C * 2);
-        const int HW = x.H * x.W, Gn = c.gn_n_groups;
+        const int HW = x.H * x.W, Gn = c.gn_n_groups, Bn = B;
         float *gw = P(g.w), *gb = P(g.b), *cs = g.chsum;
-        const bool slab = !have && !ss && !drop.ctl && use_slab(x.C, x.H, x.W);
-        if (have && real() && !ss && !drop.ctl) {
-            auto it = gn_finish.find(x.p);
-            if (it != gn_finish.end()) {
-                auto pp = it->second;
-                gn_finish.erase(it);
-                if (x.ld == pp->ldo && x.C == pp->Cout && pp->stats == cs &&
-                    igemm_conv_gn_finish_fwd(pp.get(), gw, gb, Gn, silu, y.p, y.ld)) {
-                    gn_finished_fwd++;
-                    return g;  // the producing conv's epilogue writes y
-                }
-            }
-        }
-        label("gn_fwd C=%d %dx%d%s", x.C, x.H, x.W, slab ? " slab" : (have ? "" : " +stats pass"));
-        split([&](int h) {
-            const View xh = mb(x, h), yh = mb(y, h);
-            float* csh = mbf(cs, h, size_t(x.C) * 2);
-            const int Bq = Bh;
-            if (slab)
-                F([=](cudaStream_t st) { gn_slab_fwd(xh.p, xh.ld, gw, gb, Bq, HW, xh.C, Gn, silu, yh.p, yh.ld, csh, st); }, 1,
-                  UB_KIND_NORM, 0, 2 * act_bytes(x.C, x.H, x.W) / nh);
-            else
-                F([=](cudaStream_t st) {
-                    if (!have) gn_stats(xh.p, xh.ld, Bq, HW, xh.C, csh, st);
-                    gn_apply(xh.p, xh.ld, csh, gw, gb, Bq, HW, xh.C, Gn, silu, yh.p, yh.ld, nullptr, st,
-                             mbf(const_cast<float*>(ss), h, size_t(2) * xh.C), drop);
-                }, have ? 1 : 2, UB_KIND_NORM, 0, (have ? 2 : 3) * act_bytes(x.C, x.H, x.W) / nh);
-        });
+        label("gn_fwd C=%d %dx%d%s", x.C, x.H, x.W, have ? "" : " +stats pass");
+        F([=](cudaStream_t st) {
+            if (!have) gn_stats(x.p, x.ld, Bn, HW, x.C, cs, st);
+            gn_apply(x.p, x.ld, cs, gw, gb, Bn, HW, x.C, Gn, silu, y.p, y.ld, nullptr, st, ss, drop);
+        }, have ? 1 : 2, UB_KIND_NORM, 0, (have ? 2 : 3) * act_bytes(x.C, x.H, x.W));
         return g;
     }
     // Fuse the first half of GroupNorm(+SiLU) backward into the epilogue of the dgrad conv that produces dL/dy:
     // that conv then writes dz = dL/d gn(x) and accumulates S (see epilogue.cuh); call gn_bwd(..., fused = true) after.
     void gn_hook(ConvEpilogue& ep, const GN& g, View x, int silu) {
-        if (!use_bwd_hook(x.C, x.H, x.W)) return;
         ep.gn_x = x.p, ep.gn_ldx = x.ld, ep.gn_chsum = g.chsum, ep.gn_gamma = P(g.w), ep.gn_beta = P(g.b);
         ep.gn_S = g.S, ep.gn_silu = silu, ep.gn_groups = c.gn_n_groups;
     }
     void gn_bwd(const GN& g, View x, View dy, int silu, View add_in, View dx, float* colsum_out, bool fused = false,
                 const float* ss = nullptr, float* dss = nullptr, DropArgs drop = DropArgs()) {
-        fused = fused && use_bwd_hook(x.C, x.H, x.W) && !ss && !drop.ctl;
-        const int HW = x.H * x.W, Gn = c.gn_n_groups;
+        fused = fused && !ss && !drop.ctl;
+        const int HW = x.H * x.W, Gn = c.gn_n_groups, Bn = B;
         float *gw = P(g.w), *gb = P(g.b), *cs = g.chsum, *S = g.S, *dgw = G(g.w), *dgb = G(g.b);
-        const bool slab = !fused && !ss && !drop.ctl && use_slab(x.C, x.H, x.W);
         const int mode = fused ? (silu ? 2 : 0) : silu;
-        if (fused && real()) {
-            auto it = gn_finish.find(dy.p);
-            if (it != gn_finish.end()) {
-                auto pp = it->second;
-                gn_finish.erase(it);
-                if (dy.ld == pp->ldo && x.C == pp->Cout && pp->gn_S == S &&
-                    igemm_conv_gn_finish_bwd(pp.get(), add_in.p, add_in.ld, dx.p, dx.ld, dgw, dgb, colsum_out)) {
-                    gn_finished_bwd++;
-                    return;  // the dgrad conv's epilogue writes dx, dgamma, dbeta and the column sums
-                }
-            }
-        }
-        label("gn_bwd C=%d %dx%d%s%s", x.C, x.H, x.W, slab ? " slab" : (fused ? "" : " +stats pass"), add_in.p ? " +add" : "");
-        split([&](int h) {
-            const View xh = mb(x, h), dyh = mb(dy, h), ah = mb(add_in, h), dxh = mb(dx, h);
-            float *csh = mbf(cs, h, size_t(x.C) * 2), *Sh = mbf(S, h, size_t(x.C) * 2), *colh = mbf(colsum_out, h, x.C);
-            const int Bq = Bh;
-            if (slab)
-                Bk([=](cudaStream_t st) {
-                    gn_slab_bwd(xh.p, xh.ld, dyh.p, dyh.ld, csh, gw, gb, Bq, HW, xh.C, Gn, silu, ah.p, ah.ld, dxh.p, dxh.ld,
-                                dgw, dgb, colh, st);
-                }, 1, UB_KIND_NORM, 0, (3 + (add_in.p ? 1 : 0)) * act_bytes(x.C, x.H, x.W) / nh);
-            else
-                Bk([=](cudaStream_t st) {
-                    const float* ssh = mbf(const_cast<float*>(ss), h, size_t(2) * xh.C);
-                    float* dssh = mbf(dss, h, size_t(2) * xh.C);
-                    if (!fused) gn_bwd_stats(xh.p, xh.ld, dyh.p, dyh.ld, csh, gw, gb, Bq, HW, xh.C, Gn, silu, Sh, st, ssh, drop);
-                    gn_bwd_apply(xh.p, xh.ld, dyh.p, dyh.ld, csh, Sh, gw, gb, Bq, HW, xh.C, Gn, mode, ah.p, ah.ld, dxh.p,
-                                 dxh.ld, dgw, dgb, colh, st, ssh, dssh, drop);
-                }, fused ? 1 : 2, UB_KIND_NORM, 0, ((fused ? 3 : 5) + (add_in.p ? 1 : 0)) * act_bytes(x.C, x.H, x.W) / nh);
-        });
+        label("gn_bwd C=%d %dx%d%s%s", x.C, x.H, x.W, fused ? "" : " +stats pass", add_in.p ? " +add" : "");
+        Bk([=](cudaStream_t st) {
+            if (!fused) gn_bwd_stats(x.p, x.ld, dy.p, dy.ld, cs, gw, gb, Bn, HW, x.C, Gn, silu, S, st, ss, drop);
+            gn_bwd_apply(x.p, x.ld, dy.p, dy.ld, cs, S, gw, gb, Bn, HW, x.C, Gn, mode, add_in.p, add_in.ld, dx.p, dx.ld,
+                         dgw, dgb, colsum_out, st, ss, dss, drop);
+        }, fused ? 1 : 2, UB_KIND_NORM, 0, ((fused ? 3 : 5) + (add_in.p ? 1 : 0)) * act_bytes(x.C, x.H, x.W));
     }
 
     int res_index = 0;
@@ -673,29 +516,23 @@ struct Builder {
     // 2x resampling of a tensor inside an up/down ResBlock (h_upd / x_upd, dev/resblock.py:78-86,125-128): ud = 1 average
     // pool, ud = 2 nearest upsample
     void resample_fwd(View x, View y, int ud) {
-        split([&](int hh) {
-            const View xm = mb(x, hh), ym = mb(y, hh);
-            const int Bq = Bh;
-            F([=](cudaStream_t st) {
-                if (ud == 1)
-                    avgpool2_fwd(xm.p, xm.ld, Bq, xm.H, xm.W, xm.C, ym.p, ym.ld, st);
-                else
-                    upsample2_fwd(xm.p, xm.ld, Bq, xm.H, xm.W, xm.C, ym.p, ym.ld, st);
-            }, 1, UB_KIND_ELTWISE, 0, 1.25 * act_bytes(x.C, std::max(x.H, y.H), std::max(x.W, y.W)) / nh);
-        });
+        const int Bn = B;
+        F([=](cudaStream_t st) {
+            if (ud == 1)
+                avgpool2_fwd(x.p, x.ld, Bn, x.H, x.W, x.C, y.p, y.ld, st);
+            else
+                upsample2_fwd(x.p, x.ld, Bn, x.H, x.W, x.C, y.p, y.ld, st);
+        }, 1, UB_KIND_ELTWISE, 0, 1.25 * act_bytes(x.C, std::max(x.H, y.H), std::max(x.W, y.W)));
     }
     // gradient of resample_fwd: dx (resolution of x) from dy (resolution of y)
     void resample_bwd(View dy, View dx, int ud) {
-        split([&](int hh) {
-            const View dm = mb(dy, hh), dxm = mb(dx, hh);
-            const int Bq = Bh;
-            Bk([=](cudaStream_t st) {
-                if (ud == 1)
-                    avgpool2_bwd(dm.p, dm.ld, Bq, dxm.H, dxm.W, dxm.C, nullptr, 0, dxm.p, dxm.ld, st);
-                else
-                    upsample2_bwd(dm.p, dm.ld, Bq, dm.H, dm.W, dm.C, dxm.p, dxm.ld, st);
-            }, 1, UB_KIND_ELTWISE, 0, 1.25 * act_bytes(dx.C, std::max(dx.H, dy.H), std::max(dx.W, dy.W)) / nh);
-        });
+        const int Bn = B;
+        Bk([=](cudaStream_t st) {
+            if (ud == 1)
+                avgpool2_bwd(dy.p, dy.ld, Bn, dx.H, dx.W, dx.C, nullptr, 0, dx.p, dx.ld, st);
+            else
+                upsample2_bwd(dy.p, dy.ld, Bn, dy.H, dy.W, dy.C, dx.p, dx.ld, st);
+        }, 1, UB_KIND_ELTWISE, 0, 1.25 * act_bytes(dx.C, std::max(dx.H, dy.H), std::max(dx.W, dy.W)));
     }
 
     // ResBlock (dev/resblock.py:107-160, train_unet.cu:2213-2384).  ud != 0 (cfg.resblock_updown, dev/unet.py:205-222,
@@ -734,7 +571,7 @@ struct Builder {
         const size_t w1 = take(size_t(Cout) * C * 9), b1 = take(Cout);
         const size_t wl = take(size_t(OCe) * Cemb), bl = take(OCe);
         View h1 = act(Cout, H, W);
-        h1.cs = stats_buf(Cout, H, W);
+        h1.cs = stats_buf(Cout);
         float* embproj = f32(size_t(B) * OCe);
         float* d_embproj = zf32(size_t(B) * OCe);
         Packed p1 = pack(w1, Cout, C, 9);
@@ -756,7 +593,7 @@ struct Builder {
             ps = pack(ws, Cout, C, 1);
         }
         View out = act(Cout, H, W);
-        out.cs = stats_buf(Cout, H, W);
+        out.cs = stats_buf(Cout);
         {
             ConvEpilogue ep;
             ep.bias = P(b2), ep.out = out.p, ep.ldo = out.ld, ep.stats = out.cs;
@@ -847,7 +684,7 @@ struct Builder {
         const size_t wp = take(size_t(C) * C), bp = take(C);
         Packed pq = pack(wq, 3 * C, C, 1), pp = pack(wp, C, C, 1);
         View qkv = act(3 * C, H, W), ao = act(C, H, W), out = act(C, H, W);
-        out.cs = stats_buf(C, H, W);
+        out.cs = stats_buf(C);
         float* lse = f32(size_t(B) * NH * Tn);
         float* dsum = f32(size_t(B) * NH * Tn);
         {
@@ -858,23 +695,19 @@ struct Builder {
         // tcgen05 attention core when the shape allows (T <= 256; head size 64, or 32 with an even head count), SIMT
         // fallback otherwise
         const bool tc = attn_tc_supported(Tn, NH, HSz);
+        const int Bn = B;
         label("attn fwd T=%d C=%d", Tn, C);
-        split([&](int h) {
-            const View qh = mb(qkv, h), aoh = mb(ao, h);
-            float* lseh = mbf(lse, h, size_t(NH) * Tn);
-            const int Bq = Bh;
-            AttnTcParams apf;
-            if (tc && real()) {
-                int r = attn_tc_plan(&apf, qh.p, qh.ld, Bq, Tn, NH, HSz, aoh.p, aoh.ld, lseh, nullptr, 0, nullptr, 0, nullptr);
-                if (r) set_err("attn_tc_plan failed (%d)", r), plan_errors++;
-            }
-            F([=](cudaStream_t st) {
-                if (tc)
-                    attn_tc_fwd(apf, st);
-                else
-                    attn_fwd(qh.p, qh.ld, Bq, Tn, NH, HSz, aoh.p, aoh.ld, lseh, st);
-            }, 1, UB_KIND_ATTN, 4.0 * Bq * NH * double(Tn) * Tn * HSz, act_bytes(4 * C, H, W) / nh);
-        });
+        AttnTcParams apf;
+        if (tc && real()) {
+            int r = attn_tc_plan(&apf, qkv.p, qkv.ld, B, Tn, NH, HSz, ao.p, ao.ld, lse, nullptr, 0, nullptr, 0, nullptr);
+            if (r) set_err("attn_tc_plan failed (%d)", r), plan_errors++;
+        }
+        F([=](cudaStream_t st) {
+            if (tc)
+                attn_tc_fwd(apf, st);
+            else
+                attn_fwd(qkv.p, qkv.ld, Bn, Tn, NH, HSz, ao.p, ao.ld, lse, st);
+        }, 1, UB_KIND_ATTN, 4.0 * B * NH * double(Tn) * Tn * HSz, act_bytes(4 * C, H, W));
         {
             ConvEpilogue ep;
             ep.bias = P(bp), ep.out = out.p, ep.ldo = out.ld, ep.residual = x.p, ep.ldr = x.ld, ep.stats = out.cs;
@@ -893,23 +726,18 @@ struct Builder {
             }
             label("attn bwd T=%d C=%d", Tn, C);
             UbTrainer* Tt = T;
-            split([&](int h) {
-                const View qh = mb(qkv, h), aoh = mb(ao, h), daoh = mb(dao, h), dqh = mb(dqkv, h);
-                float *lseh = mbf(lse, h, size_t(NH) * Tn), *dsh = mbf(dsum, h, size_t(NH) * Tn);
-                const int Bq = Bh;
-                AttnTcParams apb;
-                if (tc && real()) {
-                    int r = attn_tc_plan(&apb, qh.p, qh.ld, Bq, Tn, NH, HSz, aoh.p, aoh.ld, lseh, daoh.p, daoh.ld, dqh.p,
-                                         dqh.ld, dsh);
-                    if (r) set_err("attn_tc_plan (bwd) failed (%d)", r), plan_errors++;
-                }
-                Bk([=](cudaStream_t st) {
-                    if (tc)
-                        attn_tc_bwd(apb, st, Tt->attn_concurrent ? Tt->aux_stream : nullptr, Tt->ev_aux_fork, Tt->ev_aux_join);
-                    else
-                        attn_bwd(qh.p, qh.ld, aoh.p, aoh.ld, daoh.p, daoh.ld, lseh, Bq, Tn, NH, HSz, dqh.p, dqh.ld, dsh, st);
-                }, 2, UB_KIND_ATTN, 10.0 * Bq * NH * double(Tn) * Tn * HSz, act_bytes(8 * C, H, W) / nh);
-            });
+            AttnTcParams apb;
+            if (tc && real()) {
+                int r = attn_tc_plan(&apb, qkv.p, qkv.ld, B, Tn, NH, HSz, ao.p, ao.ld, lse, dao.p, dao.ld, dqkv.p, dqkv.ld,
+                                     dsum);
+                if (r) set_err("attn_tc_plan (bwd) failed (%d)", r), plan_errors++;
+            }
+            Bk([=](cudaStream_t st) {
+                if (tc)
+                    attn_tc_bwd(apb, st, Tt->attn_concurrent ? Tt->aux_stream : nullptr, Tt->ev_aux_fork, Tt->ev_aux_join);
+                else
+                    attn_bwd(qkv.p, qkv.ld, ao.p, ao.ld, dao.p, dao.ld, lse, Bn, Tn, NH, HSz, dqkv.p, dqkv.ld, dsum, st);
+            }, 2, UB_KIND_ATTN, 10.0 * B * NH * double(Tn) * Tn * HSz, act_bytes(8 * C, H, W));
             wgrad_op(dqkv, g, C, 3 * C, 1, G(wq), gbq);
             {
                 ConvEpilogue ep;
@@ -994,12 +822,7 @@ int Builder::build() {
         float *w = P(wi), *b = P(bi), *gw = G(wi), *gb = G(bi);
         const int Cin = c.C_in;
         View hv = h;
-        split([&](int hh) {
-            const View hm = mb(hv, hh);
-            const size_t xoff = size_t(hh) * Bh * img;
-            const int Bq = Bh;
-            F([=](cudaStream_t st) { conv_in_fwd(Tt->xt + xoff, w, b, Bq, Cin, hm.C, hm.H, hm.W, hm.p, hm.ld, st); });
-        });
+        F([=](cudaStream_t st) { conv_in_fwd(Tt->xt, w, b, Bn, Cin, hv.C, hv.H, hv.W, hv.p, hv.ld, st); });
         nd.out = h, nd.pushed = true;
         nd.bwd = [=](View dout) -> View {
             Bk([=](cudaStream_t st) {
@@ -1007,12 +830,7 @@ int Builder::build() {
                               Tt->small_scratch_floats, st);
             }, 1, UB_KIND_SMALL, 0, 0, tail_aux() ? 0 : 1);  // (one launch with the row kernel; two on its fallback path)
             if (Tt->cfg.compute_dinput)
-                split([&](int hh) {
-                    const View dm = mb(dout, hh);
-                    const size_t xoff = size_t(hh) * Bh * img;
-                    const int Bq = Bh;
-                    Bk([=](cudaStream_t st) { conv_in_dgrad(dm.p, dm.ld, w, Bq, Cin, hv.C, hv.H, hv.W, Tt->dxt + xoff, st); }, 1);
-                });
+                Bk([=](cudaStream_t st) { conv_in_dgrad(dout.p, dout.ld, w, Bn, Cin, hv.C, hv.H, hv.W, Tt->dxt, st); }, 1);
             return View{};
         };
         nodes.push_back(nd);
@@ -1021,11 +839,8 @@ int Builder::build() {
     std::vector<View> skip_views = {h};
 
     const int nlev = c.n_levels;
-    level_mb(H0, W0);
-    sync_nh();
     for (int level = 0; level < nlev; ++level) {
         const int cout = c.channel_mult[level] * Cm;
-        level_mb(H0 >> level, W0 >> level);
         for (int i = 0; i < c.n_res_blocks; ++i) {
             h = resblock(h, cout);
             if (level >= c.att_start_level) h = attnblock(h);
@@ -1042,22 +857,14 @@ int Builder::build() {
             Node nd;
             nd.param_begin = poff;
             View x = h, y = act(h.C, h.H / 2, h.W / 2);
-            split([&](int hh) {
-                const View xm = mb(x, hh), ym = mb(y, hh);
-                const int Bq = Bh;
-                F([=](cudaStream_t st) { avgpool2_fwd(xm.p, xm.ld, Bq, xm.H, xm.W, xm.C, ym.p, ym.ld, st); }, 1,
-                  UB_KIND_ELTWISE, 0, 1.25 * act_bytes(x.C, x.H, x.W) / nh);
-            });
+            F([=](cudaStream_t st) { avgpool2_fwd(x.p, x.ld, Bn, x.H, x.W, x.C, y.p, y.ld, st); }, 1, UB_KIND_ELTWISE, 0,
+              1.25 * act_bytes(x.C, x.H, x.W));
             nd.out = y, nd.pushed = true;
             nd.bwd = [=](View dout) -> View {
                 View dx = act(x.C, x.H, x.W);
-                split([&](int hh) {
-                    const View dm = mb(dout, hh), dxm = mb(dx, hh);
-                    const int Bq = Bh;
-                    Bk([=](cudaStream_t st) {
-                        avgpool2_bwd(dm.p, dm.ld, Bq, x.H, x.W, x.C, nullptr, 0, dxm.p, dxm.ld, st);
-                    }, 1, UB_KIND_ELTWISE, 0, 1.25 * act_bytes(x.C, x.H, x.W) / nh);
-                });
+                Bk([=](cudaStream_t st) {
+                    avgpool2_bwd(dout.p, dout.ld, Bn, x.H, x.W, x.C, nullptr, 0, dx.p, dx.ld, st);
+                }, 1, UB_KIND_ELTWISE, 0, 1.25 * act_bytes(x.C, x.H, x.W));
                 return dx;
             };
             nodes.push_back(nd);
@@ -1066,7 +873,6 @@ int Builder::build() {
             skip_views.push_back(h);
         }
     }
-    sync_nh();
     // ---- middle (dev/unet.py:224-243)
     h = resblock(h, h.C);
     h = attnblock(h);
@@ -1075,8 +881,6 @@ int Builder::build() {
     bool pending_up = false;
     for (int level = nlev - 1; level >= 0; --level) {
         const int cout = c.channel_mult[level] * Cm;
-        sync_nh();
-        level_mb(H0 >> level, W0 >> level);
         for (int i = 0; i <= c.n_res_blocks; ++i) {
             const int src = skip_stack.back();
             View sk = skip_views.back();
@@ -1087,13 +891,9 @@ int Builder::build() {
             const int C1 = h.C, C2 = sk.C, Hc = sk.H, Wc = sk.W, up = pending_up ? 1 : 0;
             View cat = act(C1 + C2, Hc, Wc), a = h;
             if (a.cs && sk.cs) cat.cs = zf32(size_t(B) * (C1 + C2) * 2);  // GroupNorm statistics of the parts, side by side
-            split([&](int hh) {
-                const View am = mb(a, hh), sm = mb(sk, hh), cm = mb(cat, hh);
-                const int Bq = Bh;
-                F([=](cudaStream_t st) {
-                    concat2(am.p, am.ld, C1, up, sm.p, sm.ld, C2, Bq, Hc, Wc, cm.p, cm.ld, am.cs, sm.cs, cm.cs, st);
-                }, 1, UB_KIND_ELTWISE, 0, 2 * act_bytes(C1 + C2, Hc, Wc) / nh);
-            });
+            F([=](cudaStream_t st) {
+                concat2(a.p, a.ld, C1, up, sk.p, sk.ld, C2, Bn, Hc, Wc, cat.p, cat.ld, a.cs, sk.cs, cat.cs, st);
+            }, 1, UB_KIND_ELTWISE, 0, 2 * act_bytes(C1 + C2, Hc, Wc));
             nd.out = cat;
             std::vector<View>* sg = &skipgrad;
             nd.bwd = [=](View d) -> View {
@@ -1102,12 +902,8 @@ int Builder::build() {
                 (*sg)[src] = skv;
                 if (up) {
                     View dlow = act(C1, Hc / 2, Wc / 2);
-                    split([&](int hh) {
-                        const View dm = mb(d, hh), lm = mb(dlow, hh);
-                        const int Bq = Bh;
-                        Bk([=](cudaStream_t st) { upsample2_bwd(dm.p, dm.ld, Bq, Hc, Wc, C1, lm.p, lm.ld, st); }, 1,
-                           UB_KIND_ELTWISE, 0, 1.25 * act_bytes(C1, Hc, Wc) / nh);
-                    });
+                    Bk([=](cudaStream_t st) { upsample2_bwd(d.p, d.ld, Bn, Hc, Wc, C1, dlow.p, dlow.ld, st); }, 1,
+                       UB_KIND_ELTWISE, 0, 1.25 * act_bytes(C1, Hc, Wc));
                     return dlow;
                 }
                 View mv = d;
@@ -1126,7 +922,6 @@ int Builder::build() {
             }
         }
     }
-    sync_nh();
     // ---- output head: GN + SiLU + conv3x3 (-> C_out) + MSE (dev/unet.py:286-290, train_unet.cu:4408-4418)
     {
         Node nd;
@@ -1147,12 +942,7 @@ int Builder::build() {
                 conv_out_wgrad(ao.p, ao.ld, Tt->dout, Bn, Cin, Co, Hh, Ww, gw, gb, Tt->small_scratch,
                                Tt->small_scratch_floats, st);
             }, 2, UB_KIND_SMALL, 0, 0, 1);  // (row kernel + bias sum; three on the fallback path)
-            split([&](int hh) {
-                const View dm = mb(dao, hh);
-                const size_t ooff = size_t(hh) * Bh * Co * Hh * Ww;
-                const int Bq = Bh;
-                Bk([=](cudaStream_t st) { conv_out_dgrad(Tt->dout + ooff, w, Bq, Cin, Co, Hh, Ww, dm.p, dm.ld, st); }, 1);
-            });
+            Bk([=](cudaStream_t st) { conv_out_dgrad(Tt->dout, w, Bn, Cin, Co, Hh, Ww, dao.p, dao.ld, st); }, 1);
             gn_bwd(g, hx, dao, 1, View{}, dh, nullptr);
             return dh;
         };
@@ -1165,11 +955,6 @@ int Builder::build() {
     // ---- backward: walk the nodes in reverse.  Gradient buckets (data parallel): parameters live in forward
     //      order, so once node i's backward has been emitted every parameter at offset >= node[i].param_begin is
     //      final (the time MLP at the head of the arena finishes last).
-    // UB_MICROBATCH_FWD=n: micro-batch chains in the FORWARD pass only -- there the device runs one kernel at a time and
-    // the 8x8 / 16x16 levels fill less than half of it, while backward already shares the device with the weight-gradient
-    // branch.  Backward ops are emitted once for the whole batch (the activations are batch-major views either way).
-    sync_nh();
-    if (T->mb_fwd_only) nh = 1, Bh = B;
     skipgrad.assign(nodes.size(), View{});
     std::vector<size_t> cuts;  // descending offsets at which a bucket is flushed
     {
@@ -1242,19 +1027,15 @@ int Builder::build() {
     View g{};
     for (int i = int(nodes.size()) - 1; i >= 0; --i) {
         Node& nd = nodes[i];
-        if (T->mb_max_hw > 0 && !T->mb_fwd_only) nh = node_nh[size_t(i)], Bh = B / nh;  // the chains of this node's level
         if (nd.pushed) {  // gradient of a tensor that also fed a skip connection: sum both contributions
             View s = skipgrad[i];
             View sum = act(nd.out.C, nd.out.H, nd.out.W);
             View a = g;
-            const size_t npix = size_t(Bh) * nd.out.H * nd.out.W;
+            const size_t npix = size_t(B) * nd.out.H * nd.out.W;
             const int C = nd.out.C;
             a.H = s.H = nd.out.H, a.W = s.W = nd.out.W;  // (channel-slice views keep the geometry of their buffer)
-            split([&](int hh) {
-                const View am = mb(a, hh), sm = mb(s, hh), um = mb(sum, hh);
-                Bk([=](cudaStream_t st) { add2(am.p, am.ld, sm.p, sm.ld, npix, C, um.p, um.ld, st); }, 1, UB_KIND_ELTWISE, 0,
-                   3 * act_bytes(C, nd.out.H, nd.out.W) / nh);
-            });
+            Bk([=](cudaStream_t st) { add2(a.p, a.ld, s.p, s.ld, npix, C, sum.p, sum.ld, st); }, 1, UB_KIND_ELTWISE, 0,
+               3 * act_bytes(C, nd.out.H, nd.out.W));
             g = sum;
         }
         if (i == 0) {  // only the 3-channel input conv is left: finalise the tcgen05 weight gradients before it
@@ -1291,9 +1072,6 @@ int Builder::build() {
             Tt->opt_stream_dirty = false;
         }
     }, 0);
-    if (real() && getenv("UB_DEBUG_GNF"))
-        fprintf(stderr, "[unet_b200] GroupNorm finished inside conv epilogues: %d forward, %d backward\n",
-                gn_finished_fwd, gn_finished_bwd);
     return plan_errors ? UB_ERR_SHAPE : UB_OK;
 }
 
@@ -1395,16 +1173,6 @@ extern "C" int ub_trainer_create(UbTrainer** out, const UbConfig* cfg, int devic
     UbTrainer* t = new UbTrainer();
     t->cfg = *cfg;
     t->device = device;
-    {   // micro-batch chains (UbTrainer::n_mb): off by default -- measured 5.18 ms/step with one chain, 5.30 with two, 5.74
-        // with four (profiles/r02_microbatch.txt): the latency that B-scaling exposes is per launch, and two chains double
-        // the launches.  UB_MICROBATCH=2 / 4 enables (B must be divisible).
-        int want = getenv("UB_MICROBATCH") ? atoi(getenv("UB_MICROBATCH")) : 1;
-        if (getenv("UB_MICROBATCH_FWD") && atoi(getenv("UB_MICROBATCH_FWD")) >= 2)
-            want = atoi(getenv("UB_MICROBATCH_FWD")), t->mb_fwd_only = true;
-        t->n_mb = (want >= 2 && want <= 8 && cfg->B % want == 0) ? want : 1;
-        if (t->n_mb == 1) t->mb_fwd_only = false;
-        t->mb_max_hw = (t->n_mb > 1 && getenv("UB_MICROBATCH_LOWRES")) ? atoi(getenv("UB_MICROBATCH_LOWRES")) : 0;
-    }
     // pass 1: count
     t->arena.counting = t->zarena.counting = true;
     {
@@ -1449,12 +1217,7 @@ extern "C" int ub_trainer_create(UbTrainer** out, const UbConfig* cfg, int devic
     cudaStreamCreateWithPriority(&t->aux_stream, cudaStreamNonBlocking, use_prio ? prio_hi : 0);
     cudaEventCreateWithFlags(&t->ev_aux_fork, cudaEventDisableTiming);
     cudaEventCreateWithFlags(&t->ev_aux_join, cudaEventDisableTiming);
-    t->attn_concurrent = !(getenv("UB_ATTN_SERIAL") && atoi(getenv("UB_ATTN_SERIAL")) != 0) && (t->n_mb == 1 || t->mb_fwd_only);
-    for (int i = 1; i < t->n_mb; ++i) {
-        cudaStream_t ms = nullptr;
-        cudaStreamCreateWithPriority(&ms, cudaStreamNonBlocking, use_prio ? prio_hi : 0);
-        t->mb_streams.push_back(ms);
-    }
+    t->attn_concurrent = !(getenv("UB_ATTN_SERIAL") && atoi(getenv("UB_ATTN_SERIAL")) != 0);
     t->side_events.resize(4096);
     for (auto& ev : t->side_events) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
     if (const char* e = getenv("UB_NO_SIDE_STREAM")) t->use_side = atoi(e) == 0;
@@ -1541,7 +1304,6 @@ extern "C" void ub_trainer_destroy(UbTrainer* t) {
     if (t->aux_stream) cudaStreamDestroy(t->aux_stream);
     if (t->ev_aux_fork) cudaEventDestroy(t->ev_aux_fork);
     if (t->ev_aux_join) cudaEventDestroy(t->ev_aux_join);
-    for (auto ms : t->mb_streams) cudaStreamDestroy(ms);
     for (auto ev : t->side_events) cudaEventDestroy(ev);
     delete t;
 }
@@ -1566,38 +1328,14 @@ static void enqueue_step(UbTrainer* t, const StepOpts& o, cudaStream_t st) {
     if (debug_sync) cudaStreamIsCapturing(st, &cap);
     bool side_dirty = false, aux_dirty = false;
     auto next_event = [&]() { return t->side_events[t->side_ev_next++ % t->side_events.size()]; };
-    // micro-batch chains: `forked` while the chains of micro-batches 1.. run beside the main stream
-    bool forked = false;
-    auto fork_mb = [&]() {
-        if (forked || t->mb_streams.empty()) return;
-        cudaEvent_t ev = next_event();
-        cudaEventRecord(ev, st);
-        for (cudaStream_t ms : t->mb_streams) cudaStreamWaitEvent(ms, ev, 0);
-        forked = true;
-    };
-    auto join_mb = [&]() {
-        if (!forked) return;
-        for (cudaStream_t ms : t->mb_streams) {
-            cudaEvent_t ev = next_event();
-            cudaEventRecord(ev, ms);
-            cudaStreamWaitEvent(st, ev, 0);
-        }
-        forked = false;
-    };
     auto run = [&](std::vector<UbTrainer::Op>& ops, std::vector<UbTrainer::OpInfo>& info, const char* what) {
         for (size_t i = 0; i < ops.size(); ++i) {
             static const bool skip_side = getenv("UB_DEBUG_SKIP_SIDE") != nullptr;  // timing experiments only
             if (info[i].side == 1 && skip_side) continue;
-            if (info[i].side == 1 && t->use_side) {  // fork: the branch sees everything enqueued on the main chains so far
+            if (info[i].side == 1 && t->use_side) {  // fork: the branch sees everything enqueued on the main stream so far
                 cudaEvent_t ev = next_event();
                 cudaEventRecord(ev, st);
                 cudaStreamWaitEvent(t->side_stream, ev, 0);
-                if (forked)
-                    for (cudaStream_t ms : t->mb_streams) {
-                        cudaEvent_t e2 = next_event();
-                        cudaEventRecord(e2, ms);
-                        cudaStreamWaitEvent(t->side_stream, e2, 0);
-                    }
                 ops[i](t->side_stream);
                 side_dirty = true;
             } else if (info[i].side == 3 && t->use_side) {  // a branch off the weight-gradient branch (time-MLP backward)
@@ -1617,22 +1355,13 @@ static void enqueue_step(UbTrainer* t, const StepOpts& o, cudaStream_t st) {
                     cudaEvent_t ev = next_event();
                     cudaEventRecord(ev, t->side_stream);
                     cudaStreamWaitEvent(st, ev, 0);
-                    if (forked)
-                        for (cudaStream_t ms : t->mb_streams) cudaStreamWaitEvent(ms, ev, 0);
                     side_dirty = false;
                 }
-            } else if (info[i].half > 0 && size_t(info[i].half) <= t->mb_streams.size()) {
-                fork_mb();
-                ops[i](t->mb_streams[info[i].half - 1]);
             } else {
-                if (info[i].half < 0 || info[i].side == 1 || info[i].side == 3) join_mb();  // whole-batch op: every chain must have arrived
-                else fork_mb();
                 ops[i](st);
             }
             if (debug_sync && cap == cudaStreamCaptureStatusNone) {
                 cudaError_t e = cudaStreamSynchronize(st);
-                for (cudaStream_t ms : t->mb_streams)
-                    if (e == cudaSuccess) e = cudaStreamSynchronize(ms);
                 if (e == cudaSuccess) e = cudaGetLastError();
                 if (e != cudaSuccess) {
                     fprintf(stderr, "[unet_b200] %s op %zu (kind %d): %s\n", what, i, info[i].kind,
@@ -1648,7 +1377,6 @@ static void enqueue_step(UbTrainer* t, const StepOpts& o, cudaStream_t st) {
     t->opt_done_lo = t->nparams;
     run(t->fwd_ops, t->fwd_info, "forward");
     run(t->bwd_ops, t->bwd_info, "backward");
-    join_mb();
     if (aux_dirty) {
         cudaEvent_t ev = next_event();
         cudaEventRecord(ev, t->aux_stream);
