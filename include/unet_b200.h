@@ -339,6 +339,44 @@ int ub_trainer_predict(UbTrainer* t, const float* xt_host, const float* t_host, 
 int ub_trainer_sample(UbTrainer* t, const float* x_init_host, int t_start, int t_end, const float* noise_host,
                       unsigned long long seed, float* out_host);
 
+/* ---- few-step sampling: guided-diffusion's image_sample.py (`--timestep_respacing`, `--use_ddim`, `clip_denoised`)
+ * on the device.  The two samplers index the schedule differently, and on purpose:
+ *   ub_trainer_sample keeps generate.py's convention -- at model input t it reads betas[t-1] / acp[t-1] -- because it
+ *     is the drop-in for that script and reproduces it bit for bit;
+ *   ub_trainer_sample_spaced follows the schedule the model was trained on: the training step's q-sample noises x0
+ *     with acp[t] at model input t, and so does guided-diffusion's sampler (acp[t_i] at model input t_i).
+ * For a model trained with this library the spaced sampler is therefore the consistent one, even with every timestep
+ * kept. */
+
+/* guided-diffusion respace.space_timesteps: writes the kept timesteps (ascending) to out[cap];
+ * returns their count, or UB_ERR_SHAPE for a malformed / unsatisfiable spec.  Needs no GPU.
+ *   "ddimN": range(0, n_timesteps, i) for the smallest stride i in 1 .. n_timesteps-1 that keeps exactly N steps;
+ *   "c0,c1,...": n_timesteps split into equal sections (the first n_timesteps % k one step longer), section j keeps
+ *     c_j steps at start + round(idx), idx = 0, f, 2f, ... accumulated in float64 with f = (size-1)/(c_j-1) (1 when
+ *     c_j <= 1), rounded half to even as Python's round.
+ * Counts are non-negative decimal integers; a spec that keeps nothing is refused. */
+int ub_space_timesteps(int n_timesteps, const char* spec, int* out, int cap);
+#define UB_SAMPLER_DDIM 0       /* ddim_sample_loop, eta in [0, 1] */
+#define UB_SAMPLER_ANCESTRAL 1  /* p_sample_loop, fixed-large variance; eta must be 0; n >= 2 */
+/* Sampling over the kept timesteps t_0 < ... < t_{n-1} (strictly ascending, in [0, n_timesteps); e.g. from
+ * ub_space_timesteps), guided-diffusion's SpacedDiffusion with rescale_timesteps = False.  Float64 tables of the
+ * trainer's linear schedule: acp = cumprod(1 - beta); beta'_i = 1 - acp[t_i] / acp[t_{i-1}] (acp[t_{-1}] = 1),
+ * acp'_i = cumprod(1 - beta'), acp'_{-1} = 1.  For i = n-1 down to 0, on all B images of the trainer at once:
+ *   eps = model(x, t_i);  x0 = sqrt(1/acp'_i) x - sqrt(1/acp'_i - 1) eps, clamped to [-1, 1] if clip_denoised;
+ *   ANCESTRAL: x <- posterior mean(x0, x) + [i > 0] sqrt(beta'_i) z                     (fixed-large variance)
+ *   DDIM:      eps' = (sqrt(1/acp'_i) x - x0) / sqrt(1/acp'_i - 1),
+ *              sigma = eta sqrt((1 - acp'_{i-1}) / (1 - acp'_i)) sqrt(1 - acp'_i / acp'_{i-1}),
+ *              x <- sqrt(acp'_{i-1}) x0 + sqrt(1 - acp'_{i-1} - sigma^2) eps' + [i > 0] sigma z
+ * x_init_host (B,C_in,H,W) may be NULL: x_T ~ N(0,1) from `seed` (as ub_trainer_sample).  noise_host may be NULL (z from
+ * the device Philox stream of `seed`; none is drawn where sigma = 0), else it holds n draws of (B,C_in,H,W), largest
+ * timestep first.  out_host receives the final x.  Labels of ub_trainer_set_labels apply; parameters, moving average,
+ * AdamW moments and step count are left untouched.  UB_ERR_SHAPE for a bad timestep list, sampler, eta or n, or
+ * C_in != C_out.  One CUDA graph per iteration, captured on the first call (again when noise_host switches between
+ * NULL and non-NULL). */
+int ub_trainer_sample_spaced(UbTrainer* t, const int* timesteps, int n, int sampler, float eta, int clip_denoised,
+                             const float* x_init_host, const float* noise_host, unsigned long long seed,
+                             float* out_host);
+
 /* ---- dataset reader: prepare_data.py:20-38 format (int32[256] header {20240620, N, C, H, W} + float32 images),
  * semantics of DataLoader / dataloader_next_batch (train_unet.cu:3035-3099): sequential batches of B images,
  * wrapping to the start when fewer than B images remain.  Batches are prefetched by a background thread into three

@@ -100,6 +100,8 @@ def _declare(L: C.CDLL) -> None:
     L.ub_trainer_predict.argtypes = [vp, fp, fp, fp]
     L.ub_trainer_profile.argtypes = [vp, i, C.POINTER(UbProfile)]
     L.ub_trainer_sample.argtypes = [vp, fp, i, i, fp, C.c_ulonglong, fp]
+    L.ub_space_timesteps.argtypes = [i, C.c_char_p, vp, i]
+    L.ub_trainer_sample_spaced.argtypes = [vp, vp, i, i, C.c_float, i, fp, fp, C.c_ulonglong, fp]
     L.ub_dataloader_open.argtypes = [C.POINTER(vp), C.c_char_p, i, i, i]
     L.ub_dataloader_info.argtypes = [vp, C.POINTER(i), C.POINTER(i), C.POINTER(i), C.POINTER(i),
                                      C.POINTER(C.c_longlong)]
@@ -133,6 +135,19 @@ def default_config(**over) -> UbConfig:
 
 def num_params(cfg: UbConfig) -> int:
     return int(lib().ub_num_params(C.byref(cfg)))
+
+
+def space_timesteps(n_timesteps: int, spec: str) -> list[int]:
+    """guided-diffusion respace.space_timesteps as a sorted list: "ddimN" or comma-separated section counts ("250",
+    "10,10,10"); raises UbError for a malformed or unsatisfiable spec.  Needs no GPU."""
+    out = np.empty(max(int(n_timesteps), 1), dtype=np.int32)
+    n = lib().ub_space_timesteps(int(n_timesteps), spec.encode(), out.ctypes.data_as(C.c_void_p), out.size)
+    if n < 0:
+        check(n, "space_timesteps")
+    return [int(v) for v in out[:n]]
+
+
+UB_SAMPLERS = {"ddim": 0, "ancestral": 1}
 
 
 def _ptr(a: Optional[np.ndarray]):
@@ -299,6 +314,26 @@ class Trainer:
         noises = None if noises is None else np.ascontiguousarray(noises, dtype=np.float32)
         out = np.empty((c.B, c.C_in, c.H, c.W), dtype=np.float32)
         check(lib().ub_trainer_sample(self._h, _ptr(x_init), t_start, t_end, _ptr(noises), seed, _ptr(out)), "sample")
+        return out
+
+    def sample_spaced(self, x_init=None, timesteps: Sequence[int] = (), sampler: str = "ddim", eta: float = 0.0,
+                      clip_denoised: bool = True, noises=None, seed: int = 0) -> np.ndarray:
+        """guided-diffusion sampling over the kept `timesteps` (ascending, e.g. space_timesteps(1000, "ddim50")):
+        sampler "ddim" (ddim_sample_loop, eta in [0, 1]) or "ancestral" (p_sample_loop, fixed-large variance).
+        noises: (len(timesteps), B, C, H, W), largest timestep first, or None (device draws from `seed`)."""
+        if sampler not in UB_SAMPLERS:
+            raise UbError(f"sampler must be one of {sorted(UB_SAMPLERS)}, got {sampler!r}")
+        c = self.cfg
+        ts = np.ascontiguousarray(timesteps, dtype=np.int32).reshape(-1)
+        x_init = None if x_init is None else np.ascontiguousarray(x_init, dtype=np.float32)
+        noises = None if noises is None else np.ascontiguousarray(noises, dtype=np.float32)
+        img = c.B * c.C_in * c.H * c.W
+        if (x_init is not None and x_init.size != img) or (noises is not None and noises.size != ts.size * img):
+            raise UbError(f"x_init must hold {img} values and noises {ts.size} x {img}")
+        out = np.empty((c.B, c.C_in, c.H, c.W), dtype=np.float32)
+        check(lib().ub_trainer_sample_spaced(self._h, ts.ctypes.data_as(C.c_void_p), ts.size, UB_SAMPLERS[sampler],
+                                             float(eta), int(bool(clip_denoised)), _ptr(x_init), _ptr(noises), seed,
+                                             _ptr(out)), "sample_spaced")
         return out
 
     def attach_dp(self, rank: int, world: int, nccl_id: bytes, n_buckets: int = 0):

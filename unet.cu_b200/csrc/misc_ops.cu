@@ -864,6 +864,42 @@ void fill_normal(float* x, size_t n, uint64_t seed, cudaStream_t st) {
     const size_t n4 = n / 4;
     launch_pdl(fill_normal_kernel, dim3(unsigned((n4 + 255) / 256)), dim3(256), 0, st, x, n4, seed);
 }
+// ---- respaced sampling
+__global__ void spaced_set_t_kernel(const int* __restrict__ ts_table, const SpacedState* __restrict__ s, int B,
+                                    float* __restrict__ tsteps) {
+    pdl_entry();
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b < B) tsteps[b] = float(ts_table[s->it]);
+}
+void spaced_set_t(const int* ts_table, const SpacedState* s, int B, float* tsteps, cudaStream_t st) {
+    launch_pdl(spaced_set_t_kernel, dim3((B + 127) / 128), dim3(128), 0, st, ts_table, s, B, tsteps);
+}
+__global__ void spaced_step_kernel(float* __restrict__ x, const float* __restrict__ eps,
+                                   const SpacedRow* __restrict__ rows, const float* __restrict__ z, size_t n4,
+                                   const SpacedState* __restrict__ s) {
+    pdl_entry();
+    const size_t i4 = size_t(blockIdx.x) * blockDim.x + threadIdx.x;
+    if (i4 >= n4) return;
+    const int it = s->it;
+    const SpacedRow c = rows[it];
+    const float4 xv = reinterpret_cast<const float4*>(x)[i4], ev = reinterpret_cast<const float4*>(eps)[i4];
+    float4 zv = make_float4(0.f, 0.f, 0.f, 0.f);
+    if (c.sigma != 0.f) zv = z ? reinterpret_cast<const float4*>(z)[i4] : philox_normal4(i4, 0x5u, uint32_t(it), s->seed);
+    auto upd = [&](float xs, float es, float zs) {
+        float x0 = c.r * xs - c.rm1 * es;
+        if (c.clip != 0.f) x0 = fminf(fmaxf(x0, -1.f), 1.f);
+        return c.c_x0 * x0 + c.c_x * xs + c.sigma * zs;
+    };
+    reinterpret_cast<float4*>(x)[i4] =
+        make_float4(upd(xv.x, ev.x, zv.x), upd(xv.y, ev.y, zv.y), upd(xv.z, ev.z, zv.z), upd(xv.w, ev.w, zv.w));
+}
+void spaced_step(float* x, const float* eps, const SpacedRow* rows, const float* z, size_t n, SpacedState* s,
+                 cudaStream_t st) {
+    const size_t n4 = n / 4;
+    launch_pdl(spaced_step_kernel, dim3(unsigned((n4 + 255) / 256)), dim3(256), 0, st, x, eps, rows, z, n4,
+               static_cast<const SpacedState*>(s));
+    increment_step(&s->it, st);
+}
 
 // Keeps the stream busy for ~`us` microseconds: the profile replay enqueues a whole step behind it, so the per-op
 // CUDA-event intervals measure device time, not how fast the host can submit launches.

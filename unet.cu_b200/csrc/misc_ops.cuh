@@ -80,6 +80,27 @@ void ddpm_step(float* x, const float* eps, const float* betas, const float* sqrt
                const float* z, size_t n, uint64_t seed, int* t_dev, int* it_dev, cudaStream_t st);
 // x ~ N(0,1) (Philox4x32-10, key = seed, stream id 0x2)
 void fill_normal(float* x, size_t n, uint64_t seed, cudaStream_t st);
+
+// ---- respaced sampling (guided-diffusion SpacedDiffusion: ddim_sample_loop / p_sample_loop).  Row `it` holds the
+//      float32 coefficients of loop iteration it (largest timestep first), built by the host in float64; both samplers
+//      share the update
+//        x0 = r * x - rm1 * eps  (clamped to [-1, 1] when clip != 0);   x <- c_x0 * x0 + c_x * x + sigma * z
+//      The iteration counter and the Philox key live in device memory, so one captured graph serves every iteration and
+//      every seed.
+struct SpacedRow {
+    float r, rm1, c_x0, c_x, sigma, clip, pad[2];
+};
+struct SpacedState {
+    int it;
+    int pad;
+    unsigned long long seed;
+};
+// tsteps[b] = float(ts_table[it]) (the model sees the original timestep)
+void spaced_set_t(const int* ts_table, const SpacedState* s, int B, float* tsteps, cudaStream_t st);
+// z: injected noise of this iteration (may be null: Philox(seed, stream id 0x5, counter = it)); no draw where sigma = 0.
+// Then it <- it + 1.
+void spaced_step(float* x, const float* eps, const SpacedRow* rows, const float* z, size_t n, SpacedState* s,
+                 cudaStream_t st);
 // occupy the stream for ~us microseconds (profiling aid: lets the host queue work ahead of the device)
 void stream_delay(unsigned us, cudaStream_t st);
 

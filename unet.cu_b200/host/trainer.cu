@@ -6,6 +6,7 @@
 #include <cuda_runtime.h>
 #include <dlfcn.h>
 
+#include <cctype>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -150,6 +151,13 @@ struct UbTrainer {
     cudaGraphExec_t samp_graph = nullptr;
     bool samp_graph_noise = false;
     float* samp_z = nullptr;  // injected noise of the current iteration (graph reads a fixed address)
+    // respaced sampling (ub_trainer_sample_spaced): coefficient rows and original timesteps of every iteration
+    // (n_timesteps rows at most), the device-side iteration counter + seed, and the graph of one iteration
+    SpacedRow* spaced_rows = nullptr;
+    int* spaced_ts = nullptr;
+    SpacedState* spaced_state = nullptr;
+    cudaGraphExec_t spaced_graph = nullptr;
+    bool spaced_graph_noise = false;
     int* step_dev = nullptr;
     float* h_loss = nullptr;  // pinned
     // Host batches are staged through the trainer's OWN page-locked double buffer: the caller's buffer (pageable or
@@ -771,6 +779,9 @@ int Builder::build() {
     T->sqrt_ac = f32(c.n_timesteps), T->sqrt_1mac = f32(c.n_timesteps), T->betas = f32(c.n_timesteps);
     T->samp_state = (int*)T->arena.alloc(256);
     T->samp_z = f32(size_t(B) * img);
+    T->spaced_rows = (SpacedRow*)T->arena.alloc(size_t(c.n_timesteps) * sizeof(SpacedRow));
+    T->spaced_ts = (int*)T->arena.alloc(size_t(c.n_timesteps) * sizeof(int));
+    T->spaced_state = (SpacedState*)T->arena.alloc(sizeof(SpacedState));
     T->step_dev = (int*)T->arena.alloc(256);
     T->hp_dev = f32(8);
     T->loss = zf32(64);
@@ -1280,6 +1291,7 @@ extern "C" void ub_trainer_destroy(UbTrainer* t) {
     cudaDeviceSynchronize();
     if (t->graph_exec) cudaGraphExecDestroy(t->graph_exec);
     if (t->samp_graph) cudaGraphExecDestroy(t->samp_graph);
+    if (t->spaced_graph) cudaGraphExecDestroy(t->spaced_graph);
     if (t->comm && nccl().ok) nccl().CommDestroy(t->comm);
     if (t->params) cudaFree(t->params);
     if (t->ema) cudaFree(t->ema);
@@ -1798,6 +1810,200 @@ extern "C" int ub_trainer_sample(UbTrainer* t, const float* x_init_host, int t_s
                                      cudaMemcpyHostToDevice, st));
         CUDA_TRY(cudaGraphLaunch(t->samp_graph, st));
         ub_count_launches((unsigned long long)(t->launches_fwd + 3));
+    }
+    CUDA_TRY(cudaMemcpyAsync(out_host, t->xt, img * sizeof(float), cudaMemcpyDeviceToHost, st));
+    CUDA_TRY(cudaStreamSynchronize(st));
+    return UB_OK;
+}
+
+// guided-diffusion respace.space_timesteps (see include/unet_b200.h).  The section strides accumulate in float64 and
+// round half to even (nearbyint in the default rounding mode), as Python's `cur_idx += frac_stride; round(cur_idx)`.
+extern "C" int ub_space_timesteps(int n_timesteps, const char* spec, int* out, int cap) {
+    const int T = n_timesteps;
+    if (T < 1 || !spec || !out) {
+        set_err("space_timesteps: needs n_timesteps >= 1, a spec and an output buffer");
+        return UB_ERR_SHAPE;
+    }
+    // a non-negative decimal integer with optional surrounding blanks, ending at `end` (Python's int() on one field)
+    auto parse = [](const char* b, const char* end, long& v) {
+        while (b < end && isspace((unsigned char)*b)) ++b;
+        while (end > b && isspace((unsigned char)end[-1])) --end;
+        if (b < end && *b == '+') ++b;
+        if (b == end || end - b > 9) return false;
+        v = 0;
+        for (; b < end; ++b) {
+            if (*b < '0' || *b > '9') return false;
+            v = v * 10 + (*b - '0');
+        }
+        return true;
+    };
+    std::vector<int> steps;
+    const char* s_end = spec + strlen(spec);
+    if (strncmp(spec, "ddim", 4) == 0) {
+        long want = 0;
+        if (!parse(spec + 4, s_end, want)) {
+            set_err("space_timesteps: malformed spec '%s'", spec);
+            return UB_ERR_SHAPE;
+        }
+        for (int i = 1; i < T && steps.empty(); ++i)
+            if ((T + i - 1) / i == want)
+                for (int k = 0; k < T; k += i) steps.push_back(k);
+        if (steps.empty()) {
+            set_err("space_timesteps: cannot create exactly %ld steps out of %d with an integer stride", want, T);
+            return UB_ERR_SHAPE;
+        }
+    } else {
+        std::vector<long> counts;
+        for (const char* b = spec;;) {
+            const char* e = strchr(b, ',');
+            if (!e) e = s_end;
+            long v = 0;
+            if (!parse(b, e, v)) {
+                set_err("space_timesteps: malformed spec '%s'", spec);
+                return UB_ERR_SHAPE;
+            }
+            counts.push_back(v);
+            if (e == s_end) break;
+            b = e + 1;
+        }
+        const int k = int(counts.size()), size_per = T / k, extra = T % k;
+        for (int i = 0, start = 0; i < k; ++i) {
+            const int size = size_per + (i < extra ? 1 : 0);
+            if (counts[i] > size) {
+                set_err("space_timesteps: cannot divide a section of %d steps into %ld", size, counts[i]);
+                return UB_ERR_SHAPE;
+            }
+            const double frac = counts[i] <= 1 ? 1.0 : double(size - 1) / double(counts[i] - 1);
+            double cur = 0.0;
+            for (long j = 0; j < counts[i]; ++j, cur += frac) steps.push_back(start + int(nearbyint(cur)));
+            start += size;
+        }
+        std::sort(steps.begin(), steps.end());
+        steps.erase(std::unique(steps.begin(), steps.end()), steps.end());
+        if (steps.empty()) {
+            set_err("space_timesteps: spec '%s' keeps no timestep", spec);
+            return UB_ERR_SHAPE;
+        }
+    }
+    if (int(steps.size()) > cap) {
+        set_err("space_timesteps: %zu timesteps do not fit the output buffer of %d", steps.size(), cap);
+        return UB_ERR_SHAPE;
+    }
+    std::copy(steps.begin(), steps.end(), out);
+    return int(steps.size());
+}
+
+// Coefficient rows of ub_trainer_sample_spaced in loop order (row k = spaced index n-1-k), from guided-diffusion's
+// SpacedDiffusion + GaussianDiffusion tables in float64: the linear betas of the trainer's schedule, acp = cumprod(1 -
+// beta), then beta'_i = 1 - acp[t_i] / acp[t_{i-1}] over the kept timesteps and the tables of that respaced chain.
+static void spaced_rows(int T, const int* ts, int n, int sampler, double eta, int clip, SpacedRow* rows) {
+    std::vector<double> acp(T);
+    const double scale = 1000.0 / T, b0 = scale * 0.0001, b1 = scale * 0.02, step = T > 1 ? (b1 - b0) / (T - 1) : 0.0;
+    double ac = 1.0;
+    for (int i = 0; i < T; ++i) {  // numpy.linspace: start + i * step, the last point exactly `stop`
+        const double beta = (T > 1 && i == T - 1) ? b1 : b0 + double(i) * step;
+        acp[i] = ac = ac * (1.0 - beta);
+    }
+    std::vector<double> bp(n), ap(n);  // beta', acp' of the respaced chain
+    double last = 1.0, cum = 1.0;
+    for (int i = 0; i < n; ++i) {
+        bp[i] = 1.0 - acp[ts[i]] / last;
+        last = acp[ts[i]];
+        ap[i] = cum = cum * (1.0 - bp[i]);
+    }
+    for (int i = 0; i < n; ++i) {
+        const double a = ap[i], a_prev = i ? ap[i - 1] : 1.0, r = sqrt(1.0 / a), rm1 = sqrt(1.0 / a - 1.0);
+        double c_x0, c_x, sigma;
+        if (sampler == UB_SAMPLER_ANCESTRAL) {  // q_posterior mean; fixed-large variance [post_var[1], beta'[1:]]
+            c_x0 = bp[i] * sqrt(a_prev) / (1.0 - a);
+            c_x = (1.0 - a_prev) * sqrt(1.0 - bp[i]) / (1.0 - a);
+            sigma = i ? sqrt(bp[i]) : 0.0;
+        } else {  // x0 * sqrt(a_prev) + k * eps', eps' = (r x - x0) / rm1, k = sqrt(1 - a_prev - sigma^2)
+            sigma = eta * sqrt((1.0 - a_prev) / (1.0 - a)) * sqrt(1.0 - a / a_prev);
+            const double k = sqrt(std::max(0.0, 1.0 - a_prev - sigma * sigma));
+            c_x0 = sqrt(a_prev) - k / rm1;
+            c_x = k * r / rm1;
+            if (!i) sigma = 0.0;
+        }
+        SpacedRow& w = rows[n - 1 - i];
+        w = SpacedRow{float(r), float(rm1), float(c_x0), float(c_x), float(sigma), clip ? 1.f : 0.f, {0.f, 0.f}};
+    }
+}
+
+// guided-diffusion ddim_sample_loop / p_sample_loop over a respaced schedule (see include/unet_b200.h)
+extern "C" int ub_trainer_sample_spaced(UbTrainer* t, const int* timesteps, int n, int sampler, float eta,
+                                        int clip_denoised, const float* x_init_host, const float* noise_host,
+                                        unsigned long long seed, float* out_host) {
+    CUDA_TRY(cudaSetDevice(t->device));
+    const UbConfig& c = t->cfg;
+    if (c.C_in != c.C_out) {
+        set_err("sampling needs C_in == C_out");
+        return UB_ERR_SHAPE;
+    }
+    if (sampler != UB_SAMPLER_DDIM && sampler != UB_SAMPLER_ANCESTRAL) {
+        set_err("sampler must be UB_SAMPLER_DDIM (0) or UB_SAMPLER_ANCESTRAL (1), got %d", sampler);
+        return UB_ERR_SHAPE;
+    }
+    if (sampler == UB_SAMPLER_DDIM ? !(eta >= 0.f && eta <= 1.f) : eta != 0.f) {
+        set_err("eta must lie in [0, 1] for DDIM and be 0 for ancestral sampling, got %g", double(eta));
+        return UB_ERR_SHAPE;
+    }
+    const int n_min = sampler == UB_SAMPLER_ANCESTRAL ? 2 : 1;  // the fixed-large variance reads post_var[1]
+    if (!timesteps || n < n_min || n > c.n_timesteps) {
+        set_err("sampling needs %d to %d timesteps, got %d", n_min, c.n_timesteps, timesteps ? n : 0);
+        return UB_ERR_SHAPE;
+    }
+    for (int i = 0; i < n; ++i)
+        if (timesteps[i] < 0 || timesteps[i] >= c.n_timesteps || (i && timesteps[i] <= timesteps[i - 1])) {
+            set_err("timesteps must be strictly ascending in [0, %d): entry %d is %d", c.n_timesteps, i, timesteps[i]);
+            return UB_ERR_SHAPE;
+        }
+    std::vector<SpacedRow> rows(n);
+    spaced_rows(c.n_timesteps, timesteps, n, sampler, double(eta), clip_denoised, rows.data());
+    std::vector<int> ts(timesteps, timesteps + n);
+    std::reverse(ts.begin(), ts.end());
+    const size_t img = size_t(c.B) * c.C_in * c.H * c.W;
+    cudaStream_t st = t->stream;
+    if (x_init_host)
+        CUDA_TRY(cudaMemcpyAsync(t->xt, x_init_host, img * sizeof(float), cudaMemcpyHostToDevice, st));
+    else
+        fill_normal(t->xt, img, seed, st);
+    const SpacedState state{0, 0, seed};
+    CUDA_TRY(cudaMemcpyAsync(t->spaced_state, &state, sizeof state, cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(t->spaced_rows, rows.data(), n * sizeof(SpacedRow), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemcpyAsync(t->spaced_ts, ts.data(), n * sizeof(int), cudaMemcpyHostToDevice, st));
+    CUDA_TRY(cudaMemsetAsync(t->noise, 0, img * sizeof(float), st));  // (the forward tape ends with the MSE vs noise)
+    const bool inject = noise_host != nullptr;
+    if (!t->spaced_graph || t->spaced_graph_noise != inject) {
+        if (t->spaced_graph) cudaGraphExecDestroy(t->spaced_graph), t->spaced_graph = nullptr;
+        cudaGraph_t graph = nullptr;
+        CUDA_TRY(cudaStreamSynchronize(st));
+        CUDA_TRY(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
+        cudaMemsetAsync(t->zero_base, 0, t->zero_bytes, st);
+        spaced_set_t(t->spaced_ts, t->spaced_state, c.B, t->tsteps, st);
+        if (t->drop_ctl) dropout_set_ctl(t->drop_ctl, 0.f, c.seed, t->step_dev, st);  // inference: no dropout
+        for (auto& op : t->fwd_ops) op(st);
+        spaced_step(t->xt, t->out, t->spaced_rows, inject ? t->samp_z : nullptr, img, t->spaced_state, st);
+        cudaError_t e = cudaStreamEndCapture(st, &graph);
+        if (e != cudaSuccess || !graph) {
+            set_err("sampling graph capture failed: %s", cudaGetErrorString(e));
+            return UB_ERR_CUDA;
+        }
+        e = cudaGraphInstantiate(&t->spaced_graph, graph, 0);
+        cudaGraphDestroy(graph);
+        if (e != cudaSuccess) {
+            set_err("sampling graph instantiate failed: %s", cudaGetErrorString(e));
+            return UB_ERR_CUDA;
+        }
+        t->spaced_graph_noise = inject;
+    }
+    const unsigned long long launches = t->launches_fwd + 3 + (t->drop_ctl ? 1 : 0);
+    for (int it = 0; it < n; ++it) {
+        if (inject)
+            CUDA_TRY(cudaMemcpyAsync(t->samp_z, noise_host + size_t(it) * img, img * sizeof(float),
+                                     cudaMemcpyHostToDevice, st));
+        CUDA_TRY(cudaGraphLaunch(t->spaced_graph, st));
+        ub_count_launches(launches);
     }
     CUDA_TRY(cudaMemcpyAsync(out_host, t->xt, img * sizeof(float), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
