@@ -413,7 +413,7 @@ int ub_trainer_profile(UbTrainer* t, int reps, UbProfile* out);
 /* ---- data parallel (SURVEY.md section 8e): one process per GPU; rank 0 creates the id, everyone attaches ---- */
 #define UB_NCCL_ID_BYTES 128
 int ub_nccl_get_unique_id(void* id_out /* UB_NCCL_ID_BYTES */);
-/* n_buckets: 0 = the library's bucket count (8 + a tail bucket, fixed when the trainer is built; UB_BUCKETS overrides) */
+/* n_buckets: 0 = the library's bucket count (8 + a tail bucket, fixed when the trainer is built) */
 int ub_trainer_attach_dp(UbTrainer* t, int rank, int world, const void* nccl_id, int n_buckets);
 
 #ifdef __cplusplus

@@ -291,77 +291,73 @@ static bool test_wgrad(int B, int H, int W, int Cin, int Cout, int ntaps, int ns
         ms /= reps, ms_red /= reps;
     }
     double flops = 2.0 * npix * Cout * double(ntaps) * Cin;
-    printf("wgrad B%d %dx%d %d->%d taps%d | MO=%d NC=%d TC=%d split=%d stages=%d | checked %zu bad %d max_err %.3g "
+    printf("wgrad B%d %dx%d %d->%d taps%d | %s MO=%d NC=%d TC=%d split=%d stages=%d | checked %zu bad %d max_err %.3g "
            "(max_ref %.3g) | %.4f ms (+%.4f reduce) %.1f TFLOP/s  %s\n",
-           B, H, W, Cin, Cout, ntaps, p.MO, p.NC, p.TC, p.nsplit, p.stages, ncheck, bad, max_err, max_ref, ms, ms_red,
+           B, H, W, Cin, Cout, ntaps, p.colmode ? "col" : "row", p.MO, p.NC, p.TC, p.nsplit, p.stages, ncheck, bad, max_err,
+           max_ref, ms, ms_red,
            ms > 0 ? flops / ms * 1e-9 : 0.0, bad ? "FAIL" : "ok");
     if (bad) g_fail++;
-    // accumulate mode (the trainer's): every CTA adds its tile into acc[tap][o][c] -- TMA reduce-add boxes (default) and
-    // per-lane REDs (tma_red = 0) -- compared with the two-pass result above, element by element
-    for (int mode = 2; mode >= 0; --mode) {  // 2 = default, 1 = one TMA producer warp, 0 = also per-lane REDs
-        float *dacc, *dbias;
-        CK(cudaMalloc(&dacc, hdw.size() * 4));
-        CK(cudaMalloc(&dbias, size_t(Cout) * 4));
-        CK(cudaMemset(dacc, 0, hdw.size() * 4));
-        CK(cudaMemset(dbias, 0, size_t(Cout) * 4));
-        IgemmWgradParams pa;
-        r = igemm_wgrad_plan_acc(&pa, ddy, Cout, dx_, Cin, B, H, W, Cin, Cout, ntaps, dacc, dbias, nullptr, 148);
-        if (r) {
-            printf("wgrad acc plan failed %d\n", r);
-            g_fail++;
-            return false;
-        }
-        if (mode < 2) pa.nprod = 1;
-        if (!mode) pa.tma_red = 0;
-        r = igemm_wgrad_launch(pa, 0);
-        e = cudaDeviceSynchronize();
-        if (r || e != cudaSuccess) {
-            printf("wgrad acc launch failed r=%d e=%s\n", r, cudaGetErrorString(e));
-            exit(3);
-        }
-        std::vector<float> hacc(hdw.size()), hb(Cout);
-        CK(cudaMemcpy(hacc.data(), dacc, hacc.size() * 4, cudaMemcpyDeviceToHost));
-        CK(cudaMemcpy(hb.data(), dbias, hb.size() * 4, cudaMemcpyDeviceToHost));
-        int bad2 = 0;
-        double me = 0;
-        for (int tap = 0; tap < ntaps; ++tap)
-            for (int o = 0; o < Cout; ++o)
-                for (int c = 0; c < Cin; ++c) {
-                    const double a = hacc[(size_t(tap) * Cout + o) * Cin + c], b = hdw[(size_t(o) * Cin + c) * ntaps + tap];
-                    const double err = fabs(a - b);
-                    if (err > me) me = err;
-                    if (!(err <= 1e-4 * (1.0 + fabs(b)) + 2e-5 * sqrt(double(npix)))) {
-                        if (bad2 < 5) printf("   acc mismatch tap=%d o=%d c=%d got=%f two-pass=%f\n", tap, o, c, a, b);
-                        bad2++;
-                    }
-                }
-        int badb = 0;
-        for (int o = 0; o < Cout; ++o) {  // bias gradient = column sums of dY
-            double sref = 0;
-            for (size_t px = 0; px < npix; ++px) sref += dy[px * Cout + o];
-            if (!(fabs(hb[o] - sref) <= 1e-3 * (1.0 + fabs(sref)) + 1e-4 * sqrt(double(npix)))) {
-                if (badb < 3) printf("   bias mismatch o=%d got=%f ref=%f\n", o, hb[o], sref);
-                badb++;
-            }
-        }
-        float msa = 0;
-        if (reps > 0) {
-            cudaEvent_t e0, e1;
-            cudaEventCreate(&e0), cudaEventCreate(&e1);
-            for (int i = 0; i < 3; ++i) igemm_wgrad_launch(pa, 0);
-            cudaEventRecord(e0);
-            for (int i = 0; i < reps; ++i) igemm_wgrad_launch(pa, 0);
-            cudaEventRecord(e1);
-            CK(cudaEventSynchronize(e1));
-            cudaEventElapsedTime(&msa, e0, e1);
-            msa /= reps;
-        }
-        printf("   acc mode %-16s max |acc - two-pass| %.3g bad %d bias bad %d | %.4f ms %.1f TFLOP/s  %s\n",
-               mode == 2 ? (pa.nprod == 2 ? "TMA red, 2 prod" : "TMA red, 1 prod*") : mode ? "TMA red, 1 prod" : "lane RED, 1 prod", me, bad2, badb, msa, msa > 0 ? flops / msa * 1e-9 : 0.0,
-               (bad2 || badb) ? "FAIL" : "ok");
-        if (bad2 || badb) g_fail++;
-        cudaFree(dacc), cudaFree(dbias);
+    // accumulate mode (the trainer's): every CTA adds its tile into acc[tap][o][c] with TMA reduce-add boxes --
+    // compared with the two-pass result above, element by element
+    float *dacc, *dbias;
+    CK(cudaMalloc(&dacc, hdw.size() * 4));
+    CK(cudaMalloc(&dbias, size_t(Cout) * 4));
+    CK(cudaMemset(dacc, 0, hdw.size() * 4));
+    CK(cudaMemset(dbias, 0, size_t(Cout) * 4));
+    IgemmWgradParams pa;
+    r = igemm_wgrad_plan_acc(&pa, ddy, Cout, dx_, Cin, B, H, W, Cin, Cout, ntaps, dacc, dbias, nullptr, 148);
+    if (r) {
+        printf("wgrad acc plan failed %d\n", r);
+        g_fail++;
+        return false;
     }
+    r = igemm_wgrad_launch(pa, 0);
+    e = cudaDeviceSynchronize();
+    if (r || e != cudaSuccess) {
+        printf("wgrad acc launch failed r=%d e=%s\n", r, cudaGetErrorString(e));
+        exit(3);
+    }
+    std::vector<float> hacc(hdw.size()), hb(Cout);
+    CK(cudaMemcpy(hacc.data(), dacc, hacc.size() * 4, cudaMemcpyDeviceToHost));
+    CK(cudaMemcpy(hb.data(), dbias, hb.size() * 4, cudaMemcpyDeviceToHost));
+    int bad2 = 0;
+    double me = 0;
+    for (int tap = 0; tap < ntaps; ++tap)
+        for (int o = 0; o < Cout; ++o)
+            for (int c = 0; c < Cin; ++c) {
+                const double a = hacc[(size_t(tap) * Cout + o) * Cin + c], b = hdw[(size_t(o) * Cin + c) * ntaps + tap];
+                const double err = fabs(a - b);
+                if (err > me) me = err;
+                if (!(err <= 1e-4 * (1.0 + fabs(b)) + 2e-5 * sqrt(double(npix)))) {
+                    if (bad2 < 5) printf("   acc mismatch tap=%d o=%d c=%d got=%f two-pass=%f\n", tap, o, c, a, b);
+                    bad2++;
+                }
+            }
+    int badb = 0;
+    for (int o = 0; o < Cout; ++o) {  // bias gradient = column sums of dY
+        double sref = 0;
+        for (size_t px = 0; px < npix; ++px) sref += dy[px * Cout + o];
+        if (!(fabs(hb[o] - sref) <= 1e-3 * (1.0 + fabs(sref)) + 1e-4 * sqrt(double(npix)))) {
+            if (badb < 3) printf("   bias mismatch o=%d got=%f ref=%f\n", o, hb[o], sref);
+            badb++;
+        }
+    }
+    float msa = 0;
+    if (reps > 0) {
+        cudaEvent_t e0, e1;
+        cudaEventCreate(&e0), cudaEventCreate(&e1);
+        for (int i = 0; i < 3; ++i) igemm_wgrad_launch(pa, 0);
+        cudaEventRecord(e0);
+        for (int i = 0; i < reps; ++i) igemm_wgrad_launch(pa, 0);
+        cudaEventRecord(e1);
+        CK(cudaEventSynchronize(e1));
+        cudaEventElapsedTime(&msa, e0, e1);
+        msa /= reps;
+    }
+    printf("   acc mode (TMA reduce-add) max |acc - two-pass| %.3g bad %d bias bad %d | %.4f ms %.1f TFLOP/s  %s\n", me,
+           bad2, badb, msa, msa > 0 ? flops / msa * 1e-9 : 0.0, (bad2 || badb) ? "FAIL" : "ok");
+    if (bad2 || badb) g_fail++;
+    cudaFree(dacc), cudaFree(dbias);
     cudaFree(dx_), cudaFree(ddy), cudaFree(dpart), cudaFree(ddw);
     return bad == 0;
 }
@@ -588,34 +584,33 @@ int main(int argc, char** argv) {
         test_conv(32, 64, 64, 512, 512, 9, 0, OUT_NHWC_BF16, true, false, false, 5000, 5, true);
     }
 wgrad_tests:
-    // column mode (default for 3x3: one halo box per filter column) and row mode (UB_WGRAD_COLMODE=0: three boxes per
-    // filter row); the plan reads the variable on every call
-    for (int colmode = 1; colmode >= 0; --colmode) {
-        setenv("UB_WGRAD_COLMODE", colmode ? "1" : "0", 1);
-        printf("== wgrad, %s mode ==\n", colmode ? "column" : "row");
-        test_wgrad(2, 8, 8, 64, 64, 9, 1 << 20, 0);
-        test_wgrad(5, 8, 8, 64, 64, 9, 1 << 20, 0);     // two images per K tile, the last tile half outside the batch
-        test_wgrad(6, 8, 8, 128, 128, 9, 1 << 20, 0);
-        test_wgrad(2, 16, 16, 128, 128, 9, 20000, 0);
-        test_wgrad(3, 8, 8, 64, 128, 1, 1 << 20, 0);
-        test_wgrad(2, 12, 20, 64, 64, 9, 1 << 20, 0);
-        test_wgrad(3, 20, 12, 64, 64, 9, 1 << 20, 0);
-        test_wgrad(4, 16, 16, 192, 64, 9, 20000, 0);
-        test_wgrad(2, 32, 32, 64, 128, 9, 20000, 0);
-        if (!quick) {
-            int reps = 20;
-            test_wgrad(32, 64, 64, 64, 64, 9, 400, reps);
-            test_wgrad(32, 64, 64, 192, 64, 9, 400, reps);
-            test_wgrad(32, 64, 64, 64, 128, 9, 400, reps);
-            test_wgrad(32, 32, 32, 128, 128, 9, 400, reps);
-            test_wgrad(32, 16, 16, 192, 192, 9, 1000, reps);
-            test_wgrad(32, 8, 8, 256, 256, 9, 2000, reps);
-            test_wgrad(32, 8, 8, 512, 256, 9, 2000, reps);
-            test_wgrad(32, 32, 32, 320, 128, 1, 2000, reps);
-            test_wgrad(32, 64, 64, 256, 256, 9, 200, reps);
-        }
+    // column mode (3x3 layers with W > 4: one halo box per filter column) and row mode (1x1 layers and 3x3 layers with
+    // W <= 4: three boxes per filter row); the plan picks the mode from the shape
+    printf("== wgrad ==\n");
+    test_wgrad(2, 8, 8, 64, 64, 9, 1 << 20, 0);
+    test_wgrad(5, 8, 8, 64, 64, 9, 1 << 20, 0);     // two images per K tile, the last tile half outside the batch
+    test_wgrad(6, 8, 8, 128, 128, 9, 1 << 20, 0);
+    test_wgrad(2, 16, 16, 128, 128, 9, 20000, 0);
+    test_wgrad(3, 8, 8, 64, 128, 1, 1 << 20, 0);
+    test_wgrad(2, 4, 4, 64, 64, 9, 1 << 20, 0);     // 3x3 row mode
+    test_wgrad(3, 4, 2, 128, 64, 9, 1 << 20, 0);
+    test_wgrad(4, 3, 3, 64, 128, 9, 1 << 20, 0);
+    test_wgrad(2, 12, 20, 64, 64, 9, 1 << 20, 0);
+    test_wgrad(3, 20, 12, 64, 64, 9, 1 << 20, 0);
+    test_wgrad(4, 16, 16, 192, 64, 9, 20000, 0);
+    test_wgrad(2, 32, 32, 64, 128, 9, 20000, 0);
+    if (!quick) {
+        int reps = 20;
+        test_wgrad(32, 64, 64, 64, 64, 9, 400, reps);
+        test_wgrad(32, 64, 64, 192, 64, 9, 400, reps);
+        test_wgrad(32, 64, 64, 64, 128, 9, 400, reps);
+        test_wgrad(32, 32, 32, 128, 128, 9, 400, reps);
+        test_wgrad(32, 16, 16, 192, 192, 9, 1000, reps);
+        test_wgrad(32, 8, 8, 256, 256, 9, 2000, reps);
+        test_wgrad(32, 8, 8, 512, 256, 9, 2000, reps);
+        test_wgrad(32, 32, 32, 320, 128, 1, 2000, reps);
+        test_wgrad(32, 64, 64, 256, 256, 9, 200, reps);
     }
-    unsetenv("UB_WGRAD_COLMODE");
     printf("== %s (%d failing groups) ==\n", g_fail ? "FAILED" : "ALL OK", g_fail);
     return g_fail ? 1 : 0;
 }

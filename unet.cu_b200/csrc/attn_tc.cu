@@ -120,7 +120,6 @@ __device__ __forceinline__ bool same_image(const AttnTcParams& p, int r, int c) 
 }
 
 __device__ __forceinline__ void prologue(Smem* sm, uint32_t ncols_tmem, int warp, int lane) {
-    pdl_trigger();
     if (warp == 0 && lane == 0) {
         mbar_init(&sm->bar_load, 1);
         mbar_init(&sm->bar_s, 1);
@@ -158,7 +157,7 @@ __global__ void __launch_bounds__(kThreads) attn_tc_fwd_kernel(const __grid_cons
     const int C = p.NH * HS;
     const uint32_t tm_cols = t.ncols > 128 ? 512 : 256;
     const uint32_t o_col = t.ncols;  // O accumulator behind the scores
-    // head split (HS = 32 only, see attn_hsplit): gridDim.z == 2 and the CTA works on ONE head of its pair
+    // head split (HS = 32 only, see attn_grid): gridDim.z == 2 and the CTA works on ONE head of its pair
     const bool hsplit = HS == 32 && gridDim.z == 2;
     const int h_lo = hsplit ? int(blockIdx.z) : 0, h_hi = hsplit ? int(blockIdx.z) + 1 : HPB;
     prologue(sm, tm_cols, warp, lane);
@@ -303,8 +302,6 @@ __global__ void __launch_bounds__(kThreads) attn_tc_dq_kernel(const __grid_const
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     constexpr int HPB = 64 / HS;  // heads per box
     const int C = p.NH * HS;
-    const bool hsplit = HS == 32 && gridDim.z == 2;  // head split
-    const int h_lo = hsplit ? int(blockIdx.z) : 0, h_hi = hsplit ? int(blockIdx.z) + 1 : HPB;
     prologue(sm, 512, warp, lane);
     const uint32_t tmem = sm->tmem_slot;
     const int nchunk = t.ncols / 128;
@@ -332,7 +329,8 @@ __global__ void __launch_bounds__(kThreads) attn_tc_dq_kernel(const __grid_const
             const uint64_t dK = make_smem_desc_sw128(smem_u32(sK), 16, 1024), dV = make_smem_desc_sw128(smem_u32(sV), 16, 1024);
             const uint64_t dS = make_smem_desc_sw128(smem_u32(sdS), 16, 1024), dKm = make_smem_desc_sw128(smem_u32(sK), 8192, 1024);
             int it = 0;
-            for (int h = h_lo; h < h_hi; ++h) {
+#pragma unroll 1
+            for (int h = 0; h < HPB; ++h) {
                 for (int cc = 0; cc < nchunk; ++cc, ++it) {
                     if (elect_one_sync()) {
 #pragma unroll
@@ -371,7 +369,6 @@ __global__ void __launch_bounds__(kThreads) attn_tc_dq_kernel(const __grid_const
         if (rvalid) {
 #pragma unroll
             for (int h = 0; h < HPB; ++h) {
-                if (h < h_lo || h >= h_hi) continue;
                 const int head = t.hp * HPB + h;
                 const uint4* gp = reinterpret_cast<const uint4*>(p.dout + size_t(gr) * p.lddo + head * HS);
                 const uint4* op = reinterpret_cast<const uint4*>(p.out + size_t(gr) * p.ldo + head * HS);
@@ -390,7 +387,9 @@ __global__ void __launch_bounds__(kThreads) attn_tc_dq_kernel(const __grid_const
             }
         }
         int it = 0;
-        for (int h = h_lo; h < h_hi; ++h) {
+#pragma unroll 1
+        for (int h = 0; h < HPB; ++h) {
+            const float Dh = Dv[h], Lh = Lv[h];  // (read once: indexed in the chunk loop they spill)
             for (int cc = 0; cc < nchunk; ++cc, ++it) {
                 mbar_wait(&sm->bar_s, it & 1);
                 tc_fence_after();
@@ -404,8 +403,8 @@ __global__ void __launch_bounds__(kThreads) attn_tc_dq_kernel(const __grid_const
 #pragma unroll
                     for (int j = 0; j < 32; ++j) {
                         const bool vis = rvalid && same_image<MASK>(p, r, cc * 128 + c0 + j);
-                        const float pr = ex2(fmaf(__uint_as_float(s[j]), c, -Lv[h]));
-                        ds[j] = vis ? pr * (__uint_as_float(d[j]) - Dv[h]) : 0.f;
+                        const float pr = ex2(fmaf(__uint_as_float(s[j]), c, -Lh));
+                        ds[j] = vis ? pr * (__uint_as_float(d[j]) - Dh) : 0.f;
                     }
                     store_row32(sdS, r, c0, ds);
                 }
@@ -415,7 +414,7 @@ __global__ void __launch_bounds__(kThreads) attn_tc_dq_kernel(const __grid_const
             }
             // dQ of this head is complete when the last chunk's MMAs are
             mbar_wait(&sm->bar_o, (it - 1) & 1);
-            if (h == h_hi - 1) pdl_trigger_late();  // all MMAs of this CTA are complete
+            if (h == HPB - 1) pdl_trigger_late();  // all MMAs of this CTA are complete
             tc_fence_after();
             uint32_t o[HS / 2];
             tmem_ld_half(trow + 256 + h * 64 + h * HS + half * (HS / 2), o);
@@ -458,8 +457,6 @@ __global__ void __launch_bounds__(kThreads) attn_tc_dkv_kernel(const __grid_cons
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     constexpr int HPB = 64 / HS;  // heads per box
     const int C = p.NH * HS;
-    const bool hsplit = HS == 32 && gridDim.z == 2;  // head split
-    const int h_lo = hsplit ? int(blockIdx.z) : 0, h_hi = hsplit ? int(blockIdx.z) + 1 : HPB;
     prologue(sm, 512, warp, lane);
     const uint32_t tmem = sm->tmem_slot;
     const int nchunk = t.ncols / 128;
@@ -489,7 +486,8 @@ __global__ void __launch_bounds__(kThreads) attn_tc_dkv_kernel(const __grid_cons
             const uint64_t dPt = make_smem_desc_sw128(smem_u32(sPt), 16, 1024), dSt = make_smem_desc_sw128(smem_u32(sdSt), 16, 1024);
             const uint64_t dQm = make_smem_desc_sw128(smem_u32(sQ), 8192, 1024), dGm = make_smem_desc_sw128(smem_u32(sdO), 8192, 1024);
             int it = 0;
-            for (int h = h_lo; h < h_hi; ++h) {
+#pragma unroll 1
+            for (int h = 0; h < HPB; ++h) {
                 for (int cc = 0; cc < nchunk; ++cc, ++it) {
                     if (elect_one_sync()) {
 #pragma unroll
@@ -550,7 +548,8 @@ __global__ void __launch_bounds__(kThreads) attn_tc_dkv_kernel(const __grid_cons
         }
         asm volatile("bar.sync 1, 256;" ::: "memory");
         int it = 0;
-        for (int h = h_lo; h < h_hi; ++h) {
+#pragma unroll 1
+        for (int h = 0; h < HPB; ++h) {
             for (int cc = 0; cc < nchunk; ++cc, ++it) {
                 mbar_wait(&sm->bar_s, it & 1);
                 tc_fence_after();
@@ -579,7 +578,7 @@ __global__ void __launch_bounds__(kThreads) attn_tc_dkv_kernel(const __grid_cons
                 mbar_arrive(&sm->bar_p);
             }
             mbar_wait(&sm->bar_o, (it - 1) & 1);
-            if (h == h_hi - 1) pdl_trigger_late();  // all MMAs of this CTA are complete
+            if (h == HPB - 1) pdl_trigger_late();  // all MMAs of this CTA are complete
             tc_fence_after();
             uint32_t dk[HS / 2], dv[HS / 2];
             tmem_ld_half(trow + 256 + h * 64 + h * HS + half * (HS / 2), dk);
@@ -672,25 +671,22 @@ int attn_tc_plan(AttnTcParams* p, const __nv_bfloat16* qkv, int ld, int B, int T
     return r;
 }
 
-// Head split (UB_ATTN_HSPLIT bit mask: 1 forward, 2 dq, 4 dkv; default 1), HS = 32 only: a CTA owns 128 rows x a PAIR
-// of heads (one 64-channel box) and works through the two heads one after the other; with the split the pair is shared
-// by two CTAs (grid z) that each load the box and take one head.  T = 256: 192 one-per-SM CTAs are two waves on 148
-// SMs, 384 half CTAs are three half-waves; T = 64: 64 CTAs become 128.  At HS = 64 a box is one head: nothing to split.
-static int attn_hsplit() {
-    static const int v = getenv("UB_ATTN_HSPLIT") ? atoi(getenv("UB_ATTN_HSPLIT")) : 1;
-    return v;
-}
-static dim3 attn_grid(const AttnTcParams& p, int bit) {
-    return dim3((p.B * p.T + 127) / 128, p.NH * p.HS / 64, (p.HS == 32 && (attn_hsplit() & bit)) ? 2 : 1);
-}
+// Head split of the forward kernel, HS = 32 only: a CTA owns 128 rows x a PAIR of heads (one 64-channel box); with the
+// split the pair is shared by two CTAs (grid z = 2) that each load the box and take one head.  T = 256: 192
+// one-per-SM CTAs are two waves on 148 SMs, 384 half CTAs are three half-waves; T = 64: 64 CTAs become 128.  The dq
+// and dkv kernels work through both heads of the pair (split: measured, removed, profiles/r02_attn_hsplit.txt).  At
+// HS = 64 a box is one head: nothing to split.
+static dim3 attn_grid(const AttnTcParams& p, int z) { return dim3((p.B * p.T + 127) / 128, p.NH * p.HS / 64, z); }
 static int attn_ncols(const AttnTcParams& p) { return p.T >= 128 ? p.T : 128; }
 
 template <int HS>
 static void attn_tc_fwd_hs(const AttnTcParams& p, cudaStream_t st) {
     if (p.T >= 128)
-        launch_pdl(attn_tc_fwd_kernel<HS, false>, dim3(attn_grid(p, 1)), dim3(kThreads), smem_fwd(attn_ncols(p)), st, p);
+        launch_pdl(attn_tc_fwd_kernel<HS, false>, dim3(attn_grid(p, HS == 32 ? 2 : 1)), dim3(kThreads),
+                   smem_fwd(attn_ncols(p)), st, p);
     else
-        launch_pdl(attn_tc_fwd_kernel<HS, true>, dim3(attn_grid(p, 1)), dim3(kThreads), smem_fwd(attn_ncols(p)), st, p);
+        launch_pdl(attn_tc_fwd_kernel<HS, true>, dim3(attn_grid(p, HS == 32 ? 2 : 1)), dim3(kThreads),
+                   smem_fwd(attn_ncols(p)), st, p);
 }
 
 int attn_tc_fwd(const AttnTcParams& p, cudaStream_t st) {
@@ -705,11 +701,11 @@ int attn_tc_fwd(const AttnTcParams& p, cudaStream_t st) {
 template <int HS>
 static void attn_tc_bwd_hs(const AttnTcParams& p, cudaStream_t st, cudaStream_t s2) {
     if (p.T >= 128) {
-        launch_pdl(attn_tc_dkv_kernel<HS, false>, dim3(attn_grid(p, 4)), dim3(kThreads), smem_dkv(attn_ncols(p)), s2, p);
-        launch_pdl(attn_tc_dq_kernel<HS, false>, dim3(attn_grid(p, 2)), dim3(kThreads), smem_dq(attn_ncols(p)), st, p);
+        launch_pdl(attn_tc_dkv_kernel<HS, false>, dim3(attn_grid(p, 1)), dim3(kThreads), smem_dkv(attn_ncols(p)), s2, p);
+        launch_pdl(attn_tc_dq_kernel<HS, false>, dim3(attn_grid(p, 1)), dim3(kThreads), smem_dq(attn_ncols(p)), st, p);
     } else {
-        launch_pdl(attn_tc_dkv_kernel<HS, true>, dim3(attn_grid(p, 4)), dim3(kThreads), smem_dkv(attn_ncols(p)), s2, p);
-        launch_pdl(attn_tc_dq_kernel<HS, true>, dim3(attn_grid(p, 2)), dim3(kThreads), smem_dq(attn_ncols(p)), st, p);
+        launch_pdl(attn_tc_dkv_kernel<HS, true>, dim3(attn_grid(p, 1)), dim3(kThreads), smem_dkv(attn_ncols(p)), s2, p);
+        launch_pdl(attn_tc_dq_kernel<HS, true>, dim3(attn_grid(p, 1)), dim3(kThreads), smem_dq(attn_ncols(p)), st, p);
     }
 }
 

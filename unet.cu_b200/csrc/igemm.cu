@@ -180,7 +180,6 @@ __device__ __forceinline__ void conv_produce_loop(const IgemmConvParams& p, int 
 // two-CTA kernel at 80 registers; the spilling epilogue cost more in the step than the main loop won.)
 template <int NACC, bool MS = false>
 __device__ __forceinline__ void igemm_conv_body(const IgemmConvParams& p) {
-    pdl_trigger();
 #ifdef UB_TRACE
     if (threadIdx.x == 0) {
         unsigned smid;
@@ -275,10 +274,7 @@ __device__ __forceinline__ void igemm_conv_body(const IgemmConvParams& p) {
         {
 #endif
             // two-stream kernels (one CTA per SM): a second producer (warp 8, see below) takes the odd K blocks
-            if (NACC == 2 && p.nprod == 2)
-                conv_produce_loop<2>(p, 0, nk, smem, full_bar, empty_bar, w0, h0, b0, n0);
-            else
-                conv_produce_loop<1>(p, 0, nk, smem, full_bar, empty_bar, w0, h0, b0, n0);
+            conv_produce_loop<NACC>(p, 0, nk, smem, full_bar, empty_bar, w0, h0, b0, n0);
             UB_TR(5, (unsigned long long)clock64());
         }
     } else if (warp == 1) {
@@ -289,7 +285,7 @@ __device__ __forceinline__ void igemm_conv_body(const IgemmConvParams& p) {
         if constexpr (NACC == 2) {  // second MMA stream first; the warp reconverges before it touches the epilogue
             if (warp == 9) conv_issue_loop<NACC>(p, 1, nk, smem, full_bar, empty_bar, tmem_full_bar, tmem_base);
             // ... and the second TMA producer (odd K blocks) on another epilogue warp that idles during the main loop
-            if (warp == 8 && p.nprod == 2) {
+            if (warp == 8) {
 #ifdef UB_TRACE
                 if (g_conv_dbg_mode < 2)
 #endif
@@ -466,7 +462,7 @@ __global__ void __launch_bounds__(kConvThreads, 2) igemm_conv_kernel(const __gri
 __global__ void __launch_bounds__(kConvThreads, 1) igemm_conv2_kernel(const __grid_constant__ IgemmConvParams p) {
     igemm_conv_body<2>(p);
 }
-// tensor-core GroupNorm statistics + TMA output store (UB_EPI_MMA=0 disables), see IgemmConvParams::ms
+// tensor-core GroupNorm statistics + TMA output store, see IgemmConvParams::ms
 __global__ void __launch_bounds__(kConvThreads, 2) igemm_conv_ms_kernel(const __grid_constant__ IgemmConvParams p) {
     igemm_conv_body<1, true>(p);
 }
@@ -478,7 +474,6 @@ __global__ void __launch_bounds__(kConvThreads, 1) igemm_conv2_ms_kernel(const _
 // wgrad: both operands MN-major (the contraction index is the pixel index, channels are contiguous)
 // =====================================================================================================
 __global__ void __launch_bounds__(kWgradThreads) igemm_wgrad_kernel(const __grid_constant__ IgemmWgradParams p) {
-    pdl_trigger();
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     const uint32_t atom = uint32_t(p.KP) * 128u;  // one 64-channel operand atom: KP pixel rows of 128 B
@@ -517,7 +512,7 @@ __global__ void __launch_bounds__(kWgradThreads) igemm_wgrad_kernel(const __grid
     if (warp == 0 && lane == 0) {
         tma_prefetch_desc(&p.tmDY);
         tma_prefetch_desc(&p.tmX);
-        if (p.tma_red) tma_prefetch_desc(&p.tmAcc);
+        if (p.acc) tma_prefetch_desc(&p.tmAcc);
         for (int i = 0; i < p.stages; ++i) {
             mbar_init(&full_bar[i], 1);
             mbar_init(&empty_bar[i], 1);
@@ -535,47 +530,46 @@ __global__ void __launch_bounds__(kWgradThreads) igemm_wgrad_kernel(const __grid
     const uint32_t tmem_base = *tmem_slot;
     pdl_wait();  // everything above touched only kernel parameters, shared memory and TMEM
 
-    if (warp == 0 || (warp == 2 && p.nprod == 2)) {
-        // TMA producer(s) (whole warp converged, TMA instructions under elect.sync: see elect_one_sync in ptx.cuh).
-        // With nprod == 2 (opt-in) the first epilogue warp -- idle until the accumulator is complete -- issues the odd
-        // K tiles: two producers lift single-box stages from ~52 to ~68 B/clk per SM (tools/tma_ingest_bench.cu), but
-        // these stages hold 3-8 boxes and one producer already reaches ~72, so it measured no gain here.
-        // Stage and phase follow from the tile index, so the producers share no state; the ring is EVEN in that case
-        // (plan), so a stage always belongs to the same producer and it waits for consecutive phases of its barriers.
-        {
-            const int step = p.nprod == 2 ? 2 : 1;
-            for (int kt = k_begin + (warp == 0 ? 0 : 1); kt < k_end; kt += step) {
-                const int kl = kt - k_begin;
-                const int stage = kl % p.stages;
-                const uint32_t phase = uint32_t(kl / p.stages) & 1u;
-                int t = kt;
-                const int w0 = (t % p.tiles_w) * p.TW;
-                t /= p.tiles_w;
-                const int h0 = (t % p.tiles_h) * p.TH;
-                const int b0 = (t / p.tiles_h) * p.TB;
-                mbar_wait(&empty_bar[stage], phase ^ 1);
-                uint8_t* sA = smem + size_t(stage) * p.stage_bytes;
-                uint8_t* sB = sA + b_off;
-                if (elect_one_sync()) {
-                    mbar_expect_tx(&full_bar[stage], p.tx_bytes);
-                    for (int a = 0; a < a_atoms; ++a)
-                        tma_load_4d(sA + a * atom, &p.tmDY, &full_bar[stage], o0 + a * 64, w0, h0, b0);
-                    if (colmode) {  // one (TH + 2)-row halo box per 64-channel atom, shifted by this CTA's dx
-                        for (int nb = 0; nb < b_atoms; ++nb)
-                            tma_load_4d(sB + nb * p.hatom, &p.tmX, &full_bar[stage], c0 + nb * 64,
-                                        w0 + int(blockIdx.y) - 1, h0 - 1, b0);
-                    } else
-                    for (int ti = 0; ti < p.TC; ++ti) {
-                        const int tap = tap0 + ti;
-                        const int dy = p.ntaps == 9 ? tap / 3 - 1 : 0;
-                        const int dx = p.ntaps == 9 ? tap % 3 - 1 : 0;
-                        for (int nb = 0; nb < b_atoms; ++nb)
-                            tma_load_4d(sB + (ti * b_atoms + nb) * atom, &p.tmX, &full_bar[stage], c0 + nb * 64, w0 + dx,
-                                        h0 + dy, b0);
-                    }
+    if (warp == 0) {
+        // TMA producer (whole warp converged, TMA instructions under elect.sync: see elect_one_sync in ptx.cuh).
+        // One producer: two lift single-box stages from ~52 to ~68 B/clk per SM (tools/tma_ingest_bench.cu), but these
+        // stages hold 3-8 boxes and one producer already reaches ~72 -- a second producer warp measured no gain here
+        // (measured, removed: profiles/r02n_wgrad_tma_red.txt).
+        for (int kt = k_begin; kt < k_end; ++kt) {
+            const int kl = kt - k_begin;
+            const int stage = kl % p.stages;
+            const uint32_t phase = uint32_t(kl / p.stages) & 1u;
+            int t = kt;
+            const int w0 = (t % p.tiles_w) * p.TW;
+            t /= p.tiles_w;
+            const int h0 = (t % p.tiles_h) * p.TH;
+            const int b0 = (t / p.tiles_h) * p.TB;
+            mbar_wait(&empty_bar[stage], phase ^ 1);
+            uint8_t* sA = smem + size_t(stage) * p.stage_bytes;
+            uint8_t* sB = sA + b_off;
+            if (elect_one_sync()) {
+                mbar_expect_tx(&full_bar[stage], p.tx_bytes);
+                // (the atom loops stay rolled: unrolled, they cost the kernel 700 instructions and 52 uniform-register
+                //  spills to registers)
+#pragma unroll 1
+                for (int a = 0; a < a_atoms; ++a)
+                    tma_load_4d(sA + a * atom, &p.tmDY, &full_bar[stage], o0 + a * 64, w0, h0, b0);
+                if (colmode) {  // one (TH + 2)-row halo box per 64-channel atom, shifted by this CTA's dx
+#pragma unroll 1
+                    for (int nb = 0; nb < b_atoms; ++nb)
+                        tma_load_4d(sB + nb * p.hatom, &p.tmX, &full_bar[stage], c0 + nb * 64,
+                                    w0 + int(blockIdx.y) - 1, h0 - 1, b0);
+                } else
+                for (int ti = 0; ti < p.TC; ++ti) {
+                    const int tap = tap0 + ti;
+                    const int dy = p.ntaps == 9 ? tap / 3 - 1 : 0;
+                    const int dx = p.ntaps == 9 ? tap % 3 - 1 : 0;
+                    for (int nb = 0; nb < b_atoms; ++nb)
+                        tma_load_4d(sB + (ti * b_atoms + nb) * atom, &p.tmX, &full_bar[stage], c0 + nb * 64, w0 + dx,
+                                    h0 + dy, b0);
                 }
-                __syncwarp();
             }
+            __syncwarp();
         }
     }
     if (warp == 1) {
@@ -669,14 +663,15 @@ __global__ void __launch_bounds__(kWgradThreads) igemm_wgrad_kernel(const __grid
         mbar_wait(tmem_full_bar, 0);
         pdl_trigger_late();  // main loop complete: the next kernel's prologue may overlap this epilogue
         tc_fence_after();
-        if (k_end > k_begin && p.tma_red) {
+        if (k_end > k_begin && p.acc) {
             // Accumulate mode through the TMA: thread = accumulator row, so a per-lane RED (or store) instruction touches
             // 32 different lines and the LSU takes one pass per lane -- 12 288 passes for a 128 x 384 tile, ~6 us, the
-            // largest phase of the low-resolution launches.  Instead every warp stages 32 columns of its MO/4 rows in
-            // the idle operand ring (fp32 rows of 128 B, 16-byte chunks XOR-swizzled with the row: conflict-free
-            // STS.128 and the layout a SWIZZLE_128B box expects) and one elected lane issues a reduce-add box per
-            // (tap, 32 columns); the L2 adds whole lines.  Warps are independent: each owns a slice of the ring and
-            // re-uses a buffer only after its bulk group has read it.
+            // largest phase of the low-resolution launches (per-lane red.global.add: 1.31 ms per step for the weight
+            // gradients against 1.19; measured, removed: profiles/r02n_wgrad_tma_red.txt).  Instead every warp stages
+            // 32 columns of its MO/4 rows in the idle operand ring (fp32 rows of 128 B, 16-byte chunks XOR-swizzled
+            // with the row: conflict-free STS.128 and the layout a SWIZZLE_128B box expects) and one elected lane
+            // issues a reduce-add box per (tap, 32 columns); the L2 adds whole lines.  Warps are independent: each
+            // owns a slice of the ring and re-uses a buffer only after its bulk group has read it.
             const int rpw = p.MO >> 2;  // accumulator rows of this warp: TMEM lanes 32q .. 32q + rpw - 1
             const uint32_t bufbytes = uint32_t(rpw) * 128u;
             const int nsub = p.NC >> 5, ntile = p.TC * nsub;
@@ -715,31 +710,21 @@ __global__ void __launch_bounds__(kWgradThreads) igemm_wgrad_kernel(const __grid
             }
             if (elect_one_sync()) bulk_wait_group0();  // (the same lane committed every group: elect.sync is deterministic)
             __syncwarp();
-        } else if (k_end > k_begin) {
+        } else if (k_end > k_begin) {  // two-pass mode: this split's partial sums, reduced by wgrad_reduce_kernel
             for (int ti = 0; ti < p.TC; ++ti) {
                 const int tap = colmode ? 3 * ti + int(blockIdx.y) : tap0 + ti;
-                float* dst = p.acc ? p.acc + (size_t(tap) * p.Cout + (o0 + row)) * p.Cin + c0
-                                   : p.partial + ((size_t(split) * p.ntaps + tap) * p.Cout + (o0 + row)) * p.Cin + c0;
+                float* dst = p.partial + ((size_t(split) * p.ntaps + tap) * p.Cout + (o0 + row)) * p.Cin + c0;
                 for (int cc = 0; cc < p.NC; cc += 16) {
                     const int tcol = colmode ? ((cc >> 6) * 3 + ti) * 64 + (cc & 63) : ti * p.NC + cc;
                     uint32_t v[16];
                     tmem_ld16(tmem_base + (uint32_t(q * 32) << 16) + uint32_t(tcol), v);
                     tmem_ld_wait();
                     if (valid) {
-                        if (p.acc) {
 #pragma unroll
-                            for (int j = 0; j < 16; j += 4)
-                                asm volatile("red.global.add.v4.f32 [%0], {%1, %2, %3, %4};" ::"l"(dst + cc + j),
-                                             "f"(__uint_as_float(v[j])), "f"(__uint_as_float(v[j + 1])),
-                                             "f"(__uint_as_float(v[j + 2])), "f"(__uint_as_float(v[j + 3]))
-                                             : "memory");
-                        } else {
-#pragma unroll
-                            for (int j = 0; j < 16; j += 4)
-                                *reinterpret_cast<float4*>(dst + cc + j) =
-                                    make_float4(__uint_as_float(v[j]), __uint_as_float(v[j + 1]),
-                                                __uint_as_float(v[j + 2]), __uint_as_float(v[j + 3]));
-                        }
+                        for (int j = 0; j < 16; j += 4)
+                            *reinterpret_cast<float4*>(dst + cc + j) =
+                                make_float4(__uint_as_float(v[j]), __uint_as_float(v[j + 1]),
+                                            __uint_as_float(v[j + 2]), __uint_as_float(v[j + 3]));
                     }
                 }
             }
@@ -909,16 +894,11 @@ int igemm_conv_plan(IgemmConvParams* p, const ConvSegDesc* segs, int nseg, int B
     for (int cand = 256; cand >= 16; cand -= 16)
         if (Cout % cand == 0 && (!gn_hook || cand % 32 == 0)) {
             if (!BN) BN = cand;
-            static const int min_bn = getenv("UB_CONV_MIN_BN") ? atoi(getenv("UB_CONV_MIN_BN")) : 64;
-            if (cand < min_bn) break;
+            if (cand < 64) break;
             BN = cand;
             if (pix_tiles * (Cout / cand) >= 128) break;
         }
     if (!BN) return -2;
-    if (const char* e = getenv("UB_CONV_FORCE_BN")) {  // experiments only
-        const int f = atoi(e);
-        if (f >= 16 && Cout % f == 0 && f <= 256 && (!gn_hook || f % 32 == 0)) BN = f;
-    }
     p->nseg = nseg;
     p->B = B, p->H = H, p->W = W, p->Cout = Cout, p->BN = BN;
     p->TW = W < 128 ? W : 128;
@@ -933,14 +913,9 @@ int igemm_conv_plan(IgemmConvParams* p, const ConvSegDesc* segs, int nseg, int B
     // columns so that a weight-gradient CTA of the side stream still finds room.
     p->nacc = 1;
     {
-        static const int want = getenv("UB_CONV_NACC") ? atoi(getenv("UB_CONV_NACC")) : 2;
         int nkb = 0;
         for (int s = 0; s < nseg; ++s) nkb += segs[s].ntaps * ceil_div_i(segs[s].Cin, 64);
-        if (want >= 2 && pix_tiles * (Cout / BN) <= 148 && BN % 32 == 0 && BN <= 128 && nkb >= 4) p->nacc = 2;
-    }
-    {
-        static const int want_np = getenv("UB_CONV2_NPROD") ? atoi(getenv("UB_CONV2_NPROD")) : 2;
-        p->nprod = (p->nacc == 2 && want_np >= 2) ? 2 : 1;  // (the two-stream ring is even: see below)
+        if (pix_tiles * (Cout / BN) <= 148 && BN % 32 == 0 && BN <= 128 && nkb >= 4) p->nacc = 2;
     }
     p->tmem_cols = next_pow2(p->nacc * BN < 32 ? 32 : p->nacc * BN);
     p->a_bytes = uint32_t(64 * p->TW * p->TH * p->TB * 2);
@@ -957,15 +932,14 @@ int igemm_conv_plan(IgemmConvParams* p, const ConvSegDesc* segs, int nseg, int B
     if (stages > kMaxStages) stages = kMaxStages;
     if (stages < 2) return -3;
     if (p->nacc == 2) {
-        // One CTA per SM: the ring may use more than the two-CTA budget (UB_CONV2_SMEM_KB; at 128 KiB a wgrad CTA of
-        // the side stream still fits beside it).  Measured round 2 (ms per step): with ONE producer warp 128 / 160 /
+        // One CTA per SM: the ring may use more than the two-CTA budget (200 KiB; at 128 KiB a wgrad CTA of the
+        // side stream still fits beside it).  Measured round 2 (ms per step): with ONE producer warp 128 / 160 /
         // 200 KiB all gave 5.09-5.10; with the second producer warp 5.02 / 4.99 / 4.975 -- default 200.  Stages of
         // TWO K blocks sharing one barrier pair (both issuers on every stage) were slower -- 890 cycles per pair of K
         // blocks in the phase trace against 2 x 322 -- and were removed again.  What bounds the main loop of these
         // layers is the TMA stream itself: the phase trace with the MMAs switched off (UB_TRACE_MODE=1) takes as long
         // as the full kernel (~77 B/clk/SM for the 4-D halo boxes), the MMA stream alone 35 % less.
-        static const int kb = getenv("UB_CONV2_SMEM_KB") ? atoi(getenv("UB_CONV2_SMEM_KB")) : 200;
-        int s2 = int((uint32_t(kb) * 1024u - tail) / p->stage_bytes);
+        int s2 = int((200u * 1024u - tail) / p->stage_bytes);
         if (s2 > kMaxStages) s2 = kMaxStages;
         if (s2 > stages) stages = s2;
     }
@@ -1020,12 +994,10 @@ int igemm_conv_plan(IgemmConvParams* p, const ConvSegDesc* segs, int nseg, int B
     {
         // tensor-core statistics + TMA output store (IgemmConvParams::ms) for the plain stats hook on full
         // 128-pixel tiles of one or two whole images with a 64- or 128-channel N tile, one or two MMA streams
-        // (measured round 2: 5.015 ms per step with, 5.043 without; parity suite green -- on by default, UB_EPI_MMA=0
-        //  switches back to the shuffle-reduce statistics)
-        static const bool want_ms = !(getenv("UB_EPI_MMA") && atoi(getenv("UB_EPI_MMA")) == 0);
+        // (measured round 2: 5.015 ms per step with, 5.043 with the shuffle-reduce statistics; measured, removed)
         const bool full_tiles = W % p->TW == 0 && H % p->TH == 0 && p->TW * p->TH * p->TB == 128;
         const size_t need = size_t(2 * (BN / 64) + 1) * 16384;  // Y atoms, Y*Y atoms, ones tile in the dead stages
-        if (want_ms && ep.stats && !ep.gn_x && p->out_mode == OUT_NHWC_BF16 && (BN == 64 || BN == 128) &&
+        if (ep.stats && !ep.gn_x && p->out_mode == OUT_NHWC_BF16 && (BN == 64 || BN == 128) &&
             p->nacc <= 2 && (p->TB == 1 || (p->TB == 2 && (p->TW * p->TH) == 64)) && full_tiles &&
             need <= size_t(p->stages) * p->stage_bytes && p->nacc * BN + 64 <= (p->nacc == 1 ? 256 : 512) &&
             make_act_map(&p->tmO, reinterpret_cast<const __nv_bfloat16*>(ep.out), Cout, p->ldo, W, H, B, p->TW, p->TH,
@@ -1034,10 +1006,8 @@ int igemm_conv_plan(IgemmConvParams* p, const ConvSegDesc* segs, int nseg, int B
             p->tmem_cols = next_pow2(p->nacc * BN + 64);
         }
         // ms == 2, store-only: a conv without any hook whose output is an NHWC bf16 tensor leaves through the same staged
-        // tile + TMA store (any whole-tile shape, N tiles of 64 .. 256 channels); UB_EPI_TMA_STORE=0 keeps the
-        // per-thread stores
-        static const bool want_st = !(getenv("UB_EPI_TMA_STORE") && atoi(getenv("UB_EPI_TMA_STORE")) == 0);
-        if (want_ms && want_st && !p->ms && !gn_hook && p->out_mode == OUT_NHWC_BF16 && BN % 64 == 0 &&
+        // tile + TMA store (any whole-tile shape, N tiles of 64 .. 256 channels)
+        if (!p->ms && !gn_hook && p->out_mode == OUT_NHWC_BF16 && BN % 64 == 0 &&
             p->nacc <= 2 && full_tiles && size_t(BN / 64) * 16384 <= size_t(p->stages) * p->stage_bytes &&
             make_act_map(&p->tmO, reinterpret_cast<const __nv_bfloat16*>(ep.out), Cout, p->ldo, W, H, B, p->TW, p->TH,
                          p->TB) == 0)
@@ -1098,19 +1068,20 @@ static int wgrad_plan_common(IgemmWgradParams* p, const __nv_bfloat16* dy, int l
     // boxes may overhang the image (TMA zero-fills), they must hold exactly KP pixels
     // K tile = KP pixels per stage.  128 halves the number of TMA issues and barrier round trips per byte (the single
     // producer thread was the pacing resource at KP = 64); 64 is kept for operands whose tiles would not fit.
-    static const int kp_env = getenv("UB_WGRAD_KP") ? atoi(getenv("UB_WGRAD_KP")) : 128;
-    int KP = (kp_env == 64 || size_t(B) * H * W < 256) ? 64 : 128;
+    int KP = size_t(B) * H * W < 256 ? 64 : 128;
     p->MO = (Cout % 128 == 0) ? 128 : 64;
     p->TC = ntaps == 9 ? 3 : 1;
     // TMEM: TC * NC columns <= 512
     p->NC = (Cin % 128 == 0) ? 128 : 64;
     const int a_atoms = p->MO / 64, b_atoms = p->NC / 64;
-    // Column mode (3x3 layers; UB_WGRAD_COLMODE=0 = row mode): a CTA owns a filter COLUMN and takes its three dy taps from
+    // Column mode (3x3 layers): a CTA owns a filter COLUMN and takes its three dy taps from
     // one halo box of TH + 2 image rows per 64-channel atom instead of three boxes of TH rows -- the main loop runs at
     // the chip-wide L2 -> shared-memory rate, so bytes are time: the activation operand shrinks to
     // (KP + 2 TW TB) / (3 KP) = 0.67 of its size at 64x64, 0.5 at 32x32, 0.42 at 16x16 and 8x8.
-    // (halo windows must start on the 8-pixel swizzle atom: image rows of the tile >= 8 pixels, i.e. W > 4)
-    p->colmode = (ntaps == 9 && next_pow2(W) >= 8 && !(getenv("UB_WGRAD_COLMODE") && atoi(getenv("UB_WGRAD_COLMODE")) == 0)) ? 1 : 0;
+    // (halo windows must start on the 8-pixel swizzle atom: image rows of the tile >= 8 pixels, i.e. W > 4; narrower
+    // 3x3 layers and 1x1 layers run row mode.  Row mode for every 3x3 layer: measured, removed,
+    // profiles/r02n_wgrad_colmode.txt)
+    p->colmode = (ntaps == 9 && next_pow2(W) >= 8) ? 1 : 0;
     for (;;) {
         p->KP = KP;
         p->TW = next_pow2(W) < KP ? next_pow2(W) : KP;
@@ -1134,25 +1105,17 @@ static int wgrad_plan_common(IgemmWgradParams* p, const __nv_bfloat16* dy, int l
     p->tmem_cols = next_pow2(p->TC * p->NC + (bias ? 16 : 0) < 32 ? 32 : p->TC * p->NC + (bias ? 16 : 0));
     if (p->tmem_cols > 512) return -3;
     p->tx_bytes = p->stage_bytes;
-    static const unsigned smem_kb = getenv("UB_WGRAD_SMEM_KB") ? unsigned(atoi(getenv("UB_WGRAD_SMEM_KB"))) : 96u;
-    int stages = int((smem_kb * 1024u) / p->stage_bytes);
+    int stages = int((96u * 1024u) / p->stage_bytes);
     if (stages < 2) stages = 2;
     if (stages > kMaxStages) stages = kMaxStages;
     if (size_t(stages) * p->stage_bytes > 220u * 1024u) return -3;
-    // two TMA producer warps (see the kernel) need an even ring: a stage must always belong to the same producer.
-    // Measured (profiles/r02n_wgrad_tma_red.txt): no gain -- the stages are multi-box, so one producer already reaches
-    // the chip-wide L2 -> shared-memory rate -- hence opt-in (UB_WGRAD_NPROD=2).
-    static const int nprod_env = getenv("UB_WGRAD_NPROD") ? atoi(getenv("UB_WGRAD_NPROD")) : 1;
-    if (nprod_env == 2 && stages > 2 && (stages & 1)) --stages;
-    p->nprod = (nprod_env == 2 && (stages & 1) == 0) ? 2 : 1;
     p->stages = stages;
     const int ktiles = p->tiles_w * p->tiles_h * p->tiles_b;
     const int base_ctas = (Cout / p->MO) * (Cin / p->NC) * (ntaps / p->TC);
     // One CTA per SM (a CTA owns the SM's smem and TMEM), and never more CTAs than SMs: a grid of 150 CTAs on 148
     // SMs runs as two waves and doubles the kernel time (ncu r01: 64->64@64x64 took 57 us as (1,3,50)).
     int nsplit = sm_count / base_ctas;
-    static const int min_kpix = getenv("UB_WGRAD_MIN_KPIX") ? atoi(getenv("UB_WGRAD_MIN_KPIX")) : 256;
-    if (nsplit > ktiles * KP / min_kpix) nsplit = ktiles * KP / min_kpix;  // at least 256 pixels of K per CTA
+    if (nsplit > ktiles * KP / 256) nsplit = ktiles * KP / 256;  // at least 256 pixels of K per CTA
     if (nsplit < 1) nsplit = 1;
     if (!acc_mode) {
         while (nsplit > 1 && igemm_wgrad_partial_floats(Cin, Cout, ntaps, nsplit) > partial_cap_floats) --nsplit;
@@ -1183,32 +1146,26 @@ int igemm_wgrad_plan_acc(IgemmWgradParams* p, const __nv_bfloat16* dy, int ldy, 
     if (!acc || (reinterpret_cast<uintptr_t>(acc) & 15)) return -16;
     p->acc = acc, p->dbias = dbias, p->dbias2 = dbias2;
     // TMA reduce-add epilogue (see the kernel): fp32 map over acc[ntaps * Cout][Cin], box = 32 columns (128 B, the
-    // swizzle span) x the MO/4 accumulator rows of one epilogue warp.  UB_WGRAD_TMA_RED=0: per-lane red.global.add.
-    static const bool tma_red = !(getenv("UB_WGRAD_TMA_RED") && atoi(getenv("UB_WGRAD_TMA_RED")) == 0);
-    if (tma_red) {
-        EncodeTiledFn fn = get_encode_fn();
-        if (!fn) return -10;
-        cuuint64_t dims[2] = {cuuint64_t(Cin), cuuint64_t(ntaps) * cuuint64_t(Cout)};
-        cuuint64_t strides[1] = {cuuint64_t(Cin) * 4};
-        cuuint32_t box[2] = {32, cuuint32_t(p->MO / 4)};
-        cuuint32_t es[2] = {1, 1};
-        CUresult cr = fn(&p->tmAcc, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, acc, dims, strides, box, es,
-                         CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
-                         CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-        if (cr != CUDA_SUCCESS) {
-            fprintf(stderr, "[unet_b200] cuTensorMapEncodeTiled(wgrad acc Cin=%d rows=%d) -> %d\n", Cin, ntaps * Cout,
-                    int(cr));
-            return -17;
-        }
-        p->tma_red = 1;
+    // swizzle span) x the MO/4 accumulator rows of one epilogue warp.
+    EncodeTiledFn fn = get_encode_fn();
+    if (!fn) return -10;
+    cuuint64_t dims[2] = {cuuint64_t(Cin), cuuint64_t(ntaps) * cuuint64_t(Cout)};
+    cuuint64_t strides[1] = {cuuint64_t(Cin) * 4};
+    cuuint32_t box[2] = {32, cuuint32_t(p->MO / 4)};
+    cuuint32_t es[2] = {1, 1};
+    CUresult cr = fn(&p->tmAcc, CU_TENSOR_MAP_DATA_TYPE_FLOAT32, 2, acc, dims, strides, box, es,
+                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_NONE,
+                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
+    if (cr != CUDA_SUCCESS) {
+        fprintf(stderr, "[unet_b200] cuTensorMapEncodeTiled(wgrad acc Cin=%d rows=%d) -> %d\n", Cin, ntaps * Cout,
+                int(cr));
+        return -17;
     }
     return 0;
 }
 
 int igemm_wgrad_finalize(const WgradFinalizeEntry* table_dev, int n_entries, size_t max_elems, cudaStream_t st) {
     if (n_entries < 1) return 0;
-    static const bool skip = getenv("UB_DEBUG_SKIP_FINALIZE") != nullptr;  // timing experiments only (wrong gradients)
-    if (skip) return 0;
     return int(launch_pdl(wgrad_finalize_kernel, dim3(unsigned((max_elems + 255) / 256), unsigned(n_entries)), dim3(288),
                           0, st, table_dev));
 }

@@ -38,8 +38,8 @@ struct IgemmConvParams {
     int BN;          // output-channel tile: multiple of 16, <= 256
     int stages;
     int tmem_cols;   // power of two >= max(32, nacc * BN)
-    int nacc;        // MMA issue streams = accumulators (1, or 2 for grids of at most one CTA per SM)
-    int nprod;       // TMA producer warps (2 with nacc == 2: even / odd K blocks)
+    int nacc;        // MMA issue streams = accumulators (1, or 2 for grids of at most one CTA per SM); nacc == 2
+                     // also has two TMA producer warps (even / odd K blocks)
     int ncomb;       // rows of the staged per-channel addend (TB when a per-image vector is fused, else 1)
     uint32_t a_bytes, b_bytes;  // TMA transaction bytes per stage
     uint32_t stage_bytes;       // smem bytes per stage (A tile 16 KiB + B tile, 1024-aligned)
@@ -63,7 +63,7 @@ struct IgemmConvParams {
     int gn_silu, gn_cpg;
     int ngimg;                      // rows of the staged GroupNorm constants (TB when gn_x is set, else 0)
     int nred;                       // BN-float rows of the cross-warp reduction scratch (8 with a hook, else 0)
-    // GroupNorm statistics on the tensor core (default for the plain statistics hook on full tiles; UB_EPI_MMA=0 off) --
+    // GroupNorm statistics on the tensor core (the plain statistics hook on full tiles) --
     // the epilogue stages the bf16 output tile Y and Y*Y in shared memory as MN-major SW128 operands (the layout TMA
     // gives the wgrad kernel), a ones-tile MMA (the wgrad kernel's bias-gradient trick) leaves sum(y) and sum(y*y)
     // of channel c in TMEM lane c, and the Y tile goes to global memory with one TMA store per 64 channels.
@@ -115,7 +115,6 @@ struct IgemmWgradParams {
     int nsplit;  // split of the pixel (K) dimension across CTAs
     int KP;      // pixels per K tile (= per stage): 64 or 128; an operand atom is KP rows of 128 B
     int stages;
-    int nprod;   // TMA producer warps: 2 = the first epilogue warp loads the odd K tiles (even ring only)
     // column mode (3x3): blockIdx.y = filter column; the three dy taps come from one halo box (64, TW, TH + 2, TB) per
     // 64-channel atom of X (tmX then has that box), hatom bytes each; accumulator columns [atom][dy][64]
     int colmode;
@@ -128,11 +127,10 @@ struct IgemmWgradParams {
     // partial buffer, no per-layer reduce launch; wgrad_finalize turns [tap][o][c] into the reference [o][c][tap]
     // layout for a whole gradient bucket at once (for 1x1 / linear layers acc IS the final gradient).
     float* acc;
-    // accumulate mode, tma_red != 0: the epilogue stages its accumulator rows in the (idle) operand ring and adds them
-    // with TMA reduce-add boxes of 32 columns x MO/4 rows (one epilogue warp's rows) instead of per-lane REDs, whose
+    // accumulate mode: the epilogue stages its accumulator rows in the (idle) operand ring and adds them with TMA
+    // reduce-add boxes of 32 columns x MO/4 rows (one epilogue warp's rows) instead of per-lane REDs, whose
     // thread-per-row addresses cost one LSU pass per lane.  tmAcc: fp32, dims (Cin, ntaps*Cout), 128B swizzle.
     CUtensorMap tmAcc;
-    int tma_red;
     // fused bias gradient: the CTAs of the centre tap / first Cin tile also contract dY with a tile of ones
     // (one extra N=16 MMA per K step), and add column 0 of that accumulator into dbias (and dbias2) atomically.
     float* dbias;

@@ -93,7 +93,6 @@ struct RowsBars {
 static size_t rows_tail_floats(int BN) { return size_t(2 + 8 + 16) * BN + (UB_EPI_SHUFFLE_REDUCE ? 0 : 8 * 32 * 36); }
 
 __global__ void __launch_bounds__(kRowsThreads, 1) igemm_rows_kernel(const __grid_constant__ IgemmRowsParams p) {
-    pdl_trigger();
     extern __shared__ uint8_t smem_raw[];
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     uint8_t* sA = smem;
@@ -408,17 +407,14 @@ int igemm_rows_plan(IgemmRowsParams* p, const ConvSegDesc* segs, int nseg, int B
     // Resident weights: a layer whose whole weight set is one ring's worth -- a single segment of <= 64 input channels and
     // one N tile (the 64 -> 64 convs of the 64x64 level) -- loads its ntaps tiles ONCE per CTA; the ring has exactly ntaps
     // stages, the MMA issuers wait for them during their first tile only and never release them.  The 72 KiB of weight
-    // traffic per 256-pixel tile (a third of the tile's bytes, nine barrier round trips) disappear.  UB_ROWS_WRES=0: off.
+    // traffic per 256-pixel tile (a third of the tile's bytes, nine barrier round trips) disappear.
     p->w_resident = 0;
-    {
-        static const bool want = !(getenv("UB_ROWS_WRES") && atoi(getenv("UB_ROWS_WRES")) == 0);
-        if (want && nseg == 1 && segs[0].Cin <= 64 && Cout == BN && ws >= segs[0].ntaps) {
-            p->w_resident = 1;
-            ws = segs[0].ntaps;
-            // the room the shorter ring frees goes to the activation ring
-            const int as2 = int((budget - size_t(ws) * p->w_stage_bytes) / p->a_stage_bytes);
-            if (as2 > as) as = as2 > kMaxAStages ? kMaxAStages : as2;
-        }
+    if (nseg == 1 && segs[0].Cin <= 64 && Cout == BN && ws >= segs[0].ntaps) {
+        p->w_resident = 1;
+        ws = segs[0].ntaps;
+        // the room the shorter ring frees goes to the activation ring
+        const int as2 = int((budget - size_t(ws) * p->w_stage_bytes) / p->a_stage_bytes);
+        if (as2 > as) as = as2 > kMaxAStages ? kMaxAStages : as2;
     }
     p->a_stages = as, p->w_stages = ws;
     for (int s = 0; s < nseg; ++s) {

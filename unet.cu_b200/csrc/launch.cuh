@@ -5,10 +5,10 @@
 // the kernel -> kernel edges become programmatic edges, which removes the ~1-2 us launch gap between the ~500 small
 // kernels of a step.
 //
-// Rules every kernel follows: (1) pdl_trigger() then pdl_wait() are executed by EVERY thread before its first access
-// to global memory that an earlier kernel may have written, and before any early return; (2) nothing before
-// pdl_wait() touches such memory (kernel parameters, including __grid_constant__ tensor maps, are fine).
-// Launched without the attribute (layer API, tools) both instructions are no-ops.
+// Rules every kernel follows: (1) pdl_wait() is executed by EVERY thread before its first access to global memory that
+// an earlier kernel may have written, and before any early return; (2) nothing before pdl_wait() touches such memory
+// (kernel parameters, including __grid_constant__ tensor maps, are fine).  Launched without the attribute (layer API,
+// tools) the griddepcontrol instructions are no-ops.
 #pragma once
 #include <cuda_runtime.h>
 
@@ -17,42 +17,23 @@
 
 namespace ub {
 
+// Where the dependent grid is released (griddepcontrol.launch_dependents), measured with bench.py at B = 32:
+// - no PDL 6.87 ms/step, the implicit trigger at grid end 6.62, an entry trigger in every kernel 7.30, an entry
+//   trigger only in the forward-pass convs 6.01 against 5.93 without: early-resident CTAs of the next kernel take SM
+//   slots, TMEM and shared memory from the kernel that is still draining and from the weight-gradient branch.  The
+//   GEMM-shaped kernels therefore trigger late (pdl_trigger_late), the others at entry (pdl_entry).
+// - round 2: the entry trigger in the elementwise / normalisation kernels gave 5.09 ms/step against 5.18 without --
+//   the launch latency of every kernel that follows a GroupNorm / data-movement kernel was exposed.
+// The early-trigger, no-late-trigger and no-entry-trigger variants were measured and removed.
 __device__ __forceinline__ void pdl_wait() { asm volatile("griddepcontrol.wait;" ::: "memory"); }
-// Measured (bench.py, B=32): no PDL 6.87 ms/step, implicit trigger 6.62, early trigger in every kernel 7.30, early
-// trigger only in the forward-pass convs 6.01 vs 5.93 without -- early-resident CTAs of the next kernel take SM slots,
-// TMEM and shared memory from the kernel that is still draining and from the weight-gradient branch.
-#ifndef UB_PDL_EARLY_TRIGGER
-#define UB_PDL_EARLY_TRIGGER 0
-#endif
-__device__ __forceinline__ void pdl_trigger() {
-#if UB_PDL_EARLY_TRIGGER
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
-}
 // Late trigger (GEMM-shaped kernels): issued by a CTA once its main loop is complete, so the next kernel's CTAs become
 // resident and run their prologue (barrier init, TMEM allocation, descriptor prefetch) under this kernel's epilogue
 // and teardown only -- they cannot take resources from a main loop that is still running.
-#ifndef UB_PDL_LATE_TRIGGER
-#define UB_PDL_LATE_TRIGGER 1
-#endif
-__device__ __forceinline__ void pdl_trigger_late() {
-#if UB_PDL_LATE_TRIGGER
-    asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#endif
-}
-// the usual kernel entry: let the dependent grid start early, then wait for our own prerequisite
-// (UB_PDL_ELT_EARLY: entry trigger only in the elementwise / normalisation kernels, whose CTAs hold no shared memory
-//  or TMEM that an early-resident dependent could be starved of.  Measured round 2, bench.py B = 32: 5.09 ms/step with,
-//  5.18 without -- the launch latency of every kernel that follows a GroupNorm / data-movement kernel was exposed.)
-#ifndef UB_PDL_ELT_EARLY
-#define UB_PDL_ELT_EARLY 1
-#endif
+__device__ __forceinline__ void pdl_trigger_late() { asm volatile("griddepcontrol.launch_dependents;" ::: "memory"); }
+// the usual kernel entry (elementwise / normalisation kernels, whose CTAs hold no shared memory or TMEM that an
+// early-resident dependent could be starved of): let the dependent grid start early, then wait for our own prerequisite
 __device__ __forceinline__ void pdl_entry() {
-#if UB_PDL_ELT_EARLY
     asm volatile("griddepcontrol.launch_dependents;" ::: "memory");
-#else
-    pdl_trigger();
-#endif
     pdl_wait();
 }
 

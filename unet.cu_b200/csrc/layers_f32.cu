@@ -87,8 +87,7 @@ __global__ void __launch_bounds__(256) nchw_to_nhwc_bf16_tile64_kernel(const flo
     }
 }
 void nchw_to_nhwc_bf16(const float* x, int B, int C, int HW, __nv_bfloat16* y, cudaStream_t st) {
-    static const bool old = getenv("UB_NCHW_CONVERT_OLD") != nullptr;  // (measurement switch)
-    if (!old && HW % 4 == 0 && C % 2 == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0 &&
+    if (HW % 4 == 0 && C % 2 == 0 && (reinterpret_cast<uintptr_t>(x) & 15) == 0 &&
         (reinterpret_cast<uintptr_t>(y) & 3) == 0) {
         dim3 grid((HW + 63) / 64, (C + 63) / 64, B);
         nchw_to_nhwc_bf16_tile64_kernel<<<grid, 256, 0, st>>>(x, C, HW, y);

@@ -746,8 +746,6 @@ __global__ void __launch_bounds__(256) pack_weights_kernel(const PackEntry* __re
     }
 }
 void pack_weights(const PackEntry* table_dev, int n_entries, int max_tiles, cudaStream_t st) {
-    static const bool skip = getenv("UB_DEBUG_SKIP_PACK") != nullptr;  // timing experiments only (stale bf16 weights)
-    if (skip) return;
     // (9 taps: 32 x 289 floats = 36 992 B of dynamic shared memory, below the 48 KiB that needs no opt-in)
     launch_pdl(pack_weights_kernel, dim3(dim3(max_tiles, n_entries)), dim3(256), size_t(32) * (32 * 9 + 1) * sizeof(float), st,
                table_dev);

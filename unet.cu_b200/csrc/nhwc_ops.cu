@@ -85,12 +85,8 @@ static RowMap make_rowmap(int B, int HW, int C, int blocks_per_sm = 3) {
     if (m.rows < 1) m.rows = 1;
     if (m.rows > HW) m.rows = HW;
     m.threads = m.C8 * m.rows;
-    static const bool one_wave = !(getenv("UB_GN_ONE_WAVE") && atoi(getenv("UB_GN_ONE_WAVE")) == 0);
-    int want = (3 * kSMs + B - 1) / B;  // chunks per image: ~3 blocks per SM, each with a long pixel loop
-    if (one_wave) {
-        want = (blocks_per_sm * kSMs) / B;  // all blocks resident at once
-        if (want < 1) want = 1;
-    }
+    int want = (blocks_per_sm * kSMs) / B;  // chunks per image: all blocks resident at once
+    if (want < 1) want = 1;
     int maxc = (HW + m.rows - 1) / m.rows;
     m.nchunks = want < maxc ? want : maxc;
     if (m.nchunks < 1) m.nchunks = 1;
@@ -960,8 +956,7 @@ __global__ void __launch_bounds__(kSmallcWarps * 32) smallc_conv_rows_kernel(
 
 static void smallc_conv(const float* xs, const float* w, const float* bias, int Cs, int Cb, int B, int H, int W,
                         int flip, bf16* y, int ldy, cudaStream_t st) {
-    static const bool use_rows = !(getenv("UB_SMALLC_ROWS") && atoi(getenv("UB_SMALLC_ROWS")) == 0);
-    if (use_rows && Cs == 3 && Cb % 64 == 0 && W % 4 == 0 && (ldy % 2) == 0) {
+    if (Cs == 3 && Cb % 64 == 0 && W % 4 == 0 && (ldy % 2) == 0) {
         const size_t smem_r = (size_t(27) * Cb + size_t(kSmallcWarps) * 9 * (W + 4)) * sizeof(float);
         if (smem_r <= 48 * 1024) {
             const long long items = (long long)B * H * (Cb / 64);
@@ -1177,8 +1172,7 @@ void nhwc_ops_init() {
 }
 static void smallc_wgrad(const float* xs, const bf16* yb, int ldy, int B, int Cs, int Cb, int H, int W, int mode,
                          float* dw, float* db, float* scratch, size_t scratch_floats, cudaStream_t st) {
-    static const bool use_rows = !(getenv("UB_SMALLC_ROWS") && atoi(getenv("UB_SMALLC_ROWS")) == 0);
-    if (use_rows && Cs == 3 && Cb % 64 == 0 && W % 4 == 0 && (ldy % 2) == 0) {
+    if (Cs == 3 && Cb % 64 == 0 && W % 4 == 0 && (ldy % 2) == 0) {
         const size_t smem_r = (size_t(kSmallcWarps) * 9 * (W + 4) + size_t(kSmallcWarps) * 56 * 32) * sizeof(float);
         if (smem_r <= 100 * 1024) {
             nhwc_ops_init();
@@ -1425,8 +1419,7 @@ __global__ void __launch_bounds__(kSmallcWarps * 32) conv_out_rows_kernel(
     }
 }
 static bool conv_out_rows_ok(int Cin, int Cout, int W) {
-    static const bool use_rows = !(getenv("UB_SMALLC_ROWS") && atoi(getenv("UB_SMALLC_ROWS")) == 0);
-    return use_rows && Cout == 3 && Cin % 64 == 0 && W % 8 == 0 &&
+    return Cout == 3 && Cin % 64 == 0 && W % 8 == 0 &&
            (size_t(3) * Cin * 9 + size_t(kSmallcWarps) * 3 * W) * sizeof(float) <= 48 * 1024;
 }
 static void conv_out_rows_launch(const bf16* a, int lda, const float* w, const float* b, int B, int Cin, int H, int W,

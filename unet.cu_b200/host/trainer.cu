@@ -115,10 +115,8 @@ struct UbTrainer {
     // attention backward's dkv kernel beside its dq kernel (attn_tc_bwd).
     cudaStream_t aux_stream = nullptr;
     cudaEvent_t ev_aux_fork = nullptr, ev_aux_join = nullptr;
-    bool attn_concurrent = true;
     std::vector<cudaEvent_t> side_events;
     size_t side_ev_next = 0;
-    bool use_side = true;
     // flat fp32 arenas in reference order
     size_t nparams = 0;
     float *params = nullptr, *grads = nullptr, *m = nullptr, *v = nullptr;
@@ -217,7 +215,7 @@ struct UbTrainer {
     int host_step = 0;
     // data parallel
     ncclComm_t comm = nullptr;
-    int rank = 0, world = 1, n_buckets = getenv("UB_BUCKETS") ? atoi(getenv("UB_BUCKETS")) : 8;
+    int rank = 0, world = 1, n_buckets = 8;
     bool comm_off = false;  // rank-local eager replays (profiling) must not enqueue collectives
     // Optimizer per gradient bucket: as soon as a bucket's gradients are final (and all-reduced), AdamW and the weight
     // re-pack of that parameter range run on the branch that finalised them, under the rest of backward; only the
@@ -358,22 +356,17 @@ struct Builder {
         // <= 64 output channels -- and (b) at wide levels with >= 192 output channels, where the basic kernel's N tile
         // is 160-192 columns: one CTA per SM, i.e. a single MMA issue stream, against the row-tile kernel's two.
         // Elsewhere (N <= 128: two CTAs per SM; 8x8 / 16x16: too few row tiles) the basic kernel is faster.
-        // UB_ROWS=0 / 2 forces never / always.
-        static const int rows_mode = getenv("UB_ROWS") ? atoi(getenv("UB_ROWS")) : 1;
         const bool rows_pref = (W >= 64 && (Cout <= 64 || Cout >= 192)) || (W >= 32 && Cout >= 192 && segs[0].ntaps == 9);
         // A one-tap conv without a hook (the 1x1 skip-conv dgrads) is all epilogue.  Measured (profiles/r02_plain_1x1.txt):
         // the row-tile kernel stays ahead of the basic kernel there even with the latter's staged tile + TMA store
-        // (64 -> 192 at 64x64: 30.6 vs 39.7 us), so the rule above stands; UB_PLAIN_1X1_BASIC=1 routes them to the basic kernel.
-        static const bool plain_basic = getenv("UB_PLAIN_1X1_BASIC") && atoi(getenv("UB_PLAIN_1X1_BASIC")) != 0;
-        const bool plain_1x1 = segs.size() == 1 && segs[0].ntaps == 1 && !ep.stats && !ep.gn_x && plain_basic;
-        const bool no_rows = rows_mode == 0 || (rows_mode == 1 && (!rows_pref || plain_1x1));
+        // (64 -> 192 at 64x64: 30.6 vs 39.7 us), so the rule above stands.
         double k = 0, bytes = act_bytes(Cout, H, W);
         for (auto& sg : segs) k += double(sg.ntaps) * sg.Cin, bytes += act_bytes(sg.Cin, H, W) + 2.0 * sg.ntaps * sg.Cin * Cout;
         const double flops = 2.0 * B * H * W * Cout * k;
         UbTrainer::Op op;
         // persistent row-tile kernel for the 16x16 .. 128x128 levels, one-CTA-per-128-pixels kernel otherwise
         IgemmRowsParams pr;
-        if (!no_rows && igemm_rows_eligible(B, H, W, Cout) &&
+        if (rows_pref && igemm_rows_eligible(B, H, W, Cout) &&
             igemm_rows_plan(&pr, segs.data(), int(segs.size()), B, H, W, Cout, ep, sm_count()) == 0) {
             op = [pr](cudaStream_t st) { igemm_rows_launch(pr, st); };
             label("conv%s %s Cin=%d%s Cout=%d %dx%d rows BN=%d stages=%d/%d%s%s", segs[0].ntaps == 9 ? "3x3" : "1x1",
@@ -405,9 +398,8 @@ struct Builder {
     void wgrad_op(View dy, View x, int Cin, int Cout, int ntaps, float* dw, float* db = nullptr, float* db2 = nullptr) {
         float* acc = ntaps == 9 ? f32(size_t(9) * Cout * Cin) : dw;
         if (!real()) return;
-        static const int wg_sms = getenv("UB_WGRAD_SMS") ? atoi(getenv("UB_WGRAD_SMS")) : sm_count();
         IgemmWgradParams p;
-        int r = igemm_wgrad_plan_acc(&p, dy.p, dy.ld, x.p, x.ld, B, x.H, x.W, Cin, Cout, ntaps, acc, db, db2, wg_sms);
+        int r = igemm_wgrad_plan_acc(&p, dy.p, dy.ld, x.p, x.ld, B, x.H, x.W, Cin, Cout, ntaps, acc, db, db2, sm_count());
         if (r) {
             set_err("igemm_wgrad_plan failed (%d) for %dx%d %d->%d", r, x.H, x.W, Cin, Cout);
             plan_errors++;
@@ -497,14 +489,10 @@ struct Builder {
     // Time-MLP backward (needs the complete d_embact, i.e. every embedding projection's backward).  Emitted on the
     // weight-gradient branch as soon as the first ResBlock has produced its embedding gradient, so that it runs under
     // the last dgrad convs instead of after them (it used to be 80 us of the step's serial tail).
-    // Step tail (UB_TAIL_AUX=0 restores the single-branch order): the time-MLP backward (six small dependent kernels)
-    // forks off the weight-gradient branch into a branch of its own, and the 3-channel input conv's weight gradient --
-    // the last gradient of the step -- runs on the main stream, which has nothing left to do: the three chains
-    // (last wgrad -> finalize -> bucket optimizer | time MLP | input-conv wgrad) overlap instead of queueing.
-    static bool tail_aux() {
-        static const bool on = !(getenv("UB_TAIL_AUX") && atoi(getenv("UB_TAIL_AUX")) == 0);
-        return on;
-    }
+    // Step tail: the time-MLP backward (six small dependent kernels) forks off the weight-gradient branch into a branch
+    // of its own, and the 3-channel input conv's weight gradient -- the last gradient of the step -- runs on the main
+    // stream, which has nothing left to do: the three chains (last wgrad -> finalize -> bucket optimizer | time MLP |
+    // input-conv wgrad) overlap instead of queueing.  (Both on the weight-gradient branch: measured, removed.)
     bool time_mlp_bwd_done = false;
     void time_mlp_bwd() {
         if (time_mlp_bwd_done) return;
@@ -518,7 +506,7 @@ struct Builder {
             small_linear_bwd(Tt->temb_table + 1, 1, Bn, Cemb, Cemb, st);
             dsilu_mul(Tt->d_h0act, Tt->h0, Tt->dh0, size_t(Bn) * Cemb, st);
             small_linear_bwd(Tt->temb_table, 1, Bn, Cemb, Cm, st);
-        }, cls ? 7 : 6, UB_KIND_SMALL, 0, 0, tail_aux() ? 3 : 1);  // 3: a branch of its own, forked from the weight-gradient branch
+        }, cls ? 7 : 6, UB_KIND_SMALL, 0, 0, 3);  // 3: a branch of its own, forked from the weight-gradient branch
     }
 
     // 2x resampling of a tensor inside an up/down ResBlock (h_upd / x_upd, dev/resblock.py:78-86,125-128): ud = 1 average
@@ -742,7 +730,7 @@ struct Builder {
             }
             Bk([=](cudaStream_t st) {
                 if (tc)
-                    attn_tc_bwd(apb, st, Tt->attn_concurrent ? Tt->aux_stream : nullptr, Tt->ev_aux_fork, Tt->ev_aux_join);
+                    attn_tc_bwd(apb, st, Tt->aux_stream, Tt->ev_aux_fork, Tt->ev_aux_join);
                 else
                     attn_bwd(qkv.p, qkv.ld, ao.p, ao.ld, dao.p, dao.ld, lse, Bn, Tn, NH, HSz, dqkv.p, dqkv.ld, dsum, st);
             }, 2, UB_KIND_ATTN, 10.0 * B * NH * double(Tn) * Tn * HSz, act_bytes(8 * C, H, W));
@@ -839,7 +827,7 @@ int Builder::build() {
             Bk([=](cudaStream_t st) {
                 conv_in_wgrad(Tt->xt, dout.p, dout.ld, Bn, Cin, hv.C, hv.H, hv.W, gw, gb, Tt->small_scratch,
                               Tt->small_scratch_floats, st);
-            }, 1, UB_KIND_SMALL, 0, 0, tail_aux() ? 0 : 1);  // (one launch with the row kernel; two on its fallback path)
+            }, 1, UB_KIND_SMALL, 0, 0, 0);  // (one launch with the row kernel; two on its fallback path)
             if (Tt->cfg.compute_dinput)
                 Bk([=](cudaStream_t st) { conv_in_dgrad(dout.p, dout.ld, w, Bn, Cin, hv.C, hv.H, hv.W, Tt->dxt, st); }, 1);
             return View{};
@@ -973,20 +961,14 @@ int Builder::build() {
         for (int k = nb - 1; k >= 1; --k) cuts.push_back(T->nparams * size_t(k) / nb);
         // A last cut right above the input conv: the bucket that must wait for the very end of backward (and whose
         // AdamW + weight re-pack are the serial tail of the step) then holds only the time MLP and the 3-channel conv.
-        static const bool tail_cut = !(getenv("UB_TAIL_CUT") && atoi(getenv("UB_TAIL_CUT")) == 0);
         // (Measured round 2: further cuts at the level boundaries of the down path, so that only the first level's
         //  small bucket waits for the end of backward, cost more in extra optimizer / re-pack launches on the tail
-        //  than the shorter last all-reduce won: 5.08 vs 5.02 ms on one GPU, 5.13 vs 5.11 on two.)
-        // UB_TAIL_NODE = n: the last bucket ends above node n (1 (default) = only the time MLP and the input conv; 2 = the
-        // first ResBlock too, so that the last full-size all-reduce is complete one ResBlock earlier).  Measured round 2:
-        // 2 costs the single GPU 0.08 ms (a longer serial optimizer tail) and changes nothing on 8 GPUs (5.015 vs 5.006).
-        static const int tail_node = getenv("UB_TAIL_NODE") ? atoi(getenv("UB_TAIL_NODE")) : 1;
-        const size_t tn = size_t(tail_node < 1 ? 1 : tail_node);
-        if (tail_cut && nodes.size() > tn && nodes[tn].param_begin > time_mlp_end && (nodes[tn].param_begin % 4) == 0 &&
-            (cuts.empty() || nodes[tn].param_begin < cuts.back()))
-            cuts.push_back(nodes[tn].param_begin);
-        else if (tail_cut && nodes.size() > 1 && nodes[1].param_begin > time_mlp_end &&
-                 (cuts.empty() || nodes[1].param_begin < cuts.back()))
+        //  than the shorter last all-reduce won: 5.08 vs 5.02 ms on one GPU, 5.13 vs 5.11 on two.  No tail cut, and a
+        //  cut above node 2 (the first ResBlock in the last bucket too, so that the last full-size all-reduce is
+        //  complete one ResBlock earlier) were measured and removed: the latter cost the single GPU 0.08 ms (a longer
+        //  serial optimizer tail) and changed nothing on 8 GPUs, 5.015 vs 5.006.)
+        if (nodes.size() > 1 && nodes[1].param_begin > time_mlp_end &&
+            (cuts.empty() || nodes[1].param_begin < cuts.back()))
             cuts.push_back(nodes[1].param_begin);
     }
     size_t flushed_hi = T->nparams;
@@ -1221,20 +1203,17 @@ extern "C" int ub_trainer_create(UbTrainer** out, const UbConfig* cfg, int devic
     // and the collectives fill the gaps (stream priorities become kernel-node priorities in the captured graph)
     int prio_lo = 0, prio_hi = 0;
     cudaDeviceGetStreamPriorityRange(&prio_lo, &prio_hi);
-    static const bool use_prio = !(getenv("UB_NO_PRIO") && atoi(getenv("UB_NO_PRIO")) != 0);
-    cudaStreamCreateWithPriority(&t->stream, cudaStreamNonBlocking, use_prio ? prio_hi : 0);
-    cudaStreamCreateWithPriority(&t->comm_stream, cudaStreamNonBlocking, use_prio ? prio_hi : 0);
-    cudaStreamCreateWithPriority(&t->side_stream, cudaStreamNonBlocking, use_prio ? prio_lo : 0);
-    cudaStreamCreateWithPriority(&t->aux_stream, cudaStreamNonBlocking, use_prio ? prio_hi : 0);
+    cudaStreamCreateWithPriority(&t->stream, cudaStreamNonBlocking, prio_hi);
+    cudaStreamCreateWithPriority(&t->comm_stream, cudaStreamNonBlocking, prio_hi);
+    cudaStreamCreateWithPriority(&t->side_stream, cudaStreamNonBlocking, prio_lo);
+    cudaStreamCreateWithPriority(&t->aux_stream, cudaStreamNonBlocking, prio_hi);
     cudaEventCreateWithFlags(&t->ev_aux_fork, cudaEventDisableTiming);
     cudaEventCreateWithFlags(&t->ev_aux_join, cudaEventDisableTiming);
-    t->attn_concurrent = !(getenv("UB_ATTN_SERIAL") && atoi(getenv("UB_ATTN_SERIAL")) != 0);
     t->side_events.resize(4096);
     for (auto& ev : t->side_events) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
-    if (const char* e = getenv("UB_NO_SIDE_STREAM")) t->use_side = atoi(e) == 0;
     cudaEventCreateWithFlags(&t->ev_join, cudaEventDisableTiming);
     cudaEventCreateWithFlags(&t->ev_join2, cudaEventDisableTiming);
-    cudaStreamCreateWithPriority(&t->opt_stream, cudaStreamNonBlocking, use_prio ? prio_lo : 0);
+    cudaStreamCreateWithPriority(&t->opt_stream, cudaStreamNonBlocking, prio_lo);
     t->bucket_events.resize(32);  // [0, 16): branch -> communication stream, [16, 32): communication -> optimizer stream
     for (auto& ev : t->bucket_events) cudaEventCreateWithFlags(&ev, cudaEventDisableTiming);
     // pass 2: build
@@ -1342,15 +1321,13 @@ static void enqueue_step(UbTrainer* t, const StepOpts& o, cudaStream_t st) {
     auto next_event = [&]() { return t->side_events[t->side_ev_next++ % t->side_events.size()]; };
     auto run = [&](std::vector<UbTrainer::Op>& ops, std::vector<UbTrainer::OpInfo>& info, const char* what) {
         for (size_t i = 0; i < ops.size(); ++i) {
-            static const bool skip_side = getenv("UB_DEBUG_SKIP_SIDE") != nullptr;  // timing experiments only
-            if (info[i].side == 1 && skip_side) continue;
-            if (info[i].side == 1 && t->use_side) {  // fork: the branch sees everything enqueued on the main stream so far
+            if (info[i].side == 1) {  // fork: the branch sees everything enqueued on the main stream so far
                 cudaEvent_t ev = next_event();
                 cudaEventRecord(ev, st);
                 cudaStreamWaitEvent(t->side_stream, ev, 0);
                 ops[i](t->side_stream);
                 side_dirty = true;
-            } else if (info[i].side == 3 && t->use_side) {  // a branch off the weight-gradient branch (time-MLP backward)
+            } else if (info[i].side == 3) {  // a branch off the weight-gradient branch (time-MLP backward)
                 cudaEvent_t ev = next_event();
                 cudaEventRecord(ev, side_dirty ? t->side_stream : st);
                 cudaStreamWaitEvent(t->aux_stream, ev, 0);
@@ -1383,8 +1360,7 @@ static void enqueue_step(UbTrainer* t, const StepOpts& o, cudaStream_t st) {
             }
         }
     };
-    static const bool opt_overlap = !(getenv("UB_NO_OPT_OVERLAP") && atoi(getenv("UB_NO_OPT_OVERLAP")) != 0);
-    t->opt_in_tape = o.update && opt_overlap && t->opt_overlap_ok;
+    t->opt_in_tape = o.update && t->opt_overlap_ok;
     t->o_lr = o.lr, t->o_b1 = o.b1, t->o_b2 = o.b2, t->o_eps = o.eps, t->o_wd = o.wd;
     t->opt_done_lo = t->nparams;
     run(t->fwd_ops, t->fwd_info, "forward");
