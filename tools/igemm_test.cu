@@ -1,7 +1,8 @@
 // Standalone GPU harness for the tcgen05 implicit-GEMM kernels (development tool, not part of the library).
-//   ./igemm_test [quick]
+//   ./igemm_test [quick | plans]
 // Checks igemm_conv (fprop, 1x1, two-segment, all epilogue modes) and igemm_wgrad against a CPU reference
 // computed from the same bf16-rounded operands, probes UMMA descriptor start-address/base_offset behaviour,
+// checks that both conv planners accept and reject the same epilogues (`plans`: only that table),
 // and prints CUDA-event timings.
 #include <cmath>
 #include <cstdio>
@@ -205,6 +206,96 @@ static bool test_conv(int B, int H, int W, int Cin, int Cout, int ntaps, int Cin
     cudaFree(dx), cudaFree(dw), cudaFree(dres), cudaFree(dbias), cudaFree(drow), cudaFree(dout);
     if (dx2) cudaFree(dx2), cudaFree(dw2);
     return bad == 0;
+}
+
+// ------------------------------------------------------------------------------------------ planner contract
+// Both conv planners must accept and reject the same epilogues, with the same codes, at a shape both kernels take
+// (B 2, 64->64 @ 64x64, 3x3).  Nothing is launched: the buffers only have to exist and be aligned.
+static void test_plan_contract() {
+    const int B = 2, H = 64, W = 64, C = 64;
+    const size_t act = size_t(B) * H * W * C, vec = size_t(B) * C * 2;
+    __nv_bfloat16 *x, *wp, *res, *gx, *out;
+    float *bias, *stats, *chsum, *gamma, *beta, *S;
+    CK(cudaMalloc(&x, act * 2));
+    CK(cudaMalloc(&wp, size_t(9) * C * C * 2));
+    CK(cudaMalloc(&res, act * 2));
+    CK(cudaMalloc(&gx, act * 2));
+    CK(cudaMalloc(&out, act * 4));  // room for an fp32 output
+    CK(cudaMalloc(&bias, 64 * 4));  // (bias, second bias, row vector: the planners only read the addresses)
+    CK(cudaMalloc(&stats, vec * 4));
+    CK(cudaMalloc(&chsum, vec * 4));
+    CK(cudaMalloc(&gamma, C * 4));
+    CK(cudaMalloc(&beta, C * 4));
+    CK(cudaMalloc(&S, vec * 4));
+    const ConvSegDesc seg = {x, C, C, wp, 9};
+    ConvEpilogue plain;
+    plain.bias = bias, plain.bias2 = bias, plain.rowvec = bias, plain.residual = res, plain.out = out;
+    ConvEpilogue st;
+    st.bias = bias, st.residual = res, st.out = out, st.stats = stats;
+    ConvEpilogue gn;
+    gn.out = out, gn.gn_x = gx, gn.gn_ldx = C, gn.gn_chsum = chsum, gn.gn_gamma = gamma, gn.gn_beta = beta;
+    gn.gn_S = S, gn.gn_silu = 1;
+    struct Case {
+        const char* name;
+        ConvEpilogue ep;
+        int want;
+    };
+    std::vector<Case> cases = {{"bias + bias2 + rowvec + residual", plain, 0}, {"statistics hook", st, 0},
+                               {"gn-bwd hook", gn, 0}};
+    auto add = [&](const char* name, ConvEpilogue ep, int want) { cases.push_back({name, ep, want}); };
+    {
+        ConvEpilogue e = gn;
+        e.stats = stats;
+        add("stats with gn_x", e, -15);
+        e = gn, e.residual = res;
+        add("gn_x with residual", e, -15);
+        e = gn, e.gn_chsum = nullptr;
+        add("gn_x without statistics", e, -15);
+        e = gn, e.gn_gamma = nullptr;
+        add("gn_x without gamma", e, -15);
+        e = gn, e.gn_beta = nullptr;
+        add("gn_x without beta", e, -15);
+        e = gn, e.gn_S = nullptr;
+        add("gn_x without S", e, -15);
+        e = gn, e.gn_groups = 24;
+        add("gn_groups not dividing Cout", e, -15);
+        e = gn, e.gn_ldx = 68;
+        add("gn_ldx % 8 != 0", e, -15);
+        e = gn, e.gn_x = gx + 1;
+        add("misaligned gn_x", e, -15);
+        e = st, e.out_mode = OUT_NHWC_F32;
+        add("stats with fp32 output", e, -15);
+        e = gn, e.out_mode = OUT_NCHW_F32;
+        add("gn_x with fp32 output", e, -15);
+        e = plain, e.bias = bias + 1;
+        add("misaligned bias", e, -8);
+        e = plain, e.bias2 = bias + 1;
+        add("misaligned bias2", e, -8);
+        e = plain, e.rowvec = bias + 1;
+        add("misaligned rowvec", e, -8);
+        e = plain, e.residual = res + 1;
+        add("misaligned residual", e, -7);
+        e = plain, e.ldr = 68;
+        add("ldr % 8 != 0", e, -7);
+        e = plain, e.out = out + 1;
+        add("misaligned output", e, -6);
+        e = plain, e.out = out + 1, e.out_mode = OUT_NHWC_F32;
+        add("misaligned fp32 output", e, -6);
+        e = plain, e.ldo = 68;
+        add("ldo % 8 != 0", e, -6);
+    }
+    printf("== planner contract (B%d %dx%d %d->%d taps9) ==\n", B, H, W, C, C);
+    for (const Case& c : cases) {
+        IgemmConvParams p;
+        IgemmRowsParams pr;
+        const int rc = igemm_conv_plan(&p, &seg, 1, B, H, W, C, c.ep);
+        const int rr = igemm_rows_plan(&pr, &seg, 1, B, H, W, C, c.ep, 148);
+        const bool ok = rc == c.want && rr == c.want;
+        printf("  %-34s conv %4d  rows %4d  (want %3d)  %s\n", c.name, rc, rr, c.want, ok ? "ok" : "FAIL");
+        if (!ok) g_fail++;
+    }
+    cudaFree(x), cudaFree(wp), cudaFree(res), cudaFree(gx), cudaFree(out), cudaFree(bias);
+    cudaFree(stats), cudaFree(chsum), cudaFree(gamma), cudaFree(beta), cudaFree(S);
 }
 
 // ------------------------------------------------------------------------------------------ wgrad test
@@ -523,6 +614,10 @@ int main(int argc, char** argv) {
                   OUT_NHWC_BF16, false, false, false, 2000, atoi(argv[9]), atoi(argv[8]) != 0);
         return g_fail ? 1 : 0;
     }
+    if (argc > 1 && !strcmp(argv[1], "plans")) {
+        test_plan_contract();
+        return g_fail ? 1 : 0;
+    }
     if (argc > 7 && !strcmp(argv[1], "wgrad")) {  // wgrad B H W Cin Cout reps
         test_wgrad(atoi(argv[2]), atoi(argv[3]), atoi(argv[4]), atoi(argv[5]), atoi(argv[6]), 9, 200, atoi(argv[7]));
         return g_fail ? 1 : 0;
@@ -535,6 +630,7 @@ int main(int argc, char** argv) {
     if (wgrad_only) goto wgrad_tests;
     printf("== descriptor probe ==\n");
     run_probe();
+    test_plan_contract();
 
     printf("== conv (fprop / 1x1 / fused) ==\n");
     // tiny shapes first: every output checked

@@ -23,6 +23,7 @@
 // Warp roles: warp 0 = TMA + MMA issue (one elected lane) + TMEM allocator; warps 1-8 = row threads (TMEM lane =
 // row; the two warps of a lane quadrant split the columns of every chunk).  mbarriers: load -> s (accumulators ready) -> p (operand written to smem) -> o (second MMA done).
 #include "attn_tc.cuh"
+#include "igemm.cuh"
 #include "launch.cuh"
 #include "ptx.cuh"
 
@@ -30,11 +31,6 @@
 #include <cstring>
 
 namespace ub {
-
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn igemm_encode_fn();
 
 namespace {
 
@@ -609,20 +605,6 @@ __global__ void __launch_bounds__(kThreads) attn_tc_dkv_kernel(const __grid_cons
     if (warp == 0) tmem_dealloc(tmem, 512);
 }
 
-int make_map_2d(CUtensorMap* m, const __nv_bfloat16* base, int cols, int rows, int ld) {
-    EncodeTiledFn fn = igemm_encode_fn();
-    if (!fn) return -10;
-    if ((reinterpret_cast<uintptr_t>(base) & 15) || (ld % 8) != 0) return -11;
-    cuuint64_t dims[2] = {cuuint64_t(cols), cuuint64_t(rows)};
-    cuuint64_t strides[1] = {cuuint64_t(ld) * 2};
-    cuuint32_t box[2] = {64, 128};
-    cuuint32_t es[2] = {1, 1};
-    CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<__nv_bfloat16*>(base), dims, strides, box, es,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    return r == CUDA_SUCCESS ? 0 : -12;
-}
-
 size_t smem_fwd(int ncols) { return 1024 + 16384 + size_t(ncols) * 512 + 4096 + 256; }
 size_t smem_dq(int ncols) { return 1024 + 32768 + size_t(ncols) * 256 + 32768 + 256; }
 size_t smem_dkv(int ncols) { return 1024 + 32768 + size_t(ncols) * 256 + 65536 + 4096 + 256; }
@@ -665,9 +647,9 @@ int attn_tc_plan(AttnTcParams* p, const __nv_bfloat16* qkv, int ld, int B, int T
     p->dsum = dsum;
     for (p->tshift = 0; (1 << p->tshift) < T; ++p->tshift) {
     }
-    int r = make_map_2d(&p->tmQKV, qkv, 3 * C, B * T, ld);
+    int r = make_bf16_map_2d(&p->tmQKV, qkv, 3 * C, B * T, ld, 128);
     if (r) return r;
-    if (dout) r = make_map_2d(&p->tmDO, dout, C, B * T, lddo);
+    if (dout) r = make_bf16_map_2d(&p->tmDO, dout, C, B * T, lddo, 128);
     return r;
 }
 

@@ -10,12 +10,9 @@
 //   * gn-bwd  : the epilogue of the dgrad conv that produces dL/d(silu(gn(x))) multiplies by silu'(gn(x)) on the
 //               spot, writes dz = dL/d(gn(x)) instead, and accumulates the per-(image, channel) sums of dz and
 //               dz * xhat (replaces gn_bwd_stats; gn_bwd_apply then needs no sigmoid at all).
-// Both reduce over the 32 pixels of a warp through a small smem transpose and add the warp totals of the CTA's
+// Both reduce over the 32 pixels of a warp by a 31-shuffle transpose-reduce and add the warp totals of the CTA's
 // epilogue warps in shared memory; one red.global.add.v2.f32 per (tile, channel) follows.
 #pragma once
-#ifndef UB_EPI_SHUFFLE_REDUCE
-#define UB_EPI_SHUFFLE_REDUCE 1
-#endif
 #include "igemm.cuh"
 #include "ptx.cuh"
 
@@ -38,6 +35,13 @@ struct EpiOut {
     int nacc = 1;
     uint32_t acc_stride = 0;
 };
+
+// the kernel-side view of a conv kernel's epilogue block (one accumulator; the two-stream kernel sets nacc, acc_stride)
+__device__ __forceinline__ EpiOut epi_out(const IgemmEpiParams& ep, int Cout, int H, int W) {
+    EpiOut e{ep.residual, ep.ldr, ep.out, ep.ldo, ep.out_mode, Cout, H, W};
+    e.stats = ep.stats, e.gx = ep.gn_x, e.ldgx = ep.gn_ldx, e.gS = ep.gn_S, e.gsilu = ep.gn_silu;
+    return e;
+}
 
 // v[0..16) = the 16 accumulator columns at taddr, summed over the kernel's accumulators
 __device__ __forceinline__ void epi_tmem_load16(const EpiOut& e, uint32_t taddr, uint32_t (&v)[16]) {
@@ -132,9 +136,6 @@ __device__ __forceinline__ void epi_chunk(const EpiOut& e, uint32_t taddr, const
 // reduction; lanes whose pixel is outside the tensor contribute zeros and store nothing.  All pixels of a warp belong
 // to one image (the plan guarantees it).  gconst = staged [4][BN] per-channel constants of that image (a = gamma*rstd,
 // bb = beta - mean*a, rstd, mean*rstd), offset to this chunk's first column (gn-bwd only); cstride = BN.
-// Column sums over the warp's 32 pixels go through a per-warp smem transpose tr[32][36] (f in columns 0..15, q in
-// 16..31; 144-byte rows keep both the 16-byte row stores and the column reads bank-conflict free): 8 STS.128 + 32
-// independent LDS per lane instead of a 5-stage shuffle butterfly -- the epilogue is latency-bound, not issue-bound.
 // xr holds the 16 channels [n, n+16) of the pixel's side input -- the residual row (stats mode) or the GroupNorm input
 // row (gn-bwd mode), never both (plan) -- fetched one chunk AHEAD (epi_side_load): a dependent global load per chunk
 // was the longest stall of the hooked epilogue.  On return xr holds the chunk at channel n_next (if n_next >= 0).
@@ -147,7 +148,7 @@ __device__ __forceinline__ void epi_side_load(const EpiOut& e, bool valid, size_
 }
 __device__ __forceinline__ void epi_chunk_gn(const EpiOut& e, uint32_t taddr, const float* comb, const float* gconst,
                                              int cstride, bool valid, size_t pix, int n, int lane, float* red,
-                                             float* tr, uint4 (&xr)[2], int n_next) {
+                                             uint4 (&xr)[2], int n_next) {
     uint32_t v[16];
     epi_tmem_load16(e, taddr, v);
     uint4 xn[2];
@@ -222,7 +223,6 @@ __device__ __forceinline__ void epi_chunk_gn(const EpiOut& e, uint32_t taddr, co
 #pragma unroll
         for (int j = 0; j < 16; ++j) f[j] = 0.f, q[j] = 0.f;
     }
-#if UB_EPI_SHUFFLE_REDUCE
     // Column sums over the warp's 32 pixels by a transpose-reduce butterfly: 31 shuffles move half as many bytes
     // through the SM's shuffle/shared-memory crossbar as the 8 STS.128 + 32 LDS of the shared-memory transpose
     // (64 wavefronts per chunk and warp; with 16 epilogue warps per SM that pipe is what bounds the hooked epilogue).
@@ -241,27 +241,6 @@ __device__ __forceinline__ void epi_chunk_gn(const EpiOut& e, uint32_t taddr, co
     }
     // lane L holds the warp's total of cs[L]: f column L for L < 16, q column L - 16 above
     sts_f32(smem_u32(red) + 4u * uint32_t(2 * (lane & 15) + (lane >> 4)), cs[0]);
-#else
-    const uint32_t tr_s = smem_u32(tr);
-    const uint32_t row_s = tr_s + uint32_t(lane) * 144u;
-#pragma unroll
-    for (int j = 0; j < 4; ++j) {
-        sts_v4(row_s + 16u * j, f[4 * j], f[4 * j + 1], f[4 * j + 2], f[4 * j + 3]);
-        sts_v4(row_s + 64u + 16u * j, q[4 * j], q[4 * j + 1], q[4 * j + 2], q[4 * j + 3]);
-    }
-    __syncwarp();
-    float s0 = 0.f, s1 = 0.f, s2 = 0.f, s3 = 0.f;
-    const uint32_t col_s = tr_s + 4u * uint32_t(lane);
-#pragma unroll
-    for (int r = 0; r < 32; r += 4) {
-        s0 += lds_f32(col_s + 144u * r), s1 += lds_f32(col_s + 144u * (r + 1));
-        s2 += lds_f32(col_s + 144u * (r + 2)), s3 += lds_f32(col_s + 144u * (r + 3));
-    }
-    __syncwarp();
-    // lane j < 16 holds the warp's total of f column j, lane 16 + j that of q column j: park them; epi_flush_stats
-    // adds the warps up and issues one vector RED per (tile, channel) (the L2 atomic unit serialises per address)
-    sts_f32(smem_u32(red) + 4u * uint32_t(2 * (lane & 15) + (lane >> 4)), (s0 + s1) + (s2 + s3));
-#endif
     xr[0] = xn[0], xr[1] = xn[1];
 }
 
@@ -293,8 +272,8 @@ __device__ __forceinline__ void epi_flush_stats(const float* red, float* dst, in
 // goes to warp i % nhalf.
 __device__ __forceinline__ void epi_row(const EpiOut& e, uint32_t trow, const float* comb, int BN, bool valid,
                                         size_t pix, int b, int h, int w, int n0, const float* gconst = nullptr,
-                                        int lane = 0, float* red = nullptr, float* tr = nullptr, int half = 0,
-                                        int nhalf = 1, uint4* side = nullptr) {
+                                        int lane = 0, float* red = nullptr, int half = 0, int nhalf = 1,
+                                        uint4* side = nullptr) {
     if (e.stats || e.gx) {  // BN % 32 == 0 (plan); red = this quadrant's [BN][2] row of the reduction scratch
         // side = the first chunk's side input, loaded by the caller (epi_side_load at channel n0 + 16 * half) before
         // it waited for the accumulator
@@ -302,7 +281,7 @@ __device__ __forceinline__ void epi_row(const EpiOut& e, uint32_t trow, const fl
         for (int c0 = 16 * half; c0 < BN; c0 += 16 * nhalf) {
             const int cn = c0 + 16 * nhalf;
             epi_chunk_gn(e, trow + uint32_t(c0), comb + c0, gconst + c0, BN, valid, pix, n0 + c0, lane, red + 2 * c0,
-                         tr, xr, cn < BN ? n0 + cn : -1);
+                         xr, cn < BN ? n0 + cn : -1);
         }
         return;
     }

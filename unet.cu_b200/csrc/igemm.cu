@@ -243,7 +243,7 @@ __device__ __forceinline__ void igemm_conv_body(const IgemmConvParams& p) {
                 l2_prefetch_bulk(p.seg[s].wp + (size_t(tap) * p.Cout + n0) * p.seg[s].Cin,
                                  uint32_t(p.BN) * uint32_t(p.seg[s].Cin) * 2u);
     }
-    if (warp == 3 && lane == 0 && p.gn_x) {
+    if (warp == 3 && lane == 0 && p.epi.gn_x) {
         // gn-bwd hook: the GroupNorm input rows of this pixel tile were written in the forward pass (long evicted);
         // fetch them into L2 now instead of at the epilogue's dependent per-chunk loads.  A pixel row of the tile is
         // contiguous over all channels; the N tiles of the grid share the rows.
@@ -252,8 +252,8 @@ __device__ __forceinline__ void igemm_conv_body(const IgemmConvParams& p) {
             const int b = b0 + r / p.TH, h = h0 + r % p.TH;
             if (b < p.B && h < p.H) {
                 const int wn = min(p.TW, p.W - w0);
-                l2_prefetch_bulk(p.gn_x + ((size_t(b) * p.H + h) * p.W + w0) * p.gn_ldx,
-                                 (uint32_t(wn - 1) * uint32_t(p.gn_ldx) + uint32_t(p.Cout)) * 2u);
+                l2_prefetch_bulk(p.epi.gn_x + ((size_t(b) * p.H + h) * p.W + w0) * p.epi.gn_ldx,
+                                 (uint32_t(wn - 1) * uint32_t(p.epi.gn_ldx) + uint32_t(p.Cout)) * 2u);
             }
         }
     }
@@ -304,19 +304,19 @@ __device__ __forceinline__ void igemm_conv_body(const IgemmConvParams& p) {
         // embedding vector is used (p.ncomb == TB), a single shared row otherwise
         const int et = threadIdx.x - 64;
         for (int i = 0; i < p.ncomb; ++i)
-            epi_stage_comb(comb + i * p.BN, p.bias, p.bias2, p.rowvec, min(b0 + i, p.B - 1), p.Cout, n0, p.BN, et,
-                           kEpiThreads);
+            epi_stage_comb(comb + i * p.BN, p.epi.bias, p.epi.bias2, p.epi.rowvec, min(b0 + i, p.B - 1), p.Cout, n0,
+                           p.BN, et, kEpiThreads);
         for (int i = 0; i < p.ngimg; ++i)
-            epi_stage_gconst(gconst + i * 4 * p.BN, p.gn_chsum, p.gn_gamma, p.gn_beta, min(b0 + i, p.B - 1), p.Cout,
-                             p.gn_cpg, p.H * p.W, n0, p.BN, et, kEpiThreads);
+            epi_stage_gconst(gconst + i * 4 * p.BN, p.epi.gn_chsum, p.epi.gn_gamma, p.epi.gn_beta, min(b0 + i, p.B - 1),
+                             p.Cout, p.epi.gn_cpg, p.H * p.W, n0, p.BN, et, kEpiThreads);
         named_bar_sync(1, kEpiThreads);
 
         const size_t pix = (size_t(b) * p.H + h) * p.W + w;
-        EpiOut eo{p.residual, p.ldr, p.out, p.ldo, p.out_mode, p.Cout, p.H, p.W};
-        eo.stats = p.stats, eo.gx = p.gn_x, eo.ldgx = p.gn_ldx, eo.gS = p.gn_S, eo.gsilu = p.gn_silu;
+        EpiOut eo = epi_out(p.epi, p.Cout, p.H, p.W);
         eo.nacc = NACC, eo.acc_stride = uint32_t(p.BN);
         uint4 side[2];
-        if (p.stats || p.gn_x) epi_side_load(eo, valid, pix, n0 + 16 * half, side);  // hidden behind the main loop
+        // (the first side-input chunk of a hook is loaded here, hidden behind the main loop)
+        if (p.epi.stats || p.epi.gn_x) epi_side_load(eo, valid, pix, n0 + 16 * half, side);
 
         mbar_wait(tmem_full_bar, 0);
         pdl_trigger_late();  // main loop complete: the next kernel's prologue may overlap this epilogue
@@ -345,15 +345,15 @@ __device__ __forceinline__ void igemm_conv_body(const IgemmConvParams& p) {
                     uint32_t v[16];
                     epi_tmem_load16(eo, tmem_base + (uint32_t(q * 32) << 16) + uint32_t(c0), v);
                     uint4 r[2];
-                    if (p.residual && valid) {
-                        const uint4* rp = reinterpret_cast<const uint4*>(p.residual + pix * p.ldr + n0 + c0);
+                    if (p.epi.residual && valid) {
+                        const uint4* rp = reinterpret_cast<const uint4*>(p.epi.residual + pix * p.epi.ldr + n0 + c0);
                         r[0] = rp[0], r[1] = rp[1];
                     }
                     tmem_ld_wait();
                     float f[16];
 #pragma unroll
                     for (int j = 0; j < 16; ++j) f[j] = valid ? __uint_as_float(v[j]) + cmb[c0 + j] : 0.f;
-                    if (p.residual && valid) {
+                    if (p.epi.residual && valid) {
 #pragma unroll
                         for (int j = 0; j < 2; ++j) {
                             float t[8];
@@ -417,7 +417,7 @@ __device__ __forceinline__ void igemm_conv_body(const IgemmConvParams& p) {
                         tmem_ld16(t_stat + (uint32_t(q * 32) << 16) + uint32_t(img * 32 + 16), qv);
                         tmem_ld_wait();
                         if (cv && b0 + img < p.B) {
-                            float* d = p.stats + (size_t(b0 + img) * p.Cout + n0 + chn) * 2;
+                            float* d = p.epi.stats + (size_t(b0 + img) * p.Cout + n0 + chn) * 2;
                             asm volatile("red.global.add.v2.f32 [%0], {%1, %2};" ::"l"(d), "f"(__uint_as_float(sv[0])),
                                          "f"(__uint_as_float(qv[0]))
                                          : "memory");
@@ -434,13 +434,11 @@ __device__ __forceinline__ void igemm_conv_body(const IgemmConvParams& p) {
         // GroupNorm hooks: all 32 pixels of a warp lie in one image of the tile (plan)
         const int lbw = min(lb, p.TB - 1);
         epi_row(eo, tmem_base + (uint32_t(q * 32) << 16), comb + (p.ncomb > 1 ? min(lb, p.ncomb - 1) : 0) * p.BN, p.BN,
-                valid, pix, b, h, w, n0, gconst + lbw * 4 * p.BN, lane, red + size_t(q) * p.BN * 2,
-                // per-warp transpose scratch: the pipeline stages are free once the accumulator is complete
-                reinterpret_cast<float*>(smem) + (warp - 2) * (32 * 36), half, 2, side);
-        if (p.stats || p.gn_x) {
+                valid, pix, b, h, w, n0, gconst + lbw * 4 * p.BN, lane, red + size_t(q) * p.BN * 2, half, 2, side);
+        if (p.epi.stats || p.epi.gn_x) {
             named_bar_sync(1, kEpiThreads);
-            epi_flush_stats(red, p.gn_x ? p.gn_S : p.stats, p.Cout, n0, p.BN, b0, p.B, p.TW * p.TH, p.TB, et,
-                            kEpiThreads);
+            epi_flush_stats(red, p.epi.gn_x ? p.epi.gn_S : p.epi.stats, p.Cout, n0, p.BN, b0, p.B, p.TW * p.TH, p.TB,
+                            et, kEpiThreads);
         }
         }  // !done_ms
         if (threadIdx.x == 64) UB_TR(9, (unsigned long long)clock64());
@@ -823,11 +821,7 @@ static EncodeTiledFn get_encode_fn() {
     return fn;
 }
 
-EncodeTiledFn igemm_encode_fn() { return get_encode_fn(); }
-
-// NHWC bf16 activation map: dims (C, W, H, B), channel pitch ld, box (64, TW, TH, TB), 128B swizzle, zero OOB fill.
-static int make_act_map(CUtensorMap* m, const __nv_bfloat16* x, int C, int ld, int W, int H, int B, int TW, int TH,
-                        int TB) {
+int make_act_map(CUtensorMap* m, const __nv_bfloat16* x, int C, int ld, int W, int H, int B, int TW, int TH, int TB) {
     EncodeTiledFn fn = get_encode_fn();
     if (!fn) return -10;
     if ((reinterpret_cast<uintptr_t>(x) & 15) || (ld % 8) != 0) return -11;
@@ -846,20 +840,20 @@ static int make_act_map(CUtensorMap* m, const __nv_bfloat16* x, int C, int ld, i
     return 0;
 }
 
-static int make_weight_map(CUtensorMap* m, const __nv_bfloat16* wp, int Cin, int rows, int BN) {
+int make_bf16_map_2d(CUtensorMap* m, const __nv_bfloat16* base, int cols, int rows, int ld, int box_rows) {
     EncodeTiledFn fn = get_encode_fn();
     if (!fn) return -10;
-    if ((reinterpret_cast<uintptr_t>(wp) & 15) || (Cin % 8) != 0) return -13;
-    cuuint64_t dims[2] = {cuuint64_t(Cin), cuuint64_t(rows)};
-    cuuint64_t strides[1] = {cuuint64_t(Cin) * 2};
-    cuuint32_t box[2] = {64, cuuint32_t(BN)};
+    if ((reinterpret_cast<uintptr_t>(base) & 15) || (ld % 8) != 0) return -13;
+    cuuint64_t dims[2] = {cuuint64_t(cols), cuuint64_t(rows)};
+    cuuint64_t strides[1] = {cuuint64_t(ld) * 2};
+    cuuint32_t box[2] = {64, cuuint32_t(box_rows)};
     cuuint32_t es[2] = {1, 1};
-    CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<__nv_bfloat16*>(wp), dims, strides, box, es,
+    CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<__nv_bfloat16*>(base), dims, strides, box, es,
                     CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
                     CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
     if (r != CUDA_SUCCESS) {
-        fprintf(stderr, "[unet_b200] cuTensorMapEncodeTiled(weight Cin=%d rows=%d BN=%d) -> %d\n", Cin, rows, BN,
-                int(r));
+        fprintf(stderr, "[unet_b200] cuTensorMapEncodeTiled(2d cols=%d rows=%d ld=%d box_rows=%d) -> %d\n", cols, rows,
+                ld, box_rows, int(r));
         return -14;
     }
     return 0;
@@ -874,18 +868,50 @@ static int ceil_div_i(int a, int b) { return (a + b - 1) / b; }
 
 static constexpr int kBarrierBytes = 256;
 
+int igemm_epi_plan(IgemmEpiParams* e, const ConvEpilogue& ep, int Cout) {
+    *e = IgemmEpiParams{};
+    e->bias = ep.bias, e->bias2 = ep.bias2, e->rowvec = ep.rowvec, e->residual = ep.residual;
+    e->ldr = ep.ldr ? ep.ldr : Cout;
+    e->out = ep.out, e->ldo = ep.ldo ? ep.ldo : Cout, e->out_mode = ep.out_mode;
+    e->stats = ep.stats;
+    e->gn_x = ep.gn_x, e->gn_ldx = ep.gn_ldx, e->gn_chsum = ep.gn_chsum, e->gn_gamma = ep.gn_gamma;
+    e->gn_beta = ep.gn_beta, e->gn_S = ep.gn_S, e->gn_silu = ep.gn_silu;
+    if (ep.stats || ep.gn_x) {
+        if ((ep.stats && ep.gn_x) || ep.out_mode != OUT_NHWC_BF16) return -15;
+        if (ep.gn_x) {
+            if (ep.residual || !ep.gn_chsum || !ep.gn_gamma || !ep.gn_beta || !ep.gn_S || ep.gn_groups < 1 ||
+                Cout % ep.gn_groups)
+                return -15;
+            if ((ep.gn_ldx % 8) != 0 || (reinterpret_cast<uintptr_t>(ep.gn_x) & 15)) return -15;
+            e->gn_cpg = Cout / ep.gn_groups;
+        }
+    }
+    if (e->out_mode != OUT_NCHW_F32) {
+        const int esz = e->out_mode == OUT_NHWC_BF16 ? 2 : 4;
+        if ((e->ldo * esz) % 16 != 0 || (reinterpret_cast<uintptr_t>(e->out) & 15)) return -6;
+    }
+    if (e->residual && ((e->ldr % 8) != 0 || (reinterpret_cast<uintptr_t>(e->residual) & 15))) return -7;
+    if (e->bias && (reinterpret_cast<uintptr_t>(e->bias) & 15)) return -8;
+    if (e->bias2 && (reinterpret_cast<uintptr_t>(e->bias2) & 15)) return -8;
+    if (e->rowvec && ((reinterpret_cast<uintptr_t>(e->rowvec) & 15) || (Cout % 4) != 0)) return -8;
+    return 0;
+}
+
 int igemm_conv_plan(IgemmConvParams* p, const ConvSegDesc* segs, int nseg, int B, int H, int W, int Cout,
                     const ConvEpilogue& ep) {
     memset(p, 0, sizeof(*p));
     if (nseg < 1 || nseg > 2) return -1;
     if (Cout % 16 != 0) return -2;
     // pixel tile first (needed to count CTAs)
-    const int TW0 = W < 128 ? W : 128;
-    int TH0 = H < 128 / TW0 ? H : 128 / TW0;
-    if (TH0 < 1) TH0 = 1;
-    int TB0 = B < 128 / (TW0 * TH0) ? B : 128 / (TW0 * TH0);
-    if (TB0 < 1) TB0 = 1;
-    const int pix_tiles = ceil_div_i(W, TW0) * ceil_div_i(H, TH0) * ceil_div_i(B, TB0);
+    p->TW = W < 128 ? W : 128;
+    p->TH = H < 128 / p->TW ? H : 128 / p->TW;
+    if (p->TH < 1) p->TH = 1;
+    p->TB = B < 128 / (p->TW * p->TH) ? B : 128 / (p->TW * p->TH);
+    if (p->TB < 1) p->TB = 1;
+    p->tiles_w = ceil_div_i(W, p->TW);
+    p->tiles_h = ceil_div_i(H, p->TH);
+    p->tiles_b = ceil_div_i(B, p->TB);
+    const int pix_tiles = p->tiles_w * p->tiles_h * p->tiles_b;
     // output-channel tile: the largest divisor of Cout that is a multiple of 16 and <= 256 -- but small problems
     // (8x8 / 16x16 layers) would then run on a handful of SMs, each limited by its own L2->SMEM bandwidth, so BN is
     // lowered (not below 64) until there are ~128 CTAs.
@@ -901,14 +927,6 @@ int igemm_conv_plan(IgemmConvParams* p, const ConvSegDesc* segs, int nseg, int B
     if (!BN) return -2;
     p->nseg = nseg;
     p->B = B, p->H = H, p->W = W, p->Cout = Cout, p->BN = BN;
-    p->TW = W < 128 ? W : 128;
-    p->TH = H < 128 / p->TW ? H : 128 / p->TW;
-    if (p->TH < 1) p->TH = 1;
-    p->TB = B < 128 / (p->TW * p->TH) ? B : 128 / (p->TW * p->TH);
-    if (p->TB < 1) p->TB = 1;
-    p->tiles_w = ceil_div_i(W, p->TW);
-    p->tiles_h = ceil_div_i(H, p->TH);
-    p->tiles_b = ceil_div_i(B, p->TB);
     // Two MMA streams for grids of at most one CTA per SM (see igemm_conv_body); both accumulators within 256 TMEM
     // columns so that a weight-gradient CTA of the side stream still finds room.
     p->nacc = 1;
@@ -959,37 +977,18 @@ int igemm_conv_plan(IgemmConvParams* p, const ConvSegDesc* segs, int nseg, int B
         if (d.Cin % 8 != 0) return -5;
         int r = make_act_map(&p->seg[s].tmA, d.x, d.Cin, d.ldx, W, H, B, p->TW, p->TH, p->TB);
         if (r) return r;
-        r = make_weight_map(&p->seg[s].tmW, d.wp, d.Cin, d.ntaps * Cout, BN);
+        r = make_bf16_map_2d(&p->seg[s].tmW, d.wp, d.Cin, d.ntaps * Cout, d.Cin, BN);
         if (r) return r;
         p->seg[s].cblocks = ceil_div_i(d.Cin, 64);
         p->seg[s].ntaps = d.ntaps;
         p->seg[s].wp = d.wp, p->seg[s].Cin = d.Cin;
     }
-    p->bias = ep.bias;
-    p->bias2 = ep.bias2;
-    p->rowvec = ep.rowvec;
-    p->residual = ep.residual;
-    p->ldr = ep.ldr ? ep.ldr : Cout;
-    p->out = ep.out;
-    p->ldo = ep.ldo ? ep.ldo : Cout;
-    p->out_mode = ep.out_mode;
-    p->ncomb = p->rowvec ? p->TB : 1;
-    p->stats = ep.stats;
-    p->gn_x = ep.gn_x, p->gn_ldx = ep.gn_ldx, p->gn_chsum = ep.gn_chsum, p->gn_gamma = ep.gn_gamma;
-    p->gn_beta = ep.gn_beta, p->gn_S = ep.gn_S, p->gn_silu = ep.gn_silu;
+    // the hooks' tiling conditions: 32-column chunks, and the 32 pixels a warp reduces over lie in one image
+    if (gn_hook && (BN % 32 != 0 || ((p->TW * p->TH) % 32 != 0 && p->TB > 1))) return -15;
+    int r = igemm_epi_plan(&p->epi, ep, Cout);
+    if (r) return r;
+    p->ncomb = ep.rowvec ? p->TB : 1;
     p->ngimg = ep.gn_x ? p->TB : 0;
-    if (gn_hook) {
-        if (ep.stats && ep.gn_x) return -15;
-        if (p->out_mode != OUT_NHWC_BF16 || BN % 32 != 0) return -15;
-        if ((p->TW * p->TH) % 32 != 0 && p->TB > 1) return -15;  // a warp's 32 pixels must share one image
-        if (ep.gn_x) {
-            if (ep.residual) return -15;
-            if (!ep.gn_chsum || !ep.gn_gamma || !ep.gn_beta || !ep.gn_S || ep.gn_groups < 1 || Cout % ep.gn_groups)
-                return -15;
-            if ((ep.gn_ldx % 8) != 0 || (reinterpret_cast<uintptr_t>(ep.gn_x) & 15)) return -15;
-            p->gn_cpg = Cout / ep.gn_groups;
-        }
-    }
     p->nred = gn_hook ? 8 : 0;
     {
         // tensor-core statistics + TMA output store (IgemmConvParams::ms) for the plain stats hook on full
@@ -997,34 +996,26 @@ int igemm_conv_plan(IgemmConvParams* p, const ConvSegDesc* segs, int nseg, int B
         // (measured round 2: 5.015 ms per step with, 5.043 with the shuffle-reduce statistics; measured, removed)
         const bool full_tiles = W % p->TW == 0 && H % p->TH == 0 && p->TW * p->TH * p->TB == 128;
         const size_t need = size_t(2 * (BN / 64) + 1) * 16384;  // Y atoms, Y*Y atoms, ones tile in the dead stages
-        if (ep.stats && !ep.gn_x && p->out_mode == OUT_NHWC_BF16 && (BN == 64 || BN == 128) &&
+        if (ep.stats && !ep.gn_x && ep.out_mode == OUT_NHWC_BF16 && (BN == 64 || BN == 128) &&
             p->nacc <= 2 && (p->TB == 1 || (p->TB == 2 && (p->TW * p->TH) == 64)) && full_tiles &&
             need <= size_t(p->stages) * p->stage_bytes && p->nacc * BN + 64 <= (p->nacc == 1 ? 256 : 512) &&
-            make_act_map(&p->tmO, reinterpret_cast<const __nv_bfloat16*>(ep.out), Cout, p->ldo, W, H, B, p->TW, p->TH,
-                         p->TB) == 0) {
+            make_act_map(&p->tmO, reinterpret_cast<const __nv_bfloat16*>(ep.out), Cout, p->epi.ldo, W, H, B, p->TW,
+                         p->TH, p->TB) == 0) {
             p->ms = 1;
             p->tmem_cols = next_pow2(p->nacc * BN + 64);
         }
         // ms == 2, store-only: a conv without any hook whose output is an NHWC bf16 tensor leaves through the same staged
         // tile + TMA store (any whole-tile shape, N tiles of 64 .. 256 channels)
-        if (!p->ms && !gn_hook && p->out_mode == OUT_NHWC_BF16 && BN % 64 == 0 &&
+        if (!p->ms && !gn_hook && ep.out_mode == OUT_NHWC_BF16 && BN % 64 == 0 &&
             p->nacc <= 2 && full_tiles && size_t(BN / 64) * 16384 <= size_t(p->stages) * p->stage_bytes &&
-            make_act_map(&p->tmO, reinterpret_cast<const __nv_bfloat16*>(ep.out), Cout, p->ldo, W, H, B, p->TW, p->TH,
-                         p->TB) == 0)
+            make_act_map(&p->tmO, reinterpret_cast<const __nv_bfloat16*>(ep.out), Cout, p->epi.ldo, W, H, B, p->TW,
+                         p->TH, p->TB) == 0)
             p->ms = 2;
     }
     if (size_t(p->ncomb + 4 * p->ngimg + p->nred) * BN * sizeof(float) > 24576) return -9;  // smem tail budget
     if (size_t(p->stages) * p->stage_bytes + 1024 + kBarrierBytes +
             size_t(p->ncomb + 4 * p->ngimg + p->nred) * BN * sizeof(float) > size_t(227) * 1024)
         return -3;
-    if (p->out_mode != OUT_NCHW_F32) {
-        const int esz = p->out_mode == OUT_NHWC_BF16 ? 2 : 4;
-        if ((p->ldo * esz) % 16 != 0 || (reinterpret_cast<uintptr_t>(p->out) & 15)) return -6;
-    }
-    if (p->residual && ((p->ldr % 8) != 0 || (reinterpret_cast<uintptr_t>(p->residual) & 15))) return -7;
-    if (p->bias && (reinterpret_cast<uintptr_t>(p->bias) & 15)) return -8;
-    if (p->bias2 && (reinterpret_cast<uintptr_t>(p->bias2) & 15)) return -8;
-    if (p->rowvec && ((reinterpret_cast<uintptr_t>(p->rowvec) & 15) || (Cout % 4) != 0)) return -8;
     return 0;
 }
 

@@ -29,6 +29,27 @@ struct IgemmSeg {
     int Cin;
 };
 
+// The resolved epilogue of both conv kernels (igemm_epi_plan): what epilogue.cuh applies to the accumulator.
+struct IgemmEpiParams {
+    const float* bias;             // [Cout] or nullptr
+    const float* bias2;            // second [Cout] bias (fused 1x1 skip conv) or nullptr
+    const float* rowvec;           // [B][Cout] per-image additive vector (time-embedding) or nullptr
+    const __nv_bfloat16* residual; // NHWC bf16 [B,H,W,ldr] added to the output, or nullptr
+    int ldr;
+    void* out;
+    int ldo;  // channel pitch of an NHWC output (>= Cout; lets a producer write into a concat buffer)
+    int out_mode;
+    // fused GroupNorm hooks (see epilogue.cuh); NHWC bf16 output
+    float* stats;                   // [B][Cout][2] += (sum, sumsq) of the output, or nullptr
+    const __nv_bfloat16* gn_x;      // gn-bwd: GroupNorm input (Cout channels, pitch gn_ldx), or nullptr
+    int gn_ldx;
+    const float* gn_chsum;          // forward statistics of gn_x [B][Cout][2]
+    const float* gn_gamma;
+    const float* gn_beta;
+    float* gn_S;                    // [B][Cout][2] += (sum dz, sum dz*xhat)
+    int gn_silu, gn_cpg;
+};
+
 struct IgemmConvParams {
     IgemmSeg seg[2];
     int nseg;
@@ -43,24 +64,7 @@ struct IgemmConvParams {
     int ncomb;       // rows of the staged per-channel addend (TB when a per-image vector is fused, else 1)
     uint32_t a_bytes, b_bytes;  // TMA transaction bytes per stage
     uint32_t stage_bytes;       // smem bytes per stage (A tile 16 KiB + B tile, 1024-aligned)
-    // epilogue
-    const float* bias;             // [Cout] or nullptr
-    const float* bias2;            // second [Cout] bias (fused 1x1 skip conv) or nullptr
-    const float* rowvec;           // [B][Cout] per-image additive vector (time-embedding) or nullptr
-    const __nv_bfloat16* residual; // NHWC bf16 [B,H,W,ldr] added to the output, or nullptr
-    int ldr;
-    void* out;
-    int ldo;  // channel pitch of an NHWC output (>= Cout; lets a producer write into a concat buffer)
-    int out_mode;
-    // fused GroupNorm hooks (see epilogue.cuh); NHWC bf16 output, BN % 32 == 0, a warp's 32 pixels in one image
-    float* stats;                   // [B][Cout][2] += (sum, sumsq) of the output, or nullptr
-    const __nv_bfloat16* gn_x;      // gn-bwd: GroupNorm input (Cout channels, pitch gn_ldx), or nullptr
-    int gn_ldx;
-    const float* gn_chsum;          // forward statistics of gn_x [B][Cout][2]
-    const float* gn_gamma;
-    const float* gn_beta;
-    float* gn_S;                    // [B][Cout][2] += (sum dz, sum dz*xhat)
-    int gn_silu, gn_cpg;
+    IgemmEpiParams epi;         // with a GroupNorm hook: BN % 32 == 0 and a warp's 32 pixels in one image
     int ngimg;                      // rows of the staged GroupNorm constants (TB when gn_x is set, else 0)
     int nred;                       // BN-float rows of the cross-warp reduction scratch (8 with a hook, else 0)
     // GroupNorm statistics on the tensor core (the plain statistics hook on full tiles) --
@@ -71,7 +75,7 @@ struct IgemmConvParams {
     CUtensorMap tmO;                // output tensor, box (64, TW, TH, TB), SWIZZLE_128B (ms only)
 };
 
-// persistent row-tile variant (igemm_rows.cu); same segments / epilogue as IgemmConvParams
+// persistent row-tile variant (igemm_rows.cu); same segments and epilogue block as IgemmConvParams
 struct IgemmRowsParams {
     IgemmSeg seg[2];  // tmA box = (64, W, box_rows, 1), tmW box = (64, BN)
     int nseg;
@@ -85,22 +89,7 @@ struct IgemmRowsParams {
     int w_resident;     // the weight ring holds the layer's whole weight set (ntaps tiles), loaded once per CTA
     int grid;
     uint32_t a_bytes, a_stage_bytes, w_bytes, w_stage_bytes;
-    const float* bias;
-    const float* bias2;
-    const float* rowvec;
-    const __nv_bfloat16* residual;
-    int ldr;
-    void* out;
-    int ldo;
-    int out_mode;
-    float* stats;
-    const __nv_bfloat16* gn_x;
-    int gn_ldx;
-    const float* gn_chsum;
-    const float* gn_gamma;
-    const float* gn_beta;
-    float* gn_S;
-    int gn_silu, gn_cpg;
+    IgemmEpiParams epi;
 };
 
 struct IgemmWgradParams {
@@ -170,6 +159,15 @@ struct ConvEpilogue {
     float* gn_S = nullptr;
     int gn_silu = 0, gn_groups = 32;
 };
+// Fills `e` from `ep` (ldr, ldo default to Cout; gn_cpg = Cout / gn_groups) and checks the epilogue contract both conv
+// kernels share.  Returns 0 or -15 (GroupNorm hook), -6 (output), -7 (residual), -8 (bias, bias2, rowvec).  The
+// planners add the checks that depend on their tiling.
+int igemm_epi_plan(IgemmEpiParams* e, const ConvEpilogue& ep, int Cout);
+// TMA maps (bf16, 128-byte swizzle, zero fill out of bounds).  make_act_map: NHWC activations, dims (C, W, H, B),
+// channel pitch ld, box (64, TW, TH, TB); -11 misaligned, -12 encode failed.  make_bf16_map_2d: row-major
+// [rows][cols] with pitch ld, box (64, box_rows); -13 misaligned, -14 encode failed.  Both: -10 no driver entry point.
+int make_act_map(CUtensorMap* m, const __nv_bfloat16* x, int C, int ld, int W, int H, int B, int TW, int TH, int TB);
+int make_bf16_map_2d(CUtensorMap* m, const __nv_bfloat16* base, int cols, int rows, int ld, int box_rows);
 // One-time kernel attribute setup (opt-in shared memory); safe to call repeatedly, call before graph capture.
 void igemm_init();
 // Fills `p` (tensor maps + tiling). Returns 0 or a negative error code (unsupported shape).

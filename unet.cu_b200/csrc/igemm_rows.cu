@@ -86,11 +86,9 @@ struct RowsBars {
     uint32_t pad_[3];
 };
 // smem tail behind the rings (floats): comb[2][BN] | gconst[2][4][BN] | red[8][BN][2]
-// (+ tr[8][32*36], the per-warp transpose scratch, only in the UB_EPI_SHUFFLE_REDUCE=0 experiment build: its 36 KiB are
-//  four more weight stages in the default build, which is what hides the ~1300-cycle TMA latency, r02b_rows_trace)
 // (16 epilogue warps -- a column split on top of quadrant x half -- measured 20 % slower: the 102-register cap of a
 // 640-thread CTA spills in the hooked chunk)
-static size_t rows_tail_floats(int BN) { return size_t(2 + 8 + 16) * BN + (UB_EPI_SHUFFLE_REDUCE ? 0 : 8 * 32 * 36); }
+static size_t rows_tail_floats(int BN) { return size_t(2 + 8 + 16) * BN; }
 
 __global__ void __launch_bounds__(kRowsThreads, 1) igemm_rows_kernel(const __grid_constant__ IgemmRowsParams p) {
     extern __shared__ uint8_t smem_raw[];
@@ -101,7 +99,6 @@ __global__ void __launch_bounds__(kRowsThreads, 1) igemm_rows_kernel(const __gri
     float* comb = reinterpret_cast<float*>(bars + 1);
     float* gconst = comb + 2 * p.BN;
     float* red = gconst + 8 * p.BN;
-    float* tr = red + 16 * p.BN;
 
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
     const int tiles_mb = p.B * p.tiles_per_img;  // pixel tiles; the N tile is the slow index of the schedule
@@ -124,11 +121,11 @@ __global__ void __launch_bounds__(kRowsThreads, 1) igemm_rows_kernel(const __gri
         tmem_alloc(&bars->tmem_slot, 512);
         tmem_relinquish();
     }
-    if (warp == 4 && lane == 0 && p.gn_x && int(blockIdx.x) < p.num_tiles) {  // first tile's GroupNorm-input rows -> L2
+    if (warp == 4 && lane == 0 && p.epi.gn_x && int(blockIdx.x) < p.num_tiles) {  // first tile's GN-input rows -> L2
         const int mt = int(blockIdx.x) % tiles_mb;
         const int b = mt / p.tiles_per_img, h0 = (mt % p.tiles_per_img) * p.TH;
-        l2_prefetch_bulk(p.gn_x + ((size_t(b) * p.H + h0) * p.W) * p.gn_ldx,
-                         (uint32_t(min(p.TH, p.H - h0) * p.W - 1) * uint32_t(p.gn_ldx) + uint32_t(p.Cout)) * 2u);
+        l2_prefetch_bulk(p.epi.gn_x + ((size_t(b) * p.H + h0) * p.W) * p.epi.gn_ldx,
+                         (uint32_t(min(p.TH, p.H - h0) * p.W - 1) * uint32_t(p.epi.gn_ldx) + uint32_t(p.Cout)) * 2u);
     }
     tc_fence_before();
     __syncthreads();
@@ -248,9 +245,8 @@ __global__ void __launch_bounds__(kRowsThreads, 1) igemm_rows_kernel(const __gri
         // ------------------------------------------------------------------ epilogue: quadrant q of M half `half`
         const int q = warp & 3, half = (warp - 4) >> 2;
         const int et = threadIdx.x - 128;
-        EpiOut eo{p.residual, p.ldr, p.out, p.ldo, p.out_mode, p.Cout, p.H, p.W};
-        eo.stats = p.stats, eo.gx = p.gn_x, eo.ldgx = p.gn_ldx, eo.gS = p.gn_S, eo.gsilu = p.gn_silu;
-        const bool hook = p.stats || p.gn_x;
+        EpiOut eo = epi_out(p.epi, p.Cout, p.H, p.W);
+        const bool hook = p.epi.stats || p.epi.gn_x;
         int it = 0;
         for (int tile = blockIdx.x; tile < p.num_tiles; tile += gridDim.x, ++it) {
             const int n0 = (tile / tiles_mb) * p.BN;
@@ -261,20 +257,20 @@ __global__ void __launch_bounds__(kRowsThreads, 1) igemm_rows_kernel(const __gri
             // double buffered: a fast warp may stage tile i+1 while a slow one still reads tile i's
             float* cb_ = comb + buf * p.BN;
             float* gc_ = gconst + buf * 4 * p.BN;
-            epi_stage_comb(cb_, p.bias, p.bias2, p.rowvec, b, p.Cout, n0, p.BN, et, kRowsEpiThreads);
-            if (p.gn_x)
-                epi_stage_gconst(gc_, p.gn_chsum, p.gn_gamma, p.gn_beta, b, p.Cout, p.gn_cpg, p.H * p.W, n0, p.BN, et,
-                                 kRowsEpiThreads);
+            epi_stage_comb(cb_, p.epi.bias, p.epi.bias2, p.epi.rowvec, b, p.Cout, n0, p.BN, et, kRowsEpiThreads);
+            if (p.epi.gn_x)
+                epi_stage_gconst(gc_, p.epi.gn_chsum, p.epi.gn_gamma, p.epi.gn_beta, b, p.Cout, p.epi.gn_cpg, p.H * p.W,
+                                 n0, p.BN, et, kRowsEpiThreads);
             named_bar_sync(1, kRowsEpiThreads);
-            if (p.gn_x && threadIdx.x == 128) {
+            if (p.epi.gn_x && threadIdx.x == 128) {
                 // the NEXT tile's GroupNorm-input rows (written in the forward pass, long evicted) -> L2
                 const int nt = tile + int(gridDim.x);
                 if (nt < p.num_tiles) {
                     const int nmt = nt % tiles_mb;
                     const int nb = nmt / p.tiles_per_img, nh0 = (nmt % p.tiles_per_img) * p.TH;
                     const int nrows = min(p.TH, p.H - nh0);
-                    l2_prefetch_bulk(p.gn_x + ((size_t(nb) * p.H + nh0) * p.W) * p.gn_ldx,
-                                     (uint32_t(nrows * p.W - 1) * uint32_t(p.gn_ldx) + uint32_t(p.Cout)) * 2u);
+                    l2_prefetch_bulk(p.epi.gn_x + ((size_t(nb) * p.H + nh0) * p.W) * p.epi.gn_ldx,
+                                     (uint32_t(nrows * p.W - 1) * uint32_t(p.epi.gn_ldx) + uint32_t(p.Cout)) * 2u);
                 }
             }
             const int row = half * 128 + q * 32 + lane;
@@ -288,8 +284,8 @@ __global__ void __launch_bounds__(kRowsThreads, 1) igemm_rows_kernel(const __gri
             if (tile + int(gridDim.x) >= p.num_tiles) pdl_trigger_late();  // last tile of this CTA
             tc_fence_after();
             const uint32_t trow = tmem_base + (uint32_t(q * 32) << 16) + uint32_t(buf * 2 * p.BN + half * p.BN);
-            epi_row(eo, trow, cb_, p.BN, valid, pix, b, h, w, n0, gc_, lane, red + size_t(warp - 4) * p.BN * 2,
-                    tr + (warp - 4) * (32 * 36), 0, 1, side);
+            epi_row(eo, trow, cb_, p.BN, valid, pix, b, h, w, n0, gc_, lane, red + size_t(warp - 4) * p.BN * 2, 0, 1,
+                    side);
             // all TMEM reads of this buffer are complete (tcgen05.wait::ld above): hand it back to the MMA warp
             tc_fence_before();
             __syncwarp();
@@ -297,7 +293,7 @@ __global__ void __launch_bounds__(kRowsThreads, 1) igemm_rows_kernel(const __gri
             if (lane == 0) mbar_arrive(&bars->t_empty[buf]);
             if (hook) {  // the 8 warps' column sums of this tile (one image) -> one vector RED per channel
                 named_bar_sync(2, kRowsEpiThreads);
-                float* dst = p.gn_x ? p.gn_S : p.stats;
+                float* dst = p.epi.gn_x ? p.epi.gn_S : p.epi.stats;
                 for (int c = et; c < p.BN; c += kRowsEpiThreads) {
                     float s0 = 0.f, s1 = 0.f;
 #pragma unroll
@@ -319,38 +315,6 @@ __global__ void __launch_bounds__(kRowsThreads, 1) igemm_rows_kernel(const __gri
 }
 
 // ------------------------------------------------------------------------------------------------ host
-typedef CUresult (*EncodeTiledFn)(CUtensorMap*, CUtensorMapDataType, cuuint32_t, void*, const cuuint64_t*,
-                                  const cuuint64_t*, const cuuint32_t*, const cuuint32_t*, CUtensorMapInterleave,
-                                  CUtensorMapSwizzle, CUtensorMapL2promotion, CUtensorMapFloatOOBfill);
-EncodeTiledFn igemm_encode_fn();  // igemm.cu
-
-static int rows_act_map(CUtensorMap* m, const __nv_bfloat16* x, int C, int ld, int W, int H, int B, int rows) {
-    EncodeTiledFn fn = igemm_encode_fn();
-    if (!fn) return -10;
-    if ((reinterpret_cast<uintptr_t>(x) & 15) || (ld % 8) != 0) return -11;
-    cuuint64_t dims[4] = {cuuint64_t(C), cuuint64_t(W), cuuint64_t(H), cuuint64_t(B)};
-    cuuint64_t strides[3] = {cuuint64_t(ld) * 2, cuuint64_t(W) * ld * 2, cuuint64_t(H) * W * ld * 2};
-    cuuint32_t box[4] = {64, cuuint32_t(W), cuuint32_t(rows), 1};
-    cuuint32_t es[4] = {1, 1, 1, 1};
-    CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 4, const_cast<__nv_bfloat16*>(x), dims, strides, box, es,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    return r == CUDA_SUCCESS ? 0 : -12;
-}
-static int rows_weight_map(CUtensorMap* m, const __nv_bfloat16* wp, int Cin, int rows, int BN) {
-    EncodeTiledFn fn = igemm_encode_fn();
-    if (!fn) return -10;
-    if ((reinterpret_cast<uintptr_t>(wp) & 15) || (Cin % 8) != 0) return -13;
-    cuuint64_t dims[2] = {cuuint64_t(Cin), cuuint64_t(rows)};
-    cuuint64_t strides[1] = {cuuint64_t(Cin) * 2};
-    cuuint32_t box[2] = {64, cuuint32_t(BN)};
-    cuuint32_t es[2] = {1, 1};
-    CUresult r = fn(m, CU_TENSOR_MAP_DATA_TYPE_BFLOAT16, 2, const_cast<__nv_bfloat16*>(wp), dims, strides, box, es,
-                    CU_TENSOR_MAP_INTERLEAVE_NONE, CU_TENSOR_MAP_SWIZZLE_128B, CU_TENSOR_MAP_L2_PROMOTION_L2_256B,
-                    CU_TENSOR_MAP_FLOAT_OOB_FILL_NONE);
-    return r == CUDA_SUCCESS ? 0 : -14;
-}
-
 bool igemm_rows_eligible(int B, int H, int W, int Cout) {
     (void)B;
     if (W < 16 || W > 128 || (256 % W) != 0) return false;
@@ -420,39 +384,15 @@ int igemm_rows_plan(IgemmRowsParams* p, const ConvSegDesc* segs, int nseg, int B
     for (int s = 0; s < nseg; ++s) {
         const ConvSegDesc& d = segs[s];
         if ((d.ntaps != 9 && d.ntaps != 1) || d.Cin % 8 != 0) return -4;
-        int r = rows_act_map(&p->seg[s].tmA, d.x, d.Cin, d.ldx, W, H, B, box_rows);
+        int r = make_act_map(&p->seg[s].tmA, d.x, d.Cin, d.ldx, W, H, B, W, box_rows, 1);
         if (r) return r;
-        r = rows_weight_map(&p->seg[s].tmW, d.wp, d.Cin, d.ntaps * Cout, BN);
+        r = make_bf16_map_2d(&p->seg[s].tmW, d.wp, d.Cin, d.ntaps * Cout, d.Cin, BN);
         if (r) return r;
         p->seg[s].cblocks = (d.Cin + 63) / 64;
         p->seg[s].ntaps = d.ntaps;
     }
-    p->bias = ep.bias, p->bias2 = ep.bias2, p->rowvec = ep.rowvec, p->residual = ep.residual;
-    p->ldr = ep.ldr ? ep.ldr : Cout;
-    p->out = ep.out;
-    p->ldo = ep.ldo ? ep.ldo : Cout;
-    p->out_mode = ep.out_mode;
-    p->stats = ep.stats;
-    p->gn_x = ep.gn_x, p->gn_ldx = ep.gn_ldx, p->gn_chsum = ep.gn_chsum, p->gn_gamma = ep.gn_gamma;
-    p->gn_beta = ep.gn_beta, p->gn_S = ep.gn_S, p->gn_silu = ep.gn_silu;
-    if (gn_hook) {
-        if ((ep.stats && ep.gn_x) || p->out_mode != OUT_NHWC_BF16) return -15;
-        if (ep.gn_x) {
-            if (ep.residual || !ep.gn_chsum || !ep.gn_gamma || !ep.gn_beta || !ep.gn_S || ep.gn_groups < 1 ||
-                Cout % ep.gn_groups)
-                return -15;
-            if ((ep.gn_ldx % 8) != 0 || (reinterpret_cast<uintptr_t>(ep.gn_x) & 15)) return -15;
-            p->gn_cpg = Cout / ep.gn_groups;
-        }
-    }
-    if (p->out_mode != OUT_NCHW_F32) {
-        const int esz = p->out_mode == OUT_NHWC_BF16 ? 2 : 4;
-        if ((p->ldo * esz) % 16 != 0 || (reinterpret_cast<uintptr_t>(p->out) & 15)) return -6;
-    }
-    if (p->residual && ((p->ldr % 8) != 0 || (reinterpret_cast<uintptr_t>(p->residual) & 15))) return -7;
-    if ((p->bias && (reinterpret_cast<uintptr_t>(p->bias) & 15)) || (p->bias2 && (reinterpret_cast<uintptr_t>(p->bias2) & 15)) ||
-        (p->rowvec && (reinterpret_cast<uintptr_t>(p->rowvec) & 15)))
-        return -8;
+    const int r = igemm_epi_plan(&p->epi, ep, Cout);
+    if (r) return r;
     p->grid = p->num_tiles < sm_count ? p->num_tiles : sm_count;
     return 0;
 }
