@@ -257,17 +257,26 @@ typedef struct {
                             (guided-diffusion's out_layers; the reference carries the option commented out,
                             dev/resblock.py:51,61, dev/unet.py:116,140) in training steps; predict / sample run without.
                             Masks are Philox draws keyed by (seed, step, block, element), never stored; 0 */
+    int super_res;       /* f >= 2: super-resolution model (guided-diffusion's SuperResModel, super_res_train.py /
+                            super_res_sample.py): the U-Net's first conv reads 2*C_in channels, cat([x_t, cond]), where
+                            cond = F.interpolate(low_res, (H, W), mode="bilinear") upsamples a (B, C_in, H/f, W/f) image.
+                            Training steps derive low_res from their own batch, F.interpolate(x0, (H/f, W/f), mode="area")
+                            (after random_flip), on the device; predict / sample / sample_spaced upsample the batch of
+                            ub_trainer_set_low_res.  Needs C_in == C_out == 3, f dividing H and W, W % 4 == 0 and
+                            W <= 256; 0 */
 } UbConfig;
 
 void ub_default_config(UbConfig* cfg);
-/* number of parameters for a config (326 tensors / 20 494 211 floats for the default) */
+/* number of parameters for a config (326 tensors / 20 494 211 floats for the default; 0 for a config that is refused) */
 size_t ub_num_params(const UbConfig* cfg);
 
 int ub_trainer_create(UbTrainer** out, const UbConfig* cfg, int device);
 void ub_trainer_destroy(UbTrainer* t);
 
 /* checkpoint, train_unet.cu:4762-4911 / train_unet.py:768-795: int32[256] header {12345678, B, C_in, C_model, C_out,
- * H, W, max_period, has_adamw, has_rng} + fp32 params [+ m + v].  The rng flag is always written 0 (the reference's
+ * H, W, max_period, has_adamw, has_rng} + fp32 params [+ m + v].  For a super-resolution model (cfg.super_res) header[2]
+ * holds the first conv's input channel count 2*C_in -- the value the reference's loader builds that conv from -- and
+ * ub_trainer_load expects it there (a plain trainer refuses such a file with UB_ERR_SHAPE).  The rng flag is always written 0 (the reference's
  * blob is a raw curandState dump); header[10] additionally stores the AdamW step count (the reference forgets it),
  * marked valid by header[11] = 0x55425354.  The reference's C writer leaves words 10..255 uninitialised
  * (train_unet.cu:4764), so ub_trainer_load trusts header[10] only behind that marker and otherwise restarts the count
@@ -275,7 +284,9 @@ void ub_trainer_destroy(UbTrainer* t);
 int ub_trainer_load(UbTrainer* t, const char* path);
 int ub_trainer_save(UbTrainer* t, const char* path, int with_adamw);
 int ub_trainer_set_step(UbTrainer* t, int step);
-/* read the {B, C_in, C_model, C_out, H, W, max_period} header of a checkpoint into cfg (other fields untouched) */
+/* read the {B, C_in, C_model, C_out, H, W, max_period} header of a checkpoint into cfg (other fields untouched).  Like
+ * head_size and channel_mult, the super-resolution factor is not stored: for a super-resolution checkpoint C_in reads
+ * 2*C_in, and the caller sets C_in = header value / 2 and super_res to the factor the model was trained with. */
 int ub_read_checkpoint_header(const char* path, UbConfig* cfg);
 
 /* host <-> device parameter access, reference parameter order (forward layer order, SURVEY.md section 8 a13) */
@@ -296,7 +307,19 @@ int ub_trainer_get_output(UbTrainer* t, float* host, size_t n); /* last forward'
 /* the flip decisions (0 / 1 per image) the last step took, when cfg.random_flip is set */
 int ub_trainer_get_flips(UbTrainer* t, int* host, size_t n);
 int ub_trainer_get_batch(UbTrainer* t, float* host, size_t n);  /* the x0 batch the last step consumed (B,C_in,H,W) */
-int ub_trainer_get_dinput(UbTrainer* t, float* host, size_t n); /* dL/d(x_t) (B,C_in,H,W); needs cfg.compute_dinput */
+/* dL/d(x_t) (B,C_in,H,W); needs cfg.compute_dinput.  For a super-resolution model this is the gradient with respect to
+ * the first C_in input channels (x_t) only; the conditioning channels are derived data, not an input of the step. */
+int ub_trainer_get_dinput(UbTrainer* t, float* host, size_t n);
+/* super-resolution model (cfg.super_res = f): the low-res images (B, C_in, H/f, W/f) fp32, scaled to [-1, 1] as
+ * super_res_sample.py passes them, that ub_trainer_predict / ub_trainer_sample / ub_trainer_sample_spaced condition on
+ * until set again (each of those calls upsamples them once, before its iterations, and returns UB_ERR_STATE while none
+ * have been set).  Training steps ignore them: they condition on their own batch.  UB_ERR_STATE on a trainer without
+ * super_res, UB_ERR_SHAPE for a wrong n. */
+int ub_trainer_set_low_res(UbTrainer* t, const float* host, size_t n);
+/* the conditioning channels (B, C_in, H, W) the last forward pass read (cfg.super_res): the bilinear upsampling of the
+ * training batch's area-downsampled (and flipped) images after a training step, of the ub_trainer_set_low_res images
+ * after an inference call */
+int ub_trainer_get_cond(UbTrainer* t, float* host, size_t n);
 
 /* One forward + backward (unet_forward + unet_backward, train_unet.cu:4335-4701) on a HOST batch x0 (B,C_in,H,W).
  * t_host (B) and noise_host (B,C_in,H,W) may be NULL: then timesteps / noise are drawn on the device (Philox).

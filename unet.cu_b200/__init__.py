@@ -31,7 +31,7 @@ class UbConfig(C.Structure):
                 ("gn_n_groups", C.c_int), ("n_timesteps", C.c_int), ("seed", C.c_ulonglong),
                 ("use_cuda_graph", C.c_int), ("compute_dinput", C.c_int), ("random_flip", C.c_int),
                 ("num_classes", C.c_int), ("ema_rate", C.c_float), ("resblock_updown", C.c_int),
-                ("use_scale_shift_norm", C.c_int), ("dropout", C.c_float)]
+                ("use_scale_shift_norm", C.c_int), ("dropout", C.c_float), ("super_res", C.c_int)]
 
 
 UB_KINDS = ("conv_igemm", "wgrad_igemm", "groupnorm", "attention", "eltwise", "small", "optimizer")
@@ -80,7 +80,8 @@ def _declare(L: C.CDLL) -> None:
     L.ub_trainer_save_ema.argtypes = [vp, C.c_char_p]
     L.ub_trainer_set_labels.argtypes = [vp, vp, C.c_size_t]
     L.ub_trainer_get_dropout_mask.argtypes = [vp, i, vp, C.c_size_t]
-    for n in ("set_params", "get_params", "get_grads", "get_output", "get_batch", "get_dinput", "get_ema", "set_ema"):
+    for n in ("set_params", "get_params", "get_grads", "get_output", "get_batch", "get_dinput", "get_ema", "set_ema",
+              "set_low_res", "get_cond"):
         getattr(L, "ub_trainer_" + n).argtypes = [vp, fp, C.c_size_t]
     L.ub_trainer_forward_backward.argtypes = [vp, fp, fp, fp, C.POINTER(C.c_float)]
     L.ub_trainer_update.argtypes = [vp] + [C.c_float] * 5
@@ -218,6 +219,17 @@ class Trainer:
     def get_dinput(self):
         c = self.cfg
         return self._get(lib().ub_trainer_get_dinput, c.B * c.C_in * c.H * c.W).reshape(c.B, c.C_in, c.H, c.W)
+
+    def set_low_res(self, low_res):
+        """Low-res images (B, C_in, H/f, W/f) in [-1, 1] that predict / sample / sample_spaced of a super-resolution
+        model (super_res = f) condition on until set again (super_res_sample.py's `low_res`)."""
+        low_res = np.ascontiguousarray(low_res, dtype=np.float32)
+        check(lib().ub_trainer_set_low_res(self._h, _ptr(low_res), low_res.size), "set_low_res")
+
+    def get_cond(self) -> np.ndarray:
+        """The conditioning channels (B, C_in, H, W) the last forward pass of a super-resolution model read."""
+        c = self.cfg
+        return self._get(lib().ub_trainer_get_cond, c.B * c.C_in * c.H * c.W).reshape(c.B, c.C_in, c.H, c.W)
 
     def get_flips(self) -> np.ndarray:
         """0 / 1 per image: the random horizontal flips of the last step (cfg.random_flip, train_unet.py:531-532)."""

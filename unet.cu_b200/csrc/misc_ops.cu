@@ -671,6 +671,61 @@ void diffusion_prepare(const float* x0, const float* sqrt_ac, const float* sqrt_
                                                                              seed, step_dev, gen_noise, t, noise, x_t, W, flips);
 }
 
+// Conditioning channels of a super-resolution model (guided-diffusion SuperResModel.forward: F.interpolate(low_res,
+// (H, W), mode="bilinear"), align_corners = False).  One block per output row of one (image, channel) plane: the two
+// low-res rows the row interpolates between are staged in shared memory, then every output pixel blends four of their
+// values.  A low-res pixel is either read from lo (B, C, H/f, W/f) or, in a training step, the f x f area mean of the
+// step's image (load_superres_data's F.interpolate(mode="area"), taken from the mirrored image where the step flipped
+// it), so the full-resolution image is read about twice rather than 4 f^2 times.  Source coordinates follow torch's
+// fp32 arithmetic (area_pixel_compute_source_index, rounded products, no contraction into an FMA).
+__device__ __forceinline__ float superres_lowres_px(const float* __restrict__ src, bool full, bool flip, size_t plane,
+                                                   int H, int W, int f, int y, int x) {
+    if (!full) return __ldg(src + (plane * (H / f) + y) * (W / f) + x);
+    float s = 0.f;
+    for (int dy = 0; dy < f; ++dy) {
+        const float* row = src + (plane * H + size_t(y) * f + dy) * W;
+        for (int dx = 0; dx < f; ++dx) s += __ldg(row + (flip ? W - 1 - (x * f + dx) : x * f + dx));
+    }
+    return s / float(f * f);
+}
+// torch's source coordinate of output index d (align_corners = False): i0, i1 and the weight of i1
+__device__ __forceinline__ void superres_src_index(int d, int n_in, int n_out, int& i0, int& i1, float& l1) {
+    const float scale = float(n_in) / float(n_out);
+    const float src = fmaxf(__fsub_rn(__fmul_rn(scale, float(d) + 0.5f), 0.5f), 0.f);
+    i0 = int(src);
+    i1 = i0 + (i0 < n_in - 1 ? 1 : 0);
+    l1 = src - float(i0);
+}
+__global__ void superres_cond_kernel(const float* __restrict__ src, int full, const int* __restrict__ flips, int C,
+                                     int H, int W, int f, float* __restrict__ cond) {
+    pdl_entry();
+    extern __shared__ float srow[];  // [2][W / f]: low-res rows y0, y1
+    const int y = blockIdx.x;
+    const size_t plane = blockIdx.y;  // b * C + c
+    const bool flip = full && flips && flips[plane / C];
+    const int hl = H / f, wl = W / f;
+    int y0, y1;
+    float ly1;
+    superres_src_index(y, hl, H, y0, y1, ly1);
+    for (int i = threadIdx.x; i < 2 * wl; i += blockDim.x)
+        srow[i] = superres_lowres_px(src, full, flip, plane, H, W, f, i < wl ? y0 : y1, i < wl ? i : i - wl);
+    __syncthreads();
+    const float ly0 = 1.f - ly1;
+    float* out = cond + (plane * H + y) * W;
+    for (int x = threadIdx.x; x < W; x += blockDim.x) {
+        int x0, x1;
+        float lx1;
+        superres_src_index(x, wl, W, x0, x1, lx1);
+        const float lx0 = 1.f - lx1;
+        out[x] = ly0 * (lx0 * srow[x0] + lx1 * srow[x1]) + ly1 * (lx0 * srow[wl + x0] + lx1 * srow[wl + x1]);
+    }
+}
+void superres_cond(const float* src, int full, const int* flips, int B, int C, int H, int W, int f, float* cond,
+                   cudaStream_t st) {
+    launch_pdl(superres_cond_kernel, dim3(unsigned(H), unsigned(B * C)), dim3(128), size_t(2) * (W / f) * sizeof(float),
+               st, src, full, flips, C, H, W, f, cond);
+}
+
 // =====================================================================================================
 // weight packing: 32x32 (o, c) tiles through smem so both packed layouts are written coalesced
 // =====================================================================================================

@@ -55,6 +55,13 @@ void diffusion_prepare(const float* x0, const float* sqrt_ac, const float* sqrt_
                        int n_timesteps, uint64_t seed, const int* step_dev, int gen_t, int gen_noise, float* t,
                        float* noise, float* x_t, cudaStream_t st, int W = 0, int* flips = nullptr);
 
+// ---- super-resolution conditioning (guided-diffusion SuperResModel): cond (B,C,H,W) fp32 = bilinear upsampling
+//      (align_corners = False) of a (B,C,H/f,W/f) image -- full = 0: src is that image (the caller's low-res batch);
+//      full = 1: src is the step's x0 (B,C,H,W) and the image is its f x f area means (super_res_train.py's condition),
+//      mirrored left-right for the images with flips[b] = 1 (flips may be null)
+void superres_cond(const float* src, int full, const int* flips, int B, int C, int H, int W, int f, float* cond,
+                   cudaStream_t st);
+
 // ---- weight packing: fp32 master (Cout, Cin, ntaps) -> bf16 fprop pack [tap][Cout][Cin] and (optional) dgrad pack
 //      [ntaps-1-tap][Cin][Cout]
 struct PackEntry {

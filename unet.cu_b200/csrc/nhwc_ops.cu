@@ -884,22 +884,36 @@ __global__ void smallc_conv_pair_kernel(const float* __restrict__ xs, const floa
     st8(y + p0 * ldy + j * 8, a0);
     st8(y + (p0 + 1) * ldy + j * 8, a1);
 }
-// Row-per-warp version for Cs == 3, Cb % 64 == 0, W % 4 == 0: a warp owns one image row and one group of 64 big
-// channels; lane l keeps the 2 x 27 weights of channels 2l, 2l+1 in registers, the zero-padded 3 x 3 x (W+2) input
-// window of the row sits in shared memory and is read as warp-uniform (broadcast) vectors -- 18 LDS per 216 FMAs, so
-// the kernel is FMA-bound (the pixel-per-thread kernels above were bound by LDS issue: one 16-byte weight read per
-// 8 FMAs, 2-way bank conflicted) -- and every pixel's 64 channels leave the warp as one 128-byte store.
+// Row-per-warp version for Cs == 3 or 6, Cb % 64 == 0, W % 4 == 0: a warp owns one image row and one group of 64
+// big channels; lane l keeps the 2 x 9 x CS weights of channels 2l, 2l+1 in registers, the zero-padded 3 x CS x (W+2)
+// input window of the row sits in shared memory and is read as warp-uniform (broadcast) vectors -- 6 CS LDS per 72 CS
+// FMAs, so the kernel is FMA-bound (the pixel-per-thread kernels above were bound by LDS issue: one 16-byte weight read
+// per 8 FMAs, 2-way bank conflicted) -- and every pixel's 64 channels leave the warp as one 128-byte store.
+// CS = 6 is the input conv of a super-resolution model (guided-diffusion's SuperResModel runs the U-Net on
+// cat([x_t, upsampled low-res])): small channels 0-2 come from xs, 3-5 from xs2, both (B, 3, H, W) fp32.
 constexpr int kSmallcWarps = 8;
-__global__ void __launch_bounds__(kSmallcWarps * 32) smallc_conv_rows_kernel(
+template <int CS>
+__device__ __forceinline__ float smallc_window_ld(const float* __restrict__ xs, const float* __restrict__ xs2, int b,
+                                                  int s_, int H, int hh, int W, int ww) {
+    if constexpr (CS == 3) {
+        return __ldg(xs + ((size_t(b) * CS + s_) * H + hh) * W + ww);
+    } else {
+        static_assert(CS == 6, "the row kernels take 3 channels from one tensor or 3 + 3 from two");
+        const float* src = s_ < 3 ? xs : xs2;
+        return __ldg(src + ((size_t(b) * 3 + (s_ < 3 ? s_ : s_ - 3)) * H + hh) * W + ww);
+    }
+}
+template <int CS, int NW>
+__global__ void __launch_bounds__(NW * 32) smallc_conv_rows_kernel(
     const float* __restrict__ xs, const float* __restrict__ w, const float* __restrict__ bias, int Cb, int B, int H,
-    int W, int flip, bf16* __restrict__ y, int ldy) {
+    int W, int flip, bf16* __restrict__ y, int ldy, const float* __restrict__ xs2) {
     pdl_entry();
-    constexpr int CS = 3;
+    constexpr int NT = 9 * CS;  // weights per big channel
     extern __shared__ float sm[];
-    float* sw = sm;                      // [27][Cb]
+    float* sw = sm;                      // [NT][Cb]
     const int WP = W + 4;                // padded row: pixel w at index w + 1, zeros at 0 and W + 1 .. W + 3
-    float* swin = sm + 27 * Cb + (threadIdx.x >> 5) * (9 * WP);  // this warp's [3 rows][CS][WP]
-    for (int i = threadIdx.x; i < Cb * 27; i += blockDim.x) {
+    float* swin = sm + NT * Cb + (threadIdx.x >> 5) * (3 * CS * WP);  // this warp's [3 rows][CS][WP]
+    for (int i = threadIdx.x; i < Cb * NT; i += blockDim.x) {
         const int cb = i % Cb, st = i / Cb;
         const int s_ = st / 9, tap = st % 9;
         sw[i] = flip ? w[(size_t(s_) * Cb + cb) * 9 + (8 - tap)] : w[(size_t(cb) * CS + s_) * 9 + tap];
@@ -907,22 +921,22 @@ __global__ void __launch_bounds__(kSmallcWarps * 32) smallc_conv_rows_kernel(
     __syncthreads();
     const int lane = threadIdx.x & 31;
     const int ngroups = Cb / 64;
-    const long long item = (long long)blockIdx.x * kSmallcWarps + (threadIdx.x >> 5);
+    const long long item = (long long)blockIdx.x * NW + (threadIdx.x >> 5);
     if (item >= (long long)B * H * ngroups) return;
     const int cg = int(item % ngroups);
     const int h = int((item / ngroups) % H);
     const int b = int(item / ((long long)ngroups * H));
-    // window rows h-1, h, h+1 of the three small channels, zero padded
-    for (int i = lane; i < 9 * WP; i += 32) {
+    // window rows h-1, h, h+1 of the small channels, zero padded
+    for (int i = lane; i < 3 * CS * WP; i += 32) {
         const int col = i % WP, rs = i / WP;  // rs = r * CS + s
         const int r = rs / CS, s_ = rs % CS;
         const int hh = h + r - 1, ww = col - 1;
-        swin[i] = (hh >= 0 && hh < H && ww >= 0 && ww < W) ? __ldg(xs + ((size_t(b) * CS + s_) * H + hh) * W + ww) : 0.f;
+        swin[i] = (hh >= 0 && hh < H && ww >= 0 && ww < W) ? smallc_window_ld<CS>(xs, xs2, b, s_, H, hh, W, ww) : 0.f;
     }
-    float wr0[27], wr1[27];
+    float wr0[NT], wr1[NT];
     const int c0 = cg * 64 + 2 * lane;
 #pragma unroll
-    for (int st = 0; st < 27; ++st) {
+    for (int st = 0; st < NT; ++st) {
         const float2 v = *reinterpret_cast<const float2*>(sw + st * Cb + c0);
         wr0[st] = v.x, wr1[st] = v.y;
     }
@@ -954,16 +968,50 @@ __global__ void __launch_bounds__(kSmallcWarps * 32) smallc_conv_rows_kernel(
     }
 }
 
-static void smallc_conv(const float* xs, const float* w, const float* bias, int Cs, int Cb, int B, int H, int W,
-                        int flip, bf16* y, int ldy, cudaStream_t st) {
-    if (Cs == 3 && Cb % 64 == 0 && W % 4 == 0 && (ldy % 2) == 0) {
-        const size_t smem_r = (size_t(27) * Cb + size_t(kSmallcWarps) * 9 * (W + 4)) * sizeof(float);
-        if (smem_r <= 48 * 1024) {
-            const long long items = (long long)B * H * (Cb / 64);
-            launch_pdl(smallc_conv_rows_kernel, dim3(unsigned((items + kSmallcWarps - 1) / kSmallcWarps)),
-                       dim3(kSmallcWarps * 32), smem_r, st, xs, w, bias, Cb, B, H, W, flip, y, ldy);
-            return;
-        }
+// Dynamic shared memory of the row kernels with NW warps per block, and the warp count the launchers use (0: the shape
+// does not fit; Cs == 3 keeps 8 warps under the default 48 KiB / the 100 KiB opt-in, Cs == 6 opts into 227 KiB and
+// halves the warps when the 8-warp window does not fit).
+static size_t smallc_conv_rows_smem(int Cs, int Cb, int W, int nw) {
+    return (size_t(9) * Cs * Cb + size_t(nw) * 3 * Cs * (W + 4)) * sizeof(float);
+}
+static size_t smallc_wgrad_rows_smem(int Cs, int W, int nw) {
+    return (size_t(nw) * 3 * Cs * (W + 4) + size_t(nw) * (18 * Cs + 2) * 32) * sizeof(float);
+}
+static int smallc_rows_warps(int Cs, int Cb, int W, bool wgrad) {
+    if (Cb % 64 || W % 4) return 0;
+    auto smem = [&](int nw) { return wgrad ? smallc_wgrad_rows_smem(Cs, W, nw) : smallc_conv_rows_smem(Cs, Cb, W, nw); };
+    if (Cs == 3) return smem(kSmallcWarps) <= (wgrad ? 100 : 48) * 1024 ? kSmallcWarps : 0;
+    if (Cs != 6) return 0;
+    for (int nw = kSmallcWarps; nw >= 4; nw /= 2)
+        if (smem(nw) <= size_t(227) * 1024) return nw;
+    return 0;
+}
+bool smallc_rows_fit(int Cs, int Cb, int W) {
+    return smallc_rows_warps(Cs, Cb, W, false) > 0 && smallc_rows_warps(Cs, Cb, W, true) > 0;
+}
+
+static void smallc_conv(const float* xs, const float* xs2, const float* w, const float* bias, int Cs, int Cb, int B,
+                        int H, int W, int flip, bf16* y, int ldy, cudaStream_t st) {
+    const int nw = (ldy % 2) == 0 ? smallc_rows_warps(Cs, Cb, W, false) : 0;
+    if (nw) {
+        const size_t smem_r = smallc_conv_rows_smem(Cs, Cb, W, nw);
+        const long long items = (long long)B * H * (Cb / 64);
+        const dim3 grid(unsigned((items + nw - 1) / nw)), block(nw * 32);
+        if (Cs == 3)
+            launch_pdl(smallc_conv_rows_kernel<3, kSmallcWarps>, grid, block, smem_r, st, xs, w, bias, Cb, B, H, W, flip,
+                       y, ldy, xs2);
+        else if (nw == kSmallcWarps)
+            launch_pdl(smallc_conv_rows_kernel<6, kSmallcWarps>, grid, block, smem_r, st, xs, w, bias, Cb, B, H, W, flip,
+                       y, ldy, xs2);
+        else
+            launch_pdl(smallc_conv_rows_kernel<6, kSmallcWarps / 2>, grid, block, smem_r, st, xs, w, bias, Cb, B, H, W,
+                       flip, y, ldy, xs2);
+        return;
+    }
+    if (xs2) {  // (super-resolution configs are validated against smallc_rows_fit)
+        fprintf(stderr, "[unet_b200] smallc_conv: %d + 3 channels at %d big channels, W = %d do not fit the row kernel\n",
+                Cs - 3, Cb, W);
+        return;
     }
     const size_t smem = size_t(Cb) * Cs * 9 * sizeof(float);
     if (W % 2 == 0) {
@@ -977,13 +1025,13 @@ static void smallc_conv(const float* xs, const float* w, const float* bias, int 
     }
 }
 
-void conv_in_fwd(const float* x, const float* w, const float* b, int B, int Cin, int Cout, int H, int W, bf16* y,
-                 int ldy, cudaStream_t st) {
-    smallc_conv(x, w, b, Cin, Cout, B, H, W, 0, y, ldy, st);
+void conv_in_fwd(const float* x, const float* x2, const float* w, const float* b, int B, int Cin, int Cout, int H,
+                 int W, bf16* y, int ldy, cudaStream_t st) {
+    smallc_conv(x, x2, w, b, Cin, Cout, B, H, W, 0, y, ldy, st);
 }
 void conv_out_dgrad(const float* dout, const float* w, int B, int Cin, int Cout, int H, int W, bf16* da, int ldda,
                     cudaStream_t st) {
-    smallc_conv(dout, w, nullptr, Cout, Cin, B, H, W, 1, da, ldda, st);
+    smallc_conv(dout, nullptr, w, nullptr, Cout, Cin, B, H, W, 1, da, ldda, st);
 }
 
 // partial[blk][cb][s*9+tap] = sum_{p in block} yb[p][cb] * xs[b][s][p + shift(tap)] ; partial[blk][cb][NT] = sum yb
@@ -1058,34 +1106,37 @@ __global__ void smallc_wgrad_reduce_kernel(const float* __restrict__ partial, in
     else
         dw[(size_t(sidx) * Cb + cb) * 9 + (8 - tap)] = s;
 }
-// Row-per-warp weight gradient of the 3-channel convs (Cs == 3, Cb % 64 == 0, W % 4 == 0), the mirror image of
-// smallc_conv_rows_kernel: lane l accumulates the 2 x 27 weight gradients (+ 2 bias sums) of big channels 2l, 2l+1 in
-// registers over whole image rows -- per 4 pixels: 4 coalesced 128-byte rows of dy, 18 broadcast LDS of the window,
-// 216 FMAs -- the 8 warps of a block are added in shared memory and every block adds its totals to dw / db with
-// 8-byte vector REDs (dw, db are zero at the start of a step like every accumulated gradient).
-// mode 0 (conv_in):  dw[cb][s][tap] ; db[cb]          mode 1 (conv_out): dw[s][cb][8 - tap] ; no db
-__global__ void __launch_bounds__(kSmallcWarps * 32) smallc_wgrad_rows_kernel(
+// Row-per-warp weight gradient of the 3- and 6-channel convs (Cs == 3 or 6, Cb % 64 == 0, W % 4 == 0), the mirror
+// image of smallc_conv_rows_kernel: lane l accumulates the 2 x 9 CS weight gradients (+ 2 bias sums) of big channels
+// 2l, 2l+1 in registers over whole image rows -- per 4 pixels: 4 coalesced 128-byte rows of dy, 6 CS broadcast LDS of
+// the window, 72 CS FMAs -- the NW warps of a block are added in shared memory and every block adds its totals to dw /
+// db with 8-byte vector REDs (dw, db are zero at the start of a step like every accumulated gradient).
+// mode 0 (conv_in):  dw[cb][s][tap] ; db[cb]          mode 1 (conv_out, Cs == 3): dw[s][cb][8 - tap] ; no db
+// With Cs == 6 small channels 0-2 come from xs and 3-5 from xs2 (the super-resolution input conv).
+template <int CS, int NW>
+__global__ void __launch_bounds__(NW * 32) smallc_wgrad_rows_kernel(
     const float* __restrict__ xs, const bf16* __restrict__ yb, int ldy, int Cb, int B, int H, int W, int mode,
-    float* __restrict__ dw, float* __restrict__ db) {
+    float* __restrict__ dw, float* __restrict__ db, const float* __restrict__ xs2) {
     pdl_entry();
-    constexpr int CS = 3;
+    constexpr int NT = 9 * CS;       // weight gradients per big channel
+    constexpr int NV = 2 * NT + 2;   // values per lane: two channels' gradients and bias sums
     extern __shared__ float sm[];
     const int WP = W + 4;
     const int warp = threadIdx.x >> 5, lane = threadIdx.x & 31;
-    float* swin = sm + warp * (9 * WP);
-    float* sred = sm + kSmallcWarps * 9 * WP;  // [warps][56][32]
+    float* swin = sm + warp * (3 * CS * WP);
+    float* sred = sm + NW * 3 * CS * WP;  // [warps][NV][32]
     const int cg = blockIdx.y;
-    float g0[27], g1[27], bs0 = 0.f, bs1 = 0.f;
+    float g0[NT], g1[NT], bs0 = 0.f, bs1 = 0.f;
 #pragma unroll
-    for (int k = 0; k < 27; ++k) g0[k] = g1[k] = 0.f;
-    for (int row = blockIdx.x * kSmallcWarps + warp; row < B * H; row += gridDim.x * kSmallcWarps) {
+    for (int k = 0; k < NT; ++k) g0[k] = g1[k] = 0.f;
+    for (int row = blockIdx.x * NW + warp; row < B * H; row += gridDim.x * NW) {
         const int b = row / H, h = row % H;
         __syncwarp();
-        for (int i = lane; i < 9 * WP; i += 32) {
+        for (int i = lane; i < 3 * CS * WP; i += 32) {
             const int col = i % WP, rs = i / WP;
             const int r = rs / CS, s_ = rs % CS;
             const int hh = h + r - 1, ww = col - 1;
-            swin[i] = (hh >= 0 && hh < H && ww >= 0 && ww < W) ? __ldg(xs + ((size_t(b) * CS + s_) * H + hh) * W + ww) : 0.f;
+            swin[i] = (hh >= 0 && hh < H && ww >= 0 && ww < W) ? smallc_window_ld<CS>(xs, xs2, b, s_, H, hh, W, ww) : 0.f;
         }
         __syncwarp();
         const bf16* yrow = yb + (size_t(row) * W) * ldy + cg * 64 + 2 * lane;
@@ -1127,33 +1178,33 @@ __global__ void __launch_bounds__(kSmallcWarps * 32) smallc_wgrad_rows_kernel(
             }
         }
     }
-    // park the warp's 56 values so that value index j of lane l is element j of the lane's contiguous output range:
-    // mode 0: [cc][s][tap] (27 per channel); mode 1: per s, [cc][8 - tap] (18 per s); then the two bias sums
-    float* mine = sred + size_t(warp) * 56 * 32 + lane;
+    // park the warp's NV values so that value index j of lane l is element j of the lane's contiguous output range:
+    // mode 0: [cc][s][tap] (NT per channel); mode 1: per s, [cc][8 - tap] (18 per s); then the two bias sums
+    float* mine = sred + size_t(warp) * NV * 32 + lane;
 #pragma unroll
     for (int s_ = 0; s_ < CS; ++s_)
 #pragma unroll
         for (int tap = 0; tap < 9; ++tap) {
             const int j0 = mode == 0 ? s_ * 9 + tap : s_ * 18 + (8 - tap);
-            const int j1 = mode == 0 ? 27 + s_ * 9 + tap : s_ * 18 + 9 + (8 - tap);
+            const int j1 = mode == 0 ? NT + s_ * 9 + tap : s_ * 18 + 9 + (8 - tap);
             mine[j0 * 32] = g0[s_ * 9 + tap];
             mine[j1 * 32] = g1[s_ * 9 + tap];
         }
-    mine[54 * 32] = bs0, mine[55 * 32] = bs1;
+    mine[2 * NT * 32] = bs0, mine[(2 * NT + 1) * 32] = bs1;
     __syncthreads();
-    for (int i = warp; i < 28; i += kSmallcWarps) {  // pair i = values 2i, 2i+1 of every lane
+    for (int i = warp; i < NT + 1; i += NW) {  // pair i = values 2i, 2i+1 of every lane
         float t0 = 0.f, t1 = 0.f;
 #pragma unroll
-        for (int w_ = 0; w_ < kSmallcWarps; ++w_) {
-            t0 += sred[(size_t(w_) * 56 + 2 * i) * 32 + lane];
-            t1 += sred[(size_t(w_) * 56 + 2 * i + 1) * 32 + lane];
+        for (int w_ = 0; w_ < NW; ++w_) {
+            t0 += sred[(size_t(w_) * NV + 2 * i) * 32 + lane];
+            t1 += sred[(size_t(w_) * NV + 2 * i + 1) * 32 + lane];
         }
         float* dst;
-        if (i == 27) {
+        if (i == NT) {
             if (mode != 0 || !db) continue;
             dst = db + cg * 64 + 2 * lane;
         } else if (mode == 0) {
-            dst = dw + (size_t(cg) * 64 + 2 * lane) * 27 + 2 * i;
+            dst = dw + (size_t(cg) * 64 + 2 * lane) * NT + 2 * i;
         } else {
             const int s_ = (2 * i) / 18, q = (2 * i) % 18;
             dst = dw + (size_t(s_) * Cb + cg * 64 + 2 * lane) * 9 + q;
@@ -1166,22 +1217,40 @@ void nhwc_ops_init() {
     static bool done = false;
     if (done) return;
     cudaFuncSetAttribute(smallc_wgrad_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
-    cudaFuncSetAttribute(smallc_wgrad_rows_kernel, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
+    cudaFuncSetAttribute(smallc_wgrad_rows_kernel<3, kSmallcWarps>, cudaFuncAttributeMaxDynamicSharedMemorySize, 100 * 1024);
+    cudaFuncSetAttribute(smallc_conv_rows_kernel<6, kSmallcWarps>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    cudaFuncSetAttribute(smallc_conv_rows_kernel<6, kSmallcWarps / 2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                         227 * 1024);
+    cudaFuncSetAttribute(smallc_wgrad_rows_kernel<6, kSmallcWarps>, cudaFuncAttributeMaxDynamicSharedMemorySize, 227 * 1024);
+    cudaFuncSetAttribute(smallc_wgrad_rows_kernel<6, kSmallcWarps / 2>, cudaFuncAttributeMaxDynamicSharedMemorySize,
+                         227 * 1024);
     gn_slab_init();
     done = true;
 }
-static void smallc_wgrad(const float* xs, const bf16* yb, int ldy, int B, int Cs, int Cb, int H, int W, int mode,
-                         float* dw, float* db, float* scratch, size_t scratch_floats, cudaStream_t st) {
-    if (Cs == 3 && Cb % 64 == 0 && W % 4 == 0 && (ldy % 2) == 0) {
-        const size_t smem_r = (size_t(kSmallcWarps) * 9 * (W + 4) + size_t(kSmallcWarps) * 56 * 32) * sizeof(float);
-        if (smem_r <= 100 * 1024) {
-            nhwc_ops_init();
-            int gx = (B * H + kSmallcWarps - 1) / kSmallcWarps;
-            if (gx > 2 * kSMs) gx = 2 * kSMs;
-            launch_pdl(smallc_wgrad_rows_kernel, dim3(unsigned(gx), unsigned(Cb / 64)), dim3(kSmallcWarps * 32), smem_r, st,
-                       xs, yb, ldy, Cb, B, H, W, mode, dw, db);
-            return;
-        }
+static void smallc_wgrad(const float* xs, const float* xs2, const bf16* yb, int ldy, int B, int Cs, int Cb, int H,
+                         int W, int mode, float* dw, float* db, float* scratch, size_t scratch_floats, cudaStream_t st) {
+    const int nw = (ldy % 2) == 0 ? smallc_rows_warps(Cs, Cb, W, true) : 0;
+    if (nw) {
+        nhwc_ops_init();
+        const size_t smem_r = smallc_wgrad_rows_smem(Cs, W, nw);
+        int gx = (B * H + nw - 1) / nw;
+        if (gx > 2 * kSMs) gx = 2 * kSMs;
+        const dim3 grid(unsigned(gx), unsigned(Cb / 64)), block(nw * 32);
+        if (Cs == 3)
+            launch_pdl(smallc_wgrad_rows_kernel<3, kSmallcWarps>, grid, block, smem_r, st, xs, yb, ldy, Cb, B, H, W, mode,
+                       dw, db, xs2);
+        else if (nw == kSmallcWarps)
+            launch_pdl(smallc_wgrad_rows_kernel<6, kSmallcWarps>, grid, block, smem_r, st, xs, yb, ldy, Cb, B, H, W, mode,
+                       dw, db, xs2);
+        else
+            launch_pdl(smallc_wgrad_rows_kernel<6, kSmallcWarps / 2>, grid, block, smem_r, st, xs, yb, ldy, Cb, B, H, W,
+                       mode, dw, db, xs2);
+        return;
+    }
+    if (xs2) {  // (super-resolution configs are validated against smallc_rows_fit)
+        fprintf(stderr, "[unet_b200] smallc_wgrad: %d + 3 channels at %d big channels, W = %d do not fit the row kernel\n",
+                Cs - 3, Cb, W);
+        return;
     }
     const int NT = Cs * 9;
     size_t nblk = 2 * kSMs;
@@ -1201,22 +1270,24 @@ static void smallc_wgrad(const float* xs, const bf16* yb, int ldy, int B, int Cs
     launch_pdl(smallc_wgrad_kernel, dim3(unsigned(nblk)), dim3(Cb * 4), smem, st, xs, yb, ldy, Cs, Cb, B, H, W, scratch);
     launch_pdl(smallc_wgrad_reduce_kernel, dim3(unsigned((per + 127) / 128)), dim3(128), 0, st, scratch, int(nblk), Cs, Cb, mode, dw, db);
 }
-void conv_in_wgrad(const float* x, const bf16* dy, int lddy, int B, int Cin, int Cout, int H, int W, float* dw,
-                   float* db, float* scratch, size_t scratch_floats, cudaStream_t st) {
-    smallc_wgrad(x, dy, lddy, B, Cin, Cout, H, W, 0, dw, db, scratch, scratch_floats, st);
+void conv_in_wgrad(const float* x, const float* x2, const bf16* dy, int lddy, int B, int Cin, int Cout, int H, int W,
+                   float* dw, float* db, float* scratch, size_t scratch_floats, cudaStream_t st) {
+    smallc_wgrad(x, x2, dy, lddy, B, Cin, Cout, H, W, 0, dw, db, scratch, scratch_floats, st);
 }
 
 // out[b][o][p] (NCHW fp32) = bias[o] + sum_tap sum_c a[p+shift][c] * w[o][c][tap] ; Cout <= 4
-// flip == 1: the same contraction with w given as (Cin, Cout, 3, 3) and taps mirrored: the input gradient of the
-// 3-channel first conv (dx[s] = sum_tap sum_cb dh[p - shift][cb] * w_in[cb][s][tap]); bias may be null.
+// flip == 1: the same contraction with w given as (Cin, ldw, 3, 3) and taps mirrored: the input gradient of the
+// 3-channel first conv (dx[s] = sum_tap sum_cb dh[p - shift][cb] * w_in[cb][s][tap]); bias may be null.  ldw is the
+// weight's input-channel count: Cout, or 2 Cout for a super-resolution model, whose first conv also reads the
+// conditioning channels -- dx is then the gradient with respect to x_t alone.
 __global__ void conv_out_fwd_kernel(const bf16* __restrict__ a, int lda, const float* __restrict__ w,
                                     const float* __restrict__ bias, int Cin, int Cout, int H, int W, size_t npix,
-                                    float* __restrict__ out, int flip) {
+                                    float* __restrict__ out, int flip, int ldw) {
     pdl_entry();
     extern __shared__ float sw[];  // [9][Cin][4]
     for (int i = threadIdx.x; i < 9 * Cin * 4; i += blockDim.x) {
         const int o = i % 4, c = (i / 4) % Cin, tap = i / (4 * Cin);
-        sw[i] = o < Cout ? (flip ? w[(size_t(c) * Cout + o) * 9 + (8 - tap)] : w[(size_t(o) * Cin + c) * 9 + tap]) : 0.f;
+        sw[i] = o < Cout ? (flip ? w[(size_t(c) * ldw + o) * 9 + (8 - tap)] : w[(size_t(o) * Cin + c) * 9 + tap]) : 0.f;
     }
     __syncthreads();
     const size_t p = size_t(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -1247,12 +1318,12 @@ __global__ void conv_out_fwd_kernel(const bf16* __restrict__ a, int lda, const f
 // (12 instead of 18 16-byte loads per 8 channels) and every weight read feeds 8 FMAs.
 __global__ void conv_out_pair_kernel(const bf16* __restrict__ a, int lda, const float* __restrict__ w,
                                      const float* __restrict__ bias, int Cin, int Cout, int H, int W, size_t npairs,
-                                     float* __restrict__ out, int flip) {
+                                     float* __restrict__ out, int flip, int ldw) {
     pdl_entry();
     extern __shared__ float sw[];  // [9][Cin][4]
     for (int i = threadIdx.x; i < 9 * Cin * 4; i += blockDim.x) {
         const int o = i % 4, c = (i / 4) % Cin, tap = i / (4 * Cin);
-        sw[i] = o < Cout ? (flip ? w[(size_t(c) * Cout + o) * 9 + (8 - tap)] : w[(size_t(o) * Cin + c) * 9 + tap]) : 0.f;
+        sw[i] = o < Cout ? (flip ? w[(size_t(c) * ldw + o) * 9 + (8 - tap)] : w[(size_t(o) * Cin + c) * 9 + tap]) : 0.f;
     }
     __syncthreads();
     const size_t pp = size_t(blockIdx.x) * blockDim.x + threadIdx.x;
@@ -1432,7 +1503,7 @@ static void conv_out_rows_launch(const bf16* a, int lda, const float* w, const f
 }
 
 static void conv_out_launch(const bf16* a, int lda, const float* w, const float* b, int B, int Cin, int Cout, int H,
-                            int W, float* out, int flip, cudaStream_t st) {
+                            int W, float* out, int flip, int ldw, cudaStream_t st) {
     if (!flip && conv_out_rows_ok(Cin, Cout, W) && (lda % 2) == 0) {
         conv_out_rows_launch(a, lda, w, b, B, Cin, H, W, out, nullptr, nullptr, nullptr, 0.f, 0.f, st);
         return;
@@ -1441,21 +1512,22 @@ static void conv_out_launch(const bf16* a, int lda, const float* w, const float*
     if (W % 2 == 0) {
         const size_t npairs = size_t(B) * H * (W / 2);
         launch_pdl(conv_out_pair_kernel, dim3(unsigned((npairs + 63) / 64)), dim3(64), smem, st, a, lda, w, b, Cin, Cout,
-                   H, W, npairs, out, flip);
+                   H, W, npairs, out, flip, ldw);
     } else {
         const size_t npix = size_t(B) * H * W;
         launch_pdl(conv_out_fwd_kernel, dim3(unsigned((npix + 127) / 128)), dim3(128), smem, st, a, lda, w, b, Cin, Cout,
-                   H, W, npix, out, flip);
+                   H, W, npix, out, flip, ldw);
     }
 }
 void conv_out_fwd(const bf16* a, int lda, const float* w, const float* b, int B, int Cin, int Cout, int H, int W,
                   float* out, cudaStream_t st) {
-    conv_out_launch(a, lda, w, b, B, Cin, Cout, H, W, out, 0, st);
+    conv_out_launch(a, lda, w, b, B, Cin, Cout, H, W, out, 0, Cout, st);
 }
 void conv_in_dgrad(const bf16* dh, int lddh, const float* w, int B, int Cin, int Cout, int H, int W, float* dx,
-                   cudaStream_t st) {
-    // dh NHWC bf16 with Cout (= model width) channels, w (Cout, Cin, 3, 3), dx NCHW fp32 with Cin <= 4 channels
-    conv_out_launch(dh, lddh, w, nullptr, B, Cout, Cin, H, W, dx, 1, st);
+                   cudaStream_t st, int Cw) {
+    // dh NHWC bf16 with Cout (= model width) channels, w (Cout, Cw, 3, 3), dx NCHW fp32: the gradient of the first
+    // Cin <= 4 input channels
+    conv_out_launch(dh, lddh, w, nullptr, B, Cout, Cin, H, W, dx, 1, Cw, st);
 }
 
 // db[o] += sum_{b,p} dout[b][o][p]   (B*Cout*H*W fp32; one block per (channel, image) plane, one atomic per block --
@@ -1488,7 +1560,7 @@ __global__ void nchw_chansum_kernel(const float* __restrict__ x, int B, int C, s
 void conv_out_wgrad(const bf16* a, int lda, const float* dout, int B, int Cin, int Cout, int H, int W, float* dw,
                     float* db, float* scratch, size_t scratch_floats, cudaStream_t st) {
     // D'[c][o][t'] = sum_p a[p][c] * dout[o][p + shift(t')]  ->  dw[o][c][8 - t']
-    smallc_wgrad(dout, a, lda, B, Cout, Cin, H, W, 1, dw, nullptr, scratch, scratch_floats, st);
+    smallc_wgrad(dout, nullptr, a, lda, B, Cout, Cin, H, W, 1, dw, nullptr, scratch, scratch_floats, st);
     launch_pdl(nchw_chansum_kernel, dim3(Cout, B), dim3(256), 0, st, dout, B, Cout, size_t(H) * W, db);
 }
 

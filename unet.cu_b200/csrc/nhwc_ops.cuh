@@ -81,15 +81,20 @@ void add2(const bf16* a, int lda, const bf16* b, int ldb, size_t npix, int C, bf
 void colsum(const bf16* x, int ldx, size_t npix, int C, float* out, float* out2, cudaStream_t st);
 
 // ---- 3-channel convolutions (first / last layer of the U-Net) -- SIMT, negligible FLOPs
-// conv_in: x NCHW fp32 (B,Cin<=4,H,W), w (Cout,Cin,3,3) fp32 -> y NHWC bf16
-void conv_in_fwd(const float* x, const float* w, const float* b, int B, int Cin, int Cout, int H, int W, bf16* y,
-                 int ldy, cudaStream_t st);
-// dW, db of conv_in from dy NHWC bf16 (overwrite); scratch >= blocks*(Cout*Cin*9 + Cout) floats
-void conv_in_wgrad(const float* x, const bf16* dy, int lddy, int B, int Cin, int Cout, int H, int W, float* dw,
-                   float* db, float* scratch, size_t scratch_floats, cudaStream_t st);
-// dx NCHW fp32 (B,Cin<=4,H,W) = conv_transpose(dh NHWC bf16 with Cout channels, w (Cout,Cin,3,3)): dL/d(x_t)
+// conv_in: x NCHW fp32 (B,Cin<=4,H,W), w (Cout,Cin,3,3) fp32 -> y NHWC bf16.  Cin = 6 (super-resolution model): input
+// channels 0-2 from x and 3-5 from x2, both (B,3,H,W) -- the row kernels only; x2 is null otherwise
+void conv_in_fwd(const float* x, const float* x2, const float* w, const float* b, int B, int Cin, int Cout, int H,
+                 int W, bf16* y, int ldy, cudaStream_t st);
+// dW, db of conv_in from dy NHWC bf16 (overwrite); scratch >= blocks*(Cout*Cin*9 + Cout) floats; x2 as conv_in_fwd
+void conv_in_wgrad(const float* x, const float* x2, const bf16* dy, int lddy, int B, int Cin, int Cout, int H, int W,
+                   float* dw, float* db, float* scratch, size_t scratch_floats, cudaStream_t st);
+// dx NCHW fp32 (B,Cin<=4,H,W) = conv_transpose(dh NHWC bf16 with Cout channels, w (Cout,Cw,3,3)) restricted to the first
+// Cin input channels: dL/d(x_t) (Cw = Cin, or 2 Cin for a super-resolution model)
 void conv_in_dgrad(const bf16* dh, int lddh, const float* w, int B, int Cin, int Cout, int H, int W, float* dx,
-                   cudaStream_t st);
+                   cudaStream_t st, int Cw);
+// true when the row-per-warp conv_in kernels (forward and weight gradient) take Cs small channels at Cb big channels
+// and width W -- what a super-resolution config (Cs = 6) needs, as no other kernel serves it
+bool smallc_rows_fit(int Cs, int Cb, int W);
 // conv_out: a NHWC bf16 (Cin = 64..), w (Cout<=4,Cin,3,3) -> out NCHW fp32
 void conv_out_fwd(const bf16* a, int lda, const float* w, const float* b, int B, int Cin, int Cout, int H, int W,
                   float* out, cudaStream_t st);

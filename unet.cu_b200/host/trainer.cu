@@ -144,6 +144,10 @@ struct UbTrainer {
     float *x0 = nullptr, *xt = nullptr, *noise = nullptr, *tsteps = nullptr, *out = nullptr, *dout = nullptr;
     float* dxt = nullptr;  // dL/d(x_t), only with cfg.compute_dinput
     int* flips = nullptr;  // per-image flip decisions of the last step, only with cfg.random_flip
+    // cfg.super_res: the conditioning channels (B,C_in,H,W) the input conv reads beside x_t -- computed from the batch
+    // by every training step, upsampled from low_res (B,C_in,H/f,W/f; ub_trainer_set_low_res) by the inference calls
+    float *cond = nullptr, *low_res = nullptr;
+    bool have_low_res = false;
     float *loss = nullptr, *sqrt_ac = nullptr, *sqrt_1mac = nullptr, *betas = nullptr;
     int* samp_state = nullptr;  // {t, iteration} of the sampling loop
     cudaGraphExec_t samp_graph = nullptr;
@@ -763,6 +767,8 @@ int Builder::build() {
     T->drop_ctl = c.dropout > 0.f ? (unsigned*)T->arena.alloc(256) : nullptr;
     T->dxt = c.compute_dinput ? f32(size_t(B) * img) : nullptr;
     T->flips = c.random_flip ? (int*)T->arena.alloc(size_t(B) * sizeof(int) + 256) : nullptr;
+    T->cond = c.super_res ? f32(size_t(B) * img) : nullptr;
+    T->low_res = c.super_res ? f32(size_t(B) * img / (size_t(c.super_res) * c.super_res)) : nullptr;
     T->out = f32(size_t(B) * c.C_out * H0 * W0), T->dout = f32(size_t(B) * c.C_out * H0 * W0);
     T->sqrt_ac = f32(c.n_timesteps), T->sqrt_1mac = f32(c.n_timesteps), T->betas = f32(c.n_timesteps);
     T->samp_state = (int*)T->arena.alloc(256);
@@ -811,25 +817,30 @@ int Builder::build() {
     }
     const size_t time_mlp_end = poff;
 
-    // ---- input conv (dev/unet.py:183-185)
+    // ---- input conv (dev/unet.py:183-185); a super-resolution model's reads cat([x_t, cond]) (SuperResModel builds
+    // UNetModel(in_channels * 2), its forward concatenates the upsampled low-res image after x_t)
     int ch = c.channel_mult[0] * Cm;
     View h = act(ch, H0, W0);
     {
         Node nd;
         nd.param_begin = poff;
-        const size_t wi = take(size_t(ch) * c.C_in * 9), bi = take(ch);
+        const int Cin = c.C_in, Cw = c.super_res ? 2 * c.C_in : c.C_in;
+        const size_t wi = take(size_t(ch) * Cw * 9), bi = take(ch);
         float *w = P(wi), *b = P(bi), *gw = G(wi), *gb = G(bi);
-        const int Cin = c.C_in;
         View hv = h;
-        F([=](cudaStream_t st) { conv_in_fwd(Tt->xt, w, b, Bn, Cin, hv.C, hv.H, hv.W, hv.p, hv.ld, st); });
+        label("input conv %d->%d", Cw, ch);
+        F([=](cudaStream_t st) { conv_in_fwd(Tt->xt, Tt->cond, w, b, Bn, Cw, hv.C, hv.H, hv.W, hv.p, hv.ld, st); });
         nd.out = h, nd.pushed = true;
         nd.bwd = [=](View dout) -> View {
+            label("input conv wgrad %d->%d", Cw, ch);
             Bk([=](cudaStream_t st) {
-                conv_in_wgrad(Tt->xt, dout.p, dout.ld, Bn, Cin, hv.C, hv.H, hv.W, gw, gb, Tt->small_scratch,
+                conv_in_wgrad(Tt->xt, Tt->cond, dout.p, dout.ld, Bn, Cw, hv.C, hv.H, hv.W, gw, gb, Tt->small_scratch,
                               Tt->small_scratch_floats, st);
             }, 1, UB_KIND_SMALL, 0, 0, 0);  // (one launch with the row kernel; two on its fallback path)
-            if (Tt->cfg.compute_dinput)
-                Bk([=](cudaStream_t st) { conv_in_dgrad(dout.p, dout.ld, w, Bn, Cin, hv.C, hv.H, hv.W, Tt->dxt, st); }, 1);
+            if (Tt->cfg.compute_dinput)  // (dL/d(x_t) only: the conditioning channels are not an input of the step)
+                Bk([=](cudaStream_t st) {
+                    conv_in_dgrad(dout.p, dout.ld, w, Bn, Cin, hv.C, hv.H, hv.W, Tt->dxt, st, Cw);
+                }, 1);
             return View{};
         };
         nodes.push_back(nd);
@@ -1115,6 +1126,15 @@ static int validate_config(const UbConfig& c) {
         set_err("C_in*H*W must be a multiple of 4");
         return UB_ERR_SHAPE;
     }
+    if (c.super_res) {
+        const int f = c.super_res, Cb = c.channel_mult[0] * c.C_model;
+        if (f < 2 || c.C_in != 3 || c.C_out != 3 || c.H % f || c.W % f || c.W % 4 || c.W > 256 ||
+            !smallc_rows_fit(2 * c.C_in, Cb, c.W)) {
+            set_err("super_res = %d needs a factor >= 2 that divides H and W, C_in == C_out == 3, W %% 4 == 0, W <= 256 "
+                    "and an input conv the 6-channel row kernels take (%d channels at W = %d)", f, Cb, c.W);
+            return UB_ERR_SHAPE;
+        }
+    }
     for (int l = 0; l < c.n_levels; ++l)
         if ((c.channel_mult[l] * c.C_model) % c.gn_n_groups) {
             set_err("channels not divisible by gn groups");
@@ -1313,6 +1333,8 @@ static void enqueue_step(UbTrainer* t, const StepOpts& o, cudaStream_t st) {
     cudaMemsetAsync(t->zero_base, 0, t->zero_bytes, st);
     diffusion_prepare(t->x0, t->sqrt_ac, t->sqrt_1mac, c.B, size_t(c.C_in) * c.H * c.W, c.n_timesteps, c.seed,
                       t->step_dev, o.gen_t ? 1 : 0, o.gen_noise ? 1 : 0, t->tsteps, t->noise, t->xt, st, c.W, t->flips);
+    // super-resolution: the condition comes from the batch itself (super_res_train.py, load_superres_data)
+    if (c.super_res) superres_cond(t->x0, 1, t->flips, c.B, c.C_in, c.H, c.W, c.super_res, t->cond, st);
     if (t->drop_ctl) dropout_set_ctl(t->drop_ctl, c.dropout, c.seed, t->step_dev, st);  // training: masks of this step
     static const bool debug_sync = getenv("UB_DEBUG_SYNC") != nullptr;  // eager runs only: find the faulting op
     cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
@@ -1601,9 +1623,11 @@ extern "C" int ub_trainer_profile(UbTrainer* t, int reps, UbProfile* out) {
     }();
     const float invR = 1.f / float(R);
     const UbConfig& c = t->cfg;
-    const size_t nops = t->fwd_ops.size() + t->bwd_ops.size() + 2;
+    const size_t n_pre = c.super_res ? 2 : 1;  // event intervals before the tape: q-sample (+ super-res condition)
+    const size_t nops = t->fwd_ops.size() + t->bwd_ops.size() + 1 + n_pre;
     std::vector<cudaEvent_t> ev(nops + 1);
     std::vector<float> op_us(nops, 0.f);
+    float cond_us = 0.f;
     for (auto& e : ev) CUDA_TRY(cudaEventCreate(&e));
     cudaStream_t st = t->stream;
     t->comm_off = true;  // a profile is rank-local: the peers are not replaying with us
@@ -1632,6 +1656,11 @@ extern "C" int ub_trainer_profile(UbTrainer* t, int reps, UbProfile* out) {
                           t->step_dev, 1, 1, t->tsteps, t->noise, t->xt, st, c.W, t->flips);
         if (t->drop_ctl) dropout_set_ctl(t->drop_ctl, c.dropout, c.seed, t->step_dev, st);
         cudaEventRecord(ev[k++], st);
+        if (c.super_res) {
+            for (int r = 0; r < R; ++r)
+                superres_cond(t->x0, 1, t->flips, c.B, c.C_in, c.H, c.W, c.super_res, t->cond, st);
+            cudaEventRecord(ev[k++], st);
+        }
         for (auto& op : t->fwd_ops) {
             for (int r = 0; r < R; ++r) op(st);
             cudaEventRecord(ev[k++], st);
@@ -1650,6 +1679,13 @@ extern "C" int ub_trainer_profile(UbTrainer* t, int reps, UbProfile* out) {
         size_t j = 1;
         cudaEventElapsedTime(&ms, ev[0], ev[1]);
         out->ms[UB_KIND_OPTIM] += ms;
+        if (c.super_res) {
+            cudaEventElapsedTime(&ms, ev[1], ev[2]);
+            ms *= invR;
+            out->ms[UB_KIND_OPTIM] += ms;
+            cond_us = ms * 1e3f;
+            j = 2;
+        }
         for (size_t i = 0; i < t->fwd_ops.size(); ++i, ++j) {
             cudaEventElapsedTime(&ms, ev[j], ev[j + 1]);
             ms *= invR;
@@ -1679,6 +1715,9 @@ extern "C" int ub_trainer_profile(UbTrainer* t, int reps, UbProfile* out) {
     for (auto& e : ev) cudaEventDestroy(e);
     if (const char* path = getenv("UB_PROFILE_DUMP")) {  // per-op times of the LAST repetition
         if (FILE* f = fopen(path, "w")) {
+            if (c.super_res)
+                fprintf(f, "pre\t0\t%d\t%.3f\t0\t%.4g\tsuper-res condition (f = %d)\n", UB_KIND_OPTIM, cond_us,
+                        2.0 * c.B * c.C_in * c.H * c.W * 4, c.super_res);
             for (size_t i = 0; i < t->fwd_ops.size(); ++i)
                 fprintf(f, "fwd\t%zu\t%d\t%.3f\t%.4g\t%.4g\t%s\n", i, t->fwd_info[i].kind, op_us[i],
                         t->fwd_info[i].flops, t->fwd_info[i].bytes, t->fwd_info[i].label.c_str());
@@ -1694,9 +1733,9 @@ extern "C" int ub_trainer_profile(UbTrainer* t, int reps, UbProfile* out) {
         for (auto& i : v) out->flops[i.kind] += i.flops, out->bytes[i.kind] += i.bytes, out->launches[i.kind] += i.launches;
     };
     acc(t->fwd_info), acc(t->bwd_info);
-    out->launches[UB_KIND_OPTIM] += 5;
+    out->launches[UB_KIND_OPTIM] += c.super_res ? 6 : 5;
     const double img = double(c.B) * c.C_in * c.H * c.W * 4;
-    out->bytes[UB_KIND_OPTIM] += 3 * img + 7.0 * 4 * t->nparams + 4.0 * t->nparams + 2.0 * 2 * t->nparams;
+    out->bytes[UB_KIND_OPTIM] += (c.super_res ? 5 : 3) * img + 7.0 * 4 * t->nparams + 4.0 * t->nparams + 2.0 * 2 * t->nparams;
     t->host_step += reps;
     return UB_OK;
 }
@@ -1712,13 +1751,28 @@ extern "C" int ub_trainer_last_loss(UbTrainer* t, float* loss_out) {
 }
 extern "C" void* ub_trainer_stream(UbTrainer* t) { return (void*)t->stream; }
 extern "C" int ub_trainer_launches_per_step(UbTrainer* t) {
-    // tapes + memset-free extras: diffusion (2), adamw, pack, step increment
-    return t->launches_fwd + t->launches_bwd + 5;
+    // tapes + memset-free extras: diffusion (2), adamw, pack, step increment (+ the super-res condition)
+    return t->launches_fwd + t->launches_bwd + 5 + (t->cfg.super_res ? 1 : 0);
+}
+
+// super-resolution model: enqueue the upsampling of the stored low-res batch into the conditioning channels that the
+// forward tape (and the sampling graphs captured from it) read; UB_ERR_STATE before ub_trainer_set_low_res
+static int prepare_inference_cond(UbTrainer* t) {
+    const UbConfig& c = t->cfg;
+    if (!c.super_res) return UB_OK;
+    if (!t->have_low_res) {
+        set_err("a super-resolution model needs its low-res images: call ub_trainer_set_low_res first");
+        return UB_ERR_STATE;
+    }
+    superres_cond(t->low_res, 0, nullptr, c.B, c.C_in, c.H, c.W, c.super_res, t->cond, t->stream);
+    CUDA_TRY(cudaGetLastError());
+    return UB_OK;
 }
 
 extern "C" int ub_trainer_predict(UbTrainer* t, const float* xt_host, const float* t_host, float* out_host) {
     CUDA_TRY(cudaSetDevice(t->device));
     const UbConfig& c = t->cfg;
+    if (int r = prepare_inference_cond(t)) return r;
     const size_t img = size_t(c.B) * c.C_in * c.H * c.W, oimg = size_t(c.B) * c.C_out * c.H * c.W;
     CUDA_TRY(cudaMemcpyAsync(t->xt, xt_host, img * sizeof(float), cudaMemcpyHostToDevice, t->stream));
     CUDA_TRY(cudaMemcpyAsync(t->tsteps, t_host, c.B * sizeof(float), cudaMemcpyHostToDevice, t->stream));
@@ -1746,6 +1800,7 @@ extern "C" int ub_trainer_sample(UbTrainer* t, const float* x_init_host, int t_s
         set_err("sampling range must satisfy 2 <= t_end <= t_start < n_timesteps");
         return UB_ERR_SHAPE;
     }
+    if (int r = prepare_inference_cond(t)) return r;
     const size_t img = size_t(c.B) * c.C_in * c.H * c.W;
     cudaStream_t st = t->stream;
     if (x_init_host)
@@ -1934,6 +1989,7 @@ extern "C" int ub_trainer_sample_spaced(UbTrainer* t, const int* timesteps, int 
             set_err("timesteps must be strictly ascending in [0, %d): entry %d is %d", c.n_timesteps, i, timesteps[i]);
             return UB_ERR_SHAPE;
         }
+    if (int r = prepare_inference_cond(t)) return r;
     std::vector<SpacedRow> rows(n);
     spaced_rows(c.n_timesteps, timesteps, n, sampler, double(eta), clip_denoised, rows.data());
     std::vector<int> ts(timesteps, timesteps + n);
@@ -2086,6 +2142,32 @@ extern "C" int ub_trainer_set_labels(UbTrainer* t, const int* labels_host, size_
     CUDA_TRY(cudaMemcpy(t->labels, labels_host, n * sizeof(int), cudaMemcpyHostToDevice));
     return UB_OK;
 }
+extern "C" int ub_trainer_set_low_res(UbTrainer* t, const float* host, size_t n) {
+    const UbConfig& c = t->cfg;
+    if (!c.super_res) {
+        set_err("not a super-resolution model: the trainer was created with cfg.super_res = 0");
+        return UB_ERR_STATE;
+    }
+    const size_t want = size_t(c.B) * c.C_in * (c.H / c.super_res) * (c.W / c.super_res);
+    if (n != want) {
+        set_err("size mismatch: got %zu low-res values, expected %zu (B, C_in, H/%d, W/%d)", n, want, c.super_res,
+                c.super_res);
+        return UB_ERR_SHAPE;
+    }
+    CUDA_TRY(cudaSetDevice(t->device));
+    CUDA_TRY(cudaStreamSynchronize(t->stream));  // (an inference call in flight may still be upsampling the old batch)
+    CUDA_TRY(cudaMemcpy(t->low_res, host, n * sizeof(float), cudaMemcpyHostToDevice));
+    t->have_low_res = true;
+    return UB_OK;
+}
+extern "C" int ub_trainer_get_cond(UbTrainer* t, float* host, size_t n) {
+    if (!t->cond) {
+        set_err("conditioning channels exist only when the trainer was created with cfg.super_res");
+        return UB_ERR_STATE;
+    }
+    const UbConfig& c = t->cfg;
+    return copy_out(t, t->cond, host, n, size_t(c.B) * c.C_in * c.H * c.W);
+}
 extern "C" int ub_trainer_get_grads(UbTrainer* t, float* host, size_t n) {
     return copy_out(t, t->grads, host, n, t->nparams);
 }
@@ -2155,7 +2237,8 @@ extern "C" int ub_trainer_load(UbTrainer* t, const char* path) {
         return UB_ERR_IO;
     }
     const UbConfig& c = t->cfg;
-    if (header[2] != c.C_in || header[3] != c.C_model || header[4] != c.C_out || header[5] != c.H ||
+    const int model_in = c.super_res ? 2 * c.C_in : c.C_in;  // (the first conv's input channels, as the file states)
+    if (header[2] != model_in || header[3] != c.C_model || header[4] != c.C_out || header[5] != c.H ||
         header[6] != c.W) {
         fclose(f);
         set_err("%s: checkpoint shape (C_in %d, C_model %d, C_out %d, %dx%d) does not match the trainer", path,
@@ -2219,7 +2302,8 @@ static int save_checkpoint(UbTrainer* t, const char* path, const float* weights,
     const UbConfig& c = t->cfg;
     int header[256];
     memset(header, 0, sizeof header);
-    header[0] = kModelMagic, header[1] = c.B, header[2] = c.C_in, header[3] = c.C_model, header[4] = c.C_out;
+    header[0] = kModelMagic, header[1] = c.B, header[2] = c.super_res ? 2 * c.C_in : c.C_in, header[3] = c.C_model;
+    header[4] = c.C_out;
     header[5] = c.H, header[6] = c.W, header[7] = c.max_period, header[8] = with_adamw ? 1 : 0, header[9] = 0;
     int step = 0;
     cudaMemcpy(&step, t->step_dev, sizeof(int), cudaMemcpyDeviceToHost);
