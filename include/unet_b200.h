@@ -264,10 +264,20 @@ typedef struct {
                             (after random_flip), on the device; predict / sample / sample_spaced upsample the batch of
                             ub_trainer_set_low_res.  Needs C_in == C_out == 3, f dividing H and W, W % 4 == 0 and
                             W <= 256; 0 */
+    int learn_sigma;     /* 1: learned-variance model (guided-diffusion's `--learn_sigma True` with improved-diffusion's
+                            hybrid loss, `use_kl False`, `rescale_learned_sigmas True`): the output conv has 2*C_out outputs
+                            [eps | v], and training minimises mse(eps, noise) + (n_timesteps / 1000) * vb, where vb is the
+                            variational bound term of the Gaussian p(x_{t-1} | x_t) with the eps-derived mean (eps detached)
+                            and the log-variance frac * log(beta_t) + (1 - frac) * log(posterior_variance_t), frac =
+                            (v + 1) / 2 -- in bits per dimension, the discretised decoder likelihood at t = 0.  eps learns
+                            from the MSE only, v from vb only.  ub_trainer_sample_spaced samples with the learned variance;
+                            ub_trainer_sample refuses the model.  Needs C_out == 3, W % 8 == 0, n_timesteps >= 2, no
+                            compute_dinput, and an output head the 6-channel row kernels take; 0 */
 } UbConfig;
 
 void ub_default_config(UbConfig* cfg);
-/* number of parameters for a config (326 tensors / 20 494 211 floats for the default; 0 for a config that is refused) */
+/* number of parameters for a config (326 tensors / 20 494 211 floats for the default; 0 for a config that is refused).
+ * learn_sigma adds C * 9 * C_out + C_out, the v rows of the output conv (C its input width) */
 size_t ub_num_params(const UbConfig* cfg);
 
 int ub_trainer_create(UbTrainer** out, const UbConfig* cfg, int device);
@@ -276,7 +286,8 @@ void ub_trainer_destroy(UbTrainer* t);
 /* checkpoint, train_unet.cu:4762-4911 / train_unet.py:768-795: int32[256] header {12345678, B, C_in, C_model, C_out,
  * H, W, max_period, has_adamw, has_rng} + fp32 params [+ m + v].  For a super-resolution model (cfg.super_res) header[2]
  * holds the first conv's input channel count 2*C_in -- the value the reference's loader builds that conv from -- and
- * ub_trainer_load expects it there (a plain trainer refuses such a file with UB_ERR_SHAPE).  The rng flag is always written 0 (the reference's
+ * ub_trainer_load expects it there (a plain trainer refuses such a file with UB_ERR_SHAPE).  Likewise header[4] holds the
+ * output conv's 2*C_out channels for a learned-variance model (cfg.learn_sigma).  The rng flag is always written 0 (the reference's
  * blob is a raw curandState dump); header[10] additionally stores the AdamW step count (the reference forgets it),
  * marked valid by header[11] = 0x55425354.  The reference's C writer leaves words 10..255 uninitialised
  * (train_unet.cu:4764), so ub_trainer_load trusts header[10] only behind that marker and otherwise restarts the count
@@ -286,7 +297,8 @@ int ub_trainer_save(UbTrainer* t, const char* path, int with_adamw);
 int ub_trainer_set_step(UbTrainer* t, int step);
 /* read the {B, C_in, C_model, C_out, H, W, max_period} header of a checkpoint into cfg (other fields untouched).  Like
  * head_size and channel_mult, the super-resolution factor is not stored: for a super-resolution checkpoint C_in reads
- * 2*C_in, and the caller sets C_in = header value / 2 and super_res to the factor the model was trained with. */
+ * 2*C_in, and the caller sets C_in = header value / 2 and super_res to the factor the model was trained with.  For a
+ * learned-variance checkpoint C_out reads 2*C_out: the caller sets C_out = header value / 2 and learn_sigma = 1. */
 int ub_read_checkpoint_header(const char* path, UbConfig* cfg);
 
 /* host <-> device parameter access, reference parameter order (forward layer order, SURVEY.md section 8 a13) */
@@ -303,7 +315,8 @@ int ub_trainer_set_labels(UbTrainer* t, const int* labels_host, size_t n);
 /* the dropout mask (0 / 1 bytes, B x H x W x C in NHWC order) the LAST training step applied in ResBlock `block`
  * (forward order), regenerated from its Philox key -- for parity checks (cfg.dropout > 0) */
 int ub_trainer_get_dropout_mask(UbTrainer* t, int block, unsigned char* host, size_t n);
-int ub_trainer_get_output(UbTrainer* t, float* host, size_t n); /* last forward's eps prediction (B,C_out,H,W) */
+/* last forward's eps prediction (B,C_out,H,W); with cfg.learn_sigma the whole head output (B,2*C_out,H,W), [eps | v] */
+int ub_trainer_get_output(UbTrainer* t, float* host, size_t n);
 /* the flip decisions (0 / 1 per image) the last step took, when cfg.random_flip is set */
 int ub_trainer_get_flips(UbTrainer* t, int* host, size_t n);
 int ub_trainer_get_batch(UbTrainer* t, float* host, size_t n);  /* the x0 batch the last step consumed (B,C_in,H,W) */
@@ -346,10 +359,15 @@ int ub_trainer_train_step_device(UbTrainer* t, const float* x0_dev, float lr, fl
                                  float weight_decay);
 int ub_trainer_sync(UbTrainer* t);
 int ub_trainer_last_loss(UbTrainer* t, float* loss_out);
+/* the last step's batch means of the two loss terms, under the synchronisation rules of ub_trainer_last_loss: mse, and
+ * the rescaled variational-bound term vb of a learned-variance model (cfg.learn_sigma; 0 without it).
+ * ub_trainer_last_loss returns mse + vb.  Either pointer may be NULL. */
+int ub_trainer_last_loss_terms(UbTrainer* t, float* mse, float* vb);
 void* ub_trainer_stream(UbTrainer* t); /* cudaStream_t the trainer launches on */
 /* kernels launched per train step (counted while building the step) */
 int ub_trainer_launches_per_step(UbTrainer* t);
-/* forward only on a device batch that is ALREADY x_t (for sampling, generate.py:29-52): out_dev (B,C_out,H,W) */
+/* forward only on a device batch that is ALREADY x_t (for sampling, generate.py:29-52): out_dev (B,C_out,H,W), or
+ * (B,2*C_out,H,W) with cfg.learn_sigma */
 int ub_trainer_predict(UbTrainer* t, const float* xt_host, const float* t_host, float* out_host);
 
 /* DDPM ancestral sampling, the loop of generate.py:29-79 on the device: for t = t_start .. t_end (descending)
@@ -358,7 +376,9 @@ int ub_trainer_predict(UbTrainer* t, const float* xt_host, const float* t_host, 
  * on all B images of the trainer at once.  generate.py runs t = n_timesteps-1 .. 2 (pass t_start = -1, t_end = -1 for
  * exactly that).  x_init_host (B,C_in,H,W) may be NULL: x_T ~ N(0,1) from `seed`.  noise_host may be NULL (z from the
  * device Philox stream of `seed`), else it holds one (B,C_in,H,W) draw per iteration, first iteration first (parity
- * runs inject the oracle's draws).  out_host (B,C_in,H,W) receives the final x.  One CUDA graph per iteration. */
+ * runs inject the oracle's draws).  out_host (B,C_in,H,W) receives the final x.  One CUDA graph per iteration.
+ * A learned-variance model (cfg.learn_sigma) gets UB_ERR_STATE: generate.py's loop has no learned variance; use
+ * ub_trainer_sample_spaced with UB_SAMPLER_ANCESTRAL and every timestep kept instead. */
 int ub_trainer_sample(UbTrainer* t, const float* x_init_host, int t_start, int t_end, const float* noise_host,
                       unsigned long long seed, float* out_host);
 
@@ -380,13 +400,16 @@ int ub_trainer_sample(UbTrainer* t, const float* x_init_host, int t_start, int t
  * Counts are non-negative decimal integers; a spec that keeps nothing is refused. */
 int ub_space_timesteps(int n_timesteps, const char* spec, int* out, int cap);
 #define UB_SAMPLER_DDIM 0       /* ddim_sample_loop, eta in [0, 1] */
-#define UB_SAMPLER_ANCESTRAL 1  /* p_sample_loop, fixed-large variance; eta must be 0; n >= 2 */
+#define UB_SAMPLER_ANCESTRAL 1  /* p_sample_loop, fixed-large (learned-range with cfg.learn_sigma) variance; eta = 0; n >= 2 */
 /* Sampling over the kept timesteps t_0 < ... < t_{n-1} (strictly ascending, in [0, n_timesteps); e.g. from
  * ub_space_timesteps), guided-diffusion's SpacedDiffusion with rescale_timesteps = False.  Float64 tables of the
  * trainer's linear schedule: acp = cumprod(1 - beta); beta'_i = 1 - acp[t_i] / acp[t_{i-1}] (acp[t_{-1}] = 1),
  * acp'_i = cumprod(1 - beta'), acp'_{-1} = 1.  For i = n-1 down to 0, on all B images of the trainer at once:
  *   eps = model(x, t_i);  x0 = sqrt(1/acp'_i) x - sqrt(1/acp'_i - 1) eps, clamped to [-1, 1] if clip_denoised;
  *   ANCESTRAL: x <- posterior mean(x0, x) + [i > 0] sqrt(beta'_i) z                     (fixed-large variance)
+ *              learned range (cfg.learn_sigma): [i > 0] exp(0.5 (frac log beta'_i + (1 - frac) lpost'_i)) z per element,
+ *              frac = (v + 1) / 2, lpost' the clipped log posterior variance of the respaced chain (eps and v are
+ *              channels 0..C_out-1 and C_out..2*C_out-1 of the model output; DDIM ignores v)
  *   DDIM:      eps' = (sqrt(1/acp'_i) x - x0) / sqrt(1/acp'_i - 1),
  *              sigma = eta sqrt((1 - acp'_{i-1}) / (1 - acp'_i)) sqrt(1 - acp'_i / acp'_{i-1}),
  *              x <- sqrt(acp'_{i-1}) x0 + sqrt(1 - acp'_{i-1} - sigma^2) eps' + [i > 0] sigma z

@@ -31,7 +31,8 @@ class UbConfig(C.Structure):
                 ("gn_n_groups", C.c_int), ("n_timesteps", C.c_int), ("seed", C.c_ulonglong),
                 ("use_cuda_graph", C.c_int), ("compute_dinput", C.c_int), ("random_flip", C.c_int),
                 ("num_classes", C.c_int), ("ema_rate", C.c_float), ("resblock_updown", C.c_int),
-                ("use_scale_shift_norm", C.c_int), ("dropout", C.c_float), ("super_res", C.c_int)]
+                ("use_scale_shift_norm", C.c_int), ("dropout", C.c_float), ("super_res", C.c_int),
+                ("learn_sigma", C.c_int)]
 
 
 UB_KINDS = ("conv_igemm", "wgrad_igemm", "groupnorm", "attention", "eltwise", "small", "optimizer")
@@ -90,6 +91,7 @@ def _declare(L: C.CDLL) -> None:
     L.ub_trainer_set_next_batch.argtypes = [vp, vp]
     L.ub_trainer_sync.argtypes = [vp]
     L.ub_trainer_last_loss.argtypes = [vp, C.POINTER(C.c_float)]
+    L.ub_trainer_last_loss_terms.argtypes = [vp, C.POINTER(C.c_float), C.POINTER(C.c_float)]
     L.ub_trainer_set_step.argtypes = [vp, i]
     L.ub_trainer_get_flips.argtypes = [vp, vp, C.c_size_t]
     L.ub_set_layer_precision.argtypes = [i]
@@ -242,9 +244,13 @@ class Trainer:
         c = self.cfg
         return self._get(lib().ub_trainer_get_batch, c.B * c.C_in * c.H * c.W).reshape(c.B, c.C_in, c.H, c.W)
 
+    def _out_channels(self) -> int:
+        """Channels of the model output: C_out, or 2 * C_out [eps | v] for a learned-variance model."""
+        return self.cfg.C_out * (2 if self.cfg.learn_sigma else 1)
+
     def get_output(self):
-        c = self.cfg
-        return self._get(lib().ub_trainer_get_output, c.B * c.C_out * c.H * c.W).reshape(c.B, c.C_out, c.H, c.W)
+        c, co = self.cfg, self._out_channels()
+        return self._get(lib().ub_trainer_get_output, c.B * co * c.H * c.W).reshape(c.B, co, c.H, c.W)
 
     def load(self, path: str):
         check(lib().ub_trainer_load(self._h, path.encode()), "ub_trainer_load")
@@ -297,6 +303,13 @@ class Trainer:
         check(lib().ub_trainer_last_loss(self._h, C.byref(loss)), "last_loss")
         return float(loss.value)
 
+    def last_loss_terms(self) -> tuple:
+        """(mse, vb) batch means of the last step; vb is the rescaled variational-bound term of a learned-variance
+        model (learn_sigma; 0 otherwise) and last_loss() their sum."""
+        mse, vb = C.c_float(), C.c_float()
+        check(lib().ub_trainer_last_loss_terms(self._h, C.byref(mse), C.byref(vb)), "last_loss_terms")
+        return float(mse.value), float(vb.value)
+
     def stream(self) -> int:
         return int(lib().ub_trainer_stream(self._h) or 0)
 
@@ -314,7 +327,7 @@ class Trainer:
         c = self.cfg
         xt = np.ascontiguousarray(xt, dtype=np.float32)
         t = np.ascontiguousarray(t, dtype=np.float32).reshape(-1)
-        out = np.empty((c.B, c.C_out, c.H, c.W), dtype=np.float32)
+        out = np.empty((c.B, self._out_channels(), c.H, c.W), dtype=np.float32)
         check(lib().ub_trainer_predict(self._h, _ptr(xt), _ptr(t), _ptr(out)), "predict")
         return out
 

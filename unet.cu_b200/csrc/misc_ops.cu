@@ -927,30 +927,52 @@ __global__ void spaced_set_t_kernel(const int* __restrict__ ts_table, const Spac
 void spaced_set_t(const int* ts_table, const SpacedState* s, int B, float* tsteps, cudaStream_t st) {
     launch_pdl(spaced_set_t_kernel, dim3((B + 127) / 128), dim3(128), 0, st, ts_table, s, B, tsteps);
 }
+// LEARNED (learned-variance model): eps and v are channels 0-2 and 3-5 of the model's (B, 6, H, W) output (img3 = the
+// 3 H W floats of one image of x), and sigma = c.sigma * exp(0.5 (frac log beta' + (1 - frac) lpost')) per element,
+// frac = (v + 1) / 2, with {log beta', lpost'} in c.pad: c.sigma is the [i > 0] draw flag of the learned-range
+// ancestral sampler; DDIM rows leave pad at 0, so that v drops out and sigma is DDIM's.
+template <bool LEARNED>
 __global__ void spaced_step_kernel(float* __restrict__ x, const float* __restrict__ eps,
                                    const SpacedRow* __restrict__ rows, const float* __restrict__ z, size_t n4,
-                                   const SpacedState* __restrict__ s) {
+                                   const SpacedState* __restrict__ s, size_t img3) {
     pdl_entry();
     const size_t i4 = size_t(blockIdx.x) * blockDim.x + threadIdx.x;
     if (i4 >= n4) return;
     const int it = s->it;
     const SpacedRow c = rows[it];
-    const float4 xv = reinterpret_cast<const float4*>(x)[i4], ev = reinterpret_cast<const float4*>(eps)[i4];
+    const float4 xv = reinterpret_cast<const float4*>(x)[i4];
+    float4 ev, sv = make_float4(c.sigma, c.sigma, c.sigma, c.sigma);
+    if constexpr (LEARNED) {
+        const size_t e = 4 * i4, bi = e / img3, o = bi * 2 * img3 + (e - bi * img3);  // (img3 % 4 == 0)
+        ev = *reinterpret_cast<const float4*>(eps + o);
+        const float4 vv = *reinterpret_cast<const float4*>(eps + o + img3);
+        auto sig = [&](float v) {
+            const float frac = 0.5f * (v + 1.f);
+            return c.sigma * expf(0.5f * (frac * c.pad[0] + (1.f - frac) * c.pad[1]));
+        };
+        sv = make_float4(sig(vv.x), sig(vv.y), sig(vv.z), sig(vv.w));
+    } else {
+        ev = reinterpret_cast<const float4*>(eps)[i4];
+    }
     float4 zv = make_float4(0.f, 0.f, 0.f, 0.f);
     if (c.sigma != 0.f) zv = z ? reinterpret_cast<const float4*>(z)[i4] : philox_normal4(i4, 0x5u, uint32_t(it), s->seed);
-    auto upd = [&](float xs, float es, float zs) {
+    auto upd = [&](float xs, float es, float zs, float ss) {
         float x0 = c.r * xs - c.rm1 * es;
         if (c.clip != 0.f) x0 = fminf(fmaxf(x0, -1.f), 1.f);
-        return c.c_x0 * x0 + c.c_x * xs + c.sigma * zs;
+        return c.c_x0 * x0 + c.c_x * xs + ss * zs;
     };
-    reinterpret_cast<float4*>(x)[i4] =
-        make_float4(upd(xv.x, ev.x, zv.x), upd(xv.y, ev.y, zv.y), upd(xv.z, ev.z, zv.z), upd(xv.w, ev.w, zv.w));
+    reinterpret_cast<float4*>(x)[i4] = make_float4(upd(xv.x, ev.x, zv.x, sv.x), upd(xv.y, ev.y, zv.y, sv.y),
+                                                   upd(xv.z, ev.z, zv.z, sv.z), upd(xv.w, ev.w, zv.w, sv.w));
 }
 void spaced_step(float* x, const float* eps, const SpacedRow* rows, const float* z, size_t n, SpacedState* s,
-                 cudaStream_t st) {
+                 cudaStream_t st, size_t img3) {
     const size_t n4 = n / 4;
-    launch_pdl(spaced_step_kernel, dim3(unsigned((n4 + 255) / 256)), dim3(256), 0, st, x, eps, rows, z, n4,
-               static_cast<const SpacedState*>(s));
+    if (img3)
+        launch_pdl(spaced_step_kernel<true>, dim3(unsigned((n4 + 255) / 256)), dim3(256), 0, st, x, eps, rows, z, n4,
+                   static_cast<const SpacedState*>(s), img3);
+    else
+        launch_pdl(spaced_step_kernel<false>, dim3(unsigned((n4 + 255) / 256)), dim3(256), 0, st, x, eps, rows, z, n4,
+                   static_cast<const SpacedState*>(s), img3);
     increment_step(&s->it, st);
 }
 

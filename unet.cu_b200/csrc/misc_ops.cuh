@@ -92,6 +92,7 @@ void fill_normal(float* x, size_t n, uint64_t seed, cudaStream_t st);
 //      float32 coefficients of loop iteration it (largest timestep first), built by the host in float64; both samplers
 //      share the update
 //        x0 = r * x - rm1 * eps  (clamped to [-1, 1] when clip != 0);   x <- c_x0 * x0 + c_x * x + sigma * z
+//      (pad: {log beta', lpost'} of a learned-variance model's ancestral rows, else 0)
 //      The iteration counter and the Philox key live in device memory, so one captured graph serves every iteration and
 //      every seed.
 struct SpacedRow {
@@ -105,9 +106,10 @@ struct SpacedState {
 // tsteps[b] = float(ts_table[it]) (the model sees the original timestep)
 void spaced_set_t(const int* ts_table, const SpacedState* s, int B, float* tsteps, cudaStream_t st);
 // z: injected noise of this iteration (may be null: Philox(seed, stream id 0x5, counter = it)); no draw where sigma = 0.
-// Then it <- it + 1.
+// Then it <- it + 1.  img3 > 0: learned-variance model -- eps is the (B, 6, H, W) model output [eps | v] with img3 =
+// 3 H W floats per image of x, and the row's pad holds {log beta', lpost'} of the learned-range variance (see misc_ops.cu)
 void spaced_step(float* x, const float* eps, const SpacedRow* rows, const float* z, size_t n, SpacedState* s,
-                 cudaStream_t st);
+                 cudaStream_t st, size_t img3 = 0);
 // occupy the stream for ~us microseconds (profiling aid: lets the host queue work ahead of the device)
 void stream_delay(unsigned us, cudaStream_t st);
 

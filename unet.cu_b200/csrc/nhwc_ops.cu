@@ -1030,8 +1030,8 @@ void conv_in_fwd(const float* x, const float* x2, const float* w, const float* b
     smallc_conv(x, x2, w, b, Cin, Cout, B, H, W, 0, y, ldy, st);
 }
 void conv_out_dgrad(const float* dout, const float* w, int B, int Cin, int Cout, int H, int W, bf16* da, int ldda,
-                    cudaStream_t st) {
-    smallc_conv(dout, nullptr, w, nullptr, Cout, Cin, B, H, W, 1, da, ldda, st);
+                    cudaStream_t st, const float* dout2) {
+    smallc_conv(dout, dout2, w, nullptr, Cout, Cin, B, H, W, 1, da, ldda, st);
 }
 
 // partial[blk][cb][s*9+tap] = sum_{p in block} yb[p][cb] * xs[b][s][p + shift(tap)] ; partial[blk][cb][NT] = sum yb
@@ -1370,26 +1370,78 @@ __global__ void conv_out_pair_kernel(const bf16* __restrict__ a, int lda, const 
             *reinterpret_cast<float2*>(out + ((b * Cout + o) * H + h) * W + w0) = make_float2(a0[o] + bv, a1[o] + bv);
         }
 }
-// Row-per-warp output head (Cout == 3, Cin % 64 == 0, W % 8 == 0): lane l owns input channels 2l, 2l+1 of a 64-channel
-// group (its 3 x 2 x 9 weights in registers), slides a 3 x 3 window of bf16 pairs along the image row -- every load is
-// one coalesced 128-byte row of a pixel -- and the 3 x 8 partial sums of 8 pixels are added across the 32 lanes with a
-// 31-shuffle transpose-reduce.  The finished row goes through shared memory so that out (NCHW fp32) is written in
-// coalesced rows; with `target` the MSE loss and its gradient (mse_kernel) are computed on the spot.
+// Row-per-warp output head (CO == 3 or 6, Cin % 64 == 0, W % 8 == 0): lane l owns input channels 2l, 2l+1 of a
+// 64-channel group (its CO x 2 x 9 weights in registers), slides a 3 x 3 window of bf16 pairs along the image row --
+// every load is one coalesced 128-byte row of a pixel -- and the CO x PX partial sums of PX pixels are added across the
+// 32 lanes with a 31-shuffle transpose-reduce (PX = 8 for CO = 3; 4 for CO = 6, so that the 24 values still fit one
+// reduce).  The finished row goes through shared memory so that out (NCHW fp32) is written in coalesced rows; with
+// `target` the MSE loss and its gradient (mse_kernel) are computed on the spot.
+// CO = 6 is the learned-variance head [eps | v]: the epilogue also evaluates the hybrid loss's vb term of the row's
+// 3 W (eps, v) pairs (see HybridLoss) and writes dL/d eps to dout and dL/d v to hl.dv, both (B, 3, H, W).
+// approx_standard_normal_cdf, 0.5 (1 + tanh z) with z = sqrt(2/pi) (x + 0.044715 x^3), written as the logistic
+// 1 / (1 + e^{-2z}): the same function, without the cancellation of 1 + tanh z in the lower tail.  It is odd-symmetric
+// about 1/2, so the upper tail is taken as 1 - cdf(-x) where it matters (see hybrid_vb).
+__device__ __forceinline__ float approx_std_normal_cdf(float x) {
+    return 1.f / (1.f + expf(-1.5957691216057308f * (x + 0.044715f * x * x * x)));
+}
+__device__ __forceinline__ float approx_std_normal_pdf(float x) {  // d/dx: 0.5 sech^2(z) dz/dx, sech^2 z = 4e/(1+e)^2
+    const float e = expf(-1.5957691216057308f * fabsf(x + 0.044715f * x * x * x));
+    return 2.f * e / ((1.f + e) * (1.f + e)) * 0.7978845608028654f * (1.f + 3.f * 0.044715f * x * x);
+}
+// vb of one element (nats, before the 1/ln 2 and T/1000 factors) and its derivative with respect to v.
+// k = {sqrt(1/acp), sqrt(1/acp - 1), c1, c2, log beta, lpost, T/1000, 0} of the element's timestep t.
+__device__ __forceinline__ float hybrid_vb(float eps, float v, float xt, float x0, int t, float4 k0, float4 k1,
+                                           float& dvb_dv) {
+    const float x0p = k0.x * xt - k0.y * eps;
+    const float mmean = k0.z * x0p + k0.w * xt, tmean = k0.z * x0 + k0.w * xt;
+    const float frac = 0.5f * (v + 1.f);
+    const float mlv = frac * k1.x + (1.f - frac) * k1.y;
+    const float dmlv_dv = 0.5f * (k1.x - k1.y);
+    if (t > 0) {  // normal_kl(true_mean, lpost, model_mean, model_logvar); -1 + e^u folded into expm1 (u ~ 0 at large t)
+        const float u = k1.y - mlv, em1 = expm1f(u), d = tmean - mmean, q = d * d * expf(-mlv);
+        dvb_dv = -0.5f * (em1 + q) * dmlv_dv;
+        return 0.5f * (em1 - u + q);
+    }
+    // -discretized_gaussian_log_likelihood(x0, model_mean, 0.5 model_logvar)
+    const float ls = 0.5f * mlv, inv = expf(-ls), cx = x0 - mmean;
+    const float pin = inv * (cx + 1.f / 255.f), min_ = inv * (cx - 1.f / 255.f);
+    float lp, dlp;  // log prob and d(log prob)/d(log scale); dpin/dls = -pin, dmin/dls = -min
+    if (x0 < -0.999f) {
+        const float cp = approx_std_normal_cdf(pin);
+        lp = logf(fmaxf(cp, 1e-12f));
+        dlp = cp >= 1e-12f ? -approx_std_normal_pdf(pin) * pin / cp : 0.f;
+    } else if (x0 > 0.999f) {
+        const float om = approx_std_normal_cdf(-min_);  // 1 - cdf(min)
+        lp = logf(fmaxf(om, 1e-12f));
+        dlp = om >= 1e-12f ? approx_std_normal_pdf(min_) * min_ / om : 0.f;
+    } else {
+        // cdf(plus) - cdf(min), from the tail the bin lies in (both values near 1 would cancel)
+        const float dl = min_ > 0.f ? approx_std_normal_cdf(-min_) - approx_std_normal_cdf(-pin)
+                                    : approx_std_normal_cdf(pin) - approx_std_normal_cdf(min_);
+        lp = logf(fmaxf(dl, 1e-12f));
+        dlp = dl >= 1e-12f ? (min_ * approx_std_normal_pdf(min_) - pin * approx_std_normal_pdf(pin)) / dl : 0.f;
+    }
+    dvb_dv = -dlp * 0.5f * dmlv_dv;
+    return -lp;
+}
+template <int CO>
 __global__ void __launch_bounds__(kSmallcWarps * 32) conv_out_rows_kernel(
     const bf16* __restrict__ a, int lda, const float* __restrict__ w, const float* __restrict__ bias, int Cin, int B,
     int H, int W, float* __restrict__ out, const float* __restrict__ target, float* __restrict__ loss,
-    float* __restrict__ dout, float inv_n, float gscale) {
+    float* __restrict__ dout, float inv_n, float gscale, HybridLoss hl) {
+    static_assert(CO == 3 || CO == 6, "the output head has 3 outputs, or 6 with a learned variance");
+    constexpr int PX = CO == 3 ? 8 : 4, PXS = CO == 3 ? 3 : 2;  // pixels per reduce, log2
     pdl_entry();
-    constexpr int CO = 3;
     extern __shared__ float sm[];
     float* sw = sm;                                         // [CO][Cin][9] as given
     float* srow = sm + CO * Cin * 9 + (threadIdx.x >> 5) * (CO * W);  // this warp's [CO][W] output row
     __shared__ float sloss[kSmallcWarps];
+    __shared__ float svb[CO == 6 ? kSmallcWarps : 1];
     for (int i = threadIdx.x; i < CO * Cin * 9; i += blockDim.x) sw[i] = w[i];
     __syncthreads();
     const int lane = threadIdx.x & 31, warp = threadIdx.x >> 5;
     const long long item = (long long)blockIdx.x * kSmallcWarps + warp;
-    float lsum = 0.f;
+    float lsum = 0.f, vsum = 0.f;
     if (item < (long long)B * H) {
         const int h = int(item % H), b = int(item / H);
         for (int i = lane; i < CO * W; i += 32) srow[i] = bias ? bias[i / W] : 0.f;
@@ -1411,30 +1463,32 @@ __global__ void __launch_bounds__(kSmallcWarps * 32) conv_out_rows_kernel(
                 rok[r] = hh >= 0 && hh < H;
                 rowp[r] = a + ((size_t(b) * H + (rok[r] ? hh : h)) * W) * lda + c0;
             }
-            // packed bf16 pairs of window columns x0-1 .. x0+8 per row: the two leading columns are carried over from
-            // the previous batch, the eight new ones are fetched with 24 independent loads (one L2 latency per 8 pixels)
-            uint32_t colw[3][10];
+            // packed bf16 pairs of window columns x0-1 .. x0+PX per row: the two leading columns are carried over from
+            // the previous batch, the PX new ones are fetched with 3 PX independent loads (one L2 latency per batch)
+            uint32_t colw[3][PX + 2];
 #pragma unroll
             for (int r = 0; r < 3; ++r) {
-                colw[r][8] = 0u;  // column -1
-                colw[r][9] = rok[r] ? *reinterpret_cast<const uint32_t*>(rowp[r]) : 0u;  // column 0
+                colw[r][PX] = 0u;  // column -1
+                colw[r][PX + 1] = rok[r] ? *reinterpret_cast<const uint32_t*>(rowp[r]) : 0u;  // column 0
             }
-            for (int x0 = 0; x0 < W; x0 += 8) {
+            for (int x0 = 0; x0 < W; x0 += PX) {
 #pragma unroll
                 for (int r = 0; r < 3; ++r) {
-                    colw[r][0] = colw[r][8], colw[r][1] = colw[r][9];
+                    colw[r][0] = colw[r][PX], colw[r][1] = colw[r][PX + 1];
 #pragma unroll
-                    for (int j = 0; j < 8; ++j)
+                    for (int j = 0; j < PX; ++j)
                         colw[r][2 + j] = (rok[r] && x0 + 1 + j < W)
                                              ? *reinterpret_cast<const uint32_t*>(rowp[r] + size_t(x0 + 1 + j) * lda)
                                              : 0u;
                 }
                 float v[32];
 #pragma unroll
-                for (int i = 24; i < 32; ++i) v[i] = 0.f;
+                for (int i = CO * PX; i < 32; ++i) v[i] = 0.f;
 #pragma unroll
-                for (int j = 0; j < 8; ++j) {
-                    float a3[CO] = {0.f, 0.f, 0.f};
+                for (int j = 0; j < PX; ++j) {
+                    float a3[CO];
+#pragma unroll
+                    for (int o = 0; o < CO; ++o) a3[o] = 0.f;
 #pragma unroll
                     for (int r = 0; r < 3; ++r)
 #pragma unroll
@@ -1448,7 +1502,7 @@ __global__ void __launch_bounds__(kSmallcWarps * 32) conv_out_rows_kernel(
                             }
                         }
 #pragma unroll
-                    for (int o = 0; o < CO; ++o) v[o * 8 + j] = a3[o];
+                    for (int o = 0; o < CO; ++o) v[o * PX + j] = a3[o];
                 }
                 // transpose-reduce: after the five steps lane L holds the warp total of v[L]
 #pragma unroll
@@ -1461,45 +1515,109 @@ __global__ void __launch_bounds__(kSmallcWarps * 32) conv_out_rows_kernel(
                         v[i] = keep + __shfl_xor_sync(0xffffffffu, send, sft);
                     }
                 }
-                if (lane < 24) srow[(lane >> 3) * W + x0 + (lane & 7)] += v[0];
+                if (lane < CO * PX) srow[(lane >> PXS) * W + x0 + (lane & (PX - 1))] += v[0];
             }
             __syncwarp();
         }
-        // the finished row: out, and optionally the loss and its gradient
-        for (int i = lane; i < CO * W; i += 32) {
-            const int o = i / W, x = i % W;
-            const size_t gi = ((size_t(b) * CO + o) * H + h) * W + x;
-            const float val = srow[i];
-            out[gi] = val;
+        if constexpr (CO == 3) {
+            // the finished row: out, and optionally the loss and its gradient
+            for (int i = lane; i < CO * W; i += 32) {
+                const int o = i / W, x = i % W;
+                const size_t gi = ((size_t(b) * CO + o) * H + h) * W + x;
+                const float val = srow[i];
+                out[gi] = val;
+                if (target) {
+                    const float d = val - target[gi];
+                    lsum += d * d;
+                    if (dout) dout[gi] = 2.f * d * inv_n * gscale;
+                }
+            }
+        } else {
+            // the finished row: out (B, 6, H, W), then per (eps, v) pair the MSE and vb terms and their gradients
+            for (int i = lane; i < CO * W; i += 32) out[((size_t(b) * CO + i / W) * H + h) * W + i % W] = srow[i];
             if (target) {
-                const float d = val - target[gi];
-                lsum += d * d;
-                if (dout) dout[gi] = 2.f * d * inv_n * gscale;
+                int t = int(hl.t[b]);
+                t = t < 0 ? 0 : (t >= hl.T ? hl.T - 1 : t);  // (predict takes any timestep from its caller)
+                const float4 k0 = reinterpret_cast<const float4*>(hl.coef)[2 * t];
+                const float4 k1 = reinterpret_cast<const float4*>(hl.coef)[2 * t + 1];
+                const bool flip = hl.flips && hl.flips[b];
+                const float gv = k1.z * 1.4426950408889634f * inv_n * gscale;  // T/1000 / ln 2 / (B C H W)
+                for (int i = lane; i < 3 * W; i += 32) {
+                    const int o = i / W, x = i % W;
+                    const size_t gi = ((size_t(b) * 3 + o) * H + h) * W + x;
+                    const float eps = srow[i], vv = srow[3 * W + i];
+                    const float d = eps - target[gi];
+                    lsum += d * d;
+                    // (the step's x0 holds the batch before random_flip: q-sample mirrors it on the fly)
+                    const float x0 = hl.x0[((size_t(b) * 3 + o) * H + h) * W + (flip ? W - 1 - x : x)];
+                    float dvb;
+                    vsum += hybrid_vb(eps, vv, hl.xt[gi], x0, t, k0, k1, dvb) * k1.z;
+                    if (dout) dout[gi] = 2.f * d * inv_n * gscale, hl.dv[gi] = dvb * gv;
+                }
             }
         }
     }
     if (target) {  // one atomic per block (the L2 atomic unit serialises same-address updates)
         for (int off = 16; off; off >>= 1) lsum += __shfl_xor_sync(0xffffffffu, lsum, off);
         if (lane == 0) sloss[warp] = lsum;
+        if constexpr (CO == 6) {
+            for (int off = 16; off; off >>= 1) vsum += __shfl_xor_sync(0xffffffffu, vsum, off);
+            if (lane == 0) svb[warp] = vsum;
+        }
         __syncthreads();
         if (threadIdx.x == 0) {
             float t = 0.f;
             for (int i = 0; i < kSmallcWarps; ++i) t += sloss[i];
             atomicAdd(loss, t * inv_n);
+            if constexpr (CO == 6) {
+                float u = 0.f;
+                for (int i = 0; i < kSmallcWarps; ++i) u += svb[i];
+                atomicAdd(loss + 1, u * inv_n * 1.4426950408889634f);
+            }
         }
     }
 }
+static size_t conv_out_rows_smem(int Cin, int Co, int W) {
+    return (size_t(Co) * Cin * 9 + size_t(kSmallcWarps) * Co * W) * sizeof(float);
+}
 static bool conv_out_rows_ok(int Cin, int Cout, int W) {
-    return Cout == 3 && Cin % 64 == 0 && W % 8 == 0 &&
-           (size_t(3) * Cin * 9 + size_t(kSmallcWarps) * 3 * W) * sizeof(float) <= 48 * 1024;
+    return Cout == 3 && Cin % 64 == 0 && W % 8 == 0 && conv_out_rows_smem(Cin, 3, W) <= 48 * 1024;
+}
+// The 6-output kernel's static shared memory (sloss, svb) counts against the same 227 KiB per-block opt-in limit as
+// its dynamic block, so the dynamic budget that the config check allows -- and that conv_out_rows_prepare6 opts into --
+// is 227 KiB minus the static part.
+constexpr size_t kHeadStaticSmem = 2 * kSmallcWarps * sizeof(float);
+constexpr size_t kHeadDynSmemMax = size_t(227) * 1024 - kHeadStaticSmem;
+bool conv_out_rows_fit6(int Cin, int W) {
+    return Cin % 64 == 0 && W % 8 == 0 && conv_out_rows_smem(Cin, 6, W) <= kHeadDynSmemMax;
+}
+cudaError_t conv_out_rows_prepare6(char* msg, size_t msg_len) {
+    cudaFuncAttributes fa;
+    cudaError_t e = cudaFuncGetAttributes(&fa, conv_out_rows_kernel<6>);
+    int dev = 0, optin = 0;
+    if (e == cudaSuccess) e = cudaGetDevice(&dev);
+    if (e == cudaSuccess) e = cudaDeviceGetAttribute(&optin, cudaDevAttrMaxSharedMemoryPerBlockOptin, dev);
+    if (e != cudaSuccess) {
+        snprintf(msg, msg_len, "output head: %s", cudaGetErrorString(e));
+        return e;
+    }
+    if (fa.sharedSizeBytes > kHeadStaticSmem || fa.sharedSizeBytes + kHeadDynSmemMax > size_t(optin)) {
+        snprintf(msg, msg_len, "output head: %zu B static + %zu B dynamic shared memory exceed the device's %d B "
+                 "per-block limit", fa.sharedSizeBytes, kHeadDynSmemMax, optin);
+        return cudaErrorInvalidValue;
+    }
+    e = cudaFuncSetAttribute(conv_out_rows_kernel<6>, cudaFuncAttributeMaxDynamicSharedMemorySize, int(kHeadDynSmemMax));
+    if (e != cudaSuccess) snprintf(msg, msg_len, "output head: shared-memory opt-in failed: %s", cudaGetErrorString(e));
+    return e;
 }
 static void conv_out_rows_launch(const bf16* a, int lda, const float* w, const float* b, int B, int Cin, int H, int W,
                                  float* out, const float* target, float* loss, float* dout, float inv_n, float gscale,
                                  cudaStream_t st) {
-    const size_t smem = (size_t(3) * Cin * 9 + size_t(kSmallcWarps) * 3 * W) * sizeof(float);
+    const size_t smem = conv_out_rows_smem(Cin, 3, W);
     const long long items = (long long)B * H;
-    launch_pdl(conv_out_rows_kernel, dim3(unsigned((items + kSmallcWarps - 1) / kSmallcWarps)), dim3(kSmallcWarps * 32),
-               smem, st, a, lda, w, b, Cin, B, H, W, out, target, loss, dout, inv_n, gscale);
+    launch_pdl(conv_out_rows_kernel<3>, dim3(unsigned((items + kSmallcWarps - 1) / kSmallcWarps)),
+               dim3(kSmallcWarps * 32), smem, st, a, lda, w, b, Cin, B, H, W, out, target, loss, dout, inv_n, gscale,
+               HybridLoss{});
 }
 
 static void conv_out_launch(const bf16* a, int lda, const float* w, const float* b, int B, int Cin, int Cout, int H,
@@ -1558,10 +1676,12 @@ __global__ void nchw_chansum_kernel(const float* __restrict__ x, int B, int C, s
     }
 }
 void conv_out_wgrad(const bf16* a, int lda, const float* dout, int B, int Cin, int Cout, int H, int W, float* dw,
-                    float* db, float* scratch, size_t scratch_floats, cudaStream_t st) {
+                    float* db, float* scratch, size_t scratch_floats, cudaStream_t st, const float* dout2) {
     // D'[c][o][t'] = sum_p a[p][c] * dout[o][p + shift(t')]  ->  dw[o][c][8 - t']
-    smallc_wgrad(dout, nullptr, a, lda, B, Cout, Cin, H, W, 1, dw, nullptr, scratch, scratch_floats, st);
-    launch_pdl(nchw_chansum_kernel, dim3(Cout, B), dim3(256), 0, st, dout, B, Cout, size_t(H) * W, db);
+    smallc_wgrad(dout, dout2, a, lda, B, Cout, Cin, H, W, 1, dw, nullptr, scratch, scratch_floats, st);
+    const int Cp = dout2 ? Cout / 2 : Cout;  // channels per plane
+    launch_pdl(nchw_chansum_kernel, dim3(Cp, B), dim3(256), 0, st, dout, B, Cp, size_t(H) * W, db);
+    if (dout2) launch_pdl(nchw_chansum_kernel, dim3(Cp, B), dim3(256), 0, st, dout2, B, Cp, size_t(H) * W, db + Cp);
 }
 
 // ------------------------------------------------------------------------------------------------ loss
@@ -1603,6 +1723,20 @@ void conv_out_fwd_mse(const bf16* a, int lda, const float* w, const float* b, in
     }
     conv_out_fwd(a, lda, w, b, B, Cin, Cout, H, W, out, st);
     mse_fwd_bwd(out, target, N, loss, dout, grad_scale, st);
+}
+void conv_out_fwd_hybrid(const bf16* a, int lda, const float* w, const float* b, int B, int Cin, int H, int W,
+                         float* out, const float* noise, float* loss2, float* deps, const HybridLoss& hl,
+                         float grad_scale, cudaStream_t st) {
+    if (!conv_out_rows_fit6(Cin, W) || (lda % 2)) {  // (learned-variance configs are validated against the fit)
+        fprintf(stderr, "[unet_b200] conv_out_fwd_hybrid: %d channels at W = %d do not fit the row kernel\n", Cin, W);
+        return;
+    }
+    const long long items = (long long)B * H;
+    const cudaError_t e = launch_pdl(conv_out_rows_kernel<6>, dim3(unsigned((items + kSmallcWarps - 1) / kSmallcWarps)),
+                                     dim3(kSmallcWarps * 32), conv_out_rows_smem(Cin, 6, W), st, a, lda, w, b, Cin, B,
+                                     H, W, out, noise, loss2, deps, 1.f / float(size_t(B) * 3 * H * W), grad_scale, hl);
+    if (e != cudaSuccess)
+        fprintf(stderr, "[unet_b200] conv_out_fwd_hybrid: launch failed: %s\n", cudaGetErrorString(e));
 }
 
 }  // namespace ub

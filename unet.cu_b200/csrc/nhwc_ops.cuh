@@ -98,16 +98,43 @@ bool smallc_rows_fit(int Cs, int Cb, int W);
 // conv_out: a NHWC bf16 (Cin = 64..), w (Cout<=4,Cin,3,3) -> out NCHW fp32
 void conv_out_fwd(const bf16* a, int lda, const float* w, const float* b, int B, int Cin, int Cout, int H, int W,
                   float* out, cudaStream_t st);
-// da NHWC bf16 = conv_transpose(dout NCHW fp32, w)
+// da NHWC bf16 = conv_transpose(dout NCHW fp32, w).  Cout = 6 (learned-variance head): dout holds the gradients of
+// output channels 0-2 and dout2 those of 3-5, both (B,3,H,W) -- the row kernels only; dout2 is null otherwise
 void conv_out_dgrad(const float* dout, const float* w, int B, int Cin, int Cout, int H, int W, bf16* da, int ldda,
-                    cudaStream_t st);
+                    cudaStream_t st, const float* dout2 = nullptr);
+// dw, db (accumulated); dout2 as conv_out_dgrad
 void conv_out_wgrad(const bf16* a, int lda, const float* dout, int B, int Cin, int Cout, int H, int W, float* dw,
-                    float* db, float* scratch, size_t scratch_floats, cudaStream_t st);
+                    float* db, float* scratch, size_t scratch_floats, cudaStream_t st, const float* dout2 = nullptr);
+// true when the 6-output row kernel of the learned-variance head (conv_out_fwd_hybrid) takes Cin channels at width W
+bool conv_out_rows_fit6(int Cin, int W);
+// opt the 6-output row kernel into the dynamic shared memory conv_out_rows_fit6 allows, on the current device; on
+// failure msg says why (a learned-variance trainer is not created then)
+cudaError_t conv_out_rows_prepare6(char* msg, size_t msg_len);
 
 // ---- loss (replaces mse_forward/backward, train_unet.cu:2981-3030): loss += mean((out-y)^2); dout = 2(out-y)/N
 void conv_out_fwd_mse(const bf16* a, int lda, const float* w, const float* b, int B, int Cin, int Cout, int H, int W,
                       float* out, const float* target, float* loss, float* dout, float grad_scale, cudaStream_t st);
 void mse_fwd_bwd(const float* out, const float* y, size_t N, float* loss, float* dout, float grad_scale,
                  cudaStream_t st);
+// Learned-variance head (guided-diffusion's learn_sigma with the hybrid loss): what the epilogue of the 6-output conv
+// reads beside the noise, and where it writes dL/dv.  coef holds 8 floats per timestep t < T, built in float64 and
+// rounded: {sqrt(1/acp), sqrt(1/acp - 1), c1, c2, log beta, lpost, T/1000, 0}, c1 / c2 the posterior-mean coefficients
+// of x0 / x_t and lpost the clipped log posterior variance.  x0 is the batch before random_flip (flips may be null).
+struct HybridLoss {
+    const float* xt;
+    const float* x0;
+    const float* t;  // (B) timesteps as floats
+    const int* flips;
+    const float* coef;
+    float* dv;  // (B,3,H,W)
+    int T;
+};
+// out (B,6,H,W) = conv3x3(a, w (6,Cin,3,3)) + b = [eps | v]; with noise: loss2[0] += mean (eps - noise)^2,
+// loss2[1] += mean vb (bits, times T/1000); deps, hl.dv (B,3,H,W) = their gradients (eps only from the MSE, v only from
+// vb) * grad_scale.  noise = null (inference): out only.  One launch; the shape must pass conv_out_rows_fit6 and
+// conv_out_rows_prepare6 must have succeeded.
+void conv_out_fwd_hybrid(const bf16* a, int lda, const float* w, const float* b, int B, int Cin, int H, int W,
+                         float* out, const float* noise, float* loss2, float* deps, const HybridLoss& hl,
+                         float grad_scale, cudaStream_t st);
 
 }  // namespace ub

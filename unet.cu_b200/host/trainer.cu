@@ -148,6 +148,12 @@ struct UbTrainer {
     // by every training step, upsampled from low_res (B,C_in,H/f,W/f; ub_trainer_set_low_res) by the inference calls
     float *cond = nullptr, *low_res = nullptr;
     bool have_low_res = false;
+    // cfg.learn_sigma: dL/dv (B,C_out,H,W) beside dL/d eps (dout), and the hybrid loss's per-timestep coefficients
+    // (HybridLoss::coef, 8 floats per timestep).  out then holds the head's (B,2*C_out,H,W) [eps | v].
+    float *dv = nullptr, *hybrid_coef = nullptr;
+    // set while predict / sample_spaced run (or capture) the forward tape: the learned-variance head then writes its
+    // output only -- no loss, no gradients -- since inference has no x0 or noise to compare with
+    bool inference = false;
     float *loss = nullptr, *sqrt_ac = nullptr, *sqrt_1mac = nullptr, *betas = nullptr;
     int* samp_state = nullptr;  // {t, iteration} of the sampling loop
     cudaGraphExec_t samp_graph = nullptr;
@@ -769,7 +775,10 @@ int Builder::build() {
     T->flips = c.random_flip ? (int*)T->arena.alloc(size_t(B) * sizeof(int) + 256) : nullptr;
     T->cond = c.super_res ? f32(size_t(B) * img) : nullptr;
     T->low_res = c.super_res ? f32(size_t(B) * img / (size_t(c.super_res) * c.super_res)) : nullptr;
-    T->out = f32(size_t(B) * c.C_out * H0 * W0), T->dout = f32(size_t(B) * c.C_out * H0 * W0);
+    const int Co_head = c.learn_sigma ? 2 * c.C_out : c.C_out;
+    T->out = f32(size_t(B) * Co_head * H0 * W0), T->dout = f32(size_t(B) * c.C_out * H0 * W0);
+    T->dv = c.learn_sigma ? f32(size_t(B) * c.C_out * H0 * W0) : nullptr;
+    T->hybrid_coef = c.learn_sigma ? f32(size_t(8) * c.n_timesteps) : nullptr;
     T->sqrt_ac = f32(c.n_timesteps), T->sqrt_1mac = f32(c.n_timesteps), T->betas = f32(c.n_timesteps);
     T->samp_state = (int*)T->arena.alloc(256);
     T->samp_z = f32(size_t(B) * img);
@@ -932,27 +941,47 @@ int Builder::build() {
             }
         }
     }
-    // ---- output head: GN + SiLU + conv3x3 (-> C_out) + MSE (dev/unet.py:286-290, train_unet.cu:4408-4418)
+    // ---- output head: GN + SiLU + conv3x3 (-> C_out) + MSE (dev/unet.py:286-290, train_unet.cu:4408-4418).  A
+    // learned-variance model's conv has 2*C_out outputs [eps | v] (UNetModel(out_channels = 6)) and its epilogue adds
+    // the hybrid loss's vb term; the backward convs take dL/d eps and dL/dv as the two 3-channel planes of the
+    // 6-channel row kernels.
     {
         Node nd;
         nd.param_begin = poff;
         View ao = act(h.C, h.H, h.W), hx = h;
         GN g = gn_fwd(h, ao, 1);
-        const size_t wo = take(size_t(c.C_out) * h.C * 9), bo = take(c.C_out);
+        const int Co = c.learn_sigma ? 2 * c.C_out : c.C_out;
+        const size_t wo = take(size_t(Co) * h.C * 9), bo = take(Co);
         float *w = P(wo), *b = P(bo), *gw = G(wo), *gb = G(bo);
-        const int Cin = h.C, Co = c.C_out, Hh = h.H, Ww = h.W;
-        const size_t N = size_t(B) * c.C_out * h.H * h.W;
-        F([=](cudaStream_t st) {
-            conv_out_fwd_mse(ao.p, ao.ld, w, b, Bn, Cin, Co, Hh, Ww, Tt->out, Tt->noise, Tt->loss, Tt->dout, 1.f, st);
-        }, 1);
+        const int Cin = h.C, Hh = h.H, Ww = h.W;
+        const bool ls = c.learn_sigma != 0;
+        // (the head's FLOPs are counted only for the learned-variance head, so that the default profile is unchanged)
+        const double hflops = ls ? 2.0 * B * Hh * Ww * Cin * 9 * Co : 0, hbytes = ls ? act_bytes(Cin, Hh, Ww) : 0;
+        label(ls ? "output conv + hybrid loss %d->%d" : "output conv + mse %d->%d", Cin, Co);
+        if (ls) {
+            F([=](cudaStream_t st) {
+                HybridLoss hl{Tt->xt, Tt->x0, Tt->tsteps, Tt->flips, Tt->hybrid_coef, Tt->dv, Tt->cfg.n_timesteps};
+                conv_out_fwd_hybrid(ao.p, ao.ld, w, b, Bn, Cin, Hh, Ww, Tt->out, Tt->inference ? nullptr : Tt->noise,
+                                    Tt->loss, Tt->dout, hl, 1.f, st);
+            }, 1, UB_KIND_SMALL, hflops, hbytes + 4.0 * B * Hh * Ww * (Co + 5 * 3));  // (+ noise, x_t, x0, dL/d eps, dL/dv)
+        } else {
+            F([=](cudaStream_t st) {
+                conv_out_fwd_mse(ao.p, ao.ld, w, b, Bn, Cin, Co, Hh, Ww, Tt->out, Tt->noise, Tt->loss, Tt->dout, 1.f, st);
+            }, 1);
+        }
         nd.out = View{};
         nd.bwd = [=](View) -> View {
             View dao = act(Cin, Hh, Ww), dh = act(Cin, Hh, Ww);
+            const float* dv = ls ? Tt->dv : nullptr;
+            label("output conv wgrad %d->%d", Cin, Co);
             Bk([=](cudaStream_t st) {
                 conv_out_wgrad(ao.p, ao.ld, Tt->dout, Bn, Cin, Co, Hh, Ww, gw, gb, Tt->small_scratch,
-                               Tt->small_scratch_floats, st);
-            }, 2, UB_KIND_SMALL, 0, 0, 1);  // (row kernel + bias sum; three on the fallback path)
-            Bk([=](cudaStream_t st) { conv_out_dgrad(Tt->dout, w, Bn, Cin, Co, Hh, Ww, dao.p, dao.ld, st); }, 1);
+                               Tt->small_scratch_floats, st, dv);
+            }, ls ? 3 : 2, UB_KIND_SMALL, hflops, ls ? hbytes + 4.0 * B * Hh * Ww * Co : 0, 1);
+            // (row kernel + bias sum -- one per plane with learn_sigma; three on the 3-channel fallback path)
+            label("output conv dgrad %d->%d", Cin, Co);
+            Bk([=](cudaStream_t st) { conv_out_dgrad(Tt->dout, w, Bn, Cin, Co, Hh, Ww, dao.p, dao.ld, st, dv); }, 1,
+               UB_KIND_SMALL, hflops, ls ? hbytes + 4.0 * B * Hh * Ww * Co : 0);
             gn_bwd(g, hx, dao, 1, View{}, dh, nullptr);
             return dh;
         };
@@ -1093,6 +1122,15 @@ extern "C" void ub_default_config(UbConfig* cfg) {
     cfg->n_timesteps = 1000, cfg->seed = 0x5eedULL, cfg->use_cuda_graph = 1;
 }
 
+// guided-diffusion's get_named_beta_schedule("linear", T) in float64: numpy.linspace(scale 1e-4, scale 0.02, T), scale =
+// 1000 / T, the last point exactly the stop value
+static std::vector<double> linear_betas(int T) {
+    std::vector<double> b(T);
+    const double scale = 1000.0 / T, b0 = scale * 0.0001, b1 = scale * 0.02, step = T > 1 ? (b1 - b0) / (T - 1) : 0.0;
+    for (int i = 0; i < T; ++i) b[i] = (T > 1 && i == T - 1) ? b1 : b0 + double(i) * step;
+    return b;
+}
+
 static int validate_config(const UbConfig& c) {
     if (c.B < 1 || c.C_in < 1 || c.C_in > 4 || c.C_out < 1 || c.C_out > 4 || c.n_levels < 1 || c.n_levels > 8) {
         set_err("bad config: B/C_in/C_out/n_levels out of range");
@@ -1132,6 +1170,31 @@ static int validate_config(const UbConfig& c) {
             !smallc_rows_fit(2 * c.C_in, Cb, c.W)) {
             set_err("super_res = %d needs a factor >= 2 that divides H and W, C_in == C_out == 3, W %% 4 == 0, W <= 256 "
                     "and an input conv the 6-channel row kernels take (%d channels at W = %d)", f, Cb, c.W);
+            return UB_ERR_SHAPE;
+        }
+    }
+    if (c.learn_sigma != 0 && c.learn_sigma != 1) {
+        set_err("bad config: learn_sigma must be 0 or 1");
+        return UB_ERR_SHAPE;
+    }
+    if (c.learn_sigma) {
+        const int Cb = c.channel_mult[0] * c.C_model;  // (the output head's input width)
+        if (c.C_out != 3) {
+            set_err("learn_sigma needs C_out == 3 (the 6-output head's kernels take two 3-channel planes)");
+            return UB_ERR_SHAPE;
+        }
+        if (c.compute_dinput) {
+            set_err("learn_sigma does not support compute_dinput (the vb term depends on x_t directly, so dL/dx_t is "
+                    "ambiguous)");
+            return UB_ERR_SHAPE;
+        }
+        if (c.n_timesteps < 2) {
+            set_err("learn_sigma needs n_timesteps >= 2 (the clipped posterior log-variance of t = 0 is that of t = 1)");
+            return UB_ERR_SHAPE;
+        }
+        if (c.W % 8 || !smallc_rows_fit(2 * c.C_out, Cb, c.W) || !conv_out_rows_fit6(Cb, c.W)) {
+            set_err("learn_sigma needs W %% 8 == 0 and an output head the 6-channel row kernels take (%d channels at "
+                    "W = %d)", Cb, c.W);
             return UB_ERR_SHAPE;
         }
     }
@@ -1183,6 +1246,14 @@ extern "C" int ub_trainer_create(UbTrainer** out, const UbConfig* cfg, int devic
     nhwc_ops_init();
     attn_init();
     attn_tc_init();
+    if (cfg->learn_sigma) {
+        char msg[256];
+        if (conv_out_rows_prepare6(msg, sizeof msg) != cudaSuccess) {
+            cudaGetLastError();  // (leave no pending error behind)
+            set_err("%s", msg);
+            return UB_ERR_CUDA;
+        }
+    }
     UbTrainer* t = new UbTrainer();
     t->cfg = *cfg;
     t->device = device;
@@ -1265,6 +1336,23 @@ extern "C" int ub_trainer_create(UbTrainer** out, const UbConfig* cfg, int devic
         cudaMemcpy(t->betas, bt.data(), n * sizeof(float), cudaMemcpyHostToDevice);
         cudaMemcpy(t->sqrt_ac, sa.data(), n * sizeof(float), cudaMemcpyHostToDevice);
         cudaMemcpy(t->sqrt_1mac, sb.data(), n * sizeof(float), cudaMemcpyHostToDevice);
+    }
+    if (cfg->learn_sigma) {  // the hybrid loss's tables (guided-diffusion's GaussianDiffusion, float64), rounded once
+        const int n = cfg->n_timesteps;
+        const std::vector<double> beta = linear_betas(n);
+        std::vector<double> acp(n), pv(n);
+        for (int i = 0; i < n; ++i) acp[i] = (i ? acp[i - 1] : 1.0) * (1.0 - beta[i]);
+        for (int i = 0; i < n; ++i) pv[i] = beta[i] * (1.0 - (i ? acp[i - 1] : 1.0)) / (1.0 - acp[i]);
+        std::vector<float> k(size_t(8) * n);
+        for (int i = 0; i < n; ++i) {
+            const double ap = i ? acp[i - 1] : 1.0;
+            const double lpost = log(i == 0 ? pv[1] : pv[i]);  // posterior_log_variance_clipped (n >= 2)
+            const double row[8] = {sqrt(1.0 / acp[i]), sqrt(1.0 / acp[i] - 1.0), beta[i] * sqrt(ap) / (1.0 - acp[i]),
+                                   (1.0 - ap) * sqrt(1.0 - beta[i]) / (1.0 - acp[i]), log(beta[i]), lpost, n / 1000.0,
+                                   0.0};
+            for (int j = 0; j < 8; ++j) k[size_t(8) * i + j] = float(row[j]);
+        }
+        cudaMemcpy(t->hybrid_coef, k.data(), k.size() * sizeof(float), cudaMemcpyHostToDevice);
     }
     const size_t img = size_t(cfg->B) * cfg->C_in * cfg->H * cfg->W;
     for (int k = 0; k < 2; ++k) {
@@ -1493,10 +1581,16 @@ extern "C" int ub_trainer_set_next_batch(UbTrainer* t, const float* next_x0_host
     return UB_OK;
 }
 
-static int fetch_loss(UbTrainer* t, float* loss_out) {
-    CUDA_TRY(cudaMemcpyAsync(t->h_loss, t->loss, sizeof(float), cudaMemcpyDeviceToHost, t->stream));
+// loss[0] = mse, loss[1] = vb (cfg.learn_sigma; zero otherwise: the loss buffer is cleared at every step)
+static int fetch_loss(UbTrainer* t, float* loss_out, float* vb_out = nullptr) {
+    const int nl = t->cfg.learn_sigma ? 2 : 1;
+    CUDA_TRY(cudaMemcpyAsync(t->h_loss, t->loss, nl * sizeof(float), cudaMemcpyDeviceToHost, t->stream));
     CUDA_TRY(cudaStreamSynchronize(t->stream));
-    *loss_out = *t->h_loss;
+    if (!vb_out) {
+        *loss_out = nl == 2 ? t->h_loss[0] + t->h_loss[1] : t->h_loss[0];
+        return UB_OK;
+    }
+    *loss_out = t->h_loss[0], *vb_out = nl == 2 ? t->h_loss[1] : 0.f;
     return UB_OK;
 }
 
@@ -1749,6 +1843,14 @@ extern "C" int ub_trainer_last_loss(UbTrainer* t, float* loss_out) {
     CUDA_TRY(cudaSetDevice(t->device));
     return fetch_loss(t, loss_out);
 }
+extern "C" int ub_trainer_last_loss_terms(UbTrainer* t, float* mse, float* vb) {
+    CUDA_TRY(cudaSetDevice(t->device));
+    float m = 0.f, v = 0.f;
+    if (int r = fetch_loss(t, &m, &v)) return r;
+    if (mse) *mse = m;
+    if (vb) *vb = v;
+    return UB_OK;
+}
 extern "C" void* ub_trainer_stream(UbTrainer* t) { return (void*)t->stream; }
 extern "C" int ub_trainer_launches_per_step(UbTrainer* t) {
     // tapes + memset-free extras: diffusion (2), adamw, pack, step increment (+ the super-res condition)
@@ -1773,13 +1875,16 @@ extern "C" int ub_trainer_predict(UbTrainer* t, const float* xt_host, const floa
     CUDA_TRY(cudaSetDevice(t->device));
     const UbConfig& c = t->cfg;
     if (int r = prepare_inference_cond(t)) return r;
-    const size_t img = size_t(c.B) * c.C_in * c.H * c.W, oimg = size_t(c.B) * c.C_out * c.H * c.W;
+    const size_t img = size_t(c.B) * c.C_in * c.H * c.W,
+                 oimg = size_t(c.B) * (c.learn_sigma ? 2 : 1) * c.C_out * c.H * c.W;
     CUDA_TRY(cudaMemcpyAsync(t->xt, xt_host, img * sizeof(float), cudaMemcpyHostToDevice, t->stream));
     CUDA_TRY(cudaMemcpyAsync(t->tsteps, t_host, c.B * sizeof(float), cudaMemcpyHostToDevice, t->stream));
     CUDA_TRY(cudaMemsetAsync(t->zero_base, 0, t->zero_bytes, t->stream));
     CUDA_TRY(cudaMemsetAsync(t->noise, 0, img * sizeof(float), t->stream));
     if (t->drop_ctl) dropout_set_ctl(t->drop_ctl, 0.f, c.seed, t->step_dev, t->stream);  // inference: no dropout
+    t->inference = true;
     for (auto& op : t->fwd_ops) op(t->stream);
+    t->inference = false;
     CUDA_TRY(cudaMemcpyAsync(out_host, t->out, oimg * sizeof(float), cudaMemcpyDeviceToHost, t->stream));
     CUDA_TRY(cudaStreamSynchronize(t->stream));
     return UB_OK;
@@ -1793,6 +1898,11 @@ extern "C" int ub_trainer_sample(UbTrainer* t, const float* x_init_host, int t_s
     if (c.C_in != c.C_out) {
         set_err("sampling needs C_in == C_out");
         return UB_ERR_SHAPE;
+    }
+    if (c.learn_sigma) {
+        set_err("ub_trainer_sample has no learned variance: sample a learn_sigma model with ub_trainer_sample_spaced "
+                "(UB_SAMPLER_ANCESTRAL, every timestep kept)");
+        return UB_ERR_STATE;
     }
     if (t_start < 0) t_start = c.n_timesteps - 1;
     if (t_end < 0) t_end = 2;
@@ -1927,14 +2037,12 @@ extern "C" int ub_space_timesteps(int n_timesteps, const char* spec, int* out, i
 // Coefficient rows of ub_trainer_sample_spaced in loop order (row k = spaced index n-1-k), from guided-diffusion's
 // SpacedDiffusion + GaussianDiffusion tables in float64: the linear betas of the trainer's schedule, acp = cumprod(1 -
 // beta), then beta'_i = 1 - acp[t_i] / acp[t_{i-1}] over the kept timesteps and the tables of that respaced chain.
-static void spaced_rows(int T, const int* ts, int n, int sampler, double eta, int clip, SpacedRow* rows) {
+static void spaced_rows(int T, const int* ts, int n, int sampler, double eta, int clip, bool learned,
+                        SpacedRow* rows) {
     std::vector<double> acp(T);
-    const double scale = 1000.0 / T, b0 = scale * 0.0001, b1 = scale * 0.02, step = T > 1 ? (b1 - b0) / (T - 1) : 0.0;
+    const std::vector<double> betas = linear_betas(T);
     double ac = 1.0;
-    for (int i = 0; i < T; ++i) {  // numpy.linspace: start + i * step, the last point exactly `stop`
-        const double beta = (T > 1 && i == T - 1) ? b1 : b0 + double(i) * step;
-        acp[i] = ac = ac * (1.0 - beta);
-    }
+    for (int i = 0; i < T; ++i) acp[i] = ac = ac * (1.0 - betas[i]);
     std::vector<double> bp(n), ap(n);  // beta', acp' of the respaced chain
     double last = 1.0, cum = 1.0;
     for (int i = 0; i < n; ++i) {
@@ -1956,8 +2064,16 @@ static void spaced_rows(int T, const int* ts, int n, int sampler, double eta, in
             c_x = k * r / rm1;
             if (!i) sigma = 0.0;
         }
+        float pad[2] = {0.f, 0.f};
+        if (learned && sampler == UB_SAMPLER_ANCESTRAL) {
+            // learned range: sigma becomes the [i > 0] draw flag; log beta'_i and the clipped log posterior variance
+            // of the respaced chain (entry 0 takes entry 1's) go to the kernel, which mixes them per element
+            auto post_var = [&](int j) { return bp[j] * (1.0 - ap[j - 1]) / (1.0 - ap[j]); };
+            pad[0] = float(log(bp[i])), pad[1] = float(log(post_var(i ? i : 1)));
+            sigma = i ? 1.0 : 0.0;
+        }
         SpacedRow& w = rows[n - 1 - i];
-        w = SpacedRow{float(r), float(rm1), float(c_x0), float(c_x), float(sigma), clip ? 1.f : 0.f, {0.f, 0.f}};
+        w = SpacedRow{float(r), float(rm1), float(c_x0), float(c_x), float(sigma), clip ? 1.f : 0.f, {pad[0], pad[1]}};
     }
 }
 
@@ -1991,7 +2107,7 @@ extern "C" int ub_trainer_sample_spaced(UbTrainer* t, const int* timesteps, int 
         }
     if (int r = prepare_inference_cond(t)) return r;
     std::vector<SpacedRow> rows(n);
-    spaced_rows(c.n_timesteps, timesteps, n, sampler, double(eta), clip_denoised, rows.data());
+    spaced_rows(c.n_timesteps, timesteps, n, sampler, double(eta), clip_denoised, c.learn_sigma != 0, rows.data());
     std::vector<int> ts(timesteps, timesteps + n);
     std::reverse(ts.begin(), ts.end());
     const size_t img = size_t(c.B) * c.C_in * c.H * c.W;
@@ -2014,8 +2130,11 @@ extern "C" int ub_trainer_sample_spaced(UbTrainer* t, const int* timesteps, int 
         cudaMemsetAsync(t->zero_base, 0, t->zero_bytes, st);
         spaced_set_t(t->spaced_ts, t->spaced_state, c.B, t->tsteps, st);
         if (t->drop_ctl) dropout_set_ctl(t->drop_ctl, 0.f, c.seed, t->step_dev, st);  // inference: no dropout
+        t->inference = true;  // (read while the tape is captured: the graph keeps the loss-free head)
         for (auto& op : t->fwd_ops) op(st);
-        spaced_step(t->xt, t->out, t->spaced_rows, inject ? t->samp_z : nullptr, img, t->spaced_state, st);
+        t->inference = false;
+        spaced_step(t->xt, t->out, t->spaced_rows, inject ? t->samp_z : nullptr, img, t->spaced_state, st,
+                    c.learn_sigma ? img / c.B : 0);
         cudaError_t e = cudaStreamEndCapture(st, &graph);
         if (e != cudaSuccess || !graph) {
             set_err("sampling graph capture failed: %s", cudaGetErrorString(e));
@@ -2173,7 +2292,7 @@ extern "C" int ub_trainer_get_grads(UbTrainer* t, float* host, size_t n) {
 }
 extern "C" int ub_trainer_get_output(UbTrainer* t, float* host, size_t n) {
     const UbConfig& c = t->cfg;
-    return copy_out(t, t->out, host, n, size_t(c.B) * c.C_out * c.H * c.W);
+    return copy_out(t, t->out, host, n, size_t(c.B) * (c.learn_sigma ? 2 : 1) * c.C_out * c.H * c.W);
 }
 extern "C" int ub_trainer_get_batch(UbTrainer* t, float* host, size_t n) {
     const UbConfig& c = t->cfg;
@@ -2238,7 +2357,8 @@ extern "C" int ub_trainer_load(UbTrainer* t, const char* path) {
     }
     const UbConfig& c = t->cfg;
     const int model_in = c.super_res ? 2 * c.C_in : c.C_in;  // (the first conv's input channels, as the file states)
-    if (header[2] != model_in || header[3] != c.C_model || header[4] != c.C_out || header[5] != c.H ||
+    const int model_out = c.learn_sigma ? 2 * c.C_out : c.C_out;  // (the output conv's channels, as the file states)
+    if (header[2] != model_in || header[3] != c.C_model || header[4] != model_out || header[5] != c.H ||
         header[6] != c.W) {
         fclose(f);
         set_err("%s: checkpoint shape (C_in %d, C_model %d, C_out %d, %dx%d) does not match the trainer", path,
@@ -2303,7 +2423,7 @@ static int save_checkpoint(UbTrainer* t, const char* path, const float* weights,
     int header[256];
     memset(header, 0, sizeof header);
     header[0] = kModelMagic, header[1] = c.B, header[2] = c.super_res ? 2 * c.C_in : c.C_in, header[3] = c.C_model;
-    header[4] = c.C_out;
+    header[4] = c.learn_sigma ? 2 * c.C_out : c.C_out;
     header[5] = c.H, header[6] = c.W, header[7] = c.max_period, header[8] = with_adamw ? 1 : 0, header[9] = 0;
     int step = 0;
     cudaMemcpy(&step, t->step_dev, sizeof(int), cudaMemcpyDeviceToHost);
