@@ -32,7 +32,7 @@ class UbConfig(C.Structure):
                 ("use_cuda_graph", C.c_int), ("compute_dinput", C.c_int), ("random_flip", C.c_int),
                 ("num_classes", C.c_int), ("ema_rate", C.c_float), ("resblock_updown", C.c_int),
                 ("use_scale_shift_norm", C.c_int), ("dropout", C.c_float), ("super_res", C.c_int),
-                ("learn_sigma", C.c_int)]
+                ("learn_sigma", C.c_int), ("noise_schedule", C.c_int)]
 
 
 UB_KINDS = ("conv_igemm", "wgrad_igemm", "groupnorm", "attention", "eltwise", "small", "optimizer")
@@ -104,6 +104,7 @@ def _declare(L: C.CDLL) -> None:
     L.ub_trainer_profile.argtypes = [vp, i, C.POINTER(UbProfile)]
     L.ub_trainer_sample.argtypes = [vp, fp, i, i, fp, C.c_ulonglong, fp]
     L.ub_space_timesteps.argtypes = [i, C.c_char_p, vp, i]
+    L.ub_beta_schedule.argtypes = [i, i, vp]
     L.ub_trainer_sample_spaced.argtypes = [vp, vp, i, i, C.c_float, i, fp, fp, C.c_ulonglong, fp]
     L.ub_dataloader_open.argtypes = [C.POINTER(vp), C.c_char_p, i, i, i]
     L.ub_dataloader_info.argtypes = [vp, C.POINTER(i), C.POINTER(i), C.POINTER(i), C.POINTER(i),
@@ -148,6 +149,20 @@ def space_timesteps(n_timesteps: int, spec: str) -> list[int]:
     if n < 0:
         check(n, "space_timesteps")
     return [int(v) for v in out[:n]]
+
+
+UB_SCHEDULE_LINEAR, UB_SCHEDULE_COSINE = 0, 1
+UB_SCHEDULES = {"linear": UB_SCHEDULE_LINEAR, "cosine": UB_SCHEDULE_COSINE}
+
+
+def beta_schedule(schedule, n_timesteps: int) -> np.ndarray:
+    """guided-diffusion's get_named_beta_schedule: the float64 betas the trainer builds its tables from, for a
+    UbConfig.noise_schedule value or its name ("linear", "cosine"); raises UbError for an unknown schedule or
+    n_timesteps < 1.  Needs no GPU."""
+    code = UB_SCHEDULES.get(schedule, -1) if isinstance(schedule, str) else int(schedule)
+    out = np.empty(max(int(n_timesteps), 1), dtype=np.float64)
+    check(lib().ub_beta_schedule(code, int(n_timesteps), out.ctypes.data_as(C.c_void_p)), "beta_schedule")
+    return out
 
 
 UB_SAMPLERS = {"ddim": 0, "ancestral": 1}
