@@ -277,6 +277,14 @@ typedef struct {
                             UB_SCHEDULE_LINEAR, the reference's (train_unet.cu:3131-3147), or UB_SCHEDULE_COSINE,
                             guided-diffusion's `--noise_schedule cosine` (ub_trainer_sample refuses such a model).  Like
                             head_size, not stored in the checkpoint header; 0 = linear */
+    float class_dropout; /* p in [0, 1), needs num_classes = K > 0: classifier-free guidance training (Ho & Salimans
+                            2022, GLIDE's p_uncond).  The label table gets a (K + 1)-th row, the null class K -- the
+                            parameter layout is exactly that of a (K + 1)-class model -- and every training step replaces
+                            each image's label with the null class with probability p: one Philox coin per (seed, step,
+                            image), stream id 0xB.  ub_trainer_set_labels then accepts -1 (the null class), and
+                            ub_trainer_set_guidance sets the guidance scale of ub_trainer_sample_spaced.  Like head_size,
+                            not stored in the checkpoint header: a trainer that only samples a guided model is created
+                            with any p > 0; 0 */
 } UbConfig;
 
 #define UB_SCHEDULE_LINEAR 0 /* numpy.linspace(s * 1e-4, s * 0.02, n_timesteps), s = 1000 / n_timesteps */
@@ -293,7 +301,8 @@ int ub_beta_schedule(int schedule, int n_timesteps, double* betas_out);
 
 void ub_default_config(UbConfig* cfg);
 /* number of parameters for a config (326 tensors / 20 494 211 floats for the default; 0 for a config that is refused).
- * learn_sigma adds C * 9 * C_out + C_out, the v rows of the output conv (C its input width) */
+ * learn_sigma adds C * 9 * C_out + C_out, the v rows of the output conv (C its input width); class_dropout > 0 adds one
+ * label row of 4 * C_model (ub_num_params({K, p > 0}) == ub_num_params({K + 1, 0})) */
 size_t ub_num_params(const UbConfig* cfg);
 
 int ub_trainer_create(UbTrainer** out, const UbConfig* cfg, int device);
@@ -328,8 +337,19 @@ int ub_trainer_get_ema(UbTrainer* t, float* host, size_t n);
 int ub_trainer_set_ema(UbTrainer* t, const float* host, size_t n);
 int ub_trainer_save_ema(UbTrainer* t, const char* path); /* parameters-only .bin of the averaged weights */
 /* class labels y (B ints in [0, num_classes)) of the batch(es) that follow (cfg.num_classes > 0, dev/unet.py:301-303);
- * used by forward_backward / train_step / predict / sample until set again */
+ * used by forward_backward / train_step / predict / sample until set again.  With cfg.class_dropout > 0, -1 is accepted
+ * too and means the null class: an explicitly unlabelled image in training, unconditional output in inference. */
 int ub_trainer_set_labels(UbTrainer* t, const int* labels_host, size_t n);
+/* cfg.class_dropout > 0: the B labels the last training step used, with -1 where it dropped the label (or the caller
+ * passed -1) -- for parity checks, like ub_trainer_get_flips.  UB_ERR_STATE on a trainer without class_dropout. */
+int ub_trainer_get_effective_labels(UbTrainer* t, int* host, size_t n);
+/* cfg.class_dropout > 0: classifier-free guidance scale s of ub_trainer_sample_spaced until set again, in GLIDE's
+ * convention (guidance_scale): eps = eps_u + s (eps_c - eps_u), eps_c the output for the labels of
+ * ub_trainer_set_labels, eps_u the output for the null class; s = 1 is plain conditional sampling (the default),
+ * s = 0 unconditional, Ho & Salimans' w = s - 1.  For s != 1 every iteration runs the model twice; a learned-variance
+ * model takes v from the conditional pass.  ub_trainer_sample refuses to run while s != 1; ub_trainer_predict stays
+ * unguided.  UB_ERR_STATE on a trainer without class_dropout, UB_ERR_SHAPE for a negative or non-finite s. */
+int ub_trainer_set_guidance(UbTrainer* t, float scale);
 /* the dropout mask (0 / 1 bytes, B x H x W x C in NHWC order) the LAST training step applied in ResBlock `block`
  * (forward order), regenerated from its Philox key -- for parity checks (cfg.dropout > 0) */
 int ub_trainer_get_dropout_mask(UbTrainer* t, int block, unsigned char* host, size_t n);
@@ -397,7 +417,8 @@ int ub_trainer_predict(UbTrainer* t, const float* xt_host, const float* t_host, 
  * runs inject the oracle's draws).  out_host (B,C_in,H,W) receives the final x.  One CUDA graph per iteration.
  * A learned-variance model (cfg.learn_sigma) or a cosine-schedule model (cfg.noise_schedule) gets UB_ERR_STATE:
  * generate.py's loop has no learned variance and only the linear schedule; use ub_trainer_sample_spaced with
- * UB_SAMPLER_ANCESTRAL and every timestep kept instead. */
+ * UB_SAMPLER_ANCESTRAL and every timestep kept instead.  So does a guided model while its guidance scale is not 1
+ * (ub_trainer_set_guidance): guidance runs in ub_trainer_sample_spaced only. */
 int ub_trainer_sample(UbTrainer* t, const float* x_init_host, int t_start, int t_end, const float* noise_host,
                       unsigned long long seed, float* out_host);
 
@@ -437,7 +458,9 @@ int ub_space_timesteps(int n_timesteps, const char* spec, int* out, int cap);
  * timestep first.  out_host receives the final x.  Labels of ub_trainer_set_labels apply; parameters, moving average,
  * AdamW moments and step count are left untouched.  UB_ERR_SHAPE for a bad timestep list, sampler, eta or n, or
  * C_in != C_out.  One CUDA graph per iteration, captured on the first call (again when noise_host switches between
- * NULL and non-NULL). */
+ * NULL and non-NULL).  With a guidance scale s != 1 (ub_trainer_set_guidance) eps is the guided
+ * eps_u + s (eps_c - eps_u) of two forward passes, and a second graph of its own (captured likewise) runs them; the
+ * scale lives in device memory, so changing it does not capture again. */
 int ub_trainer_sample_spaced(UbTrainer* t, const int* timesteps, int n, int sampler, float eta, int clip_denoised,
                              const float* x_init_host, const float* noise_host, unsigned long long seed,
                              float* out_host);

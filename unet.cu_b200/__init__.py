@@ -32,7 +32,7 @@ class UbConfig(C.Structure):
                 ("use_cuda_graph", C.c_int), ("compute_dinput", C.c_int), ("random_flip", C.c_int),
                 ("num_classes", C.c_int), ("ema_rate", C.c_float), ("resblock_updown", C.c_int),
                 ("use_scale_shift_norm", C.c_int), ("dropout", C.c_float), ("super_res", C.c_int),
-                ("learn_sigma", C.c_int), ("noise_schedule", C.c_int)]
+                ("learn_sigma", C.c_int), ("noise_schedule", C.c_int), ("class_dropout", C.c_float)]
 
 
 UB_KINDS = ("conv_igemm", "wgrad_igemm", "groupnorm", "attention", "eltwise", "small", "optimizer")
@@ -94,6 +94,8 @@ def _declare(L: C.CDLL) -> None:
     L.ub_trainer_last_loss_terms.argtypes = [vp, C.POINTER(C.c_float), C.POINTER(C.c_float)]
     L.ub_trainer_set_step.argtypes = [vp, i]
     L.ub_trainer_get_flips.argtypes = [vp, vp, C.c_size_t]
+    L.ub_trainer_get_effective_labels.argtypes = [vp, vp, C.c_size_t]
+    L.ub_trainer_set_guidance.argtypes = [vp, C.c_float]
     L.ub_set_layer_precision.argtypes = [i]
     L.ub_groupnorm_nhwc_forward.argtypes = [vp, vp, vp, vp, vp, i, i, i, i, i, i, i]
     L.ub_groupnorm_nhwc_backward.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i, i, i, i, i, i, i]
@@ -223,9 +225,23 @@ class Trainer:
         check(lib().ub_trainer_save_ema(self._h, path.encode()), "ub_trainer_save_ema")
 
     def set_labels(self, y):
-        """Class labels of the batches that follow (cfg.num_classes > 0; `y` of UNetModel.forward, dev/unet.py:301-303)."""
+        """Class labels of the batches that follow (cfg.num_classes > 0; `y` of UNetModel.forward, dev/unet.py:301-303);
+        with cfg.class_dropout > 0, -1 stands for the null class."""
         y = np.ascontiguousarray(y, dtype=np.int32).reshape(-1)
         check(lib().ub_trainer_set_labels(self._h, y.ctypes.data_as(C.c_void_p), y.size), "set_labels")
+
+    def get_effective_labels(self) -> np.ndarray:
+        """The labels the last training step of a classifier-free guidance model (cfg.class_dropout > 0) used, with -1
+        where it dropped the label or the caller passed -1."""
+        out = np.empty(self.cfg.B, dtype=np.int32)
+        check(lib().ub_trainer_get_effective_labels(self._h, out.ctypes.data_as(C.c_void_p), out.size),
+              "get_effective_labels")
+        return out
+
+    def set_guidance(self, scale: float):
+        """Classifier-free guidance scale of sample_spaced (GLIDE's guidance_scale: 1 = conditional, the default; 0 =
+        unconditional; Ho & Salimans' w = scale - 1); needs cfg.class_dropout > 0."""
+        check(lib().ub_trainer_set_guidance(self._h, float(scale)), "set_guidance")
 
     def get_dropout_mask(self, block: int, C_: int, H: int, W: int) -> np.ndarray:
         """Keep-mask (B, C, H, W) of 0 / 1 the last training step applied in ResBlock `block` (cfg.dropout > 0)."""

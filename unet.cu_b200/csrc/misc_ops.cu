@@ -671,6 +671,27 @@ void diffusion_prepare(const float* x0, const float* sqrt_ac, const float* sqrt_
                                                                              seed, step_dev, gen_noise, t, noise, x_t, W, flips);
 }
 
+// classifier-free guidance labels (see misc_ops.cuh); one thread per image
+__global__ void cfg_labels_kernel(const int* __restrict__ labels, int* __restrict__ eff, int B, int K, int mode,
+                                  float p, uint64_t seed, const int* __restrict__ step_dev) {
+    pdl_entry();
+    const int b = blockIdx.x * blockDim.x + threadIdx.x;
+    if (b >= B) return;
+    int y = mode == CFG_LABELS_NULL ? K : labels[b];
+    if (y < 0) y = K;
+    if (mode == CFG_LABELS_TRAIN) {
+        const uint4 r = philox4x32_10(make_uint4(uint32_t(b), 0u, 0xBu, uint32_t(*step_dev)),
+                                      make_uint2(uint32_t(seed), uint32_t(seed >> 32)));
+        if (u01(r.x) < p) y = K;
+        eff[B + b] = y;
+    }
+    eff[b] = y;
+}
+void cfg_labels(const int* labels, int* eff, int B, int K, int mode, float p, uint64_t seed, const int* step_dev,
+                cudaStream_t st) {
+    launch_pdl(cfg_labels_kernel, dim3((B + 127) / 128), dim3(128), 0, st, labels, eff, B, K, mode, p, seed, step_dev);
+}
+
 // Conditioning channels of a super-resolution model (guided-diffusion SuperResModel.forward: F.interpolate(low_res,
 // (H, W), mode="bilinear"), align_corners = False).  One block per output row of one (image, channel) plane: the two
 // low-res rows the row interpolates between are staged in shared memory, then every output pixel blends four of their
@@ -931,10 +952,13 @@ void spaced_set_t(const int* ts_table, const SpacedState* s, int B, float* tstep
 // 3 H W floats of one image of x), and sigma = c.sigma * exp(0.5 (frac log beta' + (1 - frac) lpost')) per element,
 // frac = (v + 1) / 2, with {log beta', lpost'} in c.pad: c.sigma is the [i > 0] draw flag of the learned-range
 // ancestral sampler; DDIM rows leave pad at 0, so that v drops out and sigma is DDIM's.
-template <bool LEARNED>
+// GUIDED (classifier-free guidance): eps is the null-class output eps_u, eps_c the conditional output in the same
+// layout; eps_u + s (eps_c - eps_u), s = *scale, replaces eps before x0 and the clip, and v is read from eps_c.
+template <bool LEARNED, bool GUIDED>
 __global__ void spaced_step_kernel(float* __restrict__ x, const float* __restrict__ eps,
                                    const SpacedRow* __restrict__ rows, const float* __restrict__ z, size_t n4,
-                                   const SpacedState* __restrict__ s, size_t img3) {
+                                   const SpacedState* __restrict__ s, size_t img3, const float* __restrict__ eps_c,
+                                   const float* __restrict__ scale) {
     pdl_entry();
     const size_t i4 = size_t(blockIdx.x) * blockDim.x + threadIdx.x;
     if (i4 >= n4) return;
@@ -942,17 +966,26 @@ __global__ void spaced_step_kernel(float* __restrict__ x, const float* __restric
     const SpacedRow c = rows[it];
     const float4 xv = reinterpret_cast<const float4*>(x)[i4];
     float4 ev, sv = make_float4(c.sigma, c.sigma, c.sigma, c.sigma);
+    auto guide = [&](float4 eu, size_t off) {
+        if constexpr (GUIDED) {
+            const float g = *scale;
+            const float4 ec = *reinterpret_cast<const float4*>(eps_c + off);
+            eu = make_float4(eu.x + g * (ec.x - eu.x), eu.y + g * (ec.y - eu.y), eu.z + g * (ec.z - eu.z),
+                             eu.w + g * (ec.w - eu.w));
+        }
+        return eu;
+    };
     if constexpr (LEARNED) {
         const size_t e = 4 * i4, bi = e / img3, o = bi * 2 * img3 + (e - bi * img3);  // (img3 % 4 == 0)
-        ev = *reinterpret_cast<const float4*>(eps + o);
-        const float4 vv = *reinterpret_cast<const float4*>(eps + o + img3);
+        ev = guide(*reinterpret_cast<const float4*>(eps + o), o);
+        const float4 vv = *reinterpret_cast<const float4*>((GUIDED ? eps_c : eps) + o + img3);
         auto sig = [&](float v) {
             const float frac = 0.5f * (v + 1.f);
             return c.sigma * expf(0.5f * (frac * c.pad[0] + (1.f - frac) * c.pad[1]));
         };
         sv = make_float4(sig(vv.x), sig(vv.y), sig(vv.z), sig(vv.w));
     } else {
-        ev = reinterpret_cast<const float4*>(eps)[i4];
+        ev = guide(reinterpret_cast<const float4*>(eps)[i4], 4 * i4);
     }
     float4 zv = make_float4(0.f, 0.f, 0.f, 0.f);
     if (c.sigma != 0.f) zv = z ? reinterpret_cast<const float4*>(z)[i4] : philox_normal4(i4, 0x5u, uint32_t(it), s->seed);
@@ -965,14 +998,13 @@ __global__ void spaced_step_kernel(float* __restrict__ x, const float* __restric
                                                    upd(xv.z, ev.z, zv.z, sv.z), upd(xv.w, ev.w, zv.w, sv.w));
 }
 void spaced_step(float* x, const float* eps, const SpacedRow* rows, const float* z, size_t n, SpacedState* s,
-                 cudaStream_t st, size_t img3) {
+                 cudaStream_t st, size_t img3, const float* eps_c, const float* scale) {
     const size_t n4 = n / 4;
-    if (img3)
-        launch_pdl(spaced_step_kernel<true>, dim3(unsigned((n4 + 255) / 256)), dim3(256), 0, st, x, eps, rows, z, n4,
-                   static_cast<const SpacedState*>(s), img3);
-    else
-        launch_pdl(spaced_step_kernel<false>, dim3(unsigned((n4 + 255) / 256)), dim3(256), 0, st, x, eps, rows, z, n4,
-                   static_cast<const SpacedState*>(s), img3);
+    const dim3 grid(unsigned((n4 + 255) / 256));
+    const SpacedState* sc = s;
+    auto kernel = eps_c ? (img3 ? spaced_step_kernel<true, true> : spaced_step_kernel<false, true>)
+                        : (img3 ? spaced_step_kernel<true, false> : spaced_step_kernel<false, false>);
+    launch_pdl(kernel, grid, dim3(256), 0, st, x, eps, rows, z, n4, sc, img3, eps_c, scale);
     increment_step(&s->it, st);
 }
 

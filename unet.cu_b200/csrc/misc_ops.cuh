@@ -45,6 +45,14 @@ void time_mlp_fwd(const float* t, int B, int Cm, int Cemb, int max_period, const
                   cudaStream_t st, const float* label_w = nullptr, const int* labels = nullptr);
 // class-conditional model (dev/unet.py:174-175, 301-303): gradient of the label-embedding rows, dw[y[b]] += demb[b]
 void label_emb_bwd(const float* demb, const int* labels, int B, int Cemb, float* dw, cudaStream_t st);
+// classifier-free guidance (UbConfig.class_dropout): the labels the embedding reads, eff[b] in [0, K], K = null class.
+//   CFG_LABELS_TRAIN: K where labels[b] == -1 or the Philox coin (seed, stream id 0xB, counter (b, step)) is below p,
+//                     else labels[b]; also copied to eff[B + b] (the last training step's labels)
+//   CFG_LABELS_COPY:  labels[b], with -1 mapped to K
+//   CFG_LABELS_NULL:  K
+enum { CFG_LABELS_TRAIN = 0, CFG_LABELS_COPY = 1, CFG_LABELS_NULL = 2 };
+void cfg_labels(const int* labels, int* eff, int B, int K, int mode, float p, uint64_t seed, const int* step_dev,
+                cudaStream_t st);
 void timestep_embedding(const float* t, int B, int dim, int max_period, float* out, cudaStream_t st);
 
 // ---- diffusion: t ~ U{0..T-1}, eps ~ N(0,1) (Philox4x32-10, counter = element index, key = (seed, step)),
@@ -108,8 +116,10 @@ void spaced_set_t(const int* ts_table, const SpacedState* s, int B, float* tstep
 // z: injected noise of this iteration (may be null: Philox(seed, stream id 0x5, counter = it)); no draw where sigma = 0.
 // Then it <- it + 1.  img3 > 0: learned-variance model -- eps is the (B, 6, H, W) model output [eps | v] with img3 =
 // 3 H W floats per image of x, and the row's pad holds {log beta', lpost'} of the learned-range variance (see misc_ops.cu)
+// eps_c != null: classifier-free guidance -- eps holds the null-class output, eps_c the conditional one (same layout),
+// and the step uses eps_u + s (eps_c - eps_u), s = *scale (device memory); a learned-variance model's v is eps_c's.
 void spaced_step(float* x, const float* eps, const SpacedRow* rows, const float* z, size_t n, SpacedState* s,
-                 cudaStream_t st, size_t img3 = 0);
+                 cudaStream_t st, size_t img3 = 0, const float* eps_c = nullptr, const float* scale = nullptr);
 // occupy the stream for ~us microseconds (profiling aid: lets the host queue work ahead of the device)
 void stream_delay(unsigned us, cudaStream_t st);
 

@@ -7,6 +7,7 @@
 #include <dlfcn.h>
 
 #include <cctype>
+#include <cfloat>
 #include <cmath>
 #include <cstdarg>
 #include <cstdio>
@@ -126,6 +127,15 @@ struct UbTrainer {
     // cfg.num_classes > 0: class labels of the current batch (ub_trainer_set_labels) and the label-embedding table
     int* labels = nullptr;
     size_t label_w_off = 0;
+    // cfg.class_dropout > 0 (classifier-free guidance): the labels the label embedding reads, in [0, K] with K the null
+    // class (cfg_labels): [0, B) those of the current pass, [B, 2B) those of the last training step.  The guidance scale
+    // of sample_spaced (host copy, and the device word the guided step reads), the conditional pass's head output and
+    // the guided sampler's graph.
+    int* eff_labels = nullptr;
+    float guidance = 1.f;
+    float *guidance_dev = nullptr, *eps_cond = nullptr;
+    cudaGraphExec_t cfg_graph = nullptr;
+    bool cfg_graph_noise = false;
     // cfg.dropout > 0: {p bits, step, seed} read by the GroupNorm kernels that regenerate the masks (DropArgs), and the
     // (C, H, W) of every ResBlock's dropped-out tensor (ub_trainer_get_dropout_mask)
     unsigned* drop_ctl = nullptr;
@@ -512,7 +522,9 @@ struct Builder {
         const bool cls = c.num_classes > 0;
         Bk([=](cudaStream_t st) {
             dsilu_mul(Tt->d_embact, Tt->emb, Tt->demb, size_t(Bn) * Cemb, st);
-            if (cls) label_emb_bwd(Tt->demb, Tt->labels, Bn, Cemb, Tt->grads + Tt->label_w_off, st);
+            if (cls)
+                label_emb_bwd(Tt->demb, Tt->eff_labels ? Tt->eff_labels : Tt->labels, Bn, Cemb,
+                              Tt->grads + Tt->label_w_off, st);
             small_linear_bwd(Tt->temb_table + 1, 1, Bn, Cemb, Cemb, st);
             dsilu_mul(Tt->d_h0act, Tt->h0, Tt->dh0, size_t(Bn) * Cemb, st);
             small_linear_bwd(Tt->temb_table, 1, Bn, Cemb, Cm, st);
@@ -770,6 +782,9 @@ int Builder::build() {
     T->x0 = f32(size_t(B) * img), T->xt = f32(size_t(B) * img), T->noise = f32(size_t(B) * img);
     T->tsteps = f32(B);
     T->labels = c.num_classes > 0 ? (int*)T->arena.alloc(size_t(B) * sizeof(int) + 256) : nullptr;
+    const bool cfg = c.class_dropout > 0.f;
+    T->eff_labels = cfg ? (int*)T->arena.alloc(2 * size_t(B) * sizeof(int) + 256) : nullptr;
+    T->guidance_dev = cfg ? f32(1) : nullptr;
     T->drop_ctl = c.dropout > 0.f ? (unsigned*)T->arena.alloc(256) : nullptr;
     T->dxt = c.compute_dinput ? f32(size_t(B) * img) : nullptr;
     T->flips = c.random_flip ? (int*)T->arena.alloc(size_t(B) * sizeof(int) + 256) : nullptr;
@@ -778,6 +793,7 @@ int Builder::build() {
     const int Co_head = c.learn_sigma ? 2 * c.C_out : c.C_out;
     T->out = f32(size_t(B) * Co_head * H0 * W0), T->dout = f32(size_t(B) * c.C_out * H0 * W0);
     T->dv = c.learn_sigma ? f32(size_t(B) * c.C_out * H0 * W0) : nullptr;
+    T->eps_cond = cfg ? f32(size_t(B) * Co_head * H0 * W0) : nullptr;
     T->hybrid_coef = c.learn_sigma ? f32(size_t(8) * c.n_timesteps) : nullptr;
     T->sqrt_ac = f32(c.n_timesteps), T->sqrt_1mac = f32(c.n_timesteps), T->betas = f32(c.n_timesteps);
     T->samp_state = (int*)T->arena.alloc(256);
@@ -809,8 +825,9 @@ int Builder::build() {
         T->h_temb = {e0, e1};
     }
     // class-conditional model: label_emb.weight (num_classes, 4*C_model) follows the time MLP in named_parameters()
-    // order (dev/unet.py:174-175); emb = time_embed(t) + label_emb[y] (dev/unet.py:301-303)
-    const size_t lw = c.num_classes > 0 ? take(size_t(c.num_classes) * Cemb) : 0;
+    // order (dev/unet.py:174-175); emb = time_embed(t) + label_emb[y] (dev/unet.py:301-303).  class_dropout adds the
+    // null class as row num_classes, and the embedding reads the labels cfg_labels wrote instead of the caller's.
+    const size_t lw = c.num_classes > 0 ? take(size_t(c.num_classes + (cfg ? 1 : 0)) * Cemb) : 0;
     if (real()) T->label_w_off = lw;
     {
         const int mp = c.max_period;
@@ -819,7 +836,7 @@ int Builder::build() {
             const SmallLinear &e0 = Tt->h_temb[0], &e1 = Tt->h_temb[1];
             time_mlp_fwd(Tt->tsteps, Bn, Cm, Cemb, mp, e0.w, e0.b, e1.w, e1.b, Tt->sin_emb, Tt->h0, Tt->emb, Tt->semb,
                          st, cls ? Tt->params + Tt->label_w_off : nullptr,
-                         Tt->labels);  // (semb = silu(emb) is the shared input of all embedding projections)
+                         Tt->eff_labels ? Tt->eff_labels : Tt->labels);  // (semb = silu(emb) feeds all projections)
             small_linear_fwd(Tt->emb_table, int(Tt->h_emb.size()), Bn, Tt->emb_max_oc, st, true);  // (Cout % 16 == 0)
         }, 2, UB_KIND_SMALL, 0, 0, 1);  // beside the input conv and the first GroupNorm
         fwd_side_pending = true;
@@ -1176,6 +1193,11 @@ static int validate_config(const UbConfig& c) {
         set_err("bad config: num_classes must be >= 0, ema_rate and dropout in [0, 1)");
         return UB_ERR_SHAPE;
     }
+    if (!(c.class_dropout >= 0.f && c.class_dropout < 1.f) || (c.class_dropout > 0.f && c.num_classes == 0)) {
+        set_err("bad config: class_dropout must lie in [0, 1) and needs num_classes > 0 (got %g with num_classes = %d)",
+                double(c.class_dropout), c.num_classes);
+        return UB_ERR_SHAPE;
+    }
     if (c.random_flip && c.W % 4) {
         set_err("random_flip needs W %% 4 == 0");
         return UB_ERR_SHAPE;
@@ -1393,6 +1415,7 @@ extern "C" int ub_trainer_create(UbTrainer** out, const UbConfig* cfg, int devic
         cudaEventCreateWithFlags(&t->ev_stage[k], cudaEventDisableTiming);
     }
     cudaMallocHost(&t->h_loss, 64);
+    if (t->guidance_dev) cudaMemcpy(t->guidance_dev, &t->guidance, sizeof(float), cudaMemcpyHostToDevice);
     e = cudaDeviceSynchronize();
     if (e != cudaSuccess) {
         set_err("trainer init failed: %s", cudaGetErrorString(e));
@@ -1410,6 +1433,7 @@ extern "C" void ub_trainer_destroy(UbTrainer* t) {
     if (t->graph_exec) cudaGraphExecDestroy(t->graph_exec);
     if (t->samp_graph) cudaGraphExecDestroy(t->samp_graph);
     if (t->spaced_graph) cudaGraphExecDestroy(t->spaced_graph);
+    if (t->cfg_graph) cudaGraphExecDestroy(t->cfg_graph);
     if (t->comm && nccl().ok) nccl().CommDestroy(t->comm);
     if (t->params) cudaFree(t->params);
     if (t->ema) cudaFree(t->ema);
@@ -1446,6 +1470,15 @@ struct StepOpts {
     float lr, b1, b2, eps, wd;
 };
 
+// classifier-free guidance model (cfg.class_dropout > 0): write the labels the embedding reads (CFG_LABELS_*); no-op
+// for any other model
+static void enqueue_cfg_labels(UbTrainer* t, int mode, cudaStream_t st) {
+    const UbConfig& c = t->cfg;
+    if (t->eff_labels)
+        cfg_labels(t->labels, t->eff_labels, c.B, c.num_classes, mode, mode == CFG_LABELS_TRAIN ? c.class_dropout : 0.f,
+                   c.seed, t->step_dev, st);
+}
+
 // everything of one step that lives on the device, in stream order (this is what gets captured into the graph)
 static void enqueue_step(UbTrainer* t, const StepOpts& o, cudaStream_t st) {
     const UbConfig& c = t->cfg;
@@ -1455,6 +1488,8 @@ static void enqueue_step(UbTrainer* t, const StepOpts& o, cudaStream_t st) {
     // super-resolution: the condition comes from the batch itself (super_res_train.py, load_superres_data)
     if (c.super_res) superres_cond(t->x0, 1, t->flips, c.B, c.C_in, c.H, c.W, c.super_res, t->cond, st);
     if (t->drop_ctl) dropout_set_ctl(t->drop_ctl, c.dropout, c.seed, t->step_dev, st);  // training: masks of this step
+    // classifier-free guidance: this step's label drops, written once before the tape (forward and backward read them)
+    enqueue_cfg_labels(t, CFG_LABELS_TRAIN, st);
     static const bool debug_sync = getenv("UB_DEBUG_SYNC") != nullptr;  // eager runs only: find the faulting op
     cudaStreamCaptureStatus cap = cudaStreamCaptureStatusNone;
     if (debug_sync) cudaStreamIsCapturing(st, &cap);
@@ -1780,6 +1815,7 @@ extern "C" int ub_trainer_profile(UbTrainer* t, int reps, UbProfile* out) {
         diffusion_prepare(t->x0, t->sqrt_ac, t->sqrt_1mac, c.B, size_t(c.C_in) * c.H * c.W, c.n_timesteps, c.seed,
                           t->step_dev, 1, 1, t->tsteps, t->noise, t->xt, st, c.W, t->flips);
         if (t->drop_ctl) dropout_set_ctl(t->drop_ctl, c.dropout, c.seed, t->step_dev, st);
+        enqueue_cfg_labels(t, CFG_LABELS_TRAIN, st);
         cudaEventRecord(ev[k++], st);
         if (c.super_res) {
             for (int r = 0; r < R; ++r)
@@ -1858,7 +1894,7 @@ extern "C" int ub_trainer_profile(UbTrainer* t, int reps, UbProfile* out) {
         for (auto& i : v) out->flops[i.kind] += i.flops, out->bytes[i.kind] += i.bytes, out->launches[i.kind] += i.launches;
     };
     acc(t->fwd_info), acc(t->bwd_info);
-    out->launches[UB_KIND_OPTIM] += c.super_res ? 6 : 5;
+    out->launches[UB_KIND_OPTIM] += (c.super_res ? 6 : 5) + (t->eff_labels ? 1 : 0);
     const double img = double(c.B) * c.C_in * c.H * c.W * 4;
     out->bytes[UB_KIND_OPTIM] += (c.super_res ? 5 : 3) * img + 7.0 * 4 * t->nparams + 4.0 * t->nparams + 2.0 * 2 * t->nparams;
     t->host_step += reps;
@@ -1884,8 +1920,9 @@ extern "C" int ub_trainer_last_loss_terms(UbTrainer* t, float* mse, float* vb) {
 }
 extern "C" void* ub_trainer_stream(UbTrainer* t) { return (void*)t->stream; }
 extern "C" int ub_trainer_launches_per_step(UbTrainer* t) {
-    // tapes + memset-free extras: diffusion (2), adamw, pack, step increment (+ the super-res condition)
-    return t->launches_fwd + t->launches_bwd + 5 + (t->cfg.super_res ? 1 : 0);
+    // tapes + memset-free extras: diffusion (2), adamw, pack, step increment (+ the super-res condition, + the label
+    // drops of classifier-free guidance)
+    return t->launches_fwd + t->launches_bwd + 5 + (t->cfg.super_res ? 1 : 0) + (t->eff_labels ? 1 : 0);
 }
 
 // super-resolution model: enqueue the upsampling of the stored low-res batch into the conditioning channels that the
@@ -1913,6 +1950,7 @@ extern "C" int ub_trainer_predict(UbTrainer* t, const float* xt_host, const floa
     CUDA_TRY(cudaMemsetAsync(t->zero_base, 0, t->zero_bytes, t->stream));
     CUDA_TRY(cudaMemsetAsync(t->noise, 0, img * sizeof(float), t->stream));
     if (t->drop_ctl) dropout_set_ctl(t->drop_ctl, 0.f, c.seed, t->step_dev, t->stream);  // inference: no dropout
+    enqueue_cfg_labels(t, CFG_LABELS_COPY, t->stream);  // unguided: the labels as set, -1 the null class
     t->inference = true;
     for (auto& op : t->fwd_ops) op(t->stream);
     t->inference = false;
@@ -1940,6 +1978,11 @@ extern "C" int ub_trainer_sample(UbTrainer* t, const float* x_init_host, int t_s
                 "ub_trainer_sample_spaced (UB_SAMPLER_ANCESTRAL, every timestep kept)");
         return UB_ERR_STATE;
     }
+    if (t->guidance != 1.f) {
+        set_err("ub_trainer_sample has no classifier-free guidance: the guidance scale is %g; sample with "
+                "ub_trainer_sample_spaced, or set the scale back to 1", double(t->guidance));
+        return UB_ERR_STATE;
+    }
     if (t_start < 0) t_start = c.n_timesteps - 1;
     if (t_end < 0) t_end = 2;
     if (t_start >= c.n_timesteps || t_end < 2 || t_end > t_start) {
@@ -1965,6 +2008,7 @@ extern "C" int ub_trainer_sample(UbTrainer* t, const float* x_init_host, int t_s
         cudaMemsetAsync(t->zero_base, 0, t->zero_bytes, st);
         sample_set_t(t->samp_state, c.B, t->tsteps, st);
         if (t->drop_ctl) dropout_set_ctl(t->drop_ctl, 0.f, c.seed, t->step_dev, st);  // inference: no dropout
+        enqueue_cfg_labels(t, CFG_LABELS_COPY, st);
         for (auto& op : t->fwd_ops) op(st);
         ddpm_step(t->xt, t->out, t->betas, t->sqrt_ac, t->sqrt_1mac, inject ? t->samp_z : nullptr, img, seed,
                   t->samp_state, t->samp_state + 1, st);
@@ -1986,7 +2030,7 @@ extern "C" int ub_trainer_sample(UbTrainer* t, const float* x_init_host, int t_s
             CUDA_TRY(cudaMemcpyAsync(t->samp_z, noise_host + size_t(it) * img, img * sizeof(float),
                                      cudaMemcpyHostToDevice, st));
         CUDA_TRY(cudaGraphLaunch(t->samp_graph, st));
-        ub_count_launches((unsigned long long)(t->launches_fwd + 3));
+        ub_count_launches((unsigned long long)(t->launches_fwd + 3 + (t->eff_labels ? 1 : 0)));
     }
     CUDA_TRY(cudaMemcpyAsync(out_host, t->xt, img * sizeof(float), cudaMemcpyDeviceToHost, st));
     CUDA_TRY(cudaStreamSynchronize(st));
@@ -2159,38 +2203,54 @@ extern "C" int ub_trainer_sample_spaced(UbTrainer* t, const int* timesteps, int 
     CUDA_TRY(cudaMemcpyAsync(t->spaced_ts, ts.data(), n * sizeof(int), cudaMemcpyHostToDevice, st));
     CUDA_TRY(cudaMemsetAsync(t->noise, 0, img * sizeof(float), st));  // (the forward tape ends with the MSE vs noise)
     const bool inject = noise_host != nullptr;
-    if (!t->spaced_graph || t->spaced_graph_noise != inject) {
-        if (t->spaced_graph) cudaGraphExecDestroy(t->spaced_graph), t->spaced_graph = nullptr;
+    // classifier-free guidance (scale != 1): a graph of its own, two forward passes per iteration
+    const bool guided = t->guidance != 1.f;
+    cudaGraphExec_t& exec = guided ? t->cfg_graph : t->spaced_graph;
+    bool& exec_noise = guided ? t->cfg_graph_noise : t->spaced_graph_noise;
+    if (!exec || exec_noise != inject) {
+        if (exec) cudaGraphExecDestroy(exec), exec = nullptr;
         cudaGraph_t graph = nullptr;
         CUDA_TRY(cudaStreamSynchronize(st));
         CUDA_TRY(cudaStreamBeginCapture(st, cudaStreamCaptureModeThreadLocal));
         cudaMemsetAsync(t->zero_base, 0, t->zero_bytes, st);
         spaced_set_t(t->spaced_ts, t->spaced_state, c.B, t->tsteps, st);
         if (t->drop_ctl) dropout_set_ctl(t->drop_ctl, 0.f, c.seed, t->step_dev, st);  // inference: no dropout
+        enqueue_cfg_labels(t, CFG_LABELS_COPY, st);
         t->inference = true;  // (read while the tape is captured: the graph keeps the loss-free head)
         for (auto& op : t->fwd_ops) op(st);
+        if (guided) {
+            // keep the conditional output; the null-class pass starts from a fresh zero region, like the first one
+            // (the tape accumulates GroupNorm statistics and the head's loss slots there)
+            const size_t oimg = size_t(c.B) * (c.learn_sigma ? 2 : 1) * c.C_out * c.H * c.W;
+            cudaMemcpyAsync(t->eps_cond, t->out, oimg * sizeof(float), cudaMemcpyDeviceToDevice, st);
+            cudaMemsetAsync(t->zero_base, 0, t->zero_bytes, st);
+            enqueue_cfg_labels(t, CFG_LABELS_NULL, st);
+            for (auto& op : t->fwd_ops) op(st);
+        }
         t->inference = false;
         spaced_step(t->xt, t->out, t->spaced_rows, inject ? t->samp_z : nullptr, img, t->spaced_state, st,
-                    c.learn_sigma ? img / c.B : 0);
+                    c.learn_sigma ? img / c.B : 0, guided ? t->eps_cond : nullptr, t->guidance_dev);
         cudaError_t e = cudaStreamEndCapture(st, &graph);
         if (e != cudaSuccess || !graph) {
             set_err("sampling graph capture failed: %s", cudaGetErrorString(e));
             return UB_ERR_CUDA;
         }
-        e = cudaGraphInstantiate(&t->spaced_graph, graph, 0);
+        e = cudaGraphInstantiate(&exec, graph, 0);
         cudaGraphDestroy(graph);
         if (e != cudaSuccess) {
             set_err("sampling graph instantiate failed: %s", cudaGetErrorString(e));
             return UB_ERR_CUDA;
         }
-        t->spaced_graph_noise = inject;
+        exec_noise = inject;
     }
-    const unsigned long long launches = t->launches_fwd + 3 + (t->drop_ctl ? 1 : 0);
+    const int passes = guided ? 2 : 1;
+    const unsigned long long launches =
+        passes * (t->launches_fwd + (t->eff_labels ? 1 : 0)) + 3 + (t->drop_ctl ? 1 : 0);
     for (int it = 0; it < n; ++it) {
         if (inject)
             CUDA_TRY(cudaMemcpyAsync(t->samp_z, noise_host + size_t(it) * img, img * sizeof(float),
                                      cudaMemcpyHostToDevice, st));
-        CUDA_TRY(cudaGraphLaunch(t->spaced_graph, st));
+        CUDA_TRY(cudaGraphLaunch(exec, st));
         ub_count_launches(launches);
     }
     CUDA_TRY(cudaMemcpyAsync(out_host, t->xt, img * sizeof(float), cudaMemcpyDeviceToHost, st));
@@ -2287,15 +2347,49 @@ extern "C" int ub_trainer_set_labels(UbTrainer* t, const int* labels_host, size_
         set_err("size mismatch: got %zu labels, batch is %d", n, t->cfg.B);
         return UB_ERR_SHAPE;
     }
+    const int lo = t->eff_labels ? -1 : 0;  // (-1: the null class of a classifier-free guidance model)
     for (size_t i = 0; i < n; ++i)
-        if (labels_host[i] < 0 || labels_host[i] >= t->cfg.num_classes) {
-            set_err("label %d of image %zu outside [0, %d)", labels_host[i], i, t->cfg.num_classes);
+        if (labels_host[i] < lo || labels_host[i] >= t->cfg.num_classes) {
+            set_err("label %d of image %zu outside [%d, %d)", labels_host[i], i, lo, t->cfg.num_classes);
             return UB_ERR_SHAPE;
         }
     CUDA_TRY(cudaSetDevice(t->device));
     // the captured step reads the labels from this fixed buffer: wait for the steps in flight, then overwrite it
     CUDA_TRY(cudaStreamSynchronize(t->stream));
     CUDA_TRY(cudaMemcpy(t->labels, labels_host, n * sizeof(int), cudaMemcpyHostToDevice));
+    return UB_OK;
+}
+extern "C" int ub_trainer_get_effective_labels(UbTrainer* t, int* host, size_t n) {
+    if (!t->eff_labels) {
+        set_err("no label dropout: the trainer was created with cfg.class_dropout = 0");
+        return UB_ERR_STATE;
+    }
+    const int B = t->cfg.B, K = t->cfg.num_classes;
+    if (n != size_t(B)) {
+        set_err("size mismatch: got %zu labels, batch is %d", n, B);
+        return UB_ERR_SHAPE;
+    }
+    CUDA_TRY(cudaSetDevice(t->device));
+    CUDA_TRY(cudaStreamSynchronize(t->stream));
+    CUDA_TRY(cudaMemcpy(host, t->eff_labels + B, n * sizeof(int), cudaMemcpyDeviceToHost));
+    for (size_t i = 0; i < n; ++i)
+        if (host[i] == K) host[i] = -1;
+    return UB_OK;
+}
+extern "C" int ub_trainer_set_guidance(UbTrainer* t, float scale) {
+    if (!t->eff_labels) {
+        set_err("no null class to guide with: the trainer was created with cfg.class_dropout = 0");
+        return UB_ERR_STATE;
+    }
+    if (!(scale >= 0.f && scale <= FLT_MAX)) {
+        set_err("guidance scale must be finite and >= 0, got %g", double(scale));
+        return UB_ERR_SHAPE;
+    }
+    CUDA_TRY(cudaSetDevice(t->device));
+    // the guided sampler's graph reads the scale from this fixed word: wait for the calls in flight, then overwrite it
+    CUDA_TRY(cudaStreamSynchronize(t->stream));
+    CUDA_TRY(cudaMemcpy(t->guidance_dev, &scale, sizeof(float), cudaMemcpyHostToDevice));
+    t->guidance = scale;
     return UB_OK;
 }
 extern "C" int ub_trainer_set_low_res(UbTrainer* t, const float* host, size_t n) {
