@@ -192,6 +192,66 @@ int ub_conv2d_nhwc_dgrad(const void* dout_bf16, const void* wd_bf16, void* dx_bf
 int ub_conv2d_nhwc_wgrad(const void* dout_bf16, const void* x_bf16, float* dweight, float* dbias, int B, int H, int W,
                          int C_in, int C_out, int ksize);
 
+/* One launch of the trainer's tcgen05 conv kernels with their whole epilogue (what each of the trainer's convolutions
+ * is): out[pix][n] = sum over segments of conv(x_seg, w_seg) + bias + bias2 + rowvec[b] + residual, for a fprop (wf
+ * pack) or a dgrad (wd pack, x = dout) of every segment.  A segment is an NHWC bf16 input with channel pitch ldx >= C_in
+ * and its packed weights; two segments (a 3x3 conv and a 1x1 skip conv of another input) sum into one output.
+ * Epilogue (one-to-one with the library's ConvEpilogue; NULL / 0 = absent, ldr / ldo 0 = C_out):
+ *   out_mode 0: NHWC bf16 [B*H*W][ldo] (ldo > C_out writes channels [0, C_out) of a wider, e.g. concat, buffer);
+ *            1: NCHW fp32 [B][C_out][H][W];  2: NHWC fp32 [B*H*W][ldo].
+ *   stats   : [B][C_out][2] += per-(image, channel) (sum, sum of squares) of the stored bf16 output (GroupNorm's
+ *             statistics; mode 0 only).
+ *   gn hook : with gn_x (NHWC bf16 [B*H*W][gn_ldx], C_out channels) the conv output is dy = dL/d act(gn(gn_x)), act =
+ *             SiLU (gn_silu 1) or identity; the kernel stores dz = dL/d gn(gn_x) = dy * act'(z) in place of dy and
+ *             accumulates gn_S [B][C_out][2] += (sum dz, sum dz * xhat), from gn_chsum (gn_x's statistics as `stats`
+ *             leaves them), gn_gamma, gn_beta, gn_groups (eps 1e-5).  Mode 0 only, no residual, not with stats.
+ *             ub_groupnorm_nhwc_backward_apply finishes the GroupNorm backward.
+ * kernel: 0 = basic kernel (one CTA per pixel tile x N tile), 1 = persistent row-tile kernel (W in {16, 32, 64, 128},
+ * H >= 256 / W); there is no fallback between them.  `info` (if non-NULL) is filled whatever the outcome: the plan the
+ * launch used (zeros where the planner stopped).  Basic kernel: nacc MMA streams (1 or 2), ms = 1 tensor-core
+ * statistics, 2 staged TMA store, 0 per-thread epilogue; pixel tile TW x TH x TB; grid = CTAs.  Row-tile kernel: TW =
+ * W, TH = rows per tile, TB = 1, stages = activation ring stages, w_resident = weights loaded once per CTA, grid =
+ * persistent CTAs, nacc = ms = 0.  UB_ERR_SHAPE (the planner's code in ub_last_error()) when the requested kernel cannot run the
+ * call; nothing is launched then.  Runs on the layer stream. */
+typedef struct {
+    const void* x_bf16;
+    int C_in;
+    int ldx;
+    const void* w_bf16;
+    int ksize;
+} UbConvSeg;
+typedef struct {
+    const float *bias, *bias2, *rowvec; /* rowvec [B][C_out] */
+    const void* residual_bf16;
+    int ldr;
+    void* out;
+    int ldo;
+    int out_mode; /* 0 NHWC bf16, 1 NCHW fp32, 2 NHWC fp32 */
+    float* stats; /* [B][C_out][2] += */
+    const void* gn_x_bf16;
+    int gn_ldx;
+    const float *gn_chsum, *gn_gamma, *gn_beta;
+    float* gn_S;
+    int gn_silu, gn_groups;
+} UbConvEpilogue;
+typedef struct {
+    int kernel, BN, nacc, ms, stages, w_resident, TW, TH, TB, grid;
+} UbConvPlanInfo;
+int ub_conv2d_nhwc_fused(const UbConvSeg* segs, int nseg, int B, int H, int W, int C_out, const UbConvEpilogue* ep,
+                         int kernel, UbConvPlanInfo* info);
+
+/* Weight gradient as the trainer computes it (accumulate mode: every CTA adds its tile with TMA reduce-add), from dout
+ * NHWC bf16 [B*H*W][lddy] and x NHWC bf16 [B*H*W][ldx]; C_in, C_out multiples of 64.
+ *   ksize 3: dweight (C_out,C_in,3,3) is OVERWRITTEN -- the kernel accumulates into a library-owned [tap][C_out][C_in]
+ *            buffer that holds zeros, and a finalize launch transposes it into dweight and zeroes it again;
+ *   ksize 1: dweight (C_out,C_in) is ACCUMULATED into (+=);
+ *   dbias / dbias2 (C_out, may be NULL; dbias2 needs dbias) are ACCUMULATED into: both += sum over pixels of dout.
+ * colmode_out (3x3: one filter column per CTA, W > 4) and nsplit_out (CTAs along the pixels) report the plan when
+ * non-NULL.  Runs on the layer stream. */
+int ub_conv2d_nhwc_wgrad_acc(const void* dout_bf16, int lddy, const void* x_bf16, int ldx, float* dweight,
+                             float* dbias, float* dbias2, int B, int H, int W, int C_in, int C_out, int ksize,
+                             int* colmode_out, int* nsplit_out);
+
 /* GroupNorm (+ optional SiLU) in the native layout (what the trainer runs; replaces groupnorm_forward / groupnorm_backward
  * fused with silu_forward / silu_backward, dev/groupnorm.cuh:3-13, dev/silu.cuh:3-13): x, y, dy, dx are NHWC bf16 [B*H*W][C].
  * Single-pass "slab" kernels when the shape allows (C % 16 == 0; impl = 0), two-pass kernels otherwise / when impl = 1.
@@ -203,6 +263,13 @@ int ub_groupnorm_nhwc_forward(const void* x_bf16, const float* weight, const flo
 int ub_groupnorm_nhwc_backward(const void* x_bf16, const void* dy_bf16, const float* chsum, const float* weight,
                                const float* bias, const void* add_in_bf16, void* dx_bf16, float* dweight, float* dbias,
                                float* scratch, int B, int H, int W, int C, int n_groups, int silu, int impl);
+/* Second half of the GroupNorm(+SiLU) backward whose first half ran in a conv epilogue (UbConvEpilogue's gn hook):
+ * dz = dL/d gn(x) (NHWC bf16, the hook's output) and S [B][C][2] (the hook's sums) -> dx = gn_bwd(dz) (+ add_in if
+ * non-NULL), overwritten; dweight / dbias (C) are ACCUMULATED into.  silu says whether SiLU followed the norm (the hook's
+ * gn_silu); the SiLU derivative is already in dz either way. */
+int ub_groupnorm_nhwc_backward_apply(const void* x_bf16, const void* dz_bf16, const float* chsum, const float* S,
+                                     const float* weight, const float* bias, const void* add_in_bf16, void* dx_bf16,
+                                     float* dweight, float* dbias, int B, int H, int W, int C, int n_groups, int silu);
 
 /* Attention core in the native layout (what the trainer runs; replaces attention_forward1 / attention_backward,
  * dev/attention.cuh:6-22, without their permutes and (B,NH,T,T) matrices): qkv is NHWC bf16 [B*T][3C], channel order

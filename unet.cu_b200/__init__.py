@@ -35,6 +35,28 @@ class UbConfig(C.Structure):
                 ("learn_sigma", C.c_int), ("noise_schedule", C.c_int), ("class_dropout", C.c_float)]
 
 
+class UbConvSeg(C.Structure):
+    """UbConvSeg of include/unet_b200.h: one input of ub_conv2d_nhwc_fused (NHWC bf16, channel pitch ldx) and its
+    packed weights."""
+    _fields_ = [("x_bf16", C.c_void_p), ("C_in", C.c_int), ("ldx", C.c_int), ("w_bf16", C.c_void_p),
+                ("ksize", C.c_int)]
+
+
+class UbConvEpilogue(C.Structure):
+    """UbConvEpilogue of include/unet_b200.h: the conv kernels' epilogue (bias, second bias, per-image row, residual,
+    output layout, GroupNorm statistics / gn-bwd hooks)."""
+    _fields_ = [("bias", C.c_void_p), ("bias2", C.c_void_p), ("rowvec", C.c_void_p), ("residual_bf16", C.c_void_p),
+                ("ldr", C.c_int), ("out", C.c_void_p), ("ldo", C.c_int), ("out_mode", C.c_int),
+                ("stats", C.c_void_p), ("gn_x_bf16", C.c_void_p), ("gn_ldx", C.c_int), ("gn_chsum", C.c_void_p),
+                ("gn_gamma", C.c_void_p), ("gn_beta", C.c_void_p), ("gn_S", C.c_void_p), ("gn_silu", C.c_int),
+                ("gn_groups", C.c_int)]
+
+
+class UbConvPlanInfo(C.Structure):
+    """UbConvPlanInfo of include/unet_b200.h: the plan ub_conv2d_nhwc_fused launched (or stopped at)."""
+    _fields_ = [(n, C.c_int) for n in ("kernel", "BN", "nacc", "ms", "stages", "w_resident", "TW", "TH", "TB", "grid")]
+
+
 UB_KINDS = ("conv_igemm", "wgrad_igemm", "groupnorm", "attention", "eltwise", "small", "optimizer")
 
 
@@ -99,6 +121,11 @@ def _declare(L: C.CDLL) -> None:
     L.ub_set_layer_precision.argtypes = [i]
     L.ub_groupnorm_nhwc_forward.argtypes = [vp, vp, vp, vp, vp, i, i, i, i, i, i, i]
     L.ub_groupnorm_nhwc_backward.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i, i, i, i, i, i, i]
+    L.ub_groupnorm_nhwc_backward_apply.argtypes = [vp, vp, vp, vp, vp, vp, vp, vp, vp, vp, i, i, i, i, i, i]
+    L.ub_conv2d_nhwc_fused.argtypes = [C.POINTER(UbConvSeg), i, i, i, i, i, C.POINTER(UbConvEpilogue), i,
+                                       C.POINTER(UbConvPlanInfo)]
+    L.ub_conv2d_nhwc_wgrad_acc.argtypes = [vp, i, vp, i, vp, vp, vp, i, i, i, i, i, i, C.POINTER(i), C.POINTER(i)]
+    L.ub_pack_conv_weight.argtypes = [vp, vp, vp, i, i, i]
     L.ub_trainer_stream.argtypes = [vp]
     L.ub_trainer_stream.restype = vp
     L.ub_trainer_launches_per_step.argtypes = [vp]

@@ -334,8 +334,8 @@ __device__ __forceinline__ void igemm_conv_body(const IgemmConvParams& p) {
                 const bool stat = p.ms == 1;
                 uint64_t* stat_bar = tmem_full_bar + 2;
                 const int atoms = p.BN / 64;
-                const uint32_t ys = smem_u32(smem), y2s = ys + uint32_t(atoms) * 16384u;
-                const uint32_t ones_s = ys + 2u * uint32_t(atoms) * 16384u;
+                const uint32_t ys = smem_u32(smem);
+                const uint32_t ones_s = ys + uint32_t(atoms) * 16384u;
                 if (stat)
                     for (int i = et; i < 1024; i += kEpiThreads)  // 128 pixel rows x 128 B of bf16 1.0
                         sts_v4_b32(ones_s + 16u * i, 0x3F803F80u, 0x3F803F80u, 0x3F803F80u, 0x3F803F80u);
@@ -362,44 +362,44 @@ __device__ __forceinline__ void igemm_conv_body(const IgemmConvParams& p) {
                             for (int i = 0; i < 8; ++i) f[j * 8 + i] += t[i];
                         }
                     }
-                    uint32_t py[8], pq[8];
+                    uint32_t py[8];
 #pragma unroll
                     for (int i = 0; i < 8; ++i) {
                         const __nv_bfloat162 h2 = __floats2bfloat162_rn(f[2 * i], f[2 * i + 1]);
-                        const float2 fr = __bfloat1622float2(h2);  // the stored values: square exactly those
-                        const __nv_bfloat162 q2 = __floats2bfloat162_rn(fr.x * fr.x, fr.y * fr.y);
                         py[i] = *reinterpret_cast<const uint32_t*>(&h2);
-                        pq[i] = *reinterpret_cast<const uint32_t*>(&q2);
                     }
                     // MN-major SW128 atom: row = pixel (128 B = 64 channels), 16-byte chunk index XOR (row % 8)
                     const uint32_t abase = uint32_t(c0 >> 6) * 16384u + rowoff;
                     const uint32_t ch = uint32_t((c0 & 63) >> 3), sw = uint32_t(row & 7);
                     sts_v4_b32(ys + abase + ((ch ^ sw) << 4), py[0], py[1], py[2], py[3]);
                     sts_v4_b32(ys + abase + (((ch + 1) ^ sw) << 4), py[4], py[5], py[6], py[7]);
-                    if (stat) {
-                        sts_v4_b32(y2s + abase + ((ch ^ sw) << 4), pq[0], pq[1], pq[2], pq[3]);
-                        sts_v4_b32(y2s + abase + (((ch + 1) ^ sw) << 4), pq[4], pq[5], pq[6], pq[7]);
-                    }
                 }
                 fence_proxy_async_smem();
                 tc_fence_before();
                 named_bar_sync(1, kEpiThreads);
-                const uint32_t t_stat = tmem_base + uint32_t(NACC * p.BN);  // [image][sum 16 cols | sumsq 16 cols]
+                // [image][16 cols]: sum y, behind the accumulators and the Gram matrices (IgemmConvParams::ms)
+                const uint32_t t_stat = tmem_base + uint32_t(max(NACC, p.TB) * p.BN);
                 if (threadIdx.x == 64) {
                     tc_fence_after();
                     for (int a = 0; a < atoms; ++a) tma_store_4d(smem + size_t(a) * 16384, &p.tmO, n0 + a * 64, w0, h0, b0);
                     bulk_commit_group();
                   if (stat) {
+                    // sum y = Y^T x ones (N = 16, column 0 used).  sum y*y = the diagonal of the Gram matrix Y^T Y (N =
+                    // BN), written over the accumulator columns, which the loop above has read: products of two bf16
+                    // values are exact in fp32, so every y*y enters the fp32 sum exactly.  (A staged Y*Y operand is
+                    // rounded to bf16, 2^-9 relative per term, which GroupNorm's E[y^2] - mean^2 amplifies by
+                    // (mean^2 + var) / var: the variance was off by 7e-3 for channels with a 4-sigma offset,
+                    // tests/test_conv_fused_gpu.py on a B200.)
                     const uint32_t idesc = make_idesc_bf16(uint32_t(p.BN), 16, 1, 1);
+                    const uint32_t gdesc = make_idesc_bf16(uint32_t(p.BN), uint32_t(p.BN), 1, 1);
                     const uint64_t dbase = make_smem_desc_sw128(0, 16384, 1024);  // LBO = 64-channel atom, SBO = 8 rows
-                    const uint64_t dY = dbase | uint64_t((ys >> 4) & 0x3FFF), dY2 = dbase | uint64_t((y2s >> 4) & 0x3FFF);
-                    const uint64_t dO = dbase | uint64_t((ones_s >> 4) & 0x3FFF);
+                    const uint64_t dY = dbase | uint64_t((ys >> 4) & 0x3FFF), dO = dbase | uint64_t((ones_s >> 4) & 0x3FFF);
                     const int kpi = 8 / p.TB;  // K steps (16 pixels) per image of the tile
                     for (int img = 0; img < p.TB; ++img)
                         for (int k = 0; k < kpi; ++k) {
                             const uint64_t ko = uint64_t((img * kpi + k) * 128);  // 16 rows x 128 B, in 16-byte units
                             umma_bf16(t_stat + uint32_t(img * 32), dY + ko, dO + ko, idesc, k != 0);
-                            umma_bf16(t_stat + uint32_t(img * 32 + 16), dY2 + ko, dO + ko, idesc, k != 0);
+                            umma_bf16(tmem_base + uint32_t(img * p.BN), dY + ko, dY + ko, gdesc, k != 0);
                         }
                     umma_commit(stat_bar);
                   }
@@ -408,18 +408,24 @@ __device__ __forceinline__ void igemm_conv_body(const IgemmConvParams& p) {
                 mbar_wait(stat_bar, 0);
                 tc_fence_after();
                 if (half == 0) {
-                    // M = 128: channel m in TMEM lane m.  M = 64: channel m in lane (m % 16) + 32 * (m / 16).
-                    const int chn = p.BN == 128 ? q * 32 + lane : q * 16 + lane;
+                    // M = 128: channel m in TMEM lane m.  M = 64: channel m in lane (m % 16) + 32 * (m / 16).  The sum
+                    // of squares of channel m is column m of its row of the Gram matrix.
+                    const int c_w = p.BN == 128 ? q * 32 : q * 16;  // first channel of this warp's lanes
+                    const int chn = c_w + lane;
                     const bool cv = p.BN == 128 || lane < 16;
+                    const uint32_t lrow = uint32_t(q * 32) << 16;
                     for (int img = 0; img < p.TB; ++img) {
-                        uint32_t sv[16], qv[16];
-                        tmem_ld16(t_stat + (uint32_t(q * 32) << 16) + uint32_t(img * 32), sv);
-                        tmem_ld16(t_stat + (uint32_t(q * 32) << 16) + uint32_t(img * 32 + 16), qv);
+                        uint32_t sv[16], gv[32];
+                        tmem_ld16(t_stat + lrow + uint32_t(img * 32), sv);
+                        tmem_ld32(tmem_base + lrow + uint32_t(img * p.BN + c_w), gv);
                         tmem_ld_wait();
+                        float ss = 0.f;
+#pragma unroll
+                        for (int j = 0; j < 32; ++j) ss = j == lane ? __uint_as_float(gv[j]) : ss;
                         if (cv && b0 + img < p.B) {
                             float* d = p.epi.stats + (size_t(b0 + img) * p.Cout + n0 + chn) * 2;
                             asm volatile("red.global.add.v2.f32 [%0], {%1, %2};" ::"l"(d), "f"(__uint_as_float(sv[0])),
-                                         "f"(__uint_as_float(qv[0]))
+                                         "f"(ss)
                                          : "memory");
                         }
                     }
@@ -995,14 +1001,19 @@ int igemm_conv_plan(IgemmConvParams* p, const ConvSegDesc* segs, int nseg, int B
         // 128-pixel tiles of one or two whole images with a 64- or 128-channel N tile, one or two MMA streams
         // (measured round 2: 5.015 ms per step with, 5.043 with the shuffle-reduce statistics; measured, removed)
         const bool full_tiles = W % p->TW == 0 && H % p->TH == 0 && p->TW * p->TH * p->TB == 128;
-        const size_t need = size_t(2 * (BN / 64) + 1) * 16384;  // Y atoms, Y*Y atoms, ones tile in the dead stages
+        // (TMEM: the accumulators, or one Gram matrix per image of the tile if more, then 64 columns of sums.  Against
+        // the staged-Y*Y version this moves two shapes: a two-image tile at BN 128 with one MMA stream (320 > 256
+        // columns: 8x8 layers at batches of ~150-255 per GPU) now takes the shuffle statistics, and one at BN 64 with
+        // one stream allocates 256 columns instead of 128.  Neither occurs in the default B = 32 step.)
+        const size_t need = size_t(BN / 64 + 1) * 16384;  // Y atoms and the ones tile in the dead stages
+        const int gcols = (p->TB > p->nacc ? p->TB : p->nacc) * BN + 64;
         if (ep.stats && !ep.gn_x && ep.out_mode == OUT_NHWC_BF16 && (BN == 64 || BN == 128) &&
             p->nacc <= 2 && (p->TB == 1 || (p->TB == 2 && (p->TW * p->TH) == 64)) && full_tiles &&
-            need <= size_t(p->stages) * p->stage_bytes && p->nacc * BN + 64 <= (p->nacc == 1 ? 256 : 512) &&
+            need <= size_t(p->stages) * p->stage_bytes && gcols <= (p->nacc == 1 ? 256 : 512) &&
             make_act_map(&p->tmO, reinterpret_cast<const __nv_bfloat16*>(ep.out), Cout, p->epi.ldo, W, H, B, p->TW,
                          p->TH, p->TB) == 0) {
             p->ms = 1;
-            p->tmem_cols = next_pow2(p->nacc * BN + 64);
+            p->tmem_cols = next_pow2(gcols);
         }
         // ms == 2, store-only: a conv without any hook whose output is an NHWC bf16 tensor leaves through the same staged
         // tile + TMA store (any whole-tile shape, N tiles of 64 .. 256 channels)

@@ -68,9 +68,10 @@ struct IgemmConvParams {
     int ngimg;                      // rows of the staged GroupNorm constants (TB when gn_x is set, else 0)
     int nred;                       // BN-float rows of the cross-warp reduction scratch (8 with a hook, else 0)
     // GroupNorm statistics on the tensor core (the plain statistics hook on full tiles) --
-    // the epilogue stages the bf16 output tile Y and Y*Y in shared memory as MN-major SW128 operands (the layout TMA
-    // gives the wgrad kernel), a ones-tile MMA (the wgrad kernel's bias-gradient trick) leaves sum(y) and sum(y*y)
-    // of channel c in TMEM lane c, and the Y tile goes to global memory with one TMA store per 64 channels.
+    // the epilogue stages the bf16 output tile Y in shared memory as an MN-major SW128 operand (the layout TMA gives
+    // the wgrad kernel), a ones-tile MMA (the wgrad kernel's bias-gradient trick) leaves sum(y) of channel c in TMEM
+    // lane c, the Gram matrix Y^T Y of each image (over the dead accumulator columns) holds the exact sum(y*y) of
+    // channel c in lane c, column c, and the Y tile goes to global memory with one TMA store per 64 channels.
     int ms;
     CUtensorMap tmO;                // output tensor, box (64, TW, TH, TB), SWIZZLE_128B (ms only)
 };

@@ -462,6 +462,17 @@ int ub_groupnorm_nhwc_backward(const void* x, const void* dy, const float* chsum
                  (const bf16*)add_in, C, (bf16*)dx, C, dweight, dbias, nullptr, st);
     return finish(2);
 }
+int ub_groupnorm_nhwc_backward_apply(const void* x, const void* dz, const float* chsum, const float* S,
+                                     const float* weight, const float* bias, const void* add_in, void* dx,
+                                     float* dweight, float* dbias, int B, int H, int W, int C, int n_groups, int silu) {
+    if (n_groups < 1 || C % n_groups || C % 8) {
+        fail("groupnorm_nhwc: needs C %% n_groups == 0 and C %% 8 == 0");
+        return UB_ERR_SHAPE;
+    }
+    gn_bwd_apply((const bf16*)x, C, (const bf16*)dz, C, chsum, S, weight, bias, B, H * W, C, n_groups, silu ? 2 : 0,
+                 (const bf16*)add_in, C, (bf16*)dx, C, dweight, dbias, nullptr, ub_layer_stream());
+    return finish(1);
+}
 int ub_conv2d_nhwc_forward(const void* x, const void* wf, const float* bias, void* out, int B, int H, int W, int C_in,
                            int C_out, int ksize) {
     if (!shape_fprop_ok(C_in, C_out)) {
@@ -524,6 +535,113 @@ int ub_conv2d_nhwc_wgrad(const void* dout, const void* x, float* dweight, float*
         colsum((const bf16*)dout, C_out, size_t(B) * H * W, C_out, dbias, nullptr, st);
         launches++;
     }
+    return finish(launches);
+}
+
+int ub_conv2d_nhwc_fused(const UbConvSeg* segs, int nseg, int B, int H, int W, int C_out, const UbConvEpilogue* ep,
+                         int kernel, UbConvPlanInfo* info) {
+    UbConvPlanInfo inf{};
+    inf.kernel = kernel;
+    if (info) *info = inf;
+    if (!segs || nseg < 1 || nseg > 2 || !ep || (kernel != 0 && kernel != 1) || B < 1 || H < 1 || W < 1) {
+        fail("conv2d_nhwc_fused: bad arguments (nseg 1 or 2, kernel 0 or 1, epilogue required)");
+        return UB_ERR_SHAPE;
+    }
+    ConvSegDesc sd[2];
+    for (int s = 0; s < nseg; ++s) {
+        if (segs[s].ksize != 1 && segs[s].ksize != 3) {
+            fail("conv2d_nhwc_fused: ksize must be 1 or 3");
+            return UB_ERR_SHAPE;
+        }
+        sd[s] = ConvSegDesc{(const bf16*)segs[s].x_bf16, segs[s].C_in, segs[s].ldx ? segs[s].ldx : segs[s].C_in,
+                            (const bf16*)segs[s].w_bf16, segs[s].ksize * segs[s].ksize};
+    }
+    ConvEpilogue e;
+    e.bias = ep->bias, e.bias2 = ep->bias2, e.rowvec = ep->rowvec;
+    e.residual = (const bf16*)ep->residual_bf16, e.ldr = ep->ldr;
+    e.out = ep->out, e.ldo = ep->ldo, e.out_mode = ep->out_mode;
+    e.stats = ep->stats;
+    e.gn_x = (const bf16*)ep->gn_x_bf16, e.gn_ldx = ep->gn_ldx ? ep->gn_ldx : C_out, e.gn_chsum = ep->gn_chsum;
+    e.gn_gamma = ep->gn_gamma, e.gn_beta = ep->gn_beta, e.gn_S = ep->gn_S;
+    e.gn_silu = ep->gn_silu, e.gn_groups = ep->gn_groups;
+    if (e.out_mode < OUT_NHWC_BF16 || e.out_mode > OUT_NHWC_F32) {
+        fail("conv2d_nhwc_fused: out_mode must be 0, 1 or 2");
+        return UB_ERR_SHAPE;
+    }
+    cudaStream_t st = ub_layer_stream();
+    if (kernel == 0) {
+        IgemmConvParams p;
+        const int r = igemm_conv_plan(&p, sd, nseg, B, H, W, C_out, e);
+        inf.BN = p.BN, inf.nacc = p.nacc, inf.ms = p.ms, inf.stages = p.stages;
+        inf.TW = p.TW, inf.TH = p.TH, inf.TB = p.TB;
+        inf.grid = p.tiles_w * p.tiles_h * p.tiles_b * (p.BN ? C_out / p.BN : 0);
+        if (info) *info = inf;
+        if (r) {
+            fail("conv2d_nhwc_fused: basic-kernel plan failed (%d)", r);
+            return UB_ERR_SHAPE;
+        }
+        igemm_conv_launch(p, st);
+    } else {
+        if (!igemm_rows_eligible(B, H, W, C_out)) {
+            fail("conv2d_nhwc_fused: the row-tile kernel needs W in {16, 32, 64, 128}, H >= 256 / W, C_out %% 16 == 0");
+            return UB_ERR_SHAPE;
+        }
+        IgemmRowsParams p;
+        const int r = igemm_rows_plan(&p, sd, nseg, B, H, W, C_out, e, sm_count());
+        inf.BN = p.BN, inf.stages = p.a_stages, inf.w_resident = p.w_resident;
+        inf.TW = W, inf.TH = p.TH, inf.TB = 1, inf.grid = p.grid;
+        if (info) *info = inf;
+        if (r) {
+            fail("conv2d_nhwc_fused: row-tile plan failed (%d)", r);
+            return UB_ERR_SHAPE;
+        }
+        igemm_rows_launch(p, st);
+    }
+    return finish(1);
+}
+
+int ub_conv2d_nhwc_wgrad_acc(const void* dout, int lddy, const void* x, int ldx, float* dweight, float* dbias,
+                             float* dbias2, int B, int H, int W, int C_in, int C_out, int ksize, int* colmode_out,
+                             int* nsplit_out) {
+    if (!shape_wgrad_ok(C_in, C_out) || (ksize != 1 && ksize != 3) || !dweight || (dbias2 && !dbias)) {
+        fail("conv2d_nhwc_wgrad_acc needs C_in %% 64 == 0, C_out %% 64 == 0, ksize 1 or 3, dweight, and dbias with dbias2");
+        return UB_ERR_SHAPE;
+    }
+    const int ntaps = ksize * ksize;
+    cudaStream_t st = ub_layer_stream();
+    std::lock_guard<std::mutex> lk(g_ws.mu);
+    float* acc = dweight;  // 1x1: [C_out][C_in] is the final layout, the kernel adds into it
+    WgradFinalizeEntry* tab = nullptr;
+    int launches = 1;
+    if (ntaps == 9) {
+        // [9][C_out][C_in] accumulator in workspace slot 4: zeroed when (re)allocated, re-zeroed by every finalize
+        static void* zeroed = nullptr;
+        static size_t zeroed_cap = 0;
+        const size_t bytes = size_t(9) * C_out * C_in * sizeof(float);
+        acc = (float*)g_ws.get(4, bytes);
+        tab = (WgradFinalizeEntry*)g_ws.get(5, sizeof(WgradFinalizeEntry));
+        if (!acc || !tab) {
+            fail("workspace allocation failed");
+            return UB_ERR_CUDA;
+        }
+        if (acc != zeroed || g_ws.cap[4] != zeroed_cap) {
+            if (cudaMemsetAsync(acc, 0, g_ws.cap[4], st) != cudaSuccess) return finish(0);
+            zeroed = acc, zeroed_cap = g_ws.cap[4];
+        }
+        const WgradFinalizeEntry e{acc, dweight, C_out, C_in};
+        if (cudaMemcpyAsync(tab, &e, sizeof e, cudaMemcpyHostToDevice, st) != cudaSuccess) return finish(0);
+    }
+    IgemmWgradParams p;
+    const int r = igemm_wgrad_plan_acc(&p, (const bf16*)dout, lddy ? lddy : C_out, (const bf16*)x, ldx ? ldx : C_in, B,
+                                       H, W, C_in, C_out, ntaps, acc, dbias, dbias2, sm_count());
+    if (colmode_out) *colmode_out = p.colmode;
+    if (nsplit_out) *nsplit_out = p.nsplit;
+    if (r) {
+        fail("conv2d_nhwc_wgrad_acc: plan failed (%d)", r);
+        return UB_ERR_SHAPE;
+    }
+    igemm_wgrad_launch(p, st);
+    if (tab) igemm_wgrad_finalize(tab, 1, size_t(C_out) * C_in, st), launches++;
     return finish(launches);
 }
 
